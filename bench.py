@@ -2,6 +2,7 @@
 """Benchmark of the nmrfit objective-evaluation hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload metric|c1|c2|c3|c4]
+                    [--dump-outputs DIR]
 
 Headline workload (`metric`): the shape BASELINE.json's metric string is quoted on - 6 peaks on a 4,096-point
 window (the configs[0] spectrum) - with one swarm generation of 65,536 particles per GPU as the batch.  A *step* is
@@ -539,7 +540,31 @@ def measure_e2e(run, steps, warmup):
         dist.all_reduce(e_ms, op=dist.ReduceOp.MAX)
     assert fx.size == S * B and np.all(np.isfinite(fx))
     return {'value': run.evals_per_step() * steps / (float(e_ms.item()) * 1e-3), 'unit': 'evals/s',
-            'h2d_bytes_per_step': int(h2d), 'd2h_bytes_per_step': int(d2h), 'api': api}
+            'h2d_bytes_per_step': int(h2d), 'd2h_bytes_per_step': int(d2h), 'api': api}, fx
+
+
+DUMP_BYTES = 64 << 20
+
+
+def swarm_outputs(run):
+    """What the last timed generation left for a caller: the swarm best (``pso_best``) and the swarm state
+    (``pso_state``: positions, velocities, personal bests and the objective values of the generation), float64, one row
+    per particle (row = spectrum * particles + particle).  When the whole exceeds DUMP_BYTES, the per-particle arrays
+    keep a fixed, seeded sample of rows, listed in ``sample_index``."""
+    x, f, it, stop = run.ctx.pso_best()
+    out = {'best_x': x, 'best_f': f, 'best_generations': it, 'best_stop': stop}
+    rows = run.B * run.S
+    per = {'swarm_' + k: a.reshape(rows, -1) if a.ndim == 3 else a.reshape(rows) for k, a in run.ctx.pso_state().items()}
+    fixed = 8 * (sum(a.size for a in out.values()) + rows)            # + the end-to-end objective values
+    row_bytes = 8 * sum(a.size // rows for a in per.values())
+    budget = DUMP_BYTES - (64 << 10)                                    # room for the .npy headers
+    if fixed + rows * row_bytes > budget:
+        keep = (budget - fixed) // (row_bytes + 8)
+        idx = np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+        per = {k: a[idx] for k, a in per.items()}
+        out['sample_index'] = idx
+    out.update(per)
+    return {k: np.asarray(a, dtype=np.float64) for k, a in out.items()}
 
 
 def secondary(name, world, rank, local, exchange, flush, steps, burst, sustained, particles=None, want_e2e=True):
@@ -561,7 +586,7 @@ def secondary(name, world, rank, local, exchange, flush, steps, burst, sustained
                                               'kernel_share_of_step', 'algorithmic_speedup', 'fp64_inst_per_peak_point',
                                               'traffic', 'hbm')}
     if want_e2e:
-        out['e2e'] = measure_e2e(run, max(3, steps // 2), 3)
+        out['e2e'], _ = measure_e2e(run, max(3, steps // 2), 3)
     run.close()
     return out
 
@@ -636,8 +661,14 @@ def run_b200(args):
     same_main = run.check_state(args.warmup + args.steps)
     total_ms = res['total_ms']
     value = run.evals_per_step() * args.steps / (total_ms * 1e-3)
+    outputs = swarm_outputs(run) if args.dump_outputs and rank == 0 else None
 
-    e2e = measure_e2e(run, args.steps, args.warmup)
+    e2e, e2e_f = measure_e2e(run, args.steps, args.warmup)
+    if outputs is not None:
+        outputs['e2e_objective'] = np.asarray(e2e_f, dtype=np.float64)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     burst, sustained = _cabi.fp64_peak(local, iters=4096, repeats=20)
     rf = roofline(args.workload, run, res, burst, sustained, clocks.get('sm_mhz'))
     tune = run.ctx.get_tuning(run.S)
@@ -809,7 +840,15 @@ def main():
     ap.add_argument('--tune', default='', help='threads,points_per_thread,exp_table_bits,particles_per_cta')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--quick', action='store_true', help='main measurement only (no CPU baseline, no secondary configs / fits)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed as DIR/<name>.npy (float64, at most '
+                         '64 MiB; rank 0\'s particles when sharded): swarm best, swarm state, and the objective values '
+                         'of the last end-to-end call.  The inputs are seeded, so two builds can be compared file by file')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to --impl b200')
     if args.warmup < 3:
         args.warmup = 3
     return run_reference(args) if args.impl == 'reference' else run_b200(args)

@@ -111,7 +111,13 @@ def main():
         f = np.array([eq.objective(x, rd.w, rd.u, rd.v, wts, False) for x in xs])
         f_ones = np.array([eq.objective(x, rd.w, rd.u, rd.v, np.ones_like(wts), False) for x in xs[:4]])
         note('objective', orc.objective_swarm(xs, data.w, data.u, data.v, wts), f)
-        out['objective_' + name] = dict(w=data.w, u=data.u, v=data.v, weights=wts, xs=xs, f=f, f_ones=f_ones,
+        # a 65,536-point axis stored whole would take the file over 1 MB: keep the np.linspace arguments instead
+        # (tests/conftest.py load_golden rebuilds it)
+        axis = dict(w=data.w)
+        if N >= 65536:
+            assert np.array_equal(np.linspace(synth.W_LO, synth.W_HI, N), data.w)
+            axis = dict(w_linspace=np.array([synth.W_LO, synth.W_HI, N], dtype=float))
+        out['objective_' + name] = dict(**axis, u=data.u, v=data.v, weights=wts, xs=xs, f=f, f_ones=f_ones,
                                         lower=np.array(lo), upper=np.array(up), true=true,
                                         peak_loc=[p.loc for p in data.peaks], peak_width=[p.width for p in data.peaks],
                                         peak_area=[p.area for p in data.peaks], peak_height=[p.height for p in data.peaks])

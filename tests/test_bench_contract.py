@@ -6,6 +6,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -54,3 +57,41 @@ def test_reference_arm_under_torchrun_ranks_other_than_zero_do_nothing():
     out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--gpus', '2'],
                          capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ''
+
+
+@pytest.mark.parametrize('extra', [['--steps', '0'], ['--impl', 'reference', '--dump-outputs', 'out']])
+def test_bench_rejects_arguments_it_cannot_honour(extra):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py')] + extra, capture_output=True, text=True,
+                         timeout=120, cwd=ROOT)
+    assert out.returncode == 2 and out.stdout == '' and 'error' in out.stderr
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize('workload', ['metric', 'c3'])
+def test_dump_outputs_writes_the_last_generation(workload, tmp_path):
+    """--dump-outputs: float64 .npy files, 64 MiB at most (c3's swarm state is larger and is sampled), taken after
+    exactly warmup + steps generations."""
+    steps, warmup = 2, 3
+    out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--quick', '--workload', workload, '--steps',
+                          str(steps), '--warmup', str(warmup), '--dump-outputs', str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert len([l for l in out.stdout.splitlines() if l.startswith('{')]) == 1
+    sys.path.insert(0, ROOT)
+    import bench
+    wl = bench.WORKLOADS[workload]
+    B, S, D = wl.get('B', 1), wl['S'], 4 + 3 * wl['P']
+    got = {f[:-4]: np.load(str(tmp_path / f)) for f in os.listdir(str(tmp_path))}
+    assert sum(os.path.getsize(str(tmp_path / f)) for f in os.listdir(str(tmp_path))) <= 64 << 20
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert got['best_x'].shape == (B, D) and np.all(got['best_generations'] == warmup + steps)
+    assert np.all(got['best_stop'] == 0) and np.all(np.isfinite(got['best_f']))
+    rows = B * S
+    if 'sample_index' in got:
+        rows = got['sample_index'].size
+        assert workload == 'c3' and rows < B * S and np.all(np.diff(got['sample_index']) > 0)
+    for k in ('x', 'v', 'p'):
+        assert got['swarm_' + k].shape == (rows, D)
+    assert got['swarm_fx'].shape == got['swarm_fp'].shape == (rows,)
+    assert np.all(got['swarm_fp'] <= got['swarm_fx'])               # a personal best is never worse than the position
+    assert got['e2e_objective'].size == B * S and np.all(np.isfinite(got['e2e_objective']))

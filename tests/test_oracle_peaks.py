@@ -12,18 +12,30 @@ CASES = ['peaks_1024x6', 'peaks_2500x12', 'peaks_4096x6', 'peaks_desc_1500x6',
          'peaks_c3_16384x6']      # the last: a BASELINE configs[2] spectrum (1,638,400 upsampled samples, window 88,554)
 
 
+def _close(got, want, scale):
+    got, want = np.asarray(got, dtype=float), np.asarray(want, dtype=float)
+    return got.shape == want.shape and np.max(np.abs(got - want), initial=0.0) <= 1e-13 * scale
+
+
 @pytest.mark.parametrize('case', CASES)
 def test_auto_peaks_matches_the_reference_class(case):
     g = load_golden(case)
     peaks, aux = orc.auto_peaks(g['w'], g['V'], float(g['thresh']), float(g['window']))
     pr = g['probe']
     assert np.array_equal(aux['wu'][pr], g['wu_probe']) and np.array_equal(aux['uu'][pr], g['uu_probe'])
-    assert np.array_equal(aux['us'][pr], g['us_probe']) and aux['baseline'] == g['baseline']
+    # The Savitzky-Golay coefficients (a least-squares solve) and peakutils' baseline (pinv, dot) go through BLAS /
+    # LAPACK, whose summation order depends on the host CPU: the smoothed signal, the baselines and the heights and
+    # areas built on them agree to rounding (at most 3e-14 of their scale between OpenBLAS's x86 kernel sets); every
+    # index, location, width and bound is exact.
+    scale = np.abs(g['V']).max()
+    assert _close(aux['us'][pr], g['us_probe'], scale) and _close(aux['baseline'], g['baseline'], scale)
     assert [p.i for p in aux['pre']] == list(g['pre_i'])
     assert [p.i for p in peaks] == list(g['i'])
-    for key in ('loc', 'height', 'width', 'area'):
+    for key in ('loc', 'width'):
         assert np.array_equal([getattr(p, key) for p in peaks], g[key]), key
-    assert np.array_equal([p.baseline for p in peaks], g['local_baseline'])
+    assert _close([p.height for p in peaks], g['height'], scale)
+    assert _close([p.area for p in peaks], g['area'], np.abs(g['area']).max())
+    assert _close([p.baseline for p in peaks], g['local_baseline'], scale)
     assert np.array_equal([p.bounds for p in peaks], g['bounds'])
     assert [p.idx_lo for p in peaks] == list(g['idx_lo']) and [p.idx_hi for p in peaks] == list(g['idx_hi'])
 
