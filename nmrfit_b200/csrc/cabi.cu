@@ -220,13 +220,18 @@ ObjTune pick_tune(const nmrfit_ctx* c, int S, bool uni) {
     if (uni && c->precision == NMRFIT_FP64 && c->user_tune.variant != 0 && t.tb == 6 && enough) {   // (built for the default table)
         t.variant = 1;
         t.occ = c->user_tune.occ == 3 ? 3 : 2;
-        const size_t budget = (t.occ == 2 ? 112 : 74) * 1024;
+        // two CTAs: the B200's 228 KB of shared memory per SM less 1 KB reserved per CTA, halved
+        const size_t budget = t.occ == 2 ? 115712 : 74 * 1024;
+        // at two CTAs per SM a warp evaluates one particle per far-field cell of a region at once (objective_stream.cu):
+        // a group that is not a multiple of that would leave lanes idle in its last step
+        const int cells = ctx_cells(c, t.r), per_warp = t.occ == 2 ? cells : 1;
         auto fit_sp = [&](int stg) {
             t.stages = stg;
             int spg = 0;
             for (int cand = 1; cand <= 16; ++cand) {
                 t.sp = cand;
-                if (objective_stream_smem_bytes(c->P, t, ctx_cells(c, t.r)) <= budget) spg = cand;
+                if (objective_stream_smem_bytes(c->P, t, cells) <= budget && (cand < per_warp || cand % per_warp == 0))
+                    spg = cand;
             }
             return spg;
         };

@@ -1,6 +1,6 @@
 // K1s: the STREAMED evaluation kernel of the uniform-axis objective (same result definition and the same
 // arithmetic, bit for bit, as objective_uniform.cu: reference equations.py:152-212 with ps2,
-// proc_autophase.py:29-36, and voigt, equations.py:141-147; both call eval_region of uniform_eval.cuh).
+// proc_autophase.py:29-36, and voigt, equations.py:141-147; both go through the per-lane steps of uniform_eval.cuh).
 //
 // What differs is how a CTA is fed.  objective_uniform_kernel gives a CTA one point tile and ONE group of
 // particles: stage the tile, wait for the group's constants, evaluate, __syncthreads, write.  ncu (profiles/
@@ -17,7 +17,12 @@
 //   * the CTA's warps take the tile's regions in rotation - group g's region q is evaluated by warp (q - g) mod NW -
 //     so every warp sees every region equally often and the regions' different costs (how many peaks are near) no
 //     longer make a CTA wait for its slowest warp;
-//   * a warp writes its region sums straight to global memory; there is no __syncthreads after the prologue.
+//   * a warp writes its region sums straight to global memory; there is no __syncthreads after the prologue;
+//   * with several far-field cells per region (real part, 2 CTAs per SM) a warp evaluates its region for `sub`
+//     particles at once, one per group of 32/sub lanes, cell by cell (eval_region_multi): the near peaks of particles
+//     in one cell hardly differ - their centres move by a few grid points, the near zone spans a thousand - while the
+//     cells of a region often differ by a peak, so the warp visits fewer peaks with idle lanes, and it reads the staged
+//     points and reduces once per `sub` particles.
 //
 // The sums are stored per REGION, partials[B][S][n_tiles][NW]; the finish / finalize kernels add the NW regions of a
 // tile first and then the tiles - the order objective_uniform_kernel and the fused swarm kernel use - so the objective
@@ -73,6 +78,9 @@ __global__ void __launch_bounds__(THREADS, (R <= 8 ? OCC * 256 : 512) / THREADS)
 objective_stream_kernel(ObjArgs a) {
     constexpr int NSUM = KK ? 2 : 1;
     constexpr int NW = THREADS / 32;
+    // several particles per warp (eval_region_multi); at 3 CTAs per SM (80 registers) its per-lane particle pointers
+    // would spill, so that build keeps one particle per warp
+    constexpr bool MULTI = SUB > 1 && !KK && OCC == 2;
     extern __shared__ __align__(16) double smem[];
     const int b = blockIdx.z;
     if (a.frozen && a.frozen[b]) return;
@@ -173,7 +181,19 @@ objective_stream_kernel(ObjArgs a) {
         const double* xs = a.x + (pb + q0) * D;
         double* out = a.partials + (((pb + q0) * n_tiles + tile) * NW + rw) * NSUM;
         mbar_wait(bars + sl, phase);                       // this fill of the slot has landed
-        for (int sp = 0; sp < nsp; ++sp) {
+        if constexpr (MULTI) {
+            // SUB particles per pass over the region, one per 32/SUB-lane group; a short last step repeats the
+            // group's last particle in the idle groups and stores nothing for them
+            constexpr int LPC = 32 / SUB;
+            const int q = lane / LPC;
+            for (int sp0 = 0; sp0 < nsp; sp0 += SUB) {
+                const int sp = min(sp0 + q, nsp - 1);
+                const double ss = eval_region_multi<R, TB, SUB>(
+                    cf + sp * s_coef, pt + sp * kPartDoubles, mk + sp * s_mask, fc + sp * s_far, an[sp * NW], MW, P, lane,
+                    xi0, inv_H, suv, swt, swf, rw * 32, THREADS, tab, xs + (size_t)sp * D, sw + tile0, N - tile0, h, w_ulp);
+                if ((lane & (LPC - 1)) == 0 && sp0 + q < nsp) out[sp * s_out] = ss;
+            }
+        } else for (int sp = 0; sp < nsp; ++sp) {
             double ssi = 0.0;
             const double ss = eval_region<R, TB, KK, false, SUB>(cf, pt, mk, fc, *an, MW, P, lane, lcell, w_first, xi0, inv_H, suv,
                                                             swt, t, THREADS, tab, xs, sw + i_first, N - i_first, h, w_ulp,

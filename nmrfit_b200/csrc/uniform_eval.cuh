@@ -8,6 +8,8 @@
 //                     two-pass path, shared memory in the fused kernel.
 //   eval_region       one warp's squared weighted residual over its region, from those constants
 //                     and the staged (u, v, weights) of the tile.
+//   eval_region_multi the same sum for `sub` particles at once, one per group of 32/sub lanes, cell by cell
+//                     (the streamed kernel); both are made of the same per-lane steps.
 //
 // Regions and cells.  A warp evaluates a REGION of 32*R consecutive points (a thread R of them).  The far-field
 // polynomial (nmrfit_math.cuh) lives on a CELL: the region itself, or one half / quarter of it (`sub` = 1, 2, 4 cells
@@ -251,16 +253,6 @@ __device__ __forceinline__ double2 stage_point(double u, double v, double wt) {
 __device__ __forceinline__ int stage_slot_uv(int t, int j, int stride) { return j * stride + (t ^ j); }
 __device__ __forceinline__ int stage_slot_wt(int t, int j, int stride) { return j * stride + (t ^ (2 * j)); }
 
-// One warp, one particle, one region: sum over the warp's 32*R points of (weights * (V_data - V_fit))^2, identical
-// in every lane on return.  cf [P][8], pt [kPartDoubles], mk [mask_words_per_region], fc [sub][kFarPoly] (16-byte aligned) and ew
-// are the particle's constants for this region (`sub` far-field cells of 32/sub lanes each, lc = lane_cell(lane, sub, P); xi0 is the lane's first
-// point's position inside ITS cell and inv_H the step of that coordinate per point); the R points of thread t of the
-// tile sit at stage_slot_uv/wt(t, j, stride) of suv / swt (SWZ) or at j*stride + t (!SWZ); w_first is the abscissa of its
-// first point.  The exact path (peaks too narrow for the recurrences) reads the particle's parameters xs and the stored
-// abscissae sw_first[0..n_valid).
-// SUBT: the number of cells when the caller knows it at compile time (0: take everything from lc).
-// KK = 1 (fit_im, reference semantics) also returns through *ss_im the same sum for the imaginary parts:
-// I_data = u sin(phi) + v cos(phi) against the last peak's Kramers-Kronig counterpart (closed form, nmrfit_math.cuh).
 // Where a lane's far-field cell keeps its mask block and its polynomial inside the region's constants: loop-invariant,
 // computed once per thread (mk_off == 0 <=> the region is one cell and has no separate union block).
 struct LaneCell { int mk_off, fc_off, mirror; };       // mirror: xor mask to the lane holding the mirror-image span
@@ -273,59 +265,68 @@ __device__ __forceinline__ LaneCell lane_cell(int lane, int sub, int P) {
     return lc;
 }
 
-template <int R, int TB, int KK = 0, bool SWZ = true, int SUBT = 0>
-__device__ __forceinline__ double eval_region(const double* __restrict__ cf, const double* __restrict__ pt,
-                                              const unsigned* __restrict__ mk, const double* __restrict__ fc,
-                                              const double2 ew, int MW, int P, int lane, const LaneCell lc, double w_first, double xi0,
-                                              double inv_H, const double2* __restrict__ suv, const double* __restrict__ swt,
-                                              int t, int stride, const double* __restrict__ tab,
-                                              const double* __restrict__ xs, const double* __restrict__ sw_first,
-                                              int n_valid, double h, double w_ulp, double* ss_im = nullptr) {
-    const unsigned* mkc = mk + lc.mk_off;                  // this lane's cell; mk itself: the union's block (prepare_particle)
-    double acc[R];
-    const double py = pt[66];                              // P*yoff: yoff is added once per peak (equations.py:147,195)
-    // all far peaks of this lane's cell at once; the accumulators start from it (and from P*yoff).  A cell without far
-    // peaks holds zeros: evaluated all the same - rare, and a branch here costs every other cell a dozen instructions.
-    {
-        const double* fcc = fc + lc.fc_off;
-        double C[kFarPoly];
+// The per-lane steps of a region's evaluation, shared by eval_region and eval_region_multi so that a point gets the
+// same arithmetic in the same order whichever of them evaluates it.
+//
+// Far field: the cell's polynomial fcc [kFarPoly] (plus P*yoff) at the lane's R points - all far peaks of the cell at
+// once.  A cell without far peaks holds zeros: evaluated all the same - rare, and a branch here costs every other cell a
+// dozen instructions.  The last R/2 points are the mirror image, inside the cell, of the first R/2 points of lane ^ mirror.
+template <int R>
+__device__ __forceinline__ void lane_far_start(const double* __restrict__ fcc, double py, double xi0, double inv_H,
+                                               int mirror, double (&acc)[R]) {
+    double C[kFarPoly];
 #pragma unroll
-        for (int n = 0; n < kFarPoly; n += 2) {
-            const double2 t2 = *reinterpret_cast<const double2*>(fcc + n);
-            C[n] = t2.x; C[n + 1] = t2.y;
-        }
-        C[0] += py;
-        double mir[R / 2];
-        far_init_half<R>(C, xi0, inv_H, acc, mir);
-        // the last R/2 points: the mirror image, inside the cell, of the first R/2 points of lane ^ (lanes per cell - 1)
+    for (int n = 0; n < kFarPoly; n += 2) {
+        const double2 t2 = *reinterpret_cast<const double2*>(fcc + n);
+        C[n] = t2.x; C[n + 1] = t2.y;
+    }
+    C[0] += py;
+    double mir[R / 2];
+    far_init_half<R>(C, xi0, inv_H, acc, mir);
 #pragma unroll
-        for (int j = 0; j < R / 2; ++j) acc[R - 1 - j] = __shfl_xor_sync(0xffffffffu, mir[j], SUBT ? 32 / SUBT - 1 : lc.mirror);
-    }
-    for (int wd = 0; wd < MW; ++wd) {
-        const unsigned mine = mkc[wd];                     // peaks near this lane's cell
-        for (unsigned m = mk[wd]; m; m &= m - 1) {         // peaks near ANY cell of the region (uniform across the warp)
-            const int kb = __ffs(m) - 1;
-            const int k = wd * 32 + kb;
-            const double2 c01 = *reinterpret_cast<const double2*>(cf + k * 8);
-            const double2 c23 = *reinterpret_cast<const double2*>(cf + k * 8 + 2);
-            const double2 c45 = *reinterpret_cast<const double2*>(cf + k * 8 + 4);
-            const double2 c67 = *reinterpret_cast<const double2*>(cf + k * 8 + 6);
-            SpanCoef c;
-            c.loc = c01.x; c.kL = c01.y; c.kG = c23.x; c.aL = c23.y;
-            c.aG = c45.x; c.dT = c45.y; c.thr = c67.x; c.c2 = c67.y;
-            // (in a cell for which the peak is far it is already inside that cell's polynomial)
-            if ((SUBT ? SUBT == 1 : lc.mk_off == 0) || ((mine >> kb) & 1u)) peak_span<R, TB>(w_first - c.loc, c, tab, acc);
-        }
-    }
-    if (pt[67] != 0.0) {                                   // rare: peaks too narrow for the uniform-axis shortcuts
+    for (int j = 0; j < R / 2; ++j) acc[R - 1 - j] = __shfl_xor_sync(0xffffffffu, mir[j], mirror);
+}
+
+// near peak k (span coefficients cf [P][8]) at the lane's R points
+template <int R, int TB>
+__device__ __forceinline__ void lane_near_peak(const double* __restrict__ cf, int k, double w_first,
+                                               const double* __restrict__ tab, double (&acc)[R]) {
+    const double2 c01 = *reinterpret_cast<const double2*>(cf + k * 8);
+    const double2 c23 = *reinterpret_cast<const double2*>(cf + k * 8 + 2);
+    const double2 c45 = *reinterpret_cast<const double2*>(cf + k * 8 + 4);
+    const double2 c67 = *reinterpret_cast<const double2*>(cf + k * 8 + 6);
+    SpanCoef c;
+    c.loc = c01.x; c.kL = c01.y; c.kG = c23.x; c.aL = c23.y;
+    c.aG = c45.x; c.dT = c45.y; c.thr = c67.x; c.c2 = c67.y;
+    peak_span<R, TB>(w_first - c.loc, c, tab, acc);
+}
+
+// rare: peaks too narrow for the uniform-axis shortcuts, from the particle's parameters xs and the stored abscissae
+template <int R, int TB>
+__device__ __forceinline__ void lane_exact_peaks(const double* __restrict__ cf, const double* __restrict__ pt, int P,
+                                                 const double* __restrict__ xs, const double* __restrict__ sw_first,
+                                                 int n_valid, double w_first, double h, double w_ulp,
+                                                 const double* __restrict__ tab, double (&acc)[R]) {
+    if (pt[67] != 0.0) {
         for (int k = 0; k < P; ++k) {
             if (!(cf[k * 8 + 6] < 0.0)) continue;
             const SpanCoef c = make_span_coef(xs[2], xs[4 + 3 * k], xs[5 + 3 * k], xs[6 + 3 * k], h, w_ulp, R);
             peak_exact<R, TB>(sw_first, n_valid, w_first, h, c, tab, acc);
         }
     }
-    // residual against the phase-rotated data; the rotation advances by p1/N per point
-    const double2 el = *reinterpret_cast<const double2*>(pt + 2 * lane);
+}
+
+// the lane's sum of squared weighted residuals against the phase-rotated data: ew = the region's phase anchor, lf = the
+// lane factor's index in the phase table (the lane's thread span inside the region); the rotation advances by p1/N per
+// point.  KK also returns the imaginary parts' sum through *ssi.
+template <int R, int KK, bool SWZ>
+__device__ __forceinline__ double lane_residual(const double (&acc)[R], const double* __restrict__ cf,
+                                                const double* __restrict__ pt, int P, const double2 ew, int lf,
+                                                const double2* __restrict__ suv, const double* __restrict__ swt, int t,
+                                                int stride, const double* __restrict__ xs,
+                                                const double* __restrict__ sw_first, int n_valid, double w_first,
+                                                double h, double w_ulp, double* ssi_out) {
+    const double2 el = *reinterpret_cast<const double2*>(pt + 2 * lf);
     const double cd = pt[64], sd = pt[65];
     double cr = fma(ew.x, el.x, -(ew.y * el.y));
     double ci = fma(ew.y, el.x, ew.x * el.y);
@@ -373,12 +374,101 @@ __device__ __forceinline__ double eval_region(const double* __restrict__ cf, con
             cr = c2;
         }
     }
+    if (KK) *ssi_out = ssi;
+    return ss;
+}
+
+// One warp, one particle, one region: sum over the warp's 32*R points of (weights * (V_data - V_fit))^2, identical
+// in every lane on return.  cf [P][8], pt [kPartDoubles], mk [mask_words_per_region], fc [sub][kFarPoly] (16-byte aligned) and ew
+// are the particle's constants for this region (`sub` far-field cells of 32/sub lanes each, lc = lane_cell(lane, sub, P); xi0 is the lane's first
+// point's position inside ITS cell and inv_H the step of that coordinate per point); the R points of thread t of the
+// tile sit at stage_slot_uv/wt(t, j, stride) of suv / swt (SWZ) or at j*stride + t (!SWZ); w_first is the abscissa of its
+// first point.  The exact path (peaks too narrow for the recurrences) reads the particle's parameters xs and the stored
+// abscissae sw_first[0..n_valid).
+// SUBT: the number of cells when the caller knows it at compile time (0: take everything from lc).
+// KK = 1 (fit_im, reference semantics) also returns through *ss_im the same sum for the imaginary parts:
+// I_data = u sin(phi) + v cos(phi) against the last peak's Kramers-Kronig counterpart (closed form, nmrfit_math.cuh).
+template <int R, int TB, int KK = 0, bool SWZ = true, int SUBT = 0>
+__device__ __forceinline__ double eval_region(const double* __restrict__ cf, const double* __restrict__ pt,
+                                              const unsigned* __restrict__ mk, const double* __restrict__ fc,
+                                              const double2 ew, int MW, int P, int lane, const LaneCell lc, double w_first, double xi0,
+                                              double inv_H, const double2* __restrict__ suv, const double* __restrict__ swt,
+                                              int t, int stride, const double* __restrict__ tab,
+                                              const double* __restrict__ xs, const double* __restrict__ sw_first,
+                                              int n_valid, double h, double w_ulp, double* ss_im = nullptr) {
+    const unsigned* mkc = mk + lc.mk_off;                  // this lane's cell; mk itself: the union's block (prepare_particle)
+    double acc[R];
+    // (P*yoff: yoff is added once per peak, equations.py:147,195)
+    lane_far_start<R>(fc + lc.fc_off, pt[66], xi0, inv_H, SUBT ? 32 / SUBT - 1 : lc.mirror, acc);
+    for (int wd = 0; wd < MW; ++wd) {
+        const unsigned mine = mkc[wd];                     // peaks near this lane's cell
+        for (unsigned m = mk[wd]; m; m &= m - 1) {         // peaks near ANY cell of the region (uniform across the warp)
+            const int kb = __ffs(m) - 1;
+            // (in a cell for which the peak is far it is already inside that cell's polynomial)
+            if ((SUBT ? SUBT == 1 : lc.mk_off == 0) || ((mine >> kb) & 1u)) lane_near_peak<R, TB>(cf, wd * 32 + kb, w_first, tab, acc);
+        }
+    }
+    lane_exact_peaks<R, TB>(cf, pt, P, xs, sw_first, n_valid, w_first, h, w_ulp, tab, acc);
+    double ssi = 0.0;
+    double ss = lane_residual<R, KK, SWZ>(acc, cf, pt, P, ew, lane, suv, swt, t, stride, xs, sw_first, n_valid, w_first,
+                                          h, w_ulp, &ssi);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         ss += __shfl_xor_sync(0xffffffffu, ss, o);
         if (KK) ssi += __shfl_xor_sync(0xffffffffu, ssi, o);
     }
     if (KK) *ss_im = ssi;
+    return ss;
+}
+
+// One warp, SUB (2 or 4) particles, one region of SUB far-field cells, real part only: the warp's 32 / SUB-lane group q
+// holds particle q and walks the region's cells one pass at a time.  In pass c lane i of a group evaluates the points
+// that lane c * 32/SUB + i evaluates in eval_region - same constants, same arithmetic, same order - so every group
+// visits only the peaks near cell c of SOME particle of the warp (near sets of particles in one cell hardly differ,
+// while the cells of one region often differ by a peak), the staged points are read once for SUB particles, and the
+// warp's reduction tree is paid once for SUB particles.  The lane's per-pass sums are added in eval_region's tree:
+// its shuffle levels 16 (and 8) pair the passes ((s0 + s2) + (s1 + s3), resp. s0 + s1), then xor 32/SUB/2 .. 1.
+// Arguments are the lane's particle's, as for eval_region, except: mk = its region's mask words (the union block
+// first), fc = its region's SUB polynomials; t0 = the region's first thread span of the tile, swf = the tile's stored
+// first abscissae per thread span, sw_tile = the w plane from the tile's first point on, n_tile = the axis' points from
+// there on.  Returns the particle's region sum in every lane of its group; the staged points sit at j*stride + t.
+template <int R, int TB, int SUB>
+__device__ __forceinline__ double eval_region_multi(const double* __restrict__ cf, const double* __restrict__ pt,
+                                                    const unsigned* __restrict__ mk, const double* __restrict__ fc,
+                                                    const double2 ew, int MW, int P, int lane, double xi0, double inv_H,
+                                                    const double2* __restrict__ suv, const double* __restrict__ swt,
+                                                    const double* __restrict__ swf, int t0, int stride,
+                                                    const double* __restrict__ tab, const double* __restrict__ xs,
+                                                    const double* __restrict__ sw_tile, int n_tile, double h, double w_ulp) {
+    static_assert(SUB == 2 || SUB == 4, "one pass per far-field cell of the region");
+    constexpr int LPC = 32 / SUB;                          // lanes per cell = lanes per particle
+    const int i = lane & (LPC - 1);
+    const double py = pt[66];
+    double se = 0.0, so = 0.0;                             // sums of the even / odd passes
+#pragma unroll 1
+    for (int c = 0; c < SUB; ++c) {
+        const int lf = c * LPC + i, t = t0 + lf;
+        const double w_first = swf[t];
+        double acc[R];
+        lane_far_start<R>(fc + c * kFarPoly, py, xi0, inv_H, LPC - 1, acc);
+        const unsigned* mkc = mk + (1 + c) * (MW + 1);
+        for (int wd = 0; wd < MW; ++wd) {
+            const unsigned mine = mkc[wd];                 // peaks near cell c of this lane's particle
+            for (unsigned m = __reduce_or_sync(0xffffffffu, mine); m; m &= m - 1) {   // ... of any particle of the warp
+                const int kb = __ffs(m) - 1;
+                if ((mine >> kb) & 1u) lane_near_peak<R, TB>(cf, wd * 32 + kb, w_first, tab, acc);
+            }
+        }
+        lane_exact_peaks<R, TB>(cf, pt, P, xs, sw_tile + t * R, n_tile - t * R, w_first, h, w_ulp, tab, acc);
+        const double s = lane_residual<R, 0, false>(acc, cf, pt, P, ew, lf, suv, swt, t, stride, xs, sw_tile + t * R,
+                                                    n_tile - t * R, w_first, h, w_ulp, nullptr);
+        // (s >= +0: a sum of squares from +0, so 0 + s == s)
+        if (c & 1) so += s;
+        else se += s;
+    }
+    double ss = se + so;
+#pragma unroll
+    for (int o = LPC / 2; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
     return ss;
 }
 
