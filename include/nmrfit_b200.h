@@ -91,6 +91,19 @@ int nmrfit_ctx_set_spectra(nmrfit_ctx* ctx, int b0, int count, const double* w, 
 int nmrfit_ctx_compute_weights(nmrfit_ctx* ctx, const double* peak_bounds, const double* peak_values, int n_windows,
                                int sweeps, double omega, double* weights_out, void* stream);
 
+/* Normal equations of the objective at one parameter vector per spectrum, from the spectra and weights the context
+ * holds (any axis; FP64 on FP32 contexts too).  With D = 4 + 3P, x = [p0, p1, r, yoff, (width, loc, area) x P],
+ *   res_i = Vdata_i(p0, p1) - Vfit_i(x),   Vdata = Re ps2(u, v, p0, p1),   Vfit = sum_k [yoff + a_k (r L_k + (1-r) G_k)]
+ * and A_i = d res_i / dx (d/dp0 = -Idata_i, d/dp1 = -Idata_i * i/N, d/dyoff = -P, d/dr = -sum_k a_k (L_k - G_k),
+ * d/da_k = -(r L_k + (1-r) G_k), and the closed-form width and location derivatives), over all n_points:
+ *   H = sum w_i^2 A_i^T A_i,  M = sum w_i^4 A_i^T A_i,  g = sum w_i^2 res_i A_i,  ssr = (sum w_i^2 res_i^2, sum res_i^2)
+ * where w_i are the weights.  x [n_spectra][D]; H, M [n_spectra][D][D] (both triangles), g [n_spectra][D],
+ * ssr [n_spectra][2].  Host or device pointers (UVA); any output may be NULL; returns when the outputs are written.
+ * Sums are in a fixed order that depends on n_points and n_peaks only: bit-reproducible, and a spectrum's result
+ * is the same alone or in a batch.  n_peaks <= 64; NMRFIT_ERR_ARG above. */
+int nmrfit_ctx_normal_equations(nmrfit_ctx* ctx, const double* x, double* H, double* M, double* g, double* ssr,
+                                void* stream);
+
 /* Which objective kernel runs (default NMRFIT_ALGO_AUTO), and which one a launch with this fit_im would use.
  * Both kernels evaluate equations.objective (equations.py:152-212); the uniform-axis one exploits
  * w_i = w_0 + i*h (what core.load builds, core.py:58-60) to replace most exponentials by a recurrence. */

@@ -51,6 +51,7 @@ SIGNATURES = {
     'nmrfit_ctx_set_spectrum': (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     'nmrfit_ctx_set_spectra': (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp]),
     'nmrfit_ctx_compute_weights': (_i, [_vp, _vp, _vp, _i, _i, _d, _vp, _vp]),
+    'nmrfit_ctx_normal_equations': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     'nmrfit_ctx_set_algorithm': (_i, [_vp, _i]),
     'nmrfit_ctx_get_algorithm': (_i, [_vp, _i, c_int_p]),
     'nmrfit_ctx_set_tuning': (_i, [_vp, _i, _i, _i, _i]),
@@ -223,6 +224,21 @@ class Context:
         check(lib().nmrfit_ctx_compute_weights(self._h, ptr(pb), ptr(pv), pb.shape[1], int(sweeps), float(omega),
                                                ptr(out), ptr(stream)))
         return out
+
+    def normal_equations(self, x, stream=None):
+        """Normal equations of the objective at ``x`` [B, D] (one parameter vector per spectrum) over the spectra and
+        weights the context holds: returns host arrays ``H`` [B, D, D] = sum w^2 A^T A, ``M`` [B, D, D] = sum w^4 A^T A,
+        ``g`` [B, D] = sum w^2 res A and ``ssr`` [B, 2] = (sum w^2 res^2, sum res^2), with res = Vdata - Vfit and
+        A = d res / dx (include/nmrfit_b200.h)."""
+        x = as_f64(x)
+        if x.shape != (self.B, self.D):
+            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        H = np.empty((self.B, self.D, self.D))
+        M = np.empty((self.B, self.D, self.D))
+        g = np.empty((self.B, self.D))
+        ssr = np.empty((self.B, 2))
+        check(lib().nmrfit_ctx_normal_equations(self._h, ptr(x), ptr(H), ptr(M), ptr(g), ptr(ssr), ptr(stream)))
+        return H, M, g, ssr
 
     def set_algorithm(self, algorithm=ALGO_AUTO):
         """ALGO_AUTO (default), ALGO_GENERAL (any axis) or ALGO_UNIFORM (require the uniform-axis kernel)."""

@@ -115,6 +115,7 @@ struct nmrfit_ctx {
     long long epoch = 0;               // fits begun on this context: part of the exchange token
     double peer_timeout_ms = 20000.0;  // wall-time bound of a wait for the peers' tokens
     DevBuf<double> wscratch, wbounds;  // batched weights: sweep scratch [B][N], windows + values
+    DevBuf<double> ne_x, ne_part, ne_out;   // normal equations: positions, chunk partials, H | M | g | ssr
     cudaStream_t pipe[2] = {nullptr, nullptr};   // nmrfit_objective_batch_host: slices of a large particle set
     double* h_f = nullptr;                       // ... and page-locked staging of their values
     size_t h_f_cap = 0;
@@ -511,6 +512,9 @@ void nmrfit_ctx_destroy(nmrfit_ctx* c) {
     c->fin_scratch.release();
     c->fin_tickets.release();
     c->wbounds.release();
+    c->ne_x.release();
+    c->ne_part.release();
+    c->ne_out.release();
     for (int k = 0; k < 2; ++k)
         if (c->pipe[k]) cudaStreamDestroy(c->pipe[k]);
     if (c->h_f) cudaFreeHost(c->h_f);
@@ -616,6 +620,36 @@ int nmrfit_ctx_compute_weights(nmrfit_ctx* c, const double* peak_bounds, const d
         CK(cudaMemcpy2DAsync(weights_out, sizeof(double) * N, c->spec.ptr + 3 * N, sizeof(double) * 4 * N,
                              sizeof(double) * N, B, cudaMemcpyDefault, st));
     CK(cudaStreamSynchronize(st));                         // the staged bounds may be pageable host memory
+    return NMRFIT_OK;
+}
+
+int nmrfit_ctx_normal_equations(nmrfit_ctx* c, const double* x, double* H, double* M, double* g, double* ssr,
+                                void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x) return fail(NMRFIT_ERR_ARG, "x must be non-NULL");
+    if (c->P > 64)
+        return fail(NMRFIT_ERR_ARG, "normal equations support at most 64 peaks (D <= 196), the context has " +
+                                        std::to_string(c->P));
+    for (char f : c->spec_set)
+        if (!f) return fail(NMRFIT_ERR_STATE, "every spectrum must be set before its normal equations are computed");
+    CK(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t B = (size_t)c->B, D = (size_t)c->D, DD = D * D, per = 2 * DD + D + 2;
+    const NormalEqPlan p = normal_eq_plan(c->N, c->P);
+    const double* xd = nullptr;
+    if (int r = stage(x, B * D, c->ne_x, st, &xd)) return r;
+    CK(c->ne_part.reserve(normal_eq_scratch_doubles(p, c->B)));
+    CK(c->ne_out.reserve(B * per));
+    cudaError_t e = launch_normal_eq(c->spec.ptr, xd, p, c->B, c->ne_part.ptr, c->ne_out.ptr, st);
+    if (e != cudaSuccess) return fail_cuda(e, "normal equations launch");
+    // per spectrum the device block is H [D][D] | M [D][D] | g [D] | ssr [2]
+    const size_t offs[4] = {0, DD, 2 * DD, 2 * DD + D}, lens[4] = {DD, DD, D, 2};
+    double* dst[4] = {H, M, g, ssr};
+    for (int k = 0; k < 4; ++k)
+        if (dst[k])
+            CK(cudaMemcpy2DAsync(dst[k], sizeof(double) * lens[k], c->ne_out.ptr + offs[k], sizeof(double) * per,
+                                 sizeof(double) * lens[k], B, cudaMemcpyDefault, st));
+    CK(cudaStreamSynchronize(st));                         // x and the outputs may be pageable host memory
     return NMRFIT_OK;
 }
 

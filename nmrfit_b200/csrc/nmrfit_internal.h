@@ -212,6 +212,21 @@ cudaError_t launch_kk(const double* w, int n, double r, double width, double loc
 cudaError_t launch_generate_result(const double* params_host, int P, const double* w, int n, double* real,
                                    double* imag, double* V, double* I, double* u, double* v, cudaStream_t st);
 
+// ---- K12 normal equations of the objective (normal_eq.cu) ---------------------------
+// Tiling of the pass: a function of N and P only, so that a spectrum's sums do not depend on the batch.
+struct NormalEqPlan {
+    int N, P;
+    int nb, ep, tri, tasks;     // 4x4 blocks per matrix edge, padded row length, blocks per triangle, both triangles
+    int ng, slices, tasks_per_slice, threads;   // point groups per CTA, CTAs per chunk, blocks per CTA, CTA size
+    int tp, chunk, n_chunks;    // points per staged tile, points per CTA, chunks per spectrum
+    size_t smem;                // dynamic shared memory of the partial kernel, bytes
+};
+NormalEqPlan normal_eq_plan(int N, int P);
+size_t normal_eq_scratch_doubles(const NormalEqPlan& p, int B);
+// x [B][D] -> out [B][2*D*D + D + 2] (H, M, g, ssr per spectrum); `part` holds normal_eq_scratch_doubles doubles
+cudaError_t launch_normal_eq(const double* spec, const double* x, const NormalEqPlan& p, int B, double* part,
+                             double* out, cudaStream_t st);
+
 // ---- probes -------------------------------------------------------------------
 cudaError_t fp64_peak_probe(int iters, int repeats, double* tflops, double* sustained, cudaStream_t st);
 

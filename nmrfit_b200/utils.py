@@ -184,6 +184,30 @@ class FitUtility:
         """Fitted areas: every third parameter from index 6 (utils.py:322)."""
         return np.array([self.params[i] for i in range(6, len(self.params), 3)])
 
+    def compute_uncertainties(self):
+        """Standard errors of ``params`` from the linearised least-squares problem at the fitted point (one pass
+        over the spectrum on the GPU, see ``compute_uncertainties_batch``).  Sets ``covariance`` [D, D], ``stderr``
+        [D] and ``uncertainty_info``, and returns ``stderr``.
+
+        Raises RuntimeError before ``fit()``, NotImplementedError with ``fit_im`` (that objective is a sum of two
+        RMSEs, not a least-squares problem) and ValueError when the spectrum has no more points than parameters."""
+        compute_uncertainties_batch([self])
+        return self.stderr
+
+    def area_fraction_stderr(self):
+        """Standard error of ``calculate_area_fraction()`` by the delta method, with the split into main peaks and
+        satellites held fixed: for f = S/T, df/da_k = (1 - f)/T for a satellite and -f/T for a main peak.  Computes
+        the covariance first if it is missing."""
+        if getattr(self, 'covariance', None) is None:
+            self.compute_uncertainties()
+        areas = self.get_areas()
+        m = np.mean(areas)
+        total = areas.sum()
+        frac = areas[areas < m].sum() / total
+        grad = np.zeros(len(self.params))
+        grad[6::3] = np.where(areas < m, (1 - frac) / total, -frac / total)
+        return float(np.sqrt(grad @ self.covariance @ grad))
+
     def _print_summary(self):
         import pandas as pd
         res = np.array(self.params)
@@ -196,6 +220,80 @@ class FitUtility:
         print('\nPeak parameters')
         print(res_peaks.to_string(index=False))
         print("Error:\t", self.error)
+
+
+# ---- parameter uncertainties (not in the reference) ---------------------------------------------------------------
+def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper):
+    """Sandwich covariance of the weighted least-squares estimate from the normal equations of one spectrum
+    (``Context.normal_equations``): ``C = s^2 H^-1 M H^-1`` with ``s^2 = sum res^2 / (N - D)``.
+
+    The dynamic weights emphasise small peaks; they are not inverse noise levels, while the spectral noise is the
+    same at every point of the unweighted data.  So the noise level comes from the unweighted residuals and the
+    weights enter through H (= A^T W^2 A) and M (= A^T W^4 A); with unit weights M = H and C = s^2 H^-1.  The estimate
+    assumes independent noise from point to point: zero-filled or apodised spectra have correlated noise, and the
+    errors are then optimistic.
+
+    H^-1 comes from a Cholesky factorisation of the Jacobi-scaled ``S H S``, S = diag(H_jj^-1/2) (H itself spans
+    many decades).  If that fails, or some H_jj = 0 (a parameter the residual does not depend on, such as the width
+    of a peak of area 0), ``C`` is all NaN and ``info['singular']`` is True.
+
+    Returns ``(C [D, D], info)``, info = dict(sigma, dof, gradient=g, at_bound, singular); ``at_bound[j]`` flags a
+    parameter within 1e-9 of its box width of a bound, where the linearisation says little."""
+    H, M, g = np.asarray(H, dtype=np.float64), np.asarray(M, dtype=np.float64), np.asarray(g, dtype=np.float64)
+    x, lb, ub = (np.asarray(a, dtype=np.float64) for a in (params, lower, upper))
+    D = H.shape[0]
+    dof = int(n_points) - D
+    sigma2 = float(ssr[1]) / dof
+    tol = 1e-9 * (ub - lb)
+    info = dict(sigma=float(np.sqrt(sigma2)), dof=dof, gradient=g.copy(),
+                at_bound=(np.abs(x - lb) <= tol) | (np.abs(ub - x) <= tol), singular=False)
+    diag = np.diag(H)
+    if not np.all(np.isfinite(H)) or np.any(diag <= 0):
+        info['singular'] = True
+        return np.full((D, D), np.nan), info
+    s = 1.0 / np.sqrt(diag)
+    try:
+        L = np.linalg.cholesky(s[:, None] * H * s[None, :])
+    except np.linalg.LinAlgError:
+        info['singular'] = True
+        return np.full((D, D), np.nan), info
+    Linv = np.linalg.solve(L, np.eye(D))
+    Hinv = s[:, None] * (Linv.T @ Linv) * s[None, :]
+    C = sigma2 * (Hinv @ M @ Hinv)
+    return 0.5 * (C + C.T), info
+
+
+def compute_uncertainties_batch(fits):
+    """``compute_uncertainties()`` for many fits of equal length and peak count (what ``fit_batch`` returns) in one
+    device pass: the normal equations of every spectrum at its fitted ``params`` with its fit's ``weights``, then
+    ``covariance_from_normal`` per fit.  Sets ``covariance``, ``stderr`` and ``uncertainty_info`` on every fit and
+    returns the list of ``stderr``."""
+    fits = list(fits)
+    if not fits:
+        return []
+    for f in fits:
+        if getattr(f, 'params', None) is None:
+            raise RuntimeError('compute_uncertainties needs a fitted model: call fit() first')
+        if f.fit_im:
+            raise NotImplementedError('uncertainties are not available with fit_im: that objective is a sum of two '
+                                      'RMSEs, not a least-squares problem')
+    N, D = len(fits[0].data.w), len(fits[0].params)
+    for f in fits:
+        if len(f.data.w) != N or len(f.params) != D:
+            raise ValueError('every fit of a batch must have the same number of points and peaks')
+    if N <= D:
+        raise ValueError('the spectrum has %d points for %d parameters: no residual degrees of freedom' % (N, D))
+    W, U, V, weights = (np.stack([_cabi.as_f64(a) for a in arrs])
+                        for arrs in zip(*[(f.data.w, f.data.u, f.data.v, f.weights) for f in fits]))
+    X = np.stack([_cabi.as_f64(f.params) for f in fits])
+    with _cabi.pooled_context(len(fits), N, (D - 4) // 3, device=fits[0].options.get('device')) as ctx:
+        ctx.set_spectra(W, U, V, weights)
+        H, M, g, ssr = ctx.normal_equations(X)
+    for b, f in enumerate(fits):
+        f.covariance, f.uncertainty_info = covariance_from_normal(H[b], M[b], g[b], ssr[b], N, f.params, f.lower,
+                                                                  f.upper)
+        f.stderr = np.sqrt(np.diag(f.covariance))
+    return [f.stderr for f in fits]
 
 
 # ---- automatic peak selection (utils.py:670-783) on the GPU ----------------------------------------------------
