@@ -103,6 +103,11 @@ int nmrfit_ctx_compute_weights(nmrfit_ctx* ctx, const double* peak_bounds, const
  * is the same alone or in a batch.  n_peaks <= 64; NMRFIT_ERR_ARG above. */
 int nmrfit_ctx_normal_equations(nmrfit_ctx* ctx, const double* x, double* H, double* M, double* g, double* ssr,
                                 void* stream);
+/* The launch plan nmrfit_ctx_normal_equations uses for n_points points and n_peaks peaks (host only, no CUDA call).
+ * out[10] = point groups per CTA, task slices per chunk, 4x4 blocks of both triangles (tasks), tasks per slice, threads
+ * per CTA, points per staged tile, points per chunk, chunks, dynamic shared memory (bytes), scratch doubles per spectrum.
+ * NMRFIT_ERR_ARG unless 1 <= n_peaks <= 64 and n_points >= 1. */
+int nmrfit_normal_eq_plan(int n_points, int n_peaks, int* out);
 
 /* Which objective kernel runs (default NMRFIT_ALGO_AUTO), and which one a launch with this fit_im would use.
  * Both kernels evaluate equations.objective (equations.py:152-212); the uniform-axis one exploits

@@ -52,6 +52,7 @@ SIGNATURES = {
     'nmrfit_ctx_set_spectra': (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp]),
     'nmrfit_ctx_compute_weights': (_i, [_vp, _vp, _vp, _i, _i, _d, _vp, _vp]),
     'nmrfit_ctx_normal_equations': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    'nmrfit_normal_eq_plan': (_i, [_i, _i, c_int_p]),
     'nmrfit_ctx_set_algorithm': (_i, [_vp, _i]),
     'nmrfit_ctx_get_algorithm': (_i, [_vp, _i, c_int_p]),
     'nmrfit_ctx_set_tuning': (_i, [_vp, _i, _i, _i, _i]),
@@ -161,6 +162,18 @@ def device_count():
     n = ctypes.c_int(0)
     check(lib().nmrfit_device_count(ctypes.byref(n)))
     return n.value
+
+
+NORMAL_EQ_PLAN_KEYS = ('point_groups', 'slices', 'tasks', 'tasks_per_slice', 'threads', 'tile_points', 'chunk_points',
+                       'n_chunks', 'smem_bytes', 'scratch_doubles')
+
+
+def normal_equations_plan(n_points, n_peaks):
+    """Launch plan of ``Context.normal_equations`` for ``n_points`` points and ``n_peaks`` peaks (host only, no CUDA
+    call): a dict of ``NORMAL_EQ_PLAN_KEYS``.  ``scratch_doubles`` is per spectrum."""
+    out = (ctypes.c_int * len(NORMAL_EQ_PLAN_KEYS))()
+    check(lib().nmrfit_normal_eq_plan(int(n_points), int(n_peaks), out))
+    return dict(zip(NORMAL_EQ_PLAN_KEYS, out))
 
 
 def default_device():

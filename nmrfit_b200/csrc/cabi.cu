@@ -653,6 +653,17 @@ int nmrfit_ctx_normal_equations(nmrfit_ctx* c, const double* x, double* H, doubl
     return NMRFIT_OK;
 }
 
+int nmrfit_normal_eq_plan(int n_points, int n_peaks, int* out) {
+    if (!out) return fail(NMRFIT_ERR_ARG, "out is NULL");
+    if (n_peaks < 1 || n_peaks > 64) return fail(NMRFIT_ERR_ARG, "n_peaks must be 1..64");
+    if (n_points < 1) return fail(NMRFIT_ERR_ARG, "n_points must be >= 1");
+    const NormalEqPlan p = normal_eq_plan(n_points, n_peaks);
+    const int v[10] = {p.ng, p.slices, p.tasks, p.tasks_per_slice, p.threads, p.tp, p.chunk, p.n_chunks,
+                       (int)p.smem, (int)normal_eq_scratch_doubles(p, 1)};
+    for (int k = 0; k < 10; ++k) out[k] = v[k];
+    return NMRFIT_OK;
+}
+
 int nmrfit_ctx_set_algorithm(nmrfit_ctx* c, int algorithm) {
     if (int r = check_ctx(c)) return r;
     if (algorithm != NMRFIT_ALGO_AUTO && algorithm != NMRFIT_ALGO_GENERAL && algorithm != NMRFIT_ALGO_UNIFORM)

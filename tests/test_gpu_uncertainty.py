@@ -1,5 +1,5 @@
 """Normal equations of the objective on the GPU (csrc/normal_eq.cu) against the numpy reference
-(linearisation_ref.py), their determinism, the calibration of the sandwich standard errors over noise realisations, and FitUtility.compute_uncertainties."""
+(linearisation_ref.py) on every branch of the launch plan and at adversarial parameters, their determinism, the calibration of the sandwich standard errors over noise realisations, and FitUtility.compute_uncertainties."""
 import numpy as np
 import pytest
 
@@ -19,14 +19,45 @@ def device_normal(ws, us, vs, wts, X, precision=_cabi.FP64):
         return ctx.normal_equations(X)
 
 
+def worst_ratio(err, tol):
+    """max(err / tol); where the tolerance is 0 only an exact 0 passes."""
+    return float(np.max(np.divide(err, tol, out=np.where(err == 0, 0.0, np.inf), where=tol > 0)))
+
+
 def assert_parity(got, want):
+    """H and M to 1e-12 sqrt(X_jj X_kk), g to 1e-10 sqrt(H_jj ssr_w), the sums of squares to 1e-10 relative.
+    Returns the largest error/tolerance ratio."""
     H, M, g, ssr = got
     Ho, Mo, go, so = want
-    for X, Xo in ((H, Ho), (M, Mo)):
-        d = np.sqrt(np.diag(Xo))
-        assert np.all(np.abs(X - Xo) <= 1e-12 * np.outer(d, d)), np.max(np.abs(X - Xo) / np.outer(d, d))
-    assert np.all(np.abs(g - go) <= 1e-10 * np.sqrt(np.diag(Ho) * so[0]))
-    assert np.all(np.abs(ssr / so - 1) <= 1e-10)
+    dh, dm = np.sqrt(np.diag(Ho)), np.sqrt(np.diag(Mo))
+    checks = (('H', np.abs(H - Ho), 1e-12 * np.outer(dh, dh)), ('M', np.abs(M - Mo), 1e-12 * np.outer(dm, dm)),
+              ('g', np.abs(g - go), 1e-10 * np.sqrt(np.diag(Ho) * so[0])), ('ssr', np.abs(ssr - so), 1e-10 * so))
+    worst = 0.0
+    for name, err, tol in checks:
+        r = worst_ratio(err, tol)
+        assert r <= 1, (name, r)
+        worst = max(worst, r)
+    return worst
+
+
+def sweep_batch(N, P, seeds):
+    """One synthetic spectrum per seed, of 6 ceil(P/6) peaks (synth.multiplet builds groups of 6), with its weights,
+    and one parameter vector each, keeping the first P peaks (the normal equations are defined at any x): the true
+    vector, a random particle of the spectrum's box, and a perturbed true vector, in turn."""
+    rng = np.random.default_rng(N + P)
+    D = 4 + 3 * P
+    ws, us, vs, wts, X = [], [], [], [], []
+    for i, s in enumerate(seeds):
+        d, true = synth.multiplet(N, 6 * -(-P // 6), seed=s)
+        lo, up = d.generate_solution_bounds()
+        if i % 3 == 0:
+            x = true[:D]
+        elif i % 3 == 1:
+            x = synth.particles(lo, up, 1, seed=s)[0, :D]
+        else:
+            x = true[:D] * (1 + 0.05 * rng.standard_normal(D)) + np.r_[0.3, -0.2, 0.0, 1e-3, np.zeros(3 * P)]
+        ws.append(d.w); us.append(d.u); vs.append(d.v); wts.append(utils.compute_weights(d.w, d.peaks)); X.append(x)
+    return tuple(np.stack(a) for a in (ws, us, vs, wts, X))
 
 
 @pytest.mark.parametrize('case', CASES)
@@ -55,6 +86,71 @@ def test_parity_on_a_nonuniform_axis_and_a_mixed_batch():
         assert_parity([a[b] for a in got], lin.normal_equations(X[b], ws[b], us[b], vs[b], wts[b]))
 
 
+@pytest.mark.parametrize('N,P', list(lin.SWEEP), ids=['%dx%d' % s for s in lin.SWEEP])
+def test_parity_across_the_launch_plan(N, P):
+    """Every branch of normal_eq_plan (lin.SWEEP): point groups other than 6, one and several task slices, 16- to
+    128-point tiles, rows without a padding column, ragged tiles and ragged last chunks, a chunk grown past 16,384
+    points.  The reference sums in long double."""
+    plan = _cabi.normal_equations_plan(N, P)
+    want = lin.SWEEP[(N, P)]
+    assert {k: plan[k] for k in want} == want, plan
+    ws, us, vs, wts, X = sweep_batch(N, P, (21,) if N > 1_000_000 else (21, 22, 23))
+    got = device_normal(ws, us, vs, wts, X)
+    worst = max(assert_parity([a[b] for a in got], lin.normal_equations(X[b], ws[b], us[b], vs[b], wts[b],
+                                                                        accumulate=np.longdouble))
+                for b in range(len(X)))
+    print('normal equations %d x %d: worst error/tolerance %.3g' % (N, P, worst))
+
+
+ZERO_AREA_PEAK = 3
+
+
+def adversarial_batch(N, P):
+    """One spectrum and three parameter vectors at the edges of the lineshape and phase arithmetic.  Spectrum 2 has
+    a stretch of zero weights and a peak of area 0."""
+    ws, us, vs, wts, X = sweep_batch(N, P, (31,))
+    w = ws[0]
+    window = w[-1] - w[0]
+    X = np.repeat(X, 3, axis=0)
+    width, loc, area = (lambda k: 4 + 3 * k), (lambda k: 5 + 3 * k), (lambda k: 6 + 3 * k)
+    # r = 0; widths of 1e-6 of the window and of twice the window; phases on both sides of 2^31, where sincos
+    # leaves its fast argument reduction (the fast path is taken for |x| < 2^31 in the PTX it compiles to)
+    X[0, 2] = 0.0
+    X[0, width(0)], X[0, width(1)] = 1e-6 * window, 2 * window
+    X[0, 0], X[0, 1] = 2.0 ** 31 - 1.0, 3.0
+    # r = 1; centres exactly on a grid point (one of them 1e-6 of the window wide) and outside the window; every
+    # phase on the slow path
+    X[1, 2] = 1.0
+    X[1, loc(0)], X[1, loc(1)], X[1, loc(2)] = w[N // 3], w[-1] + 0.1 * window, w[N // 2]
+    X[1, width(2)] = 1e-6 * window
+    X[1, 0], X[1, 1] = -5e9, 40.0
+    # zero weights over a third of the spectrum, across chunk boundaries; a peak of area 0, whose width and
+    # location drop out of the residual
+    X[2, area(ZERO_AREA_PEAK)] = 0.0
+    ws, us, vs, wts = (np.repeat(a, 3, axis=0) for a in (ws, us, vs, wts))
+    wts[2, N // 5:N // 5 + N // 3] = 0.0
+    return ws, us, vs, wts, X
+
+
+@pytest.mark.parametrize('N,P', [(5000, 11), (2500, 28)], ids=['5000x11', '2500x28'])
+def test_parity_at_adversarial_parameters(N, P):
+    """Point groups (5000 x 11: ng = 2) and task slices (2500 x 28: 2 slices), both with ragged last chunks."""
+    ws, us, vs, wts, X = adversarial_batch(N, P)
+    got = device_normal(ws, us, vs, wts, X)
+    worst = max(assert_parity([a[b] for a in got], lin.normal_equations(X[b], ws[b], us[b], vs[b], wts[b],
+                                                                        accumulate=np.longdouble))
+                for b in range(len(X)))
+    print('normal equations %d x %d, adversarial: worst error/tolerance %.3g' % (N, P, worst))
+    # the zero-area peak: exactly zero rows and columns for its width and location, and a singular covariance
+    H, M, g, ssr = (a[2] for a in got)
+    zero = [4 + 3 * ZERO_AREA_PEAK, 5 + 3 * ZERO_AREA_PEAK]
+    for Z in (H, M):
+        assert np.all(Z[zero, :] == 0) and np.all(Z[:, zero] == 0)
+    assert np.all(g[zero] == 0)
+    C, info = utils.covariance_from_normal(H, M, g, ssr, N, X[2], X[2] - 1, X[2] + 1)
+    assert info['singular'] and np.all(np.isnan(C))
+
+
 @pytest.mark.parametrize('case', ['c1_4096x6', 'p24_1536'])
 def test_ssr_is_the_library_objective(case):
     gd = load_golden('objective_' + case)
@@ -75,19 +171,22 @@ def test_deterministic_and_independent_of_the_batch():
     ws, us, vs = (np.stack([getattr(d, k) for d, _ in spectra]) for k in ('w', 'u', 'v'))
     wts = np.stack([utils.compute_weights(d.w, d.peaks) for d, _ in spectra])
     X = np.stack([gd['xs'][1], spectra[1][1], gd['xs'][2]])
-    first = device_normal(ws, us, vs, wts, X)
-    again = device_normal(ws, us, vs, wts, X)
-    for a, b in zip(first, again):
-        assert np.array_equal(a, b)
-    for b in range(3):
-        alone = device_normal(ws[b:b + 1], us[b:b + 1], vs[b:b + 1], wts[b:b + 1], X[b:b + 1])
-        for a, s in zip(first, alone):
-            assert np.array_equal(a[b], s[0])
-    f32 = device_normal(ws, us, vs, wts, X, precision=_cabi.FP32)     # the pass is FP64 on FP32 contexts too
-    for a, b in zip(first, f32):
-        assert np.array_equal(a, b)
-    H = first[0]
-    assert np.array_equal(H, np.transpose(H, (0, 2, 1)))
+    # one task slice, then several (2 and 5 slices per chunk, ragged last chunks)
+    batches = [(ws, us, vs, wts, X)] + [sweep_batch(N, P, (3, 4, 5)) for N, P in ((2500, 28), (1000, 64))]
+    for ws, us, vs, wts, X in batches:
+        first = device_normal(ws, us, vs, wts, X)
+        again = device_normal(ws, us, vs, wts, X)
+        for a, b in zip(first, again):
+            assert np.array_equal(a, b)
+        for b in range(3):
+            alone = device_normal(ws[b:b + 1], us[b:b + 1], vs[b:b + 1], wts[b:b + 1], X[b:b + 1])
+            for a, s in zip(first, alone):
+                assert np.array_equal(a[b], s[0])
+        f32 = device_normal(ws, us, vs, wts, X, precision=_cabi.FP32)     # the pass is FP64 on FP32 contexts too
+        for a, b in zip(first, f32):
+            assert np.array_equal(a, b)
+        H = first[0]
+        assert np.array_equal(H, np.transpose(H, (0, 2, 1)))
 
 
 def test_sandwich_errors_are_calibrated():
@@ -126,29 +225,42 @@ def small_fit_options(**kw):
 
 
 def test_fit_then_uncertainties():
-    data, true = synth.multiplet(2048, 6, seed=2)
-    lo, up = data.generate_solution_bounds()
-    f = utils.FitUtility(data, lo, up, summary=False, options=small_fit_options())
-    with pytest.raises(RuntimeError):
-        f.compute_uncertainties()
-    f.fit()
-    se = f.compute_uncertainties()
-    assert se.shape == (len(true),) and np.all(np.isfinite(se)) and np.all(se > 0)
-    assert f.covariance.shape == (len(true), len(true)) and not f.uncertainty_info['singular']
-    fe = f.area_fraction_stderr()
-    assert np.isfinite(fe) and fe > 0
+    # 36 peaks: two task slices per chunk and a ragged last chunk (3,000 = 11 x 256 + 184)
+    for N, P in ((2048, 6), (3000, 36)):
+        data, true = synth.multiplet(N, P, seed=2)
+        lo, up = data.generate_solution_bounds()
+        f = utils.FitUtility(data, lo, up, summary=False, options=small_fit_options())
+        with pytest.raises(RuntimeError):
+            f.compute_uncertainties()
+        f.fit()
+        se = f.compute_uncertainties()
+        assert se.shape == (len(true),) and np.all(np.isfinite(se)) and np.all(se > 0)
+        assert f.covariance.shape == (len(true), len(true)) and not f.uncertainty_info['singular']
+        fe = f.area_fraction_stderr()
+        assert np.isfinite(fe) and fe > 0
+        if P == 36:
+            # against the covariance of the reference normal equations at the fitted point, to 1e-11 of the
+            # condition number of the Jacobi-scaled H that covariance_from_normal factorises
+            H, M, g, ssr = lin.normal_equations(f.params, data.w, data.u, data.v, f.weights, accumulate=np.longdouble)
+            C, info = utils.covariance_from_normal(H, M, g, ssr, N, f.params, lo, up)
+            s = 1 / np.sqrt(np.diag(H))
+            cond = np.linalg.cond(s[:, None] * H * s[None, :])
+            se_ref = np.sqrt(np.diag(C))
+            assert not info['singular']
+            assert np.all(np.abs(se - se_ref) <= 1e-11 * cond * se_ref), (cond, np.max(np.abs(se / se_ref - 1)))
 
 
 def test_batch_equals_per_fit():
-    datas = [synth.multiplet(2048, 6, seed=s)[0] for s in (5, 6, 7)]
-    bounds = [d.generate_solution_bounds() for d in datas]
-    fits = core.fit_batch(datas, [b[0] for b in bounds], [b[1] for b in bounds],
-                          options=small_fit_options(rng='device', seed=3))
-    batch = [s.copy() for s in utils.compute_uncertainties_batch(fits)]
-    covs = [f.covariance.copy() for f in fits]
-    for f, s, c in zip(fits, batch, covs):
-        assert np.array_equal(f.compute_uncertainties(), s)
-        assert np.array_equal(f.covariance, c)
+    for N, P in ((2048, 6), (3000, 36)):
+        datas = [synth.multiplet(N, P, seed=s)[0] for s in (5, 6, 7)]
+        bounds = [d.generate_solution_bounds() for d in datas]
+        fits = core.fit_batch(datas, [b[0] for b in bounds], [b[1] for b in bounds],
+                              options=small_fit_options(rng='device', seed=3))
+        batch = [s.copy() for s in utils.compute_uncertainties_batch(fits)]
+        covs = [f.covariance.copy() for f in fits]
+        for f, s, c in zip(fits, batch, covs):
+            assert np.array_equal(f.compute_uncertainties(), s)
+            assert np.array_equal(f.covariance, c)
 
 
 def test_error_paths():

@@ -7,6 +7,7 @@ from conftest import load_golden
 from nmrfit_b200 import utils
 import linearisation_ref as lin
 from oracle import nmrfit_oracle as orc
+from test_cabi_symbols import built  # noqa: F401  (builds the library; the plan query makes no CUDA call)
 
 LN2 = np.log(2.0)
 
@@ -151,6 +152,58 @@ def test_area_fraction_stderr_is_the_delta_method():
         grad[j] = (orc.area_fraction(orc.get_areas(xp)) - orc.area_fraction(orc.get_areas(xm))) / (2 * h)
     want = np.sqrt(grad @ f.covariance @ grad)
     assert f.area_fraction_stderr() == pytest.approx(want, rel=1e-8)
+
+
+PLAN_POINTS = (1, 37, 255, 256, 257, 1000, 4096, 5000, 65536, 2_100_000)
+
+
+def test_normal_equations_plan_invariants(built):
+    """What csrc/normal_eq.cu relies on, for every peak count it accepts: the CTA fits __launch_bounds__(512), the
+    point groups or task slices cover every 4x4 block, the tile keeps the staged rows near 48 KB, the chunks cover
+    the spectrum in at most 128 partials, and the shared memory holds both the staged tile and the end-of-chunk
+    reduction within the 200 KiB the launch opts into."""
+    from nmrfit_b200 import _cabi
+    for P in range(1, 65):
+        E = 5 + 3 * P
+        nb = -(-E // 4)
+        ep = 4 * nb
+        for N in PLAN_POINTS:
+            p = _cabi.normal_equations_plan(N, P)
+            where = (N, P, p)
+            ng, tasks, tps, threads, tp, ch = (p[k] for k in ('point_groups', 'tasks', 'tasks_per_slice', 'threads',
+                                                              'tile_points', 'chunk_points'))
+            assert tasks == nb * (nb + 1), where                      # upper triangles of both matrices
+            assert threads % 32 == 0 and 0 < threads <= 512, where
+            if ng > 1:
+                assert p['slices'] == 1 and tps == tasks and ng * tasks <= threads, where
+            else:
+                assert ng == 1 and tps <= threads, where
+                assert p['slices'] * tps >= tasks and (p['slices'] - 1) * tps < tasks, where
+            assert tp in (16, 32, 64, 128), where
+            assert tp == 16 or 2 * tp * ep <= 6144, where
+            assert ch >= 256 and ch & (ch - 1) == 0 and ch % tp == 0, where
+            assert p['n_chunks'] == -(-N // ch) and p['n_chunks'] <= 128, where
+            stage = 2 * tp * ep + 2 * tp * P + 8 * P                  # rows, model values, d/dr terms, peak constants
+            assert p['smem_bytes'] == 8 * max(stage, 16 * threads) <= 200 * 1024, where
+            assert p['scratch_doubles'] == p['n_chunks'] * tasks * 16, where
+
+
+def test_normal_equations_plan_pins(built):
+    """The sizes DESIGN §4 K12 states, and the branch every shape of the GPU parity sweep must take."""
+    from nmrfit_b200 import _cabi
+    c3 = _cabi.normal_equations_plan(16384, 6)
+    assert (c3['n_chunks'], c3['chunk_points']) == (4, 4096)
+    assert round(c3['scratch_doubles'] * 8 * 1024 / 1e6) == 22            # MB for 1,024 spectra
+    c4 = _cabi.normal_equations_plan(65536, 24)
+    assert (c4['n_chunks'], c4['chunk_points']) == (128, 512)
+    assert round(c4['scratch_doubles'] * 8 / 1e6, 1) == 6.9
+    for (N, P), want in lin.SWEEP.items():
+        got = _cabi.normal_equations_plan(N, P)
+        assert {k: got[k] for k in want} == want, (N, P, got)
+    for N, P in ((0, 6), (-5, 6), (100, 0), (100, 65)):
+        with pytest.raises(_cabi.NmrfitError) as e:
+            _cabi.normal_equations_plan(N, P)
+        assert e.value.code == -1
 
 
 def test_compute_uncertainties_errors_before_any_device_call():
