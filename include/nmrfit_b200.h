@@ -109,6 +109,28 @@ int nmrfit_ctx_normal_equations(nmrfit_ctx* ctx, const double* x, double* H, dou
  * NMRFIT_ERR_ARG unless 1 <= n_peaks <= 64 and n_points >= 1. */
 int nmrfit_normal_eq_plan(int n_points, int n_peaks, int* out);
 
+/* How nmrfit_ctx_refine left a spectrum. */
+#define NMRFIT_REFINE_CONVERGED 1   /* an accepted step was at most xtol of every parameter's diagonal noise scale */
+#define NMRFIT_REFINE_STALLED 2     /* the damping passed 1e16 without a descent step: a numerical minimum */
+#define NMRFIT_REFINE_MAX_ITER 3    /* max_iter passes of the normal equations */
+#define NMRFIT_REFINE_NONFINITE 4   /* H, g or s is not finite at the start; x is left as it was */
+
+/* Bounded Levenberg-Marquardt refinement of one parameter vector per spectrum to the least-squares optimum of the
+ * weighted residual (DESIGN K13), from the spectra and weights the context holds, looping on the device.  Each pass
+ * forms the normal equations at a trial point (as nmrfit_ctx_normal_equations does); one CTA per spectrum accepts the
+ * trial if its s = sum w^2 res^2 is finite and strictly below the current one, updates the damping lam (1e-3 at the
+ * start; /10 down to 1e-12 on acceptance, *10 on rejection), and solves (S H S + lam I) y = -S g, S = diag(H_jj^-1/2),
+ * over the parameters not frozen (H_jj = 0, or at a bound with the gradient pointing out), for the next trial
+ * clip(x + S y, lb, ub).  A spectrum stops CONVERGED when an accepted step has max_j |dx_j| sqrt(H_jj (N-D)/s) <= xtol
+ * (H and s of the point the step was built from), or STALLED, MAX_ITER (max_iter passes, counting the one at the start)
+ * or NONFINITE.  x_inout [n_spectra][D]: the start in, the refined point out (bit for bit the start if no step was
+ * accepted); lb, ub [n_spectra][D]; f_out = sqrt(s/N) at the returned point, passes_out, accepted_out, status_out
+ * [n_spectra] (any of the four may be NULL).  Host or device pointers; returns when the outputs are written.  The
+ * result of a spectrum is bit-reproducible and the same alone or in a batch, on FP32 contexts too.  NMRFIT_ERR_ARG for
+ * more than 64 peaks, n_points <= D, lb_j >= ub_j, a start outside its box, max_iter < 1 or xtol <= 0. */
+int nmrfit_ctx_refine(nmrfit_ctx* ctx, double* x_inout, const double* lb, const double* ub, int max_iter, double xtol,
+                      double* f_out, int* passes_out, int* accepted_out, int* status_out, void* stream);
+
 /* Which objective kernel runs (default NMRFIT_ALGO_AUTO), and which one a launch with this fit_im would use.
  * Both kernels evaluate equations.objective (equations.py:152-212); the uniform-axis one exploits
  * w_i = w_0 + i*h (what core.load builds, core.py:58-60) to replace most exponentials by a recurrence. */

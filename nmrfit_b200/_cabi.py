@@ -18,6 +18,7 @@ REAL_ONLY, IM_REFERENCE, IM_SUM = 0, 1, 2
 ALGO_AUTO, ALGO_GENERAL, ALGO_UNIFORM = 0, 1, 2
 FUSED_AUTO, FUSED_OFF, FUSED_REQUIRE = 0, 1, 2
 RUNNING, STOP_MINFUNC, STOP_MINSTEP, STOP_MAXITER, STOP_PEER_LOST = 0, 1, 2, 3, 4
+REFINE_CONVERGED, REFINE_STALLED, REFINE_MAX_ITER, REFINE_NONFINITE = 1, 2, 3, 4
 
 c_double_p = ctypes.POINTER(ctypes.c_double)
 c_int_p = ctypes.POINTER(ctypes.c_int)
@@ -53,6 +54,7 @@ SIGNATURES = {
     'nmrfit_ctx_compute_weights': (_i, [_vp, _vp, _vp, _i, _i, _d, _vp, _vp]),
     'nmrfit_ctx_normal_equations': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     'nmrfit_normal_eq_plan': (_i, [_i, _i, c_int_p]),
+    'nmrfit_ctx_refine': (_i, [_vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
     'nmrfit_ctx_set_algorithm': (_i, [_vp, _i]),
     'nmrfit_ctx_get_algorithm': (_i, [_vp, _i, c_int_p]),
     'nmrfit_ctx_set_tuning': (_i, [_vp, _i, _i, _i, _i]),
@@ -176,6 +178,32 @@ def normal_equations_plan(n_points, n_peaks):
     return dict(zip(NORMAL_EQ_PLAN_KEYS, out))
 
 
+def check_refine_args(x, lb, ub, max_iter, xtol, B, N, P):
+    """The checks ``Context.refine`` makes before any CUDA call (the library makes them again): returns fresh
+    C-contiguous float64 copies of ``x`` [B, D] and of ``lb``, ``ub`` broadcast to [B, D].  ValueError otherwise."""
+    D = 4 + 3 * P
+    if P > 64:
+        raise ValueError('refinement supports at most 64 peaks (D <= 196), got %d' % P)
+    if N <= D:
+        raise ValueError('the spectrum has %d points for %d parameters: no residual degrees of freedom' % (N, D))
+    x = np.array(x, dtype=np.float64, order='C')
+    if x.shape != (B, D):
+        raise ValueError('x must have shape (%d, %d), got %s' % (B, D, x.shape))
+    try:
+        lb, ub = (np.ascontiguousarray(np.broadcast_to(np.asarray(a, dtype=np.float64), (B, D))) for a in (lb, ub))
+    except ValueError:
+        raise ValueError('lb and ub must have shape (%d, %d) or (%d,)' % (B, D, D)) from None
+    if int(max_iter) < 1:
+        raise ValueError('max_iter must be >= 1')
+    if not float(xtol) > 0:
+        raise ValueError('xtol must be > 0')
+    if not np.all(ub > lb):
+        raise ValueError('every lower bound must be below its upper bound')
+    if not np.all((x >= lb) & (x <= ub)):
+        raise ValueError('the start must lie inside its box')
+    return x, lb, ub
+
+
 def default_device():
     """LOCAL_RANK under torchrun, else NMRFIT_DEVICE, else 0."""
     for key in ('NMRFIT_DEVICE', 'LOCAL_RANK'):
@@ -252,6 +280,19 @@ class Context:
         ssr = np.empty((self.B, 2))
         check(lib().nmrfit_ctx_normal_equations(self._h, ptr(x), ptr(H), ptr(M), ptr(g), ptr(ssr), ptr(stream)))
         return H, M, g, ssr
+
+    def refine(self, x, lb, ub, max_iter=50, xtol=1e-6, stream=None):
+        """Bounded Levenberg-Marquardt refinement of ``x`` [B, D] (one start per spectrum) to the least-squares optimum
+        of the weighted residual within [``lb``, ``ub``] ([B, D], or [D] for every spectrum), looping on the device
+        (include/nmrfit_b200.h, DESIGN K13).  Returns ``(x, f, passes, accepted, status)``: the refined [B, D] (the
+        start, bit for bit, where no step was accepted), sqrt(s/N) there [B], the passes of the normal equations,
+        the accepted steps and the ``REFINE_*`` status [B]."""
+        x, lb, ub = check_refine_args(x, lb, ub, max_iter, xtol, self.B, self.N, self.P)
+        f = np.empty(self.B)
+        passes, accepted, status = (np.empty(self.B, dtype=np.int32) for _ in range(3))
+        check(lib().nmrfit_ctx_refine(self._h, ptr(x), ptr(lb), ptr(ub), int(max_iter), float(xtol), ptr(f),
+                                      ptr(passes), ptr(accepted), ptr(status), ptr(stream)))
+        return x, f, passes, accepted, status
 
     def set_algorithm(self, algorithm=ALGO_AUTO):
         """ALGO_AUTO (default), ALGO_GENERAL (any axis) or ALGO_UNIFORM (require the uniform-axis kernel)."""

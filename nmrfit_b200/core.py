@@ -33,11 +33,15 @@ def fit_batch(datas, lowers, uppers, expon=0.5, dynamic_weighting=True, fit_im=F
     Equivalent to ``[fit(d, lo, up, ...) for d, lo, up in zip(...)]`` but all swarms
     advance together, one launch per generation.  With options['rng'] == 'host' and
     options['seeds'] = [k_0, k_1, ...], spectrum b reproduces the reference fit run
-    after ``np.random.seed(k_b)``.  Returns a list of ``FitUtility``.
+    after ``np.random.seed(k_b)``.  With options['refine'] every fit is then refined (``utils.refine_batch``) in the
+    same context, where the spectra and weights already are.  Returns a list of ``FitUtility``.
     """
     fits = [utils.FitUtility(d, lo, up, expon, dynamic_weighting, fit_im, 1, summary, options)
             for d, lo, up in zip(datas, lowers, uppers)]
     opt = options
+    refine = opt.get('refine', False)
+    if refine and fits:
+        utils._check_refinable(fits[0])
     B = len(fits)
     lb = np.array(lowers, dtype=np.float64)
     n_peaks = (lb.shape[1] - 4) // 3
@@ -60,11 +64,14 @@ def fit_batch(datas, lowers, uppers, expon=0.5, dynamic_weighting=True, fit_im=F
             rng=opt.get('rng', 'device'), seeds=opt.get('seeds'), seed=opt.get('seed', 0),
             chunk=opt.get('chunk', 16), fused=opt.get('fused', 'auto'), ctx=ctx,
             spectrum_offset=opt.get('spectrum_offset', 0))
-    for b, f in enumerate(fits):
-        f.weights = weights[b]
-        f.params = x[b].copy()
-        f.error = float(fbest[b])
-        f.fit_info = dict(generations=int(it[b]), stop=int(stop[b]))
+        for b, f in enumerate(fits):
+            f.weights = weights[b]
+            f.params = x[b].copy()
+            f.error = float(fbest[b])
+            f.fit_info = dict(generations=int(it[b]), stop=int(stop[b]))
+        if refine:
+            utils.apply_refinement(fits, *ctx.refine(x, lowers, uppers))
+    for f in fits:
         if summary is True:
             f._print_summary()
     return fits

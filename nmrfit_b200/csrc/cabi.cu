@@ -116,6 +116,9 @@ struct nmrfit_ctx {
     double peer_timeout_ms = 20000.0;  // wall-time bound of a wait for the peers' tokens
     DevBuf<double> wscratch, wbounds;  // batched weights: sweep scratch [B][N], windows + values
     DevBuf<double> ne_x, ne_part, ne_out;   // normal equations: positions, chunk partials, H | M | g | ssr
+    DevBuf<double> rf_x, rf_cur;       // refinement: current, trial, lb, ub [4][B][D]; H | g | s at the current point
+    DevBuf<RefineState> rf_state;
+    DevBuf<int> rf_active;             // spectra still running after the last polled step
     cudaStream_t pipe[2] = {nullptr, nullptr};   // nmrfit_objective_batch_host: slices of a large particle set
     double* h_f = nullptr;                       // ... and page-locked staging of their values
     size_t h_f_cap = 0;
@@ -515,6 +518,10 @@ void nmrfit_ctx_destroy(nmrfit_ctx* c) {
     c->ne_x.release();
     c->ne_part.release();
     c->ne_out.release();
+    c->rf_x.release();
+    c->rf_cur.release();
+    c->rf_state.release();
+    c->rf_active.release();
     for (int k = 0; k < 2; ++k)
         if (c->pipe[k]) cudaStreamDestroy(c->pipe[k]);
     if (c->h_f) cudaFreeHost(c->h_f);
@@ -650,6 +657,71 @@ int nmrfit_ctx_normal_equations(nmrfit_ctx* c, const double* x, double* H, doubl
             CK(cudaMemcpy2DAsync(dst[k], sizeof(double) * lens[k], c->ne_out.ptr + offs[k], sizeof(double) * per,
                                  sizeof(double) * lens[k], B, cudaMemcpyDefault, st));
     CK(cudaStreamSynchronize(st));                         // x and the outputs may be pageable host memory
+    return NMRFIT_OK;
+}
+
+constexpr int kRefinePoll = 8;   // refinement iterations queued between host reads of the running count
+
+int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* ub, int max_iter, double xtol,
+                      double* f_out, int* passes_out, int* accepted_out, int* status_out, void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
+    if (c->P > 64)
+        return fail(NMRFIT_ERR_ARG, "refinement supports at most 64 peaks (D <= 196), the context has " +
+                                        std::to_string(c->P));
+    if (c->N <= c->D) return fail(NMRFIT_ERR_ARG, "refinement needs more points than parameters");
+    if (max_iter < 1) return fail(NMRFIT_ERR_ARG, "max_iter must be >= 1");
+    if (!(xtol > 0.0)) return fail(NMRFIT_ERR_ARG, "xtol must be > 0");
+    for (char f : c->spec_set)
+        if (!f) return fail(NMRFIT_ERR_STATE, "every spectrum must be set before it is refined");
+    CK(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t B = (size_t)c->B, D = (size_t)c->D, BD = B * D;
+    // [x | x | lb | ub]: the start is the first current point and the first trial
+    std::vector<double> h(4 * BD);
+    CK(cudaMemcpy(h.data(), x, sizeof(double) * BD, cudaMemcpyDefault));
+    CK(cudaMemcpy(h.data() + 2 * BD, lb, sizeof(double) * BD, cudaMemcpyDefault));
+    CK(cudaMemcpy(h.data() + 3 * BD, ub, sizeof(double) * BD, cudaMemcpyDefault));
+    std::copy(h.begin(), h.begin() + BD, h.begin() + BD);
+    for (size_t i = 0; i < BD; ++i) {
+        const double xi = h[i], lo = h[2 * BD + i], hi = h[3 * BD + i];
+        if (!(hi > lo)) return fail(NMRFIT_ERR_ARG, "every lower bound must be below its upper bound");
+        if (!(xi >= lo && xi <= hi)) return fail(NMRFIT_ERR_ARG, "the start must lie inside its box");
+    }
+    const NormalEqPlan p = normal_eq_plan(c->N, c->P);
+    CK(c->ne_part.reserve(normal_eq_scratch_doubles(p, c->B)));
+    CK(c->ne_out.reserve(B * (2 * D * D + D + 2)));
+    CK(c->rf_x.reserve(4 * BD));
+    CK(c->rf_cur.reserve(B * (D * D + D + 1)));
+    CK(c->rf_state.reserve(B));
+    CK(c->rf_active.reserve(1));
+    double *xc = c->rf_x.ptr, *xt = xc + BD, *lbd = xc + 2 * BD, *ubd = xc + 3 * BD;
+    CK(cudaMemcpyAsync(xc, h.data(), sizeof(double) * 4 * BD, cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(c->rf_state.ptr, 0, sizeof(RefineState) * B, st));
+    // every running spectrum has had the same number of passes, so max_iter iterations finish them all
+    for (int it = 0; it < max_iter; ++it) {
+        cudaError_t e = launch_normal_eq(c->spec.ptr, xt, p, c->B, c->ne_part.ptr, c->ne_out.ptr, st);
+        if (e != cudaSuccess) return fail_cuda(e, "refinement: normal equations launch");
+        const bool poll = (it + 1) % kRefinePoll == 0 && it + 1 < max_iter;
+        if (poll) CK(cudaMemsetAsync(c->rf_active.ptr, 0, sizeof(int), st));
+        e = launch_refine_step(c->ne_out.ptr, c->rf_cur.ptr, c->rf_state.ptr, xc, xt, lbd, ubd, c->B, c->N, c->D,
+                               max_iter, xtol, poll ? c->rf_active.ptr : nullptr, st);
+        if (e != cudaSuccess) return fail_cuda(e, "refinement step launch");
+        if (poll) {
+            CK(cudaMemcpyAsync(c->h_flags, c->rf_active.ptr, sizeof(int), cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            if (c->h_flags[0] == 0) break;
+        }
+    }
+    CK(cudaMemcpyAsync(x, xc, sizeof(double) * BD, cudaMemcpyDefault, st));
+    const RefineState* rs = c->rf_state.ptr;
+    const size_t pitch = sizeof(RefineState);
+    if (f_out) CK(cudaMemcpy2DAsync(f_out, sizeof(double), &rs->f, pitch, sizeof(double), B, cudaMemcpyDefault, st));
+    int* outs[3] = {passes_out, accepted_out, status_out};
+    const int* srcs[3] = {&rs->passes, &rs->accepted, &rs->status};
+    for (int k = 0; k < 3; ++k)
+        if (outs[k]) CK(cudaMemcpy2DAsync(outs[k], sizeof(int), srcs[k], pitch, sizeof(int), B, cudaMemcpyDefault, st));
+    CK(cudaStreamSynchronize(st));                         // the staged starts and the outputs may be pageable memory
     return NMRFIT_OK;
 }
 

@@ -227,6 +227,19 @@ size_t normal_eq_scratch_doubles(const NormalEqPlan& p, int B);
 cudaError_t launch_normal_eq(const double* spec, const double* x, const NormalEqPlan& p, int B, double* part,
                              double* out, cudaStream_t st);
 
+// ---- K13 bounded Levenberg-Marquardt refinement on K12 (refine.cu) --------------------
+#define NMRFIT_REFINE_RUNNING 0
+struct RefineState {
+    double lam, f;              // damping of the next trial; sqrt(s/N) at the current point
+    int status, passes, accepted, pad;
+};
+size_t refine_step_smem(int D);
+// trial [B][2*D*D + D + 2] is launch_normal_eq's output at xt; cur [B][D*D + D + 1] holds H | g | s at xc.
+// `active` (or null) gains one per spectrum still running after the step.
+cudaError_t launch_refine_step(const double* trial, double* cur, RefineState* state, double* xc, double* xt,
+                               const double* lb, const double* ub, int B, int N, int D, int max_iter, double xtol,
+                               int* active, cudaStream_t st);
+
 // ---- probes -------------------------------------------------------------------
 cudaError_t fp64_peak_probe(int iters, int repeats, double* tflops, double* sustained, cudaStream_t st);
 

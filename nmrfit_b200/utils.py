@@ -98,6 +98,7 @@ class FitUtility:
       ``fused``     'auto' (default) | 'off' | 'require': run the generations of a small swarm in one
                     cooperative launch (bit-identical to the per-step kernels).
       ``device``    CUDA device index.
+      ``refine``    True: ``refine()`` after the swarm (default False).
     ``processes`` is accepted and ignored (the GPU evaluates every particle at once).
     """
 
@@ -114,7 +115,10 @@ class FitUtility:
         self.options = options
 
     def fit(self):
-        """Minimise the objective over the box [lower, upper] with the swarm."""
+        """Minimise the objective over the box [lower, upper] with the swarm (then ``refine()`` with
+        ``options['refine']``)."""
+        if self.options.get('refine', False):
+            _check_refinable(self)
         self.weights = self._compute_weights()
         if self.dynamic_weighting is False:
             self.weights = np.ones_like(self.weights)
@@ -132,6 +136,8 @@ class FitUtility:
         self.params = xopt
         self.error = fopt
         self.fit_info = info
+        if opt.get('refine', False):
+            self.refine()
 
         if self.summary is True:
             self._print_summary()
@@ -184,10 +190,24 @@ class FitUtility:
         """Fitted areas: every third parameter from index 6 (utils.py:322)."""
         return np.array([self.params[i] for i in range(6, len(self.params), 3)])
 
+    def refine(self, max_iter=50, xtol=1e-6):
+        """Refine the swarm's ``params`` to the least-squares optimum of the weighted residual within the box, by
+        bounded Levenberg-Marquardt on the GPU (see ``refine_batch``).  Replaces ``params`` and ``error`` (which
+        becomes sqrt(s/N) from the normal equations at the new point; both stay bit for bit as they were if no step
+        was accepted) and sets ``refine_info`` = dict(start_params, start_error, passes, accepted, status), status one
+        of ``_cabi.REFINE_CONVERGED``, ``_STALLED``, ``_MAX_ITER``, ``_NONFINITE``.
+
+        Raises RuntimeError before ``fit()`` and NotImplementedError with ``fit_im``."""
+        refine_batch([self], max_iter, xtol)
+        return self.params
+
     def compute_uncertainties(self):
         """Standard errors of ``params`` from the linearised least-squares problem at the fitted point (one pass
         over the spectrum on the GPU, see ``compute_uncertainties_batch``).  Sets ``covariance`` [D, D], ``stderr``
         [D] and ``uncertainty_info``, and returns ``stderr``.
+
+        The errors assume that ``params`` is the least-squares optimum; the swarm stops short of it, and ``refine()``
+        takes ``params`` there first.
 
         Raises RuntimeError before ``fit()``, NotImplementedError with ``fit_im`` (that objective is a sum of two
         RMSEs, not a least-squares problem) and ValueError when the spectrum has no more points than parameters."""
@@ -294,6 +314,48 @@ def compute_uncertainties_batch(fits):
                                                                   f.upper)
         f.stderr = np.sqrt(np.diag(f.covariance))
     return [f.stderr for f in fits]
+
+
+def _check_refinable(f, fitted=False):
+    if fitted and getattr(f, 'params', None) is None:
+        raise RuntimeError('refine needs a fitted model: call fit() first')
+    if f.fit_im:
+        raise NotImplementedError('refinement is not available with fit_im: that objective is a sum of two RMSEs, '
+                                  'not a least-squares problem')
+
+
+def apply_refinement(fits, x, fval, passes, accepted, status):
+    """Store the result of ``Context.refine`` on the fits it refined (see ``FitUtility.refine``)."""
+    for b, f in enumerate(fits):
+        f.refine_info = dict(start_params=np.array(f.params, dtype=np.float64), start_error=f.error,
+                             passes=int(passes[b]), accepted=int(accepted[b]), status=int(status[b]))
+        if accepted[b] > 0:
+            f.params = x[b].copy()
+            f.error = float(fval[b])
+
+
+def refine_batch(fits, max_iter=50, xtol=1e-6):
+    """``refine()`` for many fits of equal length and peak count (what ``fit_batch`` returns) in one device call:
+    the spectra and each fit's ``weights`` go to a pooled context, and every spectrum runs bounded Levenberg-Marquardt
+    (``Context.refine``, DESIGN K13) from its ``params`` within its box.  Returns the list of refined ``params``."""
+    fits = list(fits)
+    if not fits:
+        return []
+    for f in fits:
+        _check_refinable(f, fitted=True)
+    N, D = len(fits[0].data.w), len(fits[0].params)
+    for f in fits:
+        if len(f.data.w) != N or len(f.params) != D:
+            raise ValueError('every fit of a batch must have the same number of points and peaks')
+    W, U, V, weights = (np.stack([_cabi.as_f64(a) for a in arrs])
+                        for arrs in zip(*[(f.data.w, f.data.u, f.data.v, f.weights) for f in fits]))
+    X, LB, UB = (np.stack([_cabi.as_f64(getattr(f, k)) for f in fits]) for k in ('params', 'lower', 'upper'))
+    _cabi.check_refine_args(X, LB, UB, max_iter, xtol, len(fits), N, (D - 4) // 3)
+    with _cabi.pooled_context(len(fits), N, (D - 4) // 3, device=fits[0].options.get('device')) as ctx:
+        ctx.set_spectra(W, U, V, weights)
+        out = ctx.refine(X, LB, UB, max_iter, xtol)
+    apply_refinement(fits, *out)
+    return [f.params for f in fits]
 
 
 # ---- automatic peak selection (utils.py:670-783) on the GPU ----------------------------------------------------
