@@ -212,21 +212,15 @@ def default_device():
     return 0
 
 
-class Context:
-    """Owner of one ``nmrfit_ctx``: a batch of spectra resident on one GPU."""
+class _Handle:
+    """Owner of one library handle ``_h``, freed by the C function named ``_destroy`` on ``close()``, at the end of a
+    ``with`` block or when the owner is collected."""
 
-    def __init__(self, n_spectra, n_points, n_peaks, device=None, precision=FP64):
-        self._h = ctypes.c_void_p()
-        self.device = default_device() if device is None else int(device)
-        self.B, self.N, self.P = int(n_spectra), int(n_points), int(n_peaks)
-        self.D = 4 + 3 * self.P
-        self.precision = precision
-        check(lib().nmrfit_ctx_create(ctypes.byref(self._h), self.device, self.B, self.N, self.P, precision))
-        self._keep = []
+    _destroy = None
 
     def close(self):
         if getattr(self, '_h', None) is not None and self._h:
-            lib().nmrfit_ctx_destroy(self._h)
+            getattr(lib(), self._destroy)(self._h)
             self._h = ctypes.c_void_p()
 
     __del__ = close
@@ -236,6 +230,21 @@ class Context:
 
     def __exit__(self, *exc):
         self.close()
+
+
+class Context(_Handle):
+    """Owner of one ``nmrfit_ctx``: a batch of spectra resident on one GPU."""
+
+    _destroy = 'nmrfit_ctx_destroy'
+
+    def __init__(self, n_spectra, n_points, n_peaks, device=None, precision=FP64):
+        self._h = ctypes.c_void_p()
+        self.device = default_device() if device is None else int(device)
+        self.B, self.N, self.P = int(n_spectra), int(n_points), int(n_peaks)
+        self.D = 4 + 3 * self.P
+        self.precision = precision
+        check(lib().nmrfit_ctx_create(ctypes.byref(self._h), self.device, self.B, self.N, self.P, precision))
+        self._keep = []
 
     # -- spectra
     def set_spectrum(self, b, w, u, v, weights):
@@ -544,8 +553,10 @@ class Context:
         return out
 
 
-class PhaseScorer:
+class PhaseScorer(_Handle):
     """Device copies of a batch of spectra (u, v: [B, N] or [N]) for phase estimation (csrc/phase.cu)."""
+
+    _destroy = 'nmrfit_phase_destroy'
 
     def __init__(self, u, v, device=None):
         u, v = as_f64(np.atleast_2d(u)), as_f64(np.atleast_2d(v))
@@ -555,19 +566,6 @@ class PhaseScorer:
         self._h = ctypes.c_void_p()
         dev = default_device() if device is None else int(device)
         check(lib().nmrfit_phase_create(ctypes.byref(self._h), dev, self.B, self.N, ptr(u), ptr(v)))
-
-    def close(self):
-        if getattr(self, '_h', None) is not None and self._h:
-            lib().nmrfit_phase_destroy(self._h)
-            self._h = ctypes.c_void_p()
-
-    __del__ = close
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     def brute(self, candidates, details=False):
         """First smallest baseline error among the upward candidates, per spectrum (containers.py:98-110)."""
@@ -615,8 +613,10 @@ class Communicator:
         return running.value, lost.value
 
 
-class PeakPicker:
+class PeakPicker(_Handle):
     """Device side of the automatic peak selection for a batch of spectra (csrc/peaks.cu): ``maxima`` then ``measure``."""
+
+    _destroy = 'nmrfit_peaks_destroy'
 
     def __init__(self, n_spectra, n_points, upsample=100, max_peaks=64, device=None):
         self._h = ctypes.c_void_p()
@@ -624,19 +624,6 @@ class PeakPicker:
         self.M = self.N * self.upsample
         dev = default_device() if device is None else int(device)
         check(lib().nmrfit_peaks_create(ctypes.byref(self._h), dev, self.B, self.N, self.upsample, self.max_peaks))
-
-    def close(self):
-        if getattr(self, '_h', None) is not None and self._h:
-            lib().nmrfit_peaks_destroy(self._h)
-            self._h = ctypes.c_void_p()
-
-    __del__ = close
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     def maxima(self, w, u, window, sg_coeffs=None, max_it=100, tol=1e-3):
         """-> (n_maxima [B], maxima [B, max_peaks] (unsorted upsampled indices), signal there, global baseline [B])"""

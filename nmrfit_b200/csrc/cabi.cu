@@ -4,10 +4,11 @@
 #include <cmath>
 #include <atomic>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <string>
+#include <utility>
 #include <vector>
 #include "../../include/nmrfit_b200.h"
 #include "nmrfit_internal.h"
@@ -39,25 +40,48 @@ int fail_cuda(cudaError_t e, const char* where) {
         if (_e != cudaSuccess) return fail_cuda(_e, #call);   \
     } while (0)
 
-template <typename T>
-struct DevBuf {
+// An array that grows on demand and is freed with its owner: device memory, or page-locked host memory.  The owner's
+// device must be current when it is destroyed.
+template <typename T, bool kPinned>
+struct Buf {
     T* ptr = nullptr;
     size_t cap = 0;
+    Buf() = default;
+    Buf(Buf&& o) noexcept : ptr(std::exchange(o.ptr, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    ~Buf() { release(); }
     cudaError_t reserve(size_t n) {
         if (n <= cap) return cudaSuccess;
-        if (ptr) cudaFree(ptr);
-        ptr = nullptr;
-        cap = 0;
-        cudaError_t e = cudaMalloc(&ptr, n * sizeof(T));
+        release();
+        cudaError_t e = kPinned ? cudaMallocHost((void**)&ptr, n * sizeof(T)) : cudaMalloc((void**)&ptr, n * sizeof(T));
         if (e == cudaSuccess) cap = n;
         return e;
     }
     void release() {
-        if (ptr) cudaFree(ptr);
+        if (ptr && kPinned) cudaFreeHost(ptr);
+        else if (ptr) cudaFree(ptr);
         ptr = nullptr;
         cap = 0;
     }
 };
+template <typename T> using DevBuf = Buf<T, false>;
+template <typename T> using PinnedBuf = Buf<T, true>;
+
+// One CUDA runtime object (stream, event, allocation, IPC mapping), destroyed with its owner
+template <typename H, cudaError_t (*Destroy)(H)>
+struct Owned {
+    H h = nullptr;
+    Owned() = default;
+    explicit Owned(H v) : h(v) {}
+    Owned(Owned&& o) noexcept : h(std::exchange(o.h, nullptr)) {}
+    ~Owned() { if (h) Destroy(h); }
+};
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+using DevAlloc = Owned<void*, cudaFree>;
+using IpcMapping = Owned<void*, cudaIpcCloseMemHandle>;
+
+// the non-blocking stream of `s`, created on first use
+cudaError_t ensure_stream(Stream& s) { return s.h ? cudaSuccess : cudaStreamCreateWithFlags(&s.h, cudaStreamNonBlocking); }
 
 bool is_device_pointer(const void* p) {
     cudaPointerAttributes at;
@@ -98,17 +122,17 @@ struct nmrfit_ctx {
     long long mt_elems = 0;            // elements of one random array (n_spectra * swarmsize * D)
     DevBuf<double> mt_a[2], mt_b[2];   // nmrfit_ctx_mt19937_begin / _end: two sets of arrays, used in turn
     DevBuf<unsigned> mt_state2, mt_words2;
-    cudaStream_t mt_stream = nullptr;
-    unsigned* mt_host = nullptr;       // page-locked [2][625]: state in, state out
+    Stream mt_stream;
+    PinnedBuf<unsigned> mt_host;       // [2][625]: state in, state out
     int mt_flip = 0, mt_pending = 0;
     DevBuf<double> fin_scratch;        // finish kernel: per-CTA candidates
     DevBuf<unsigned> fin_tickets;
     // record exchange over peer memory (particle sharding without a collective call)
-    void* peer_win = nullptr;          // this context's window: records [2][R][B][D+2], then tokens [R][B]
+    DevAlloc peer_win;                 // this context's window: records [2][R][B][D+2], then tokens [R][B]
     size_t peer_rec_bytes = 0;
     int peer_ranks = 0, peer_rank = 0;
     bool peers_ready = false;
-    std::vector<void*> peer_opened;    // windows of other processes opened through CUDA IPC
+    std::vector<IpcMapping> peer_opened;   // windows of other processes opened through CUDA IPC
     DevBuf<double*> peer_recs_dev;
     DevBuf<long long*> peer_tok_dev;
     DevBuf<int> peer_err;
@@ -119,18 +143,17 @@ struct nmrfit_ctx {
     DevBuf<double> rf_x, rf_cur;       // refinement: current, trial, lb, ub [4][B][D]; H | g | s at the current point
     DevBuf<RefineState> rf_state;
     DevBuf<int> rf_active;             // spectra still running after the last polled step
-    cudaStream_t pipe[2] = {nullptr, nullptr};   // nmrfit_objective_batch_host: slices of a large particle set
-    double* h_f = nullptr;                       // ... and page-locked staging of their values
-    size_t h_f_cap = 0;
+    Stream pipe[2];                    // nmrfit_objective_batch_host: slices of a large particle set
+    PinnedBuf<double> h_f;             // ... and staging of their values
     int far_cells = 0;                 // far-field cells per region: 0 = far_cells_per_region(N, R), else 1 | 2 | 4
     int fused_mode = NMRFIT_FUSED_AUTO;
     DevBuf<long long> ftiming;         // optional per-phase cycle counters of the fused kernel
     bool fused_timing = false;
     long long fused_launches = 0;
-    int* h_flags = nullptr;            // pinned [2*B]
+    PinnedBuf<int> h_flags;            // [2*B]
     // optional per-launch timing of the objective kernel (nmrfit_ctx_profile)
     bool profiling = false;
-    std::vector<cudaEvent_t> prof_events;   // pairs
+    std::vector<Event> prof_events;    // triples
     size_t prof_used = 0;
 };
 
@@ -280,11 +303,30 @@ int check_ctx(const nmrfit_ctx* c) {
     return NMRFIT_OK;
 }
 
-int run_objective(nmrfit_ctx* c, const double* x_dev, int S, int fit_im, double* f_dev, const int* frozen,
-                  cudaStream_t st, const MoveArgs* mv = nullptr, int* tiles_out = nullptr, int* nsum_out = nullptr,
-                  int* nw_out = nullptr, size_t slot0 = 0, size_t slots_total = 0, const double* x_in = nullptr) {
-    // slot0 / slots_total (one spectrum only): this launch is one slice of a larger particle set evaluated in pieces on
-    // several streams (nmrfit_objective_batch_host); it owns the scratch of particle slots [slot0, slot0 + S + pad)
+// every spectrum of the context has been set; `what` completes the error message otherwise
+int require_spectra(const nmrfit_ctx* c, const char* what) {
+    for (char f : c->spec_set)
+        if (!f) return fail(NMRFIT_ERR_STATE, std::string("every spectrum must be set before ") + what);
+    return NMRFIT_OK;
+}
+
+// optional inputs of run_objective
+struct ObjIn {
+    const double* x_in = nullptr;      // the positions as the device sees them in page-locked host memory (FP64 uniform axis)
+    // (one spectrum only) this launch is one slice of a larger particle set evaluated in pieces on several streams
+    // (nmrfit_objective_batch_host); it owns the scratch of particle slots [slot0, slot0 + S + pad) of slots_total
+    size_t slot0 = 0, slots_total = 0;
+    const int* frozen = nullptr;       // per-spectrum stop flags of the swarm: stopped spectra are skipped
+    const MoveArgs* move = nullptr;    // move the swarm before evaluating it
+};
+
+// what a launch of run_objective left in c->partials for the finish kernel
+struct ObjOut {
+    int n_tiles = 0, nsum = 1, nw = 1;
+};
+
+int run_objective(nmrfit_ctx* c, const double* x_dev, int S, int fit_im, double* f_dev, cudaStream_t st,
+                  const ObjIn& in = {}, ObjOut* out = nullptr) {
     for (int b = 0; b < c->B; ++b)
         if (!c->spec_set[b]) return fail(NMRFIT_ERR_STATE, "spectrum " + std::to_string(b) + " was never set");
     if (fit_im < 0 || fit_im > 2) return fail(NMRFIT_ERR_ARG, "fit_im must be 0, 1 or 2");
@@ -300,28 +342,28 @@ int run_objective(nmrfit_ctx* c, const double* x_dev, int S, int fit_im, double*
                                         : "points_per_thread must be 2, 4 or 8 for the general kernel");
     int n_tiles = objective_tiles(c->N, t);
     const size_t part_per = (size_t)n_tiles * 2 * (t.variant == 1 ? t.threads / 32 : 1);
-    CK(c->partials.reserve(std::max((size_t)c->B * S, slots_total) * part_per));
+    CK(c->partials.reserve(std::max((size_t)c->B * S, in.slots_total) * part_per));
     ObjArgs a{};
     const int sub = (uni && c->precision == NMRFIT_FP64) ? ctx_cells(c, t.r) : 1;
     if (uni) {
         size_t nc, np, nf, na, nm;
         int pad = 0;
         objective_uniform_prep_sizes(c->N, c->P, t, sub, &nc, &np, &nf, &na, &nm, &pad);
-        const size_t slots = std::max((size_t)c->B * S, slots_total) + pad;
+        const size_t slots = std::max((size_t)c->B * S, in.slots_total) + pad;
         CK(c->prep_coef.reserve(slots * nc));
         CK(c->prep_part.reserve(slots * np));
         CK(c->prep_far.reserve(slots * nf));
         CK(c->prep_anchor.reserve(slots * na));
         CK(c->prep_mask.reserve(slots * nm));
-        a.prep_coef = c->prep_coef.ptr + slot0 * nc; a.prep_part = c->prep_part.ptr + slot0 * np;
-        a.prep_far = c->prep_far.ptr + slot0 * nf; a.prep_anchor = c->prep_anchor.ptr + slot0 * na;
-        a.prep_mask = c->prep_mask.ptr + slot0 * nm;
+        a.prep_coef = c->prep_coef.ptr + in.slot0 * nc; a.prep_part = c->prep_part.ptr + in.slot0 * np;
+        a.prep_far = c->prep_far.ptr + in.slot0 * nf; a.prep_anchor = c->prep_anchor.ptr + in.slot0 * na;
+        a.prep_mask = c->prep_mask.ptr + in.slot0 * nm;
     }
     a.spec = c->spec.ptr;
     a.x = x_dev;
-    a.x_in = x_in;                                         // (two-pass FP64 path only: the caller checks)
-    a.partials = c->partials.ptr + slot0 * part_per;
-    a.frozen = frozen;
+    a.x_in = in.x_in;                                      // (two-pass FP64 path only: the caller checks)
+    a.partials = c->partials.ptr + in.slot0 * part_per;
+    a.frozen = in.frozen;
     a.grid_h = c->grid_h.ptr;
     a.N = c->N; a.P = c->P; a.S = S; a.kk = fit_im; a.sp = t.sp; a.sub = sub;
     // profiling: three events per launch - before the prepare pass, between it and the evaluation kernel, after
@@ -331,12 +373,12 @@ int run_objective(nmrfit_ctx* c, const double* x_dev, int S, int fit_im, double*
             for (int k = 0; k < 3; ++k) {
                 cudaEvent_t ev;
                 CK(cudaEventCreate(&ev));
-                c->prof_events.push_back(ev);
+                c->prof_events.emplace_back(ev);
             }
         }
-        ev0 = c->prof_events[c->prof_used];
-        evm = c->prof_events[c->prof_used + 1];
-        ev1 = c->prof_events[c->prof_used + 2];
+        ev0 = c->prof_events[c->prof_used].h;
+        evm = c->prof_events[c->prof_used + 1].h;
+        ev1 = c->prof_events[c->prof_used + 2].h;
         c->prof_used += 3;
     }
     const bool two_pass = uni && c->precision == NMRFIT_FP64;
@@ -345,17 +387,19 @@ int run_objective(nmrfit_ctx* c, const double* x_dev, int S, int fit_im, double*
         CK(cudaEventRecord(evm, st));
         ev0 = nullptr;
     }
+    const MoveArgs* mv = in.move;
     const bool move_in_prepare = mv && uni && c->precision == NMRFIT_FP64;
     if (mv && !move_in_prepare) {                          // paths without a prepare pass move the swarm on their own
         cudaError_t em = launch_swarm_move(mv->s, mv->rp, mv->rg, mv->generation, st);
         if (em != cudaSuccess) return fail_cuda(em, "swarm move");
     }
-    if (nsum_out) *nsum_out = c->precision == NMRFIT_FP32 ? 1 : (fit_im ? 2 : 1);
-    if (nw_out) *nw_out = 1;
-    cudaError_t e = c->precision == NMRFIT_FP32 ? launch_objective_f32(a, t, c->B, f_dev, uni, st, ev0, ev1, tiles_out)
-                    : uni ? launch_objective_uniform(a, t, c->B, f_dev, st, ev0, ev1, move_in_prepare ? mv : nullptr, tiles_out, evm, nw_out)
-                          : launch_objective(a, t, c->B, f_dev, st, ev0, ev1, tiles_out);
+    ObjOut o;
+    o.nsum = c->precision == NMRFIT_FP32 ? 1 : (fit_im ? 2 : 1);
+    cudaError_t e = c->precision == NMRFIT_FP32 ? launch_objective_f32(a, t, c->B, f_dev, uni, st, ev0, ev1, &o.n_tiles)
+                    : uni ? launch_objective_uniform(a, t, c->B, f_dev, st, ev0, ev1, move_in_prepare ? mv : nullptr, &o.n_tiles, evm, &o.nw)
+                          : launch_objective(a, t, c->B, f_dev, st, ev0, ev1, &o.n_tiles);
     if (e != cudaSuccess) return fail_cuda(e, "objective launch");
+    if (out) *out = o;
     return NMRFIT_OK;
 }
 
@@ -430,15 +474,63 @@ int swarm_generation(nmrfit_ctx* c, bool move, const double* rp_d, const double*
     SwarmState& s = c->sw;
     if (commit == 2 && !c->peers_ready) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_peer_open has not been called");
     const PeerArgs pa = commit == 2 ? make_peer_args(c) : PeerArgs{};
-    MoveArgs mv{s, rp_d, rg_d, c->generation};
-    int n_tiles = 0, nsum = 1, nw = 1;
-    if (int rc = run_objective(c, s.x, s.S, c->kk, nullptr, move ? s.stop : nullptr, st, move ? &mv : nullptr, &n_tiles, &nsum,
-                               &nw))
-        return rc;
-    cudaError_t e = launch_swarm_finish(s, c->partials.ptr, n_tiles, nsum, c->N, s.rec, c->fin_scratch.ptr,
-                                        c->fin_tickets.ptr, commit, c->maxiter, st, nw, commit == 2 ? &pa : nullptr);
+    const MoveArgs mv{s, rp_d, rg_d, c->generation};
+    ObjIn in;
+    if (move) {
+        in.frozen = s.stop;
+        in.move = &mv;
+    }
+    ObjOut o;
+    if (int rc = run_objective(c, s.x, s.S, c->kk, nullptr, st, in, &o)) return rc;
+    cudaError_t e = launch_swarm_finish(s, c->partials.ptr, o.n_tiles, o.nsum, c->N, s.rec, c->fin_scratch.ptr,
+                                        c->fin_tickets.ptr, commit, c->maxiter, st, o.nw, commit == 2 ? &pa : nullptr);
     if (e != cudaSuccess) return fail_cuda(e, "swarm finish");
     return NMRFIT_OK;
+}
+
+int require_swarm(const nmrfit_ctx* c) {
+    if (int rc = check_ctx(c)) return rc;
+    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
+    return NMRFIT_OK;
+}
+
+// The random arrays of `n` generations, [n][B][S][D] each: both given (host arrays are staged into rnd_a / rnd_b,
+// device arrays are used in place) or both null (the swarm draws its own).  `names` is how the caller calls them.
+int stage_random(nmrfit_ctx* c, int n, const double* rp, const double* rg, const char* names, cudaStream_t st,
+                 const double** rp_d, const double** rg_d) {
+    *rp_d = *rg_d = nullptr;
+    if ((rp == nullptr) != (rg == nullptr)) return fail(NMRFIT_ERR_ARG, std::string(names) + " must both be given or both be NULL");
+    if (n <= 0) return NMRFIT_OK;
+    const size_t nsd = (size_t)c->sw.B * c->sw.S * c->sw.D * n;
+    if (int rc = stage(rp, nsd, c->rnd_a, st, rp_d)) return rc;
+    return stage(rg, nsd, c->rnd_b, st, rg_d);
+}
+
+// `n` generations of the per-step path on `st`, with the random arrays of stage_random
+int queue_generations(nmrfit_ctx* c, int n, const double* rp_d, const double* rg_d, int commit, cudaStream_t st) {
+    const size_t nsd = (size_t)c->sw.B * c->sw.S * c->sw.D;
+    for (int k = 0; k < n; ++k) {
+        c->generation += 1;
+        if (int rc = swarm_generation(c, true, rp_d ? rp_d + nsd * k : nullptr, rg_d ? rg_d + nsd * k : nullptr, commit, st))
+            return rc;
+    }
+    return NMRFIT_OK;
+}
+
+// Queue the host copy of the stop flags into h_flags [0, B) and of an optional device error word into h_flags [B] (0
+// without one).  Once `st` has been synchronised, running_spectra counts the spectra whose swarm has not stopped.
+int queue_stop_flags(nmrfit_ctx* c, const int* err_dev, cudaStream_t st) {
+    const int B = c->sw.B;
+    CK(cudaMemcpyAsync(c->h_flags.ptr, c->sw.stop, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
+    c->h_flags.ptr[B] = 0;
+    if (err_dev) CK(cudaMemcpyAsync(c->h_flags.ptr + B, err_dev, sizeof(int), cudaMemcpyDeviceToHost, st));
+    return NMRFIT_OK;
+}
+
+int running_spectra(const nmrfit_ctx* c) {
+    int running = 0;
+    for (int b = 0; b < c->sw.B; ++b) running += c->h_flags.ptr[b] == 0;
+    return running;
 }
 
 }  // namespace
@@ -467,66 +559,22 @@ int nmrfit_ctx_create(nmrfit_ctx** out, int device, int n_spectra, int n_points,
     CK(cudaGetDeviceCount(&ndev));
     if (device < 0 || device >= ndev) return fail(NMRFIT_ERR_ARG, "no such CUDA device");
     CK(cudaSetDevice(device));
-    nmrfit_ctx* c = new (std::nothrow) nmrfit_ctx();
+    std::unique_ptr<nmrfit_ctx> c(new (std::nothrow) nmrfit_ctx());
     if (!c) return fail(NMRFIT_ERR_NOMEM, "out of host memory");
     c->device = device; c->B = n_spectra; c->N = n_points; c->P = n_peaks; c->D = 4 + 3 * n_peaks;
     c->precision = precision;
     c->spec_set.assign(n_spectra, 0);
     c->uniform.assign(n_spectra, 0);
-    cudaError_t e = c->spec.reserve((size_t)n_spectra * 4 * n_points);
-    if (e == cudaSuccess) e = c->grid_h.reserve(2 * (size_t)n_spectra);
-    if (e == cudaSuccess) e = cudaMallocHost(&c->h_flags, sizeof(int) * 2 * n_spectra);
-    if (e != cudaSuccess) {
-        nmrfit_ctx_destroy(c);
-        return fail_cuda(e, "ctx allocation");
-    }
-    *out = c;
+    CK(c->spec.reserve((size_t)n_spectra * 4 * n_points));
+    CK(c->grid_h.reserve(2 * (size_t)n_spectra));
+    CK(c->h_flags.reserve(2 * (size_t)n_spectra));
+    *out = c.release();
     return NMRFIT_OK;
 }
 
 void nmrfit_ctx_destroy(nmrfit_ctx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
-    c->prep_mask.release();
-    for (DevBuf<double>* b : {&c->prep_coef, &c->prep_part, &c->prep_far, &c->prep_anchor, &c->spec, &c->grid_h, &c->partials, &c->x_stage, &c->f_stage, &c->sx, &c->sv, &c->sp, &c->sfx,
-                              &c->sfp, &c->sg, &c->sfg, &c->sbx, &c->sbf, &c->slb, &c->sub, &c->srec, &c->rnd_a,
-                              &c->rnd_b})
-        b->release();
-    c->sstop.release();
-    c->sit.release();
-    c->frec_f.release();
-    c->frec_x.release();
-    c->fbarrier.release();
-    c->ferror.release();
-    c->mt_state.release();
-    for (int k = 0; k < 2; ++k) { c->mt_a[k].release(); c->mt_b[k].release(); }
-    c->mt_state2.release();
-    c->mt_words2.release();
-    if (c->mt_stream) cudaStreamDestroy(c->mt_stream);
-    if (c->mt_host) cudaFreeHost(c->mt_host);
-    c->mt_words.release();
-    c->ftiming.release();
-    for (void* p : c->peer_opened) cudaIpcCloseMemHandle(p);
-    if (c->peer_win) cudaFree(c->peer_win);
-    c->peer_recs_dev.release();
-    c->peer_tok_dev.release();
-    c->peer_err.release();
-    c->wscratch.release();
-    c->fin_scratch.release();
-    c->fin_tickets.release();
-    c->wbounds.release();
-    c->ne_x.release();
-    c->ne_part.release();
-    c->ne_out.release();
-    c->rf_x.release();
-    c->rf_cur.release();
-    c->rf_state.release();
-    c->rf_active.release();
-    for (int k = 0; k < 2; ++k)
-        if (c->pipe[k]) cudaStreamDestroy(c->pipe[k]);
-    if (c->h_f) cudaFreeHost(c->h_f);
-    if (c->h_flags) cudaFreeHost(c->h_flags);
-    for (cudaEvent_t ev : c->prof_events) cudaEventDestroy(ev);
     delete c;
 }
 
@@ -610,8 +658,7 @@ int nmrfit_ctx_compute_weights(nmrfit_ctx* c, const double* peak_bounds, const d
     if (!peak_bounds || !peak_values) return fail(NMRFIT_ERR_ARG, "peak_bounds and peak_values must be non-NULL");
     if (n_windows < 1 || n_windows > 4096) return fail(NMRFIT_ERR_ARG, "n_windows must be 1..4096");
     if (sweeps < 0) return fail(NMRFIT_ERR_ARG, "sweeps must be >= 0");
-    for (char f : c->spec_set)
-        if (!f) return fail(NMRFIT_ERR_STATE, "every spectrum must be set before its weights are computed");
+    if (int r = require_spectra(c, "its weights are computed")) return r;
     CK(cudaSetDevice(c->device));
     for (auto& sh : c->shadow) sh.clear();                 // the weights plane is rewritten on the device
     cudaStream_t st = (cudaStream_t)stream;
@@ -637,8 +684,7 @@ int nmrfit_ctx_normal_equations(nmrfit_ctx* c, const double* x, double* H, doubl
     if (c->P > 64)
         return fail(NMRFIT_ERR_ARG, "normal equations support at most 64 peaks (D <= 196), the context has " +
                                         std::to_string(c->P));
-    for (char f : c->spec_set)
-        if (!f) return fail(NMRFIT_ERR_STATE, "every spectrum must be set before its normal equations are computed");
+    if (int r = require_spectra(c, "its normal equations are computed")) return r;
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     const size_t B = (size_t)c->B, D = (size_t)c->D, DD = D * D, per = 2 * DD + D + 2;
@@ -672,8 +718,7 @@ int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* 
     if (c->N <= c->D) return fail(NMRFIT_ERR_ARG, "refinement needs more points than parameters");
     if (max_iter < 1) return fail(NMRFIT_ERR_ARG, "max_iter must be >= 1");
     if (!(xtol > 0.0)) return fail(NMRFIT_ERR_ARG, "xtol must be > 0");
-    for (char f : c->spec_set)
-        if (!f) return fail(NMRFIT_ERR_STATE, "every spectrum must be set before it is refined");
+    if (int r = require_spectra(c, "it is refined")) return r;
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     const size_t B = (size_t)c->B, D = (size_t)c->D, BD = B * D;
@@ -708,9 +753,9 @@ int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* 
                                max_iter, xtol, poll ? c->rf_active.ptr : nullptr, st);
         if (e != cudaSuccess) return fail_cuda(e, "refinement step launch");
         if (poll) {
-            CK(cudaMemcpyAsync(c->h_flags, c->rf_active.ptr, sizeof(int), cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(c->h_flags.ptr, c->rf_active.ptr, sizeof(int), cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
-            if (c->h_flags[0] == 0) break;
+            if (c->h_flags.ptr[0] == 0) break;
         }
     }
     CK(cudaMemcpyAsync(x, xc, sizeof(double) * BD, cudaMemcpyDefault, st));
@@ -843,10 +888,10 @@ int nmrfit_ctx_profile_read_split(nmrfit_ctx* c, double* prepare_ms, double* eva
     CK(cudaSetDevice(c->device));
     double prep = 0.0, eval = 0.0;
     for (size_t i = 0; i + 2 < c->prof_used; i += 3) {
-        CK(cudaEventSynchronize(c->prof_events[i + 2]));
+        CK(cudaEventSynchronize(c->prof_events[i + 2].h));
         float a = 0.f, b = 0.f;
-        CK(cudaEventElapsedTime(&a, c->prof_events[i], c->prof_events[i + 1]));
-        CK(cudaEventElapsedTime(&b, c->prof_events[i + 1], c->prof_events[i + 2]));
+        CK(cudaEventElapsedTime(&a, c->prof_events[i].h, c->prof_events[i + 1].h));
+        CK(cudaEventElapsedTime(&b, c->prof_events[i + 1].h, c->prof_events[i + 2].h));
         prep += a;
         eval += b;
     }
@@ -869,14 +914,13 @@ int nmrfit_objective_batch(nmrfit_ctx* c, const double* x_dev, int S, int fit_im
     if (!x_dev || !f_dev) return fail(NMRFIT_ERR_ARG, "x_dev and f_dev must be non-NULL");
     if (S < 1) return fail(NMRFIT_ERR_ARG, "n_particles must be >= 1");
     CK(cudaSetDevice(c->device));
-    return run_objective(c, x_dev, S, fit_im, f_dev, nullptr, (cudaStream_t)stream);
+    return run_objective(c, x_dev, S, fit_im, f_dev, (cudaStream_t)stream);
 }
 
 namespace {
 // Page-locked host positions as the device sees them (null: pageable memory, or a path without the prepare pass)
 const double* mapped_positions(const nmrfit_ctx* c, const double* x_host, int fit_im) {
-    static const bool kZeroCopy = [] { const char* e = getenv("NMRFIT_E2E_ZEROCOPY"); return !(e && atoi(e) == 0); }();
-    if (!kZeroCopy || !use_uniform(c, fit_im) || c->precision != NMRFIT_FP64) return nullptr;
+    if (!use_uniform(c, fit_im) || c->precision != NMRFIT_FP64) return nullptr;
     cudaPointerAttributes at{};
     const cudaError_t pe = cudaPointerGetAttributes(&at, x_host);
     if (pe != cudaSuccess) (void)cudaGetLastError();
@@ -896,50 +940,38 @@ int nmrfit_objective_batch_host(nmrfit_ctx* c, const double* x_host, int S, int 
     // k + 1's positions are on their way in and slice k - 1's values on their way out (each slice has its own scratch).
     // Page-locked host positions (cudaHostAlloc / cudaHostRegister: mapped into the device under unified addressing) are
     // read by the prepare pass ITSELF, each element crossing PCIe once while other CTAs compute - no staging copy in
-    // front of the kernels (NMRFIT_E2E_ZEROCOPY=0 turns this off).  Pageable arrays take the copies below.
+    // front of the kernels.  Pageable arrays take the copies below.
     const double* x_map = mapped_positions(c, x_host, fit_im);     // the caller's array as the device sees it, or null
     constexpr int kPad = 64;
     // (slices of ~12k particles, two to six of them: 1.24 / 1.15 / 1.13 / 1.12 ms per call with 1 / 2 / 4 / 6 slices
-    // at 65,536 particles of 6 peaks x 4,096 points, tools/e2e_probe.py; NMRFIT_E2E_SLICES overrides)
-    static const int kEnvSlices = [] { const char* e = getenv("NMRFIT_E2E_SLICES"); const int v = e ? atoi(e) : 0; return v < 0 ? 0 : (v > 16 ? 16 : v); }();
+    // at 65,536 particles of 6 peaks x 4,096 points, tools/e2e_probe.py)
     // (in-place reads are not sliced: 1.048 / 1.084 / 1.105 ms with 1 / 2 / 3 slices - and 1.136 ms for the best copy path)
-    const int kSlices = kEnvSlices ? kEnvSlices : x_map ? 1 : std::min(6, std::max(2, S / 12288));
+    const int kSlices = x_map ? 1 : std::min(6, std::max(2, S / 12288));
     if (c->B == 1 && S >= 4 * 4096 && !c->profiling && kSlices > 1) {
-        for (int k = 0; k < 2; ++k)
-            if (!c->pipe[k]) CK(cudaStreamCreateWithFlags(&c->pipe[k], cudaStreamNonBlocking));
-        if (c->h_f_cap < nf) {
-            if (c->h_f) cudaFreeHost(c->h_f);
-            c->h_f = nullptr;
-            c->h_f_cap = 0;
-            CK(cudaMallocHost(&c->h_f, sizeof(double) * nf));
-            c->h_f_cap = nf;
-        }
+        for (Stream& ps : c->pipe) CK(ensure_stream(ps));
+        CK(c->h_f.reserve(nf));
         const int chunk = ((S + kSlices - 1) / kSlices + 63) & ~63;
         const size_t total = (size_t)kSlices * (chunk + kPad);
         for (int k = 0, s0 = 0; s0 < S; ++k, s0 += chunk) {
             const int ns = std::min(chunk, S - s0);
-            cudaStream_t ps = c->pipe[k & 1];
+            cudaStream_t ps = c->pipe[k & 1].h;
             if (!x_map)
                 CK(cudaMemcpyAsync(c->x_stage.ptr + (size_t)s0 * c->D, x_host + (size_t)s0 * c->D, sizeof(double) * ns * c->D,
                                    cudaMemcpyHostToDevice, ps));
-            if (int rc = run_objective(c, c->x_stage.ptr + (size_t)s0 * c->D, ns, fit_im, c->f_stage.ptr + s0, nullptr, ps,
-                                       nullptr, nullptr, nullptr, nullptr, (size_t)k * (chunk + kPad), total,
-                                       x_map ? x_map + (size_t)s0 * c->D : nullptr))
+            const ObjIn slice{x_map ? x_map + (size_t)s0 * c->D : nullptr, (size_t)k * (chunk + kPad), total};
+            if (int rc = run_objective(c, c->x_stage.ptr + (size_t)s0 * c->D, ns, fit_im, c->f_stage.ptr + s0, ps, slice))
                 return rc;
             // (into page-locked staging: an "async" copy into the caller's pageable array would block the host until
             // the slice has been evaluated, and the slices would run one after the other)
-            CK(cudaMemcpyAsync(c->h_f + s0, c->f_stage.ptr + s0, sizeof(double) * ns, cudaMemcpyDeviceToHost, ps));
+            CK(cudaMemcpyAsync(c->h_f.ptr + s0, c->f_stage.ptr + s0, sizeof(double) * ns, cudaMemcpyDeviceToHost, ps));
         }
-        CK(cudaStreamSynchronize(c->pipe[0]));
-        CK(cudaStreamSynchronize(c->pipe[1]));
-        std::memcpy(f_host, c->h_f, sizeof(double) * nf);
+        for (Stream& ps : c->pipe) CK(cudaStreamSynchronize(ps.h));
+        std::memcpy(f_host, c->h_f.ptr, sizeof(double) * nf);
         return NMRFIT_OK;
     }
     cudaStream_t st = 0;
     if (!x_map) CK(cudaMemcpyAsync(c->x_stage.ptr, x_host, nx * sizeof(double), cudaMemcpyHostToDevice, st));
-    if (int rc = run_objective(c, c->x_stage.ptr, S, fit_im, c->f_stage.ptr, nullptr, st, nullptr, nullptr, nullptr, nullptr, 0, 0,
-                               x_map))
-        return rc;
+    if (int rc = run_objective(c, c->x_stage.ptr, S, fit_im, c->f_stage.ptr, st, ObjIn{x_map})) return rc;
     CK(cudaMemcpyAsync(f_host, c->f_stage.ptr, nf * sizeof(double), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return NMRFIT_OK;
@@ -968,9 +1000,7 @@ int nmrfit_objective_spectrum_host(nmrfit_ctx* c, const double* w, const double*
     CK(c->x_stage.reserve((size_t)S * c->D));
     CK(c->f_stage.reserve((size_t)S));
     cudaStream_t st = 0;
-    if (int rc = run_objective(c, c->x_stage.ptr, S, fit_im, c->f_stage.ptr, nullptr, st, nullptr, nullptr, nullptr, nullptr, 0, 0,
-                               x_map))
-        return rc;
+    if (int rc = run_objective(c, c->x_stage.ptr, S, fit_im, c->f_stage.ptr, st, ObjIn{x_map})) return rc;
     const double* src[4] = {w, u, v, weights};
     bool same = true;
     for (int k = 0; same && k < 4; ++k) same = std::memcmp(c->shadow[0].data() + (size_t)k * N, src[k], sizeof(double) * N) == 0;
@@ -1038,58 +1068,63 @@ int nmrfit_pso_begin(nmrfit_ctx* c, const double* lb, const double* ub, const nm
     return swarm_generation(c, false, nullptr, nullptr, 0, st);
 }
 
-int nmrfit_pso_advance(nmrfit_ctx* c, const double* rp, const double* rg, void* stream) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
-    if ((rp == nullptr) != (rg == nullptr)) return fail(NMRFIT_ERR_ARG, "rp and rg must both be given or both be NULL");
+namespace {
+// One generation of nmrfit_pso_advance (commit 0), nmrfit_pso_step (1) or nmrfit_pso_step_peers (2)
+int pso_generation(nmrfit_ctx* c, const double* rp, const double* rg, int commit, void* stream) {
+    if (int rc = require_swarm(c)) return rc;
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
-    SwarmState& s = c->sw;
-    size_t nsd = (size_t)s.B * s.S * s.D;
-    const double *rp_d = nullptr, *rg_d = nullptr;
-    if (int rc = stage(rp, nsd, c->rnd_a, st, &rp_d)) return rc;
-    if (int rc = stage(rg, nsd, c->rnd_b, st, &rg_d)) return rc;
-    c->generation += 1;
-    return swarm_generation(c, true, rp_d, rg_d, 0, st);
+    const double *rp_d, *rg_d;
+    if (int rc = stage_random(c, 1, rp, rg, "rp and rg", st, &rp_d, &rg_d)) return rc;
+    return queue_generations(c, 1, rp_d, rg_d, commit, st);
+}
+
+// the argument checks of nmrfit_ctx_mt19937 and nmrfit_ctx_mt19937_begin
+int mt_check(const nmrfit_ctx* c, int pos, long long n_arrays) {
+    if (pos < 0 || pos > 624) return fail(NMRFIT_ERR_ARG, "MT19937 position must be 0..624");
+    if (n_arrays < 2 || (n_arrays & 1)) return fail(NMRFIT_ERR_ARG, "n_arrays must be even: arrays come in (first, second) pairs");
+    if (c->mt_elems == 0) return fail(NMRFIT_ERR_STATE, "call nmrfit_ctx_mt19937_shape first");
+    return NMRFIT_OK;
+}
+
+// Queue on `st` the generation of n_arrays arrays into (a, b) in turn, from the state (key [624] + position) at
+// `state_in`; the advanced state goes back to `state_out`.  Each caller has its own buffers: nmrfit_ctx_mt19937 may
+// run while a nmrfit_ctx_mt19937_begin is pending.
+int mt_queue(nmrfit_ctx* c, long long n_arrays, DevBuf<double>& a, DevBuf<double>& b, DevBuf<unsigned>& state,
+             DevBuf<unsigned>& words, const unsigned* state_in, unsigned* state_out, cudaStream_t st) {
+    const long long nsd = c->mt_elems, pairs = n_arrays / 2;
+    CK(a.reserve((size_t)(pairs * nsd)));
+    CK(b.reserve((size_t)(pairs * nsd)));
+    CK(state.reserve(625));
+    CK(words.reserve((size_t)(2 * n_arrays * nsd)));
+    CK(cudaMemcpyAsync(state.ptr, state_in, sizeof(unsigned) * 625, cudaMemcpyHostToDevice, st));
+    cudaError_t e = launch_mt19937(state.ptr, reinterpret_cast<int*>(state.ptr + 624), n_arrays * nsd, words.ptr, a.ptr,
+                                   b.ptr, nsd, st);
+    if (e != cudaSuccess) return fail_cuda(e, "MT19937 launch");
+    CK(cudaMemcpyAsync(state_out, state.ptr, sizeof(unsigned) * 625, cudaMemcpyDeviceToHost, st));
+    return NMRFIT_OK;
+}
+}  // namespace
+
+int nmrfit_pso_advance(nmrfit_ctx* c, const double* rp, const double* rg, void* stream) {
+    return pso_generation(c, rp, rg, 0, stream);
 }
 
 int nmrfit_pso_step(nmrfit_ctx* c, const double* rp, const double* rg, void* stream) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
-    if ((rp == nullptr) != (rg == nullptr)) return fail(NMRFIT_ERR_ARG, "rp and rg must both be given or both be NULL");
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    SwarmState& s = c->sw;
-    size_t nsd = (size_t)s.B * s.S * s.D;
-    const double *rp_d = nullptr, *rg_d = nullptr;
-    if (int rc = stage(rp, nsd, c->rnd_a, st, &rp_d)) return rc;
-    if (int rc = stage(rg, nsd, c->rnd_b, st, &rg_d)) return rc;
-    c->generation += 1;
-    return swarm_generation(c, true, rp_d, rg_d, 1, st);
+    return pso_generation(c, rp, rg, 1, stream);
 }
 
 int nmrfit_ctx_mt19937(nmrfit_ctx* c, unsigned* key, int* pos, long long n_arrays, double** a_dev, double** b_dev,
                        void* stream) {
     if (int rc = check_ctx(c)) return rc;
     if (!key || !pos || !a_dev || !b_dev) return fail(NMRFIT_ERR_ARG, "NULL argument");
-    if (*pos < 0 || *pos > 624) return fail(NMRFIT_ERR_ARG, "MT19937 position must be 0..624");
-    if (n_arrays < 2 || (n_arrays & 1)) return fail(NMRFIT_ERR_ARG, "n_arrays must be even: arrays come in (first, second) pairs");
-    if (c->mt_elems == 0) return fail(NMRFIT_ERR_STATE, "call nmrfit_ctx_mt19937_shape first");
+    if (int rc = mt_check(c, *pos, n_arrays)) return rc;
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
-    const long long nsd = c->mt_elems, pairs = n_arrays / 2;
-    CK(c->rnd_a.reserve((size_t)(pairs * nsd)));
-    CK(c->rnd_b.reserve((size_t)(pairs * nsd)));
-    CK(c->mt_state.reserve(625));
-    CK(c->mt_words.reserve((size_t)(2 * n_arrays * nsd)));
     unsigned host[625];
     std::memcpy(host, key, sizeof(unsigned) * 624);
     host[624] = (unsigned)*pos;
-    CK(cudaMemcpyAsync(c->mt_state.ptr, host, sizeof(host), cudaMemcpyHostToDevice, st));
-    cudaError_t e = launch_mt19937(c->mt_state.ptr, reinterpret_cast<int*>(c->mt_state.ptr + 624), n_arrays * nsd,
-                                   c->mt_words.ptr, c->rnd_a.ptr, c->rnd_b.ptr, nsd, st);
-    if (e != cudaSuccess) return fail_cuda(e, "MT19937 launch");
-    CK(cudaMemcpyAsync(host, c->mt_state.ptr, sizeof(host), cudaMemcpyDeviceToHost, st));
+    if (int rc = mt_queue(c, n_arrays, c->rnd_a, c->rnd_b, c->mt_state, c->mt_words, host, host, st)) return rc;
     CK(cudaStreamSynchronize(st));
     std::memcpy(key, host, sizeof(unsigned) * 624);
     *pos = (int)host[624];
@@ -1105,28 +1140,18 @@ int nmrfit_ctx_mt19937(nmrfit_ctx* c, unsigned* key, int* pos, long long n_array
 int nmrfit_ctx_mt19937_begin(nmrfit_ctx* c, const unsigned* key, int pos, long long n_arrays, double** a_dev, double** b_dev) {
     if (int rc = check_ctx(c)) return rc;
     if (!key || !a_dev || !b_dev) return fail(NMRFIT_ERR_ARG, "NULL argument");
-    if (pos < 0 || pos > 624) return fail(NMRFIT_ERR_ARG, "MT19937 position must be 0..624");
-    if (n_arrays < 2 || (n_arrays & 1)) return fail(NMRFIT_ERR_ARG, "n_arrays must be even: arrays come in (first, second) pairs");
-    if (c->mt_elems == 0) return fail(NMRFIT_ERR_STATE, "call nmrfit_ctx_mt19937_shape first");
+    if (int rc = mt_check(c, pos, n_arrays)) return rc;
     if (c->mt_pending) return fail(NMRFIT_ERR_STATE, "nmrfit_ctx_mt19937_end has not been called for the previous begin");
     CK(cudaSetDevice(c->device));
-    if (!c->mt_stream) CK(cudaStreamCreateWithFlags(&c->mt_stream, cudaStreamNonBlocking));
-    if (!c->mt_host) CK(cudaMallocHost(&c->mt_host, sizeof(unsigned) * 2 * 625));
-    const long long nsd = c->mt_elems, pairs = n_arrays / 2;
+    CK(ensure_stream(c->mt_stream));
+    CK(c->mt_host.reserve(2 * 625));
     const int k = c->mt_flip;
+    std::memcpy(c->mt_host.ptr, key, sizeof(unsigned) * 624);
+    c->mt_host.ptr[624] = (unsigned)pos;
     // (growing a buffer frees and allocates: an implicit device synchronisation, first calls only)
-    CK(c->mt_a[k].reserve((size_t)(pairs * nsd)));
-    CK(c->mt_b[k].reserve((size_t)(pairs * nsd)));
-    CK(c->mt_state2.reserve(625));
-    CK(c->mt_words2.reserve((size_t)(2 * n_arrays * nsd)));
-    std::memcpy(c->mt_host, key, sizeof(unsigned) * 624);
-    c->mt_host[624] = (unsigned)pos;
-    cudaStream_t st = c->mt_stream;
-    CK(cudaMemcpyAsync(c->mt_state2.ptr, c->mt_host, sizeof(unsigned) * 625, cudaMemcpyHostToDevice, st));
-    cudaError_t e = launch_mt19937(c->mt_state2.ptr, reinterpret_cast<int*>(c->mt_state2.ptr + 624), n_arrays * nsd,
-                                   c->mt_words2.ptr, c->mt_a[k].ptr, c->mt_b[k].ptr, nsd, st);
-    if (e != cudaSuccess) return fail_cuda(e, "MT19937 launch");
-    CK(cudaMemcpyAsync(c->mt_host + 625, c->mt_state2.ptr, sizeof(unsigned) * 625, cudaMemcpyDeviceToHost, st));
+    if (int rc = mt_queue(c, n_arrays, c->mt_a[k], c->mt_b[k], c->mt_state2, c->mt_words2, c->mt_host.ptr,
+                          c->mt_host.ptr + 625, c->mt_stream.h))
+        return rc;
     *a_dev = c->mt_a[k].ptr;
     *b_dev = c->mt_b[k].ptr;
     c->mt_flip ^= 1;
@@ -1138,10 +1163,10 @@ int nmrfit_ctx_mt19937_end(nmrfit_ctx* c, unsigned* key_out, int* pos_out) {
     if (int rc = check_ctx(c)) return rc;
     if (!c->mt_pending) return fail(NMRFIT_ERR_STATE, "no nmrfit_ctx_mt19937_begin is pending");
     CK(cudaSetDevice(c->device));
-    CK(cudaStreamSynchronize(c->mt_stream));
+    CK(cudaStreamSynchronize(c->mt_stream.h));
     c->mt_pending = 0;
-    if (key_out) std::memcpy(key_out, c->mt_host + 625, sizeof(unsigned) * 624);
-    if (pos_out) *pos_out = (int)c->mt_host[625 + 624];
+    if (key_out) std::memcpy(key_out, c->mt_host.ptr + 625, sizeof(unsigned) * 624);
+    if (pos_out) *pos_out = (int)c->mt_host.ptr[625 + 624];
     return NMRFIT_OK;
 }
 
@@ -1157,7 +1182,7 @@ int nmrfit_ctx_mt19937_shape(nmrfit_ctx* c, long long elements_per_array) {
 int nmrfit_pso_peer_export(nmrfit_ctx* c, int n_ranks, int rank, void* ipc_handle_out, void** base_out) {
     if (int rc = check_ctx(c)) return rc;
     if (n_ranks < 1 || n_ranks > 64 || rank < 0 || rank >= n_ranks) return fail(NMRFIT_ERR_ARG, "bad rank / n_ranks");
-    if (c->peer_win) return fail(NMRFIT_ERR_STATE, "the exchange window of this context already exists");
+    if (c->peer_win.h) return fail(NMRFIT_ERR_STATE, "the exchange window of this context already exists");
     CK(cudaSetDevice(c->device));
     const size_t W = (size_t)c->D + 2;
     c->peer_rec_bytes = (2 * (size_t)n_ranks * c->B * W * sizeof(double) + 15) & ~(size_t)15;
@@ -1165,24 +1190,24 @@ int nmrfit_pso_peer_export(nmrfit_ctx* c, int n_ranks, int rank, void* ipc_handl
     // 2 MiB granule), so that a peer that opens the handle cannot reach any other allocation of this process
     const size_t granule = (size_t)2 << 20;
     const size_t bytes = ((c->peer_rec_bytes + (size_t)n_ranks * c->B * sizeof(long long) + granule - 1) / granule) * granule;
-    CK(cudaMalloc(&c->peer_win, bytes));
-    CK(cudaMemset(c->peer_win, 0, bytes));                 // tokens start at 0; the first real token is (1 << 32)
+    CK(cudaMalloc(&c->peer_win.h, bytes));
+    CK(cudaMemset(c->peer_win.h, 0, bytes));               // tokens start at 0; the first real token is (1 << 32)
     CK(cudaDeviceSynchronize());
     c->peer_ranks = n_ranks;
     c->peer_rank = rank;
     if (ipc_handle_out) {
         static_assert(sizeof(cudaIpcMemHandle_t) == 64, "CUDA IPC handles are 64 bytes");
         cudaIpcMemHandle_t h;
-        CK(cudaIpcGetMemHandle(&h, c->peer_win));
+        CK(cudaIpcGetMemHandle(&h, c->peer_win.h));
         std::memcpy(ipc_handle_out, &h, sizeof(h));
     }
-    if (base_out) *base_out = c->peer_win;
+    if (base_out) *base_out = c->peer_win.h;
     return NMRFIT_OK;
 }
 
 int nmrfit_pso_peer_open(nmrfit_ctx* c, const void* ipc_handles, void* const* local_bases) {
     if (int rc = check_ctx(c)) return rc;
-    if (!c->peer_win) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_peer_export has not been called");
+    if (!c->peer_win.h) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_peer_export has not been called");
     if (!ipc_handles && !local_bases) return fail(NMRFIT_ERR_ARG, "ipc_handles or local_bases must be given");
     CK(cudaSetDevice(c->device));
     const int R = c->peer_ranks;
@@ -1191,14 +1216,14 @@ int nmrfit_pso_peer_open(nmrfit_ctx* c, const void* ipc_handles, void* const* lo
     for (int q = 0; q < R; ++q) {
         void* base = nullptr;
         if (q == c->peer_rank) {
-            base = c->peer_win;
+            base = c->peer_win.h;
         } else if (local_bases && local_bases[q]) {
             base = local_bases[q];                          // another context of this process
         } else {
             cudaIpcMemHandle_t h;
             std::memcpy(&h, (const char*)ipc_handles + (size_t)q * sizeof(h), sizeof(h));
             CK(cudaIpcOpenMemHandle(&base, h, cudaIpcMemLazyEnablePeerAccess));
-            c->peer_opened.push_back(base);
+            c->peer_opened.emplace_back(base);
         }
         recs[q] = (double*)base;
         toks[q] = (long long*)((char*)base + c->peer_rec_bytes);
@@ -1224,54 +1249,28 @@ int exchange_commit(nmrfit_ctx* c, cudaStream_t st) {
 }  // namespace
 
 int nmrfit_pso_commit_peers(nmrfit_ctx* c, void* stream) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
+    if (int rc = require_swarm(c)) return rc;
     CK(cudaSetDevice(c->device));
     return exchange_commit(c, (cudaStream_t)stream);
 }
 
 int nmrfit_pso_step_peers(nmrfit_ctx* c, const double* rp, const double* rg, void* stream) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
-    if ((rp == nullptr) != (rg == nullptr)) return fail(NMRFIT_ERR_ARG, "rp and rg must both be given or both be NULL");
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    SwarmState& s = c->sw;
-    size_t nsd = (size_t)s.B * s.S * s.D;
-    const double *rp_d = nullptr, *rg_d = nullptr;
-    if (int rc = stage(rp, nsd, c->rnd_a, st, &rp_d)) return rc;
-    if (int rc = stage(rg, nsd, c->rnd_b, st, &rg_d)) return rc;
-    c->generation += 1;
-    return swarm_generation(c, true, rp_d, rg_d, 2, st);
+    return pso_generation(c, rp, rg, 2, stream);
 }
 
 int nmrfit_pso_run_peers(nmrfit_ctx* c, int n_generations, const double* rp_all, const double* rg_all, int* n_running,
                          int* timed_out, void* stream) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
-    if ((rp_all == nullptr) != (rg_all == nullptr)) return fail(NMRFIT_ERR_ARG, "rp_all and rg_all must both be given or both be NULL");
+    if (int rc = require_swarm(c)) return rc;
     if (n_generations < 0) return fail(NMRFIT_ERR_ARG, "n_generations must be >= 0");
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
-    SwarmState& s = c->sw;
-    size_t nsd = (size_t)s.B * s.S * s.D;
-    const double *rp_d = nullptr, *rg_d = nullptr;
-    if (n_generations > 0) {
-        if (int rc = stage(rp_all, nsd * n_generations, c->rnd_a, st, &rp_d)) return rc;
-        if (int rc = stage(rg_all, nsd * n_generations, c->rnd_b, st, &rg_d)) return rc;
-    }
-    for (int k = 0; k < n_generations; ++k) {
-        c->generation += 1;
-        if (int rc = swarm_generation(c, true, rp_d ? rp_d + nsd * k : nullptr, rg_d ? rg_d + nsd * k : nullptr, 2, st))
-            return rc;
-    }
-    CK(cudaMemcpyAsync(c->h_flags, s.stop, sizeof(int) * s.B, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(c->h_flags + s.B, c->peer_err.ptr, sizeof(int), cudaMemcpyDeviceToHost, st));
+    const double *rp_d, *rg_d;
+    if (int rc = stage_random(c, n_generations, rp_all, rg_all, "rp_all and rg_all", st, &rp_d, &rg_d)) return rc;
+    if (int rc = queue_generations(c, n_generations, rp_d, rg_d, 2, st)) return rc;
+    if (int rc = queue_stop_flags(c, c->peer_err.ptr, st)) return rc;
     CK(cudaStreamSynchronize(st));
-    int running = 0;
-    for (int b = 0; b < s.B; ++b) running += c->h_flags[b] == 0;
-    if (n_running) *n_running = running;
-    if (timed_out) *timed_out = c->h_flags[s.B];
+    if (n_running) *n_running = running_spectra(c);
+    if (timed_out) *timed_out = c->h_flags.ptr[c->sw.B];
     return NMRFIT_OK;
 }
 
@@ -1308,9 +1307,9 @@ int nmrfit_comm_init_all(nmrfit_ctx* const* ctxs, int n) {
 namespace {
 int comm_stream(nmrfit_ctx* c, cudaStream_t* st) {
     CK(cudaSetDevice(c->device));
-    if (!c->pipe[0]) CK(cudaStreamCreateWithFlags(&c->pipe[0], cudaStreamNonBlocking));
+    CK(ensure_stream(c->pipe[0]));
     CK(cudaStreamSynchronize(0));                          // nmrfit_pso_begin and friends ran on the default stream
-    *st = c->pipe[0];
+    *st = c->pipe[0].h;
     return NMRFIT_OK;
 }
 }  // namespace
@@ -1328,7 +1327,7 @@ int nmrfit_comm_commit(nmrfit_ctx* const* ctxs, int n) {
     }
     for (int r = 0; r < n; ++r) {
         CK(cudaSetDevice(ctxs[r]->device));
-        CK(cudaStreamSynchronize(ctxs[r]->pipe[0]));
+        CK(cudaStreamSynchronize(ctxs[r]->pipe[0].h));
     }
     return NMRFIT_OK;
 }
@@ -1336,20 +1335,17 @@ int nmrfit_comm_commit(nmrfit_ctx* const* ctxs, int n) {
 int nmrfit_comm_run(nmrfit_ctx* const* ctxs, int n, int n_generations, const double* const* rp_all,
                     const double* const* rg_all, int* n_running, int* timed_out) {
     if (!ctxs || n < 1) return fail(NMRFIT_ERR_ARG, "ctxs must hold at least one context");
-    if ((rp_all == nullptr) != (rg_all == nullptr)) return fail(NMRFIT_ERR_ARG, "rp_all and rg_all must both be given or both be NULL");
     if (n_generations < 0) return fail(NMRFIT_ERR_ARG, "n_generations must be >= 0");
-    std::vector<const double*> rp_d(n, nullptr), rg_d(n, nullptr);
+    std::vector<const double*> rp_d(n), rg_d(n);
     std::vector<cudaStream_t> sts(n);
     for (int r = 0; r < n; ++r) {
         nmrfit_ctx* c = ctxs[r];
         if (int rc = check_ctx(c)) return rc;
         if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called on every context");
         if (int rc = comm_stream(c, &sts[r])) return rc;
-        const size_t nsd = (size_t)c->sw.B * c->sw.S * c->sw.D;
-        if (rp_all && n_generations > 0) {
-            if (int rc = stage(rp_all[r], nsd * n_generations, c->rnd_a, sts[r], &rp_d[r])) return rc;
-            if (int rc = stage(rg_all[r], nsd * n_generations, c->rnd_b, sts[r], &rg_d[r])) return rc;
-        }
+        if (int rc = stage_random(c, n_generations, rp_all ? rp_all[r] : nullptr, rg_all ? rg_all[r] : nullptr,
+                                  "rp_all and rg_all", sts[r], &rp_d[r], &rg_d[r]))
+            return rc;
     }
     // generation by generation over the contexts: every rank's kernels are queued before the host waits for anything
     for (int k = 0; k < n_generations; ++k) {
@@ -1357,25 +1353,22 @@ int nmrfit_comm_run(nmrfit_ctx* const* ctxs, int n, int n_generations, const dou
             nmrfit_ctx* c = ctxs[r];
             CK(cudaSetDevice(c->device));
             const size_t nsd = (size_t)c->sw.B * c->sw.S * c->sw.D;
-            c->generation += 1;
-            if (int rc = swarm_generation(c, true, rp_d[r] ? rp_d[r] + nsd * k : nullptr, rg_d[r] ? rg_d[r] + nsd * k : nullptr,
-                                          2, sts[r]))
+            if (int rc = queue_generations(c, 1, rp_d[r] ? rp_d[r] + nsd * k : nullptr, rg_d[r] ? rg_d[r] + nsd * k : nullptr,
+                                           2, sts[r]))
                 return rc;
         }
+    }
+    for (int r = 0; r < n; ++r) {
+        CK(cudaSetDevice(ctxs[r]->device));
+        if (int rc = queue_stop_flags(ctxs[r], ctxs[r]->peer_err.ptr, sts[r])) return rc;
     }
     int running = 0, lost = 0;
     for (int r = 0; r < n; ++r) {
         nmrfit_ctx* c = ctxs[r];
         CK(cudaSetDevice(c->device));
-        CK(cudaMemcpyAsync(c->h_flags, c->sw.stop, sizeof(int) * c->sw.B, cudaMemcpyDeviceToHost, sts[r]));
-        CK(cudaMemcpyAsync(c->h_flags + c->sw.B, c->peer_err.ptr, sizeof(int), cudaMemcpyDeviceToHost, sts[r]));
-    }
-    for (int r = 0; r < n; ++r) {
-        nmrfit_ctx* c = ctxs[r];
-        CK(cudaSetDevice(c->device));
         CK(cudaStreamSynchronize(sts[r]));
-        lost |= c->h_flags[c->sw.B];
-        if (r == 0) for (int b = 0; b < c->sw.B; ++b) running += c->h_flags[b] == 0;     // identical on every rank
+        lost |= c->h_flags.ptr[c->sw.B];
+        if (r == 0) running = running_spectra(c);          // identical on every rank
     }
     if (n_running) *n_running = running;
     if (timed_out) *timed_out = lost;
@@ -1400,16 +1393,14 @@ int nmrfit_pso_peer_error(nmrfit_ctx* c, int* timed_out) {
 }
 
 int nmrfit_pso_record(nmrfit_ctx* c, double** rec_dev, int* n_doubles) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
+    if (int rc = require_swarm(c)) return rc;
     if (rec_dev) *rec_dev = c->sw.rec;
     if (n_doubles) *n_doubles = c->B * (c->D + 2);
     return NMRFIT_OK;
 }
 
 int nmrfit_pso_commit(nmrfit_ctx* c, const double* recs_dev, int n_ranks, void* stream) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
+    if (int rc = require_swarm(c)) return rc;
     if (recs_dev && n_ranks < 1) return fail(NMRFIT_ERR_ARG, "n_ranks must be >= 1");
     CK(cudaSetDevice(c->device));
     const double* recs = recs_dev ? recs_dev : c->sw.rec;
@@ -1421,18 +1412,12 @@ int nmrfit_pso_commit(nmrfit_ctx* c, const double* recs_dev, int n_ranks, void* 
 
 int nmrfit_pso_run(nmrfit_ctx* c, int n_generations, const double* rp_all, const double* rg_all, int* n_running,
                    void* stream) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
-    if ((rp_all == nullptr) != (rg_all == nullptr)) return fail(NMRFIT_ERR_ARG, "rp_all and rg_all must both be given or both be NULL");
+    if (int rc = require_swarm(c)) return rc;
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
-    SwarmState& s = c->sw;
-    size_t nsd = (size_t)s.B * s.S * s.D;
-    const double *rp_d = nullptr, *rg_d = nullptr;
-    if (n_generations > 0) {
-        if (int rc = stage(rp_all, nsd * n_generations, c->rnd_a, st, &rp_d)) return rc;
-        if (int rc = stage(rg_all, nsd * n_generations, c->rnd_b, st, &rg_d)) return rc;
-    }
+    const SwarmState& s = c->sw;
+    const double *rp_d, *rg_d;
+    if (int rc = stage_random(c, n_generations, rp_all, rg_all, "rp_all and rg_all", st, &rp_d, &rg_d)) return rc;
     FusedArgs fa;
     FusedPlan plan{};
     if (n_generations > 0)
@@ -1447,27 +1432,18 @@ int nmrfit_pso_run(nmrfit_ctx* c, int n_generations, const double* rp_all, const
         c->fused_launches += 1;
         n_generations = 0;
     }
-    for (int k = 0; k < n_generations; ++k) {
-        c->generation += 1;
-        if (int rc = swarm_generation(c, true, rp_d ? rp_d + nsd * k : nullptr, rg_d ? rg_d + nsd * k : nullptr, 1, st))
-            return rc;
-    }
-    CK(cudaMemcpyAsync(c->h_flags, s.stop, sizeof(int) * s.B, cudaMemcpyDeviceToHost, st));
-    c->h_flags[s.B] = 0;
-    if (c->ferror.ptr) CK(cudaMemcpyAsync(c->h_flags + s.B, c->ferror.ptr, sizeof(int), cudaMemcpyDeviceToHost, st));
+    if (int rc = queue_generations(c, n_generations, rp_d, rg_d, 1, st)) return rc;
+    if (int rc = queue_stop_flags(c, c->ferror.ptr, st)) return rc;
     CK(cudaStreamSynchronize(st));
-    if (c->h_flags[s.B])
+    if (c->h_flags.ptr[s.B])
         return fail(NMRFIT_ERR_STATE, "fused swarm kernel: the barrier among the CTAs of a spectrum timed out (a CTA died); "
                                       "the swarm state is undefined");
-    int running = 0;
-    for (int b = 0; b < s.B; ++b) running += c->h_flags[b] == 0;
-    if (n_running) *n_running = running;
+    if (n_running) *n_running = running_spectra(c);
     return NMRFIT_OK;
 }
 
 int nmrfit_pso_get_best(nmrfit_ctx* c, double* x_best, double* f_best, int* generations, int* stop_reason) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
+    if (int rc = require_swarm(c)) return rc;
     CK(cudaSetDevice(c->device));
     CK(cudaDeviceSynchronize());
     const SwarmState& s = c->sw;
@@ -1479,8 +1455,7 @@ int nmrfit_pso_get_best(nmrfit_ctx* c, double* x_best, double* f_best, int* gene
 }
 
 int nmrfit_pso_get_state(nmrfit_ctx* c, double* x, double* v, double* p, double* fx, double* fp) {
-    if (int rc = check_ctx(c)) return rc;
-    if (!c->swarm) return fail(NMRFIT_ERR_STATE, "nmrfit_pso_begin has not been called");
+    if (int rc = require_swarm(c)) return rc;
     CK(cudaSetDevice(c->device));
     CK(cudaDeviceSynchronize());
     const SwarmState& s = c->sw;
@@ -1647,26 +1622,21 @@ int nmrfit_phase_create(nmrfit_phase** out, int device, int n_spectra, int n_poi
     CK(cudaGetDeviceCount(&ndev));
     if (device < 0 || device >= ndev) return fail(NMRFIT_ERR_ARG, "no such CUDA device");
     CK(cudaSetDevice(device));
-    nmrfit_phase* h = new (std::nothrow) nmrfit_phase();
+    std::unique_ptr<nmrfit_phase> h(new (std::nothrow) nmrfit_phase());
     if (!h) return fail(NMRFIT_ERR_NOMEM, "out of host memory");
     h->device = device; h->B = n_spectra; h->N = n_points;
     const size_t n = (size_t)n_spectra * n_points;
-    cudaError_t e = h->u.reserve(n);
-    if (e == cudaSuccess) e = h->v.reserve(n);
-    if (e == cudaSuccess) e = cudaMemcpy(h->u.ptr, u, sizeof(double) * n, cudaMemcpyDefault);
-    if (e == cudaSuccess) e = cudaMemcpy(h->v.ptr, v, sizeof(double) * n, cudaMemcpyDefault);
-    if (e != cudaSuccess) {
-        nmrfit_phase_destroy(h);
-        return fail_cuda(e, "phase allocation");
-    }
-    *out = h;
+    CK(h->u.reserve(n));
+    CK(h->v.reserve(n));
+    CK(cudaMemcpy(h->u.ptr, u, sizeof(double) * n, cudaMemcpyDefault));
+    CK(cudaMemcpy(h->v.ptr, v, sizeof(double) * n, cudaMemcpyDefault));
+    *out = h.release();
     return NMRFIT_OK;
 }
 
 void nmrfit_phase_destroy(nmrfit_phase* h) {
     if (!h) return;
     cudaSetDevice(h->device);
-    h->u.release(); h->v.release(); h->cands.release(); h->out.release(); h->ok.release();
     delete h;
 }
 
@@ -1724,42 +1694,34 @@ int nmrfit_peaks_create(nmrfit_peaks** out, int device, int n_spectra, int n_poi
     CK(cudaGetDeviceCount(&ndev));
     if (device < 0 || device >= ndev) return fail(NMRFIT_ERR_ARG, "no such CUDA device");
     CK(cudaSetDevice(device));
-    nmrfit_peaks* h = new (std::nothrow) nmrfit_peaks();
+    std::unique_ptr<nmrfit_peaks> h(new (std::nothrow) nmrfit_peaks());
     if (!h) return fail(NMRFIT_ERR_NOMEM, "out of host memory");
     h->device = device; h->B = n_spectra; h->N = n_points; h->upsample = upsample; h->max_peaks = max_peaks;
     h->M = (long long)n_points * upsample;
     h->nblk = (int)((h->M + 1023) / 1024);
     const size_t BN = (size_t)n_spectra * n_points, BM = (size_t)n_spectra * h->M, BK = (size_t)n_spectra * max_peaks;
-    cudaError_t e = h->w.reserve(BN);
-    if (e == cudaSuccess) e = h->u.reserve(BN);
-    if (e == cudaSuccess) e = h->uu.reserve(BM);
-    if (e == cudaSuccess) e = h->us.reserve(BM);
-    if (e == cudaSuccess) e = h->bmax.reserve((size_t)n_spectra * h->nblk);
-    if (e == cudaSuccess) e = h->base.reserve(n_spectra);
-    if (e == cudaSuccess) e = h->uu_at.reserve(BK);
-    if (e == cudaSuccess) e = h->pk_h.reserve(BK);
-    if (e == cudaSuccess) e = h->sg.reserve(121);
-    if (e == cudaSuccess) e = h->maxima.reserve(BK);
-    if (e == cudaSuccess) e = h->pk_i.reserve(BK);
-    if (e == cudaSuccess) e = h->cross.reserve(2 * BK);
-    if (e == cudaSuccess) e = h->n_maxima.reserve(n_spectra);
-    if (e == cudaSuccess) e = h->n_pk.reserve(n_spectra);
-    if (e == cudaSuccess) e = h->out.reserve(BK * peaks_out_bytes());
-    if (e != cudaSuccess) {
-        nmrfit_peaks_destroy(h);
-        return fail_cuda(e, "peak-selector allocation");
-    }
-    *out = h;
+    CK(h->w.reserve(BN));
+    CK(h->u.reserve(BN));
+    CK(h->uu.reserve(BM));
+    CK(h->us.reserve(BM));
+    CK(h->bmax.reserve((size_t)n_spectra * h->nblk));
+    CK(h->base.reserve(n_spectra));
+    CK(h->uu_at.reserve(BK));
+    CK(h->pk_h.reserve(BK));
+    CK(h->sg.reserve(121));
+    CK(h->maxima.reserve(BK));
+    CK(h->pk_i.reserve(BK));
+    CK(h->cross.reserve(2 * BK));
+    CK(h->n_maxima.reserve(n_spectra));
+    CK(h->n_pk.reserve(n_spectra));
+    CK(h->out.reserve(BK * peaks_out_bytes()));
+    *out = h.release();
     return NMRFIT_OK;
 }
 
 void nmrfit_peaks_destroy(nmrfit_peaks* h) {
     if (!h) return;
     cudaSetDevice(h->device);
-    for (DevBuf<double>* b : {&h->w, &h->u, &h->uu, &h->us, &h->bmax, &h->base, &h->uu_at, &h->pk_h, &h->sg, &h->probe_out})
-        b->release();
-    for (DevBuf<long long>* b : {&h->maxima, &h->pk_i, &h->cross, &h->probe_idx}) b->release();
-    h->n_maxima.release(); h->n_pk.release(); h->out.release();
     delete h;
 }
 
