@@ -109,6 +109,25 @@ int nmrfit_ctx_normal_equations(nmrfit_ctx* ctx, const double* x, double* H, dou
  * NMRFIT_ERR_ARG unless 1 <= n_peaks <= 64 and n_points >= 1. */
 int nmrfit_normal_eq_plan(int n_points, int n_peaks, int* out);
 
+/* Correlated noise (DESIGN K14), from the spectra and weights the context holds, at one x [n_spectra][D] per spectrum,
+ * with res_i and A_i as in nmrfit_ctx_normal_equations and L = max_lag:
+ *   nmrfit_ctx_residual_acf:    r_out [n_spectra][L+1],  r_k = sum_{i=0}^{N-1-k} res_i res_{i+k}  (r_0 = ssr[1]);
+ *   nmrfit_ctx_normal_m_lagged: M_out [n_spectra][D][D] = sum_i sum_{|k| <= L, 0 <= i+k < N} rho_|k| a_i^T a_{i+k},
+ *                               a_i = w_i^2 A_i, from rho [n_spectra][L+1]  (L = 0, rho = 1: the M of K12).
+ * Host or device pointers; they return when the outputs are written.  Sums are in a fixed order that depends on
+ * n_points, n_peaks and L only: bit-reproducible, the same alone or in a batch; M_out is exactly symmetric.
+ * NMRFIT_ERR_ARG for NULL pointers, more than 64 peaks, max_lag < 0, max_lag >= n_points, max_lag above the cap of
+ * nmrfit_lagged_plan, or a non-finite rho. */
+int nmrfit_ctx_residual_acf(nmrfit_ctx* ctx, const double* x, int max_lag, double* r_out, void* stream);
+int nmrfit_ctx_normal_m_lagged(nmrfit_ctx* ctx, const double* x, const double* rho, int max_lag, double* M_out,
+                               void* stream);
+/* The launch plan of both lagged passes (host only, no CUDA call).  out[14] = point groups per CTA, task slices per
+ * chunk, 4x4 blocks of the upper triangle (tasks), tasks per slice, threads per CTA, points per staged tile, points per
+ * chunk, chunks, dynamic shared memory (bytes), scratch doubles per spectrum (M pass); the largest max_lag at n_peaks;
+ * points per chunk, chunks and scratch doubles per spectrum of the residual pass.  NMRFIT_ERR_ARG unless
+ * 1 <= n_peaks <= 64, n_points >= 1 and 0 <= max_lag <= the cap (query max_lag = 0 to learn the cap). */
+int nmrfit_lagged_plan(int n_points, int n_peaks, int max_lag, int* out);
+
 /* How nmrfit_ctx_refine left a spectrum. */
 #define NMRFIT_REFINE_CONVERGED 1   /* an accepted step was at most xtol of every parameter's diagonal noise scale */
 #define NMRFIT_REFINE_STALLED 2     /* the damping passed 1e16 without a descent step: a numerical minimum */

@@ -55,6 +55,9 @@ SIGNATURES = {
     'nmrfit_ctx_normal_equations': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     'nmrfit_normal_eq_plan': (_i, [_i, _i, c_int_p]),
     'nmrfit_ctx_refine': (_i, [_vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
+    'nmrfit_ctx_residual_acf': (_i, [_vp, _vp, _i, _vp, _vp]),
+    'nmrfit_ctx_normal_m_lagged': (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
+    'nmrfit_lagged_plan': (_i, [_i, _i, _i, c_int_p]),
     'nmrfit_ctx_set_algorithm': (_i, [_vp, _i]),
     'nmrfit_ctx_get_algorithm': (_i, [_vp, _i, c_int_p]),
     'nmrfit_ctx_set_tuning': (_i, [_vp, _i, _i, _i, _i]),
@@ -176,6 +179,49 @@ def normal_equations_plan(n_points, n_peaks):
     out = (ctypes.c_int * len(NORMAL_EQ_PLAN_KEYS))()
     check(lib().nmrfit_normal_eq_plan(int(n_points), int(n_peaks), out))
     return dict(zip(NORMAL_EQ_PLAN_KEYS, out))
+
+
+LAGGED_PLAN_KEYS = ('point_groups', 'slices', 'tasks', 'tasks_per_slice', 'threads', 'tile_points', 'chunk_points',
+                    'n_chunks', 'smem_bytes', 'scratch_doubles', 'max_lag', 'acf_chunk_points', 'acf_n_chunks',
+                    'acf_scratch_doubles')
+
+
+def lagged_plan(n_points, n_peaks, max_lag=0):
+    """Launch plan of ``Context.residual_acf`` and ``Context.normal_m_lagged`` (host only, no CUDA call): a dict of
+    ``LAGGED_PLAN_KEYS``; ``max_lag`` is the largest lag the passes take at ``n_peaks``.  Scratch sizes are per
+    spectrum."""
+    out = (ctypes.c_int * len(LAGGED_PLAN_KEYS))()
+    check(lib().nmrfit_lagged_plan(int(n_points), int(n_peaks), int(max_lag), out))
+    return dict(zip(LAGGED_PLAN_KEYS, out))
+
+
+def check_lag(max_lag, N, P):
+    """The lag checks of the lagged passes (the library makes them again): returns int(max_lag), else ValueError."""
+    if P > 64:
+        raise ValueError('the lagged passes support at most 64 peaks (D <= 196), got %d' % P)
+    if isinstance(max_lag, bool) or int(max_lag) != max_lag:
+        raise ValueError('max_lag must be an integer, got %r' % (max_lag,))
+    L = int(max_lag)
+    if L < 0:
+        raise ValueError('max_lag must be >= 0')
+    if L >= N:
+        raise ValueError('max_lag must be below the number of points, %d' % N)
+    cap = lagged_plan(N, P)['max_lag']
+    if L > cap:
+        raise ValueError('max_lag %d is above the cap of %d at %d peaks' % (L, cap, P))
+    return L
+
+
+def check_rho(rho, B, N, P):
+    """``rho`` [L+1] (every spectrum) or [B, L+1] as a fresh C-contiguous [B, L+1] float64 array, with its lag
+    checked and every value finite.  ValueError otherwise."""
+    rho = np.asarray(rho, dtype=np.float64)
+    if rho.ndim not in (1, 2) or rho.shape[-1] < 1 or (rho.ndim == 2 and rho.shape[0] != B):
+        raise ValueError('rho must have shape (L+1,) or (%d, L+1), got %s' % (B, rho.shape))
+    check_lag(rho.shape[-1] - 1, N, P)
+    if not np.all(np.isfinite(rho)):
+        raise ValueError('every rho must be finite')
+    return np.array(np.broadcast_to(rho, (B, rho.shape[-1])), dtype=np.float64, order='C')
 
 
 def check_refine_args(x, lb, ub, max_iter, xtol, B, N, P):
@@ -302,6 +348,30 @@ class Context(_Handle):
         check(lib().nmrfit_ctx_refine(self._h, ptr(x), ptr(lb), ptr(ub), int(max_iter), float(xtol), ptr(f),
                                       ptr(passes), ptr(accepted), ptr(status), ptr(stream)))
         return x, f, passes, accepted, status
+
+    def residual_acf(self, x, max_lag, stream=None):
+        """Residual autocorrelation at ``x`` [B, D] over the spectra the context holds: returns ``r`` [B, L+1] on the
+        host, r_k = sum_{i < N-k} res_i res_{i+k} (the biased form; r_0 is ``normal_equations``' ssr[:, 1]).
+        ``max_lag`` = L, 0 <= L < N and at most ``lagged_plan(N, P)['max_lag']``."""
+        L = check_lag(max_lag, self.N, self.P)
+        x = as_f64(x)
+        if x.shape != (self.B, self.D):
+            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        r = np.empty((self.B, L + 1))
+        check(lib().nmrfit_ctx_residual_acf(self._h, ptr(x), L, ptr(r), ptr(stream)))
+        return r
+
+    def normal_m_lagged(self, x, rho, stream=None):
+        """Lag-weighted M at ``x`` [B, D]: returns [B, D, D] = sum_i sum_{|k| <= L} rho_|k| a_i^T a_{i+k}, a_i = w_i^2 A_i
+        (rows outside the spectrum are zero), from ``rho`` [L+1] or [B, L+1].  With rho = [1] it is ``normal_equations``'
+        M.  The result is exactly symmetric."""
+        rho = check_rho(rho, self.B, self.N, self.P)
+        x = as_f64(x)
+        if x.shape != (self.B, self.D):
+            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        M = np.empty((self.B, self.D, self.D))
+        check(lib().nmrfit_ctx_normal_m_lagged(self._h, ptr(x), ptr(rho), rho.shape[1] - 1, ptr(M), ptr(stream)))
+        return M
 
     def set_algorithm(self, algorithm=ALGO_AUTO):
         """ALGO_AUTO (default), ALGO_GENERAL (any axis) or ALGO_UNIFORM (require the uniform-axis kernel)."""

@@ -140,6 +140,7 @@ struct nmrfit_ctx {
     double peer_timeout_ms = 20000.0;  // wall-time bound of a wait for the peers' tokens
     DevBuf<double> wscratch, wbounds;  // batched weights: sweep scratch [B][N], windows + values
     DevBuf<double> ne_x, ne_part, ne_out;   // normal equations: positions, chunk partials, H | M | g | ssr
+    DevBuf<double> lg_rho, lg_part, lg_out;   // lagged passes: rho, chunk partials, r or M_rho
     DevBuf<double> rf_x, rf_cur;       // refinement: current, trial, lb, ub [4][B][D]; H | g | s at the current point
     DevBuf<RefineState> rf_state;
     DevBuf<int> rf_active;             // spectra still running after the last polled step
@@ -703,6 +704,84 @@ int nmrfit_ctx_normal_equations(nmrfit_ctx* c, const double* x, double* H, doubl
             CK(cudaMemcpy2DAsync(dst[k], sizeof(double) * lens[k], c->ne_out.ptr + offs[k], sizeof(double) * per,
                                  sizeof(double) * lens[k], B, cudaMemcpyDefault, st));
     CK(cudaStreamSynchronize(st));                         // x and the outputs may be pageable host memory
+    return NMRFIT_OK;
+}
+
+// the checks of both lagged passes past the NULL pointers; fills the plan
+static int lagged_check(const nmrfit_ctx* c, int max_lag, LaggedPlan* plan) {
+    if (c->P > 64)
+        return fail(NMRFIT_ERR_ARG, "the lagged passes support at most 64 peaks (D <= 196), the context has " +
+                                        std::to_string(c->P));
+    if (max_lag < 0) return fail(NMRFIT_ERR_ARG, "max_lag must be >= 0");
+    if (max_lag >= c->N)
+        return fail(NMRFIT_ERR_ARG, "max_lag must be below the number of points, " + std::to_string(c->N));
+    *plan = lagged_plan(c->N, c->P, max_lag);
+    if (max_lag > plan->max_lag)
+        return fail(NMRFIT_ERR_ARG, "max_lag " + std::to_string(max_lag) + " is above the cap of " +
+                                        std::to_string(plan->max_lag) + " at " + std::to_string(c->P) + " peaks");
+    return NMRFIT_OK;
+}
+
+int nmrfit_ctx_residual_acf(nmrfit_ctx* c, const double* x, int max_lag, double* r_out, void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !r_out) return fail(NMRFIT_ERR_ARG, "x and r_out must be non-NULL");
+    LaggedPlan p;
+    if (int r = lagged_check(c, max_lag, &p)) return r;
+    if (int r = require_spectra(c, "its residual autocorrelation is computed")) return r;
+    CK(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t B = (size_t)c->B, K = (size_t)max_lag + 1;
+    const double* xd = nullptr;
+    if (int r = stage(x, B * c->D, c->ne_x, st, &xd)) return r;
+    CK(c->lg_part.reserve(residual_acf_scratch_doubles(p, c->B)));
+    CK(c->lg_out.reserve(B * K));
+    cudaError_t e = launch_residual_acf(c->spec.ptr, xd, p, c->B, c->lg_part.ptr, c->lg_out.ptr, st);
+    if (e != cudaSuccess) return fail_cuda(e, "residual autocorrelation launch");
+    CK(cudaMemcpyAsync(r_out, c->lg_out.ptr, sizeof(double) * B * K, cudaMemcpyDefault, st));
+    CK(cudaStreamSynchronize(st));                         // x and r_out may be pageable host memory
+    return NMRFIT_OK;
+}
+
+int nmrfit_ctx_normal_m_lagged(nmrfit_ctx* c, const double* x, const double* rho, int max_lag, double* M_out,
+                               void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !rho || !M_out) return fail(NMRFIT_ERR_ARG, "x, rho and M_out must be non-NULL");
+    LaggedPlan p;
+    if (int r = lagged_check(c, max_lag, &p)) return r;
+    CK(cudaSetDevice(c->device));
+    const size_t B = (size_t)c->B, K = (size_t)max_lag + 1, D = (size_t)c->D;
+    std::vector<double> h(B * K);
+    CK(cudaMemcpy(h.data(), rho, sizeof(double) * B * K, cudaMemcpyDefault));
+    for (double v : h)
+        if (!std::isfinite(v)) return fail(NMRFIT_ERR_ARG, "every rho must be finite");
+    if (int r = require_spectra(c, "its lagged M is computed")) return r;
+    cudaStream_t st = (cudaStream_t)stream;
+    const double* xd = nullptr;
+    if (int r = stage(x, B * D, c->ne_x, st, &xd)) return r;
+    CK(c->lg_rho.reserve(B * K));
+    CK(cudaMemcpyAsync(c->lg_rho.ptr, h.data(), sizeof(double) * B * K, cudaMemcpyHostToDevice, st));
+    CK(c->lg_part.reserve(lagged_m_scratch_doubles(p, c->B)));
+    CK(c->lg_out.reserve(B * D * D));
+    cudaError_t e = launch_lagged_m(c->spec.ptr, xd, c->lg_rho.ptr, p, c->B, c->lg_part.ptr, c->lg_out.ptr, st);
+    if (e != cudaSuccess) return fail_cuda(e, "lagged M launch");
+    CK(cudaMemcpyAsync(M_out, c->lg_out.ptr, sizeof(double) * B * D * D, cudaMemcpyDefault, st));
+    CK(cudaStreamSynchronize(st));                         // x, rho and M_out may be pageable host memory
+    return NMRFIT_OK;
+}
+
+int nmrfit_lagged_plan(int n_points, int n_peaks, int max_lag, int* out) {
+    if (!out) return fail(NMRFIT_ERR_ARG, "out is NULL");
+    if (n_peaks < 1 || n_peaks > 64) return fail(NMRFIT_ERR_ARG, "n_peaks must be 1..64");
+    if (n_points < 1) return fail(NMRFIT_ERR_ARG, "n_points must be >= 1");
+    if (max_lag < 0) return fail(NMRFIT_ERR_ARG, "max_lag must be >= 0");
+    const LaggedPlan p = lagged_plan(n_points, n_peaks, max_lag);
+    if (max_lag > p.max_lag)
+        return fail(NMRFIT_ERR_ARG, "max_lag " + std::to_string(max_lag) + " is above the cap of " +
+                                        std::to_string(p.max_lag) + " at " + std::to_string(n_peaks) + " peaks");
+    const int v[14] = {p.ng, p.slices, p.tasks, p.tasks_per_slice, p.threads, p.tp, p.chunk, p.n_chunks, (int)p.smem,
+                       (int)lagged_m_scratch_doubles(p, 1), p.max_lag, p.acf_chunk, p.acf_n_chunks,
+                       (int)residual_acf_scratch_doubles(p, 1)};
+    for (int k = 0; k < 14; ++k) out[k] = v[k];
     return NMRFIT_OK;
 }
 

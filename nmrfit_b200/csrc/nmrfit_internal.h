@@ -227,6 +227,28 @@ size_t normal_eq_scratch_doubles(const NormalEqPlan& p, int B);
 cudaError_t launch_normal_eq(const double* spec, const double* x, const NormalEqPlan& p, int B, double* part,
                              double* out, cudaStream_t st);
 
+// ---- K14 residual autocorrelation and lag-weighted M (lagged.cu) --------------------
+// Tiling of both passes: a function of N, P and the largest lag L only.
+struct LaggedPlan {
+    int N, P, L;
+    int nb, ep, tasks;          // 4x4 blocks per edge of M, padded row length, blocks of its upper triangle
+    int ng, slices, tasks_per_slice, threads;   // as NormalEqPlan
+    int tp, chunk, n_chunks;    // points per tile (staged with L rows of halo on each side), per CTA, chunks
+    size_t smem;                // dynamic shared memory of the M partial kernel, bytes
+    int max_lag;                // largest L the shared memory holds at this P
+    int acf_chunk, acf_n_chunks, acf_threads, acf_segments;   // residual autocorrelation pass: points per CTA,
+    size_t acf_smem;                                          // chunks, CTA size, segments of a chunk per lag
+};
+LaggedPlan lagged_plan(int N, int P, int L);
+size_t lagged_m_scratch_doubles(const LaggedPlan& p, int B);
+size_t residual_acf_scratch_doubles(const LaggedPlan& p, int B);
+// x [B][D] -> r [B][L+1], r_k = sum_{i < N-k} res_i res_{i+k}; `part` holds residual_acf_scratch_doubles doubles
+cudaError_t launch_residual_acf(const double* spec, const double* x, const LaggedPlan& p, int B, double* part,
+                                double* r, cudaStream_t st);
+// x [B][D], rho [B][L+1] -> M [B][D][D] = sum_i sum_{|k| <= L} rho_|k| a_i^T a_{i+k}, a_i = w_i^2 A_i
+cudaError_t launch_lagged_m(const double* spec, const double* x, const double* rho, const LaggedPlan& p, int B,
+                            double* part, double* M, cudaStream_t st);
+
 // ---- K13 bounded Levenberg-Marquardt refinement on K12 (refine.cu) --------------------
 #define NMRFIT_REFINE_RUNNING 0
 struct RefineState {

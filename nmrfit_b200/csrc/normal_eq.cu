@@ -14,17 +14,13 @@
 #include <cuda_runtime.h>
 #include <algorithm>
 #include "nmrfit_internal.h"
+#include "normal_eq_rows.cuh"
 
 namespace nmrfit {
 
 namespace {
 
 constexpr int RB = 4;                  // register block edge
-constexpr double kSqrtLn2 = 0.83255461115769775635;
-constexpr double kSqrtLn2OverPi = 0.46971863934982566;   // sqrt(ln 2 / pi)
-constexpr double kInvPi = 0.31830988618379067154;
-
-struct PeakK { double loc, gam, area, kL, kG, cL, cG, igam; };
 
 // upper-triangle block q of an nb x nb block grid -> (row block, column block), row-major over bi <= bj
 __device__ __forceinline__ void tri_block(int q, int nb, int* bi, int* bj) {
@@ -53,12 +49,7 @@ __global__ void __launch_bounds__(512) normal_eq_partial_kernel(const double* __
     const double p0 = x[0], p1 = x[1], r = x[2], yoff = x[3];
     for (int k = tid; k < P; k += nt) {
         PeakK c;
-        c.gam = x[4 + 3 * k]; c.loc = x[5 + 3 * k]; c.area = x[6 + 3 * k];
-        c.igam = 1.0 / c.gam;
-        c.kL = 2.0 * c.igam;
-        c.kG = 2.0 * kSqrtLn2 * c.igam;
-        c.cL = c.kL * kInvPi;
-        c.cG = c.kL * kSqrtLn2OverPi;
+        ne_peak_constants(x, k, c);
         pk[k] = c;
     }
     for (int idx = tid; idx < 2 * TP * EP; idx += nt) rows[idx] = 0.0;    // padding columns stay zero
@@ -95,21 +86,10 @@ __global__ void __launch_bounds__(512) normal_eq_partial_kernel(const double* __
             }
             const double wt = sw[3 * N + pt], wt2 = wt * wt;
             const PeakK c = pk[k];
-            const double d = sw[pt] - c.loc;
-            const double t = d * c.kL, s = d * c.kG;
-            const double q = fma(t, t, 1.0);
-            const double iq = 1.0 / q;
-            const double L = c.cL * iq;
-            const double G = c.cG * exp(-(s * s));
-            const double mix = fma(r, L, (1.0 - r) * G);
-            const double dl_loc = L * (2.0 * t) * iq * c.kL, dg_loc = G * (2.0 * s) * c.kG;
-            const double dl_gam = L * c.igam * (fma(t, t, -1.0) * iq), dg_gam = G * c.igam * fma(2.0 * s, s, -1.0);
-            const double a_gam = -c.area * fma(r, dl_gam, (1.0 - r) * dg_gam);
-            const double a_loc = -c.area * fma(r, dl_loc, (1.0 - r) * dg_loc);
-            row[0] = wt * a_gam; row[1] = wt * a_loc; row[2] = wt * -mix;
-            rowm[0] = wt2 * a_gam; rowm[1] = wt2 * a_loc; rowm[2] = wt2 * -mix;
-            cfit[idx] = fma(c.area, mix, yoff);
-            cdr[idx] = c.area * (L - G);
+            ne_peak_terms(c, sw[pt], r, yoff, [&](double a_gam, double a_loc, double a_area) {
+                row[0] = wt * a_gam; row[1] = wt * a_loc; row[2] = wt * a_area;
+                rowm[0] = wt2 * a_gam; rowm[1] = wt2 * a_loc; rowm[2] = wt2 * a_area;
+            }, &cfit[idx], &cdr[idx]);
         }
         __syncthreads();
         // per point: phase, residual, the four global columns; peaks summed in index order
@@ -126,12 +106,9 @@ __global__ void __launch_bounds__(512) normal_eq_partial_kernel(const double* __
                 fit += cfit[i * P + k];
                 dr += cdr[i * P + k];
             }
-            double sn, cs;
-            sincos(p0 + (p1 * (double)pt) / rN, &sn, &cs);
-            const double u = sw[N + pt], v = sw[2 * N + pt];
-            const double vd = fma(u, cs, -(v * sn)), id = fma(u, sn, v * cs);
-            const double a[4] = {-id, -id * ((double)pt / rN), -dr, -(double)P};
-            const double wt = sw[3 * N + pt], wt2 = wt * wt, res = vd - fit;
+            double a[4], wt, res;
+            ne_point_terms(p0, p1, pt, N, rN, sw, fit, dr, P, a, &wt, &res);
+            const double wt2 = wt * wt;
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 rh[j] = wt * a[j];

@@ -107,6 +107,20 @@ def multiplet(n_points, n_peaks=6, seed=0, noise=1e-4, jitter=None):
     return data, np.array(true)
 
 
+def processed_noise(n_points, sigma, broadening=3.0, zero_fill=2, n_realisations=1, seed=0):
+    """Noise of a processed spectrum, for ``u`` and ``v``: white complex noise on an FID of n_points / zero_fill
+    samples, exponential line broadening of ``broadening`` spectral points (the FWHM it gives a Lorentzian line;
+    0 for none), zero-filled to n_points, FFT.  Scaled so that the real part has standard deviation ``sigma``.
+    Its real part then has the autocorrelation rho_k ~ b^2 / (b^2 + k^2) at b = broadening.  Returns
+    ``(noise_u, noise_v)``, each [n_realisations, n_points], from ``default_rng(seed)``."""
+    rng = np.random.default_rng(seed)
+    n_fid = n_points // zero_fill
+    window = np.exp(-np.pi * broadening * np.arange(n_fid) / n_points)
+    fid = (rng.standard_normal((n_realisations, n_fid)) + 1j * rng.standard_normal((n_realisations, n_fid))) * window
+    spec = np.fft.fft(fid, n=n_points, axis=1) * (sigma / np.sqrt(np.sum(window * window)))
+    return spec.real, spec.imag
+
+
 def particles(lower, upper, n_particles, seed=7):
     """Objective-parity particle positions: lb + U(0,1)*(ub-lb), default_rng(seed)."""
     lb = np.asarray(lower, dtype=float)

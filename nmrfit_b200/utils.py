@@ -201,17 +201,19 @@ class FitUtility:
         refine_batch([self], max_iter, xtol)
         return self.params
 
-    def compute_uncertainties(self):
+    def compute_uncertainties(self, noise='white', max_lag=32, noise_acf=None):
         """Standard errors of ``params`` from the linearised least-squares problem at the fitted point (one pass
         over the spectrum on the GPU, see ``compute_uncertainties_batch``).  Sets ``covariance`` [D, D], ``stderr``
         [D] and ``uncertainty_info``, and returns ``stderr``.
 
         The errors assume that ``params`` is the least-squares optimum; the swarm stops short of it, and ``refine()``
-        takes ``params`` there first.
+        takes ``params`` there first.  ``noise='correlated'`` accounts for noise that is correlated from point to point,
+        as line broadening makes it (see ``compute_uncertainties_batch`` for it and for ``max_lag`` and ``noise_acf``).
 
         Raises RuntimeError before ``fit()``, NotImplementedError with ``fit_im`` (that objective is a sum of two
-        RMSEs, not a least-squares problem) and ValueError when the spectrum has no more points than parameters."""
-        compute_uncertainties_batch([self])
+        RMSEs, not a least-squares problem) and ValueError when the spectrum has no more points than parameters or
+        an argument is out of range."""
+        compute_uncertainties_batch([self], noise=noise, max_lag=max_lag, noise_acf=noise_acf)
         return self.stderr
 
     def area_fraction_stderr(self):
@@ -283,11 +285,58 @@ def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper):
     return 0.5 * (C + C.T), info
 
 
-def compute_uncertainties_batch(fits):
+def bartlett_taper(rho):
+    """``rho_k (1 - k/(L+1))`` along the last axis of ``rho`` [..., L+1]: the Bartlett (triangle) window.  The biased
+    autocorrelation of a sequence and the triangle are both positive-semidefinite sequences, and so is their
+    product (Schur), so the lag-weighted M formed from a tapered estimate is positive semidefinite by construction."""
+    rho = np.asarray(rho, dtype=np.float64)
+    L = rho.shape[-1] - 1
+    return rho * (1.0 - np.arange(L + 1) / (L + 1))
+
+
+def _check_noise_args(noise, max_lag, noise_acf, B, N, P):
+    """The checks ``compute_uncertainties_batch`` makes before any CUDA call: returns (L, rho) with rho None unless
+    ``noise_acf`` is given (then [B, L+1]); ValueError otherwise."""
+    if noise not in ('white', 'correlated'):
+        raise ValueError("noise must be 'white' or 'correlated', got %r" % (noise,))
+    if isinstance(max_lag, bool) or not isinstance(max_lag, (int, np.integer)) or max_lag < 0:
+        raise ValueError('max_lag must be an integer >= 0, got %r' % (max_lag,))
+    if noise == 'white':
+        if noise_acf is not None:
+            raise ValueError("noise_acf is used with noise='correlated' only")
+        return 0, None
+    if noise_acf is None:
+        return _cabi.check_lag(min(int(max_lag), N - 1), N, P), None
+    rho = _cabi.check_rho(noise_acf, B, N, P)
+    if not np.all(rho[:, 0] == 1.0):
+        raise ValueError('noise_acf must have rho_0 = 1')
+    if not np.all(np.abs(rho) <= 1.0):
+        raise ValueError('noise_acf must have |rho_k| <= 1')
+    return rho.shape[1] - 1, rho
+
+
+def compute_uncertainties_batch(fits, noise='white', max_lag=32, noise_acf=None):
     """``compute_uncertainties()`` for many fits of equal length and peak count (what ``fit_batch`` returns) in one
     device pass: the normal equations of every spectrum at its fitted ``params`` with its fit's ``weights``, then
     ``covariance_from_normal`` per fit.  Sets ``covariance``, ``stderr`` and ``uncertainty_info`` on every fit and
-    returns the list of ``stderr``."""
+    returns the list of ``stderr``.
+
+    ``noise='white'`` (the default) assumes noise independent from point to point.  ``noise='correlated'`` uses
+    ``C = s^2 H^-1 M_rho H^-1`` with ``M_rho = sum_i sum_{|k| <= L} rho_|k| a_i^T a_{i+k}``, a_i = w_i^2 A_i
+    (``Context.normal_m_lagged``, DESIGN K14), and L = min(max_lag, N - 1):
+      * by default rho is estimated from the residuals at ``params`` (``Context.residual_acf``), rho_k = r_k / r_0,
+        and tapered by ``bartlett_taper``, which keeps M_rho positive semidefinite;
+      * ``noise_acf`` [L+1] or [B, L+1] (rho_0 = 1, |rho_k| <= 1) is a known correlation used as given, with no
+        taper, for example the autocorrelation of a signal-free region of the full spectrum.
+    s^2 stays sum res^2 / (N - D).  These errors assume stationary noise and a residual that is noise: call
+    ``refine()`` first, because after an unrefined swarm the lineshape misfit shows up as correlation.  s^2 and the
+    estimated rho carry biases of order D * sum(rho) / N (a few per cent in s^2 at 4,096 points and 6 peaks with
+    sum(rho) near 10).  At a correlation length of 3 points, the taper at the default L = 32 loses 4-7 % of the
+    standard error, 2-4 % at L = 64.
+
+    ``uncertainty_info`` also holds ``noise``, ``noise_acf`` (the rho used, [L+1]; [1.] for white noise),
+    ``max_lag`` (L) and ``inflation`` (the correlated over the white standard error of each parameter; ones for
+    white noise)."""
     fits = list(fits)
     if not fits:
         return []
@@ -303,16 +352,33 @@ def compute_uncertainties_batch(fits):
             raise ValueError('every fit of a batch must have the same number of points and peaks')
     if N <= D:
         raise ValueError('the spectrum has %d points for %d parameters: no residual degrees of freedom' % (N, D))
+    B, P = len(fits), (D - 4) // 3
+    L, rho = _check_noise_args(noise, max_lag, noise_acf, B, N, P)
     W, U, V, weights = (np.stack([_cabi.as_f64(a) for a in arrs])
                         for arrs in zip(*[(f.data.w, f.data.u, f.data.v, f.weights) for f in fits]))
     X = np.stack([_cabi.as_f64(f.params) for f in fits])
-    with _cabi.pooled_context(len(fits), N, (D - 4) // 3, device=fits[0].options.get('device')) as ctx:
+    with _cabi.pooled_context(B, N, P, device=fits[0].options.get('device')) as ctx:
         ctx.set_spectra(W, U, V, weights)
         H, M, g, ssr = ctx.normal_equations(X)
+        if noise == 'correlated':
+            if rho is None:
+                r = ctx.residual_acf(X, L)
+                r0 = r[:, :1]
+                rho = bartlett_taper(np.where(r0 > 0, r / np.where(r0 > 0, r0, 1.0), np.eye(1, L + 1)))
+            M_rho = ctx.normal_m_lagged(X, rho)
     for b, f in enumerate(fits):
         f.covariance, f.uncertainty_info = covariance_from_normal(H[b], M[b], g[b], ssr[b], N, f.params, f.lower,
                                                                   f.upper)
         f.stderr = np.sqrt(np.diag(f.covariance))
+        inflation = np.ones(D)
+        if noise == 'correlated':
+            white = f.stderr
+            f.covariance, f.uncertainty_info = covariance_from_normal(H[b], M_rho[b], g[b], ssr[b], N, f.params,
+                                                                      f.lower, f.upper)
+            f.stderr = np.sqrt(np.diag(f.covariance))
+            inflation = f.stderr / white
+        f.uncertainty_info.update(noise=noise, noise_acf=np.ones(1) if rho is None else rho[b].copy(), max_lag=L,
+                                  inflation=inflation)
     return [f.stderr for f in fits]
 
 
