@@ -150,6 +150,29 @@ int nmrfit_lagged_plan(int n_points, int n_peaks, int max_lag, int* out);
 int nmrfit_ctx_refine(nmrfit_ctx* ctx, double* x_inout, const double* lb, const double* ub, int max_iter, double xtol,
                       double* f_out, int* passes_out, int* accepted_out, int* status_out, void* stream);
 
+/* nmrfit_ctx_refine with fixed and linked parameters (DESIGN K15).  tie_master, tie_scale, tie_offset [n_spectra][D]
+ * give each parameter j of a spectrum one of three roles:
+ *   free    tie_master[j] = j;
+ *   fixed   tie_master[j] = -1: x_j = tie_offset[j];
+ *   linked  tie_master[j] = k != j, k free: x_j = tie_scale[j] * x_k + tie_offset[j] (no chains).
+ * Scale and offset are read for linked parameters (scale finite and non-zero, offset finite) and the offset for fixed
+ * ones (finite); the box of a fixed parameter is not read.  The d free parameters theta, in index order, are refined
+ * as nmrfit_ctx_refine refines x, within the reduced box: the master's own box intersected with each dependent's box
+ * mapped through its tie, [(lb_j - c_j)/a_j, (ub_j - c_j)/a_j] (swapped for a_j < 0).  H and g of theta are
+ * H_theta[m][n] = sum_{j in G(m)} sum_{k in G(n)} a_j a_k H_jk and g_theta[m] = sum_{j in G(m)} a_j g_j, G(m) the master
+ * (a = 1) and its dependents in ascending index, summed in that order without FMA (the identity map gives H and g
+ * exactly); the convergence test uses H_theta and N - d.  A trial is expanded as x_j = a_j * theta_m + c_j rounded
+ * twice, so numpy's `a * t + c` gives the same bits; dependents are not clipped to their own box and leave it at a
+ * reduced bound only by that rounding.  The start: free entries of x_inout are clipped into the reduced box (NaN to
+ * its lower end), the others are recomputed by the expansion; no start is refused.  Outputs as nmrfit_ctx_refine, x
+ * expanded.  Spectra of one batch may carry different maps.  NMRFIT_ERR_ARG, with the spectrum and parameter named, for
+ * a master out of [-1, D), a chain (a master that is itself linked), a fixed master, a zero or non-finite scale, a
+ * non-finite offset, an empty or single-point reduced box, n_points <= d, and for what nmrfit_ctx_refine refuses
+ * besides the box and the start. */
+int nmrfit_ctx_refine_tied(nmrfit_ctx* ctx, double* x_inout, const double* lb, const double* ub, const int* tie_master,
+                           const double* tie_scale, const double* tie_offset, int max_iter, double xtol, double* f_out,
+                           int* passes_out, int* accepted_out, int* status_out, void* stream);
+
 /* Which objective kernel runs (default NMRFIT_ALGO_AUTO), and which one a launch with this fit_im would use.
  * Both kernels evaluate equations.objective (equations.py:152-212); the uniform-axis one exploits
  * w_i = w_0 + i*h (what core.load builds, core.py:58-60) to replace most exponentials by a recurrence. */

@@ -55,6 +55,7 @@ SIGNATURES = {
     'nmrfit_ctx_normal_equations': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     'nmrfit_normal_eq_plan': (_i, [_i, _i, c_int_p]),
     'nmrfit_ctx_refine': (_i, [_vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
+    'nmrfit_ctx_refine_tied': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
     'nmrfit_ctx_residual_acf': (_i, [_vp, _vp, _i, _vp, _vp]),
     'nmrfit_ctx_normal_m_lagged': (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     'nmrfit_lagged_plan': (_i, [_i, _i, _i, c_int_p]),
@@ -224,13 +225,14 @@ def check_rho(rho, B, N, P):
     return np.array(np.broadcast_to(rho, (B, rho.shape[-1])), dtype=np.float64, order='C')
 
 
-def check_refine_args(x, lb, ub, max_iter, xtol, B, N, P):
+def check_refine_args(x, lb, ub, max_iter, xtol, B, N, P, box=True):
     """The checks ``Context.refine`` makes before any CUDA call (the library makes them again): returns fresh
-    C-contiguous float64 copies of ``x`` [B, D] and of ``lb``, ``ub`` broadcast to [B, D].  ValueError otherwise."""
+    C-contiguous float64 copies of ``x`` [B, D] and of ``lb``, ``ub`` broadcast to [B, D].  ValueError otherwise.
+    ``box=False`` leaves the box, the start and the degrees of freedom to ``check_ties``."""
     D = 4 + 3 * P
     if P > 64:
         raise ValueError('refinement supports at most 64 peaks (D <= 196), got %d' % P)
-    if N <= D:
+    if box and N <= D:
         raise ValueError('the spectrum has %d points for %d parameters: no residual degrees of freedom' % (N, D))
     x = np.array(x, dtype=np.float64, order='C')
     if x.shape != (B, D):
@@ -243,11 +245,102 @@ def check_refine_args(x, lb, ub, max_iter, xtol, B, N, P):
         raise ValueError('max_iter must be >= 1')
     if not float(xtol) > 0:
         raise ValueError('xtol must be > 0')
+    if not box:
+        return x, lb, ub
     if not np.all(ub > lb):
         raise ValueError('every lower bound must be below its upper bound')
     if not np.all((x >= lb) & (x <= ub)):
         raise ValueError('the start must lie inside its box')
     return x, lb, ub
+
+
+def reduced_box(master, scale, offset, lb, ub):
+    """The box of the free parameters of one tie map [D] (DESIGN K15): ``(free, lo, hi)``, ``free`` their indices in
+    ascending order and [lo, hi] each one's own box intersected with the box of every dependent mapped through its tie,
+    computed as the library computes it.  ``lb``, ``ub`` are [D], or [n, D] for n spectra sharing the map (then lo, hi
+    are [n, d]).  ValueError, naming the parameter and its master, where a box is empty or a single point.  The map
+    itself must have passed ``check_tie_map``."""
+    lb, ub = np.asarray(lb, dtype=np.float64), np.asarray(ub, dtype=np.float64)
+    D = len(master)
+    free = np.flatnonzero(master == np.arange(D))
+    lo, hi = lb[..., free].copy(), ub[..., free].copy()
+    for m, j in enumerate(free):
+        if not np.all(hi[..., m] > lo[..., m]):
+            raise ValueError('parameter %d (a master or free): its box is empty or a single point' % j)
+        for i in np.flatnonzero(master == j):
+            if i == j:
+                continue
+            li, ui = (lb[..., i] - offset[i]) / scale[i], (ub[..., i] - offset[i]) / scale[i]
+            if scale[i] < 0:
+                li, ui = ui, li
+            lo[..., m], hi[..., m] = np.maximum(lo[..., m], li), np.minimum(hi[..., m], ui)
+            if not np.all((hi[..., m] > lo[..., m]) & ~np.isnan(li) & ~np.isnan(ui)):
+                raise ValueError('parameter %d and its master %d: the reduced box is empty or a single point' % (i, j))
+    return free, lo, hi
+
+
+def check_tie_map(master, scale, offset):
+    """One tie map [D] (``master`` int, ``scale``, ``offset`` float64; DESIGN K15): ValueError, naming the parameter,
+    for a master out of [-1, D), a chain, a fixed master, a zero or non-finite scale of a linked parameter and a
+    non-finite offset of a fixed or linked one."""
+    D = len(master)
+    for j in range(D):
+        m = int(master[j])
+        if m < -1 or m >= D:
+            raise ValueError('parameter %d: master %d is out of range (-1 fixed, j free, else a free parameter below '
+                             '%d)' % (j, m, D))
+        if m == j:
+            continue
+        if not np.isfinite(offset[j]):
+            raise ValueError('parameter %d: offset is not finite' % j)
+        if m == -1:
+            continue
+        if not np.isfinite(scale[j]) or scale[j] == 0:
+            raise ValueError('parameter %d: scale must be finite and non-zero (fix the parameter instead of a zero '
+                             'scale)' % j)
+        if master[m] == -1:
+            raise ValueError('parameter %d: its master %d is fixed' % (j, m))
+        if master[m] != m:
+            raise ValueError('parameter %d: its master %d is itself linked (no chains)' % (j, m))
+
+
+def check_ties(master, scale, offset, lb, ub, B, N, P):
+    """The checks ``Context.refine(ties=...)`` makes before any CUDA call, as ``nmrfit_ctx_refine_tied`` makes them:
+    ``master``, ``scale``, ``offset`` of shape [D] (every spectrum) or [B, D], ``lb``, ``ub`` [B, D] or [D].  Returns
+    C-contiguous [B, D] int32 / float64 / float64 copies of the map, else ValueError naming the spectrum and the
+    parameter (a malformed map, an empty or single-point reduced box, or no more points than free parameters)."""
+    D = 4 + 3 * P
+    try:
+        master = np.broadcast_to(np.asarray(master), (B, D))
+        scale, offset, lb, ub = (np.broadcast_to(np.asarray(a, dtype=np.float64), (B, D))
+                                 for a in (scale, offset, lb, ub))
+    except ValueError:
+        raise ValueError('the tie arrays, lb and ub must have shape (%d, %d) or (%d,)' % (B, D, D)) from None
+    if master.dtype.kind not in 'iu' and not np.all(master == np.round(master)):
+        raise ValueError('tie masters must be integers')
+    master = np.ascontiguousarray(master, dtype=np.int32)
+    # each distinct map is checked once, its reduced box over all the spectra that carry it at once; a refusal is
+    # then located spectrum by spectrum for its message
+    maps = np.concatenate([master.view(np.uint32).astype(np.uint64), scale.view(np.uint64), offset.view(np.uint64)],
+                          axis=1)
+    _, first, which = np.unique(maps, axis=0, return_index=True, return_inverse=True)
+    for k, b0 in enumerate(first):
+        group = np.flatnonzero(which.ravel() == k)
+        m, s, o = master[b0], scale[b0], offset[b0]
+        try:
+            check_tie_map(m, s, o)
+            free = reduced_box(m, s, o, lb[group], ub[group])[0]
+        except ValueError:
+            for b in group:
+                try:
+                    check_tie_map(m, s, o)
+                    reduced_box(m, s, o, lb[b], ub[b])
+                except ValueError as e:
+                    raise ValueError('spectrum %d, %s' % (b, e)) from None
+        if N <= free.size:
+            raise ValueError('spectrum %d: %d points for %d free parameters: no residual degrees of freedom'
+                             % (group[0], N, free.size))
+    return master, np.ascontiguousarray(scale), np.ascontiguousarray(offset)
 
 
 def default_device():
@@ -336,17 +429,30 @@ class Context(_Handle):
         check(lib().nmrfit_ctx_normal_equations(self._h, ptr(x), ptr(H), ptr(M), ptr(g), ptr(ssr), ptr(stream)))
         return H, M, g, ssr
 
-    def refine(self, x, lb, ub, max_iter=50, xtol=1e-6, stream=None):
+    def refine(self, x, lb, ub, max_iter=50, xtol=1e-6, stream=None, ties=None):
         """Bounded Levenberg-Marquardt refinement of ``x`` [B, D] (one start per spectrum) to the least-squares optimum
         of the weighted residual within [``lb``, ``ub``] ([B, D], or [D] for every spectrum), looping on the device
         (include/nmrfit_b200.h, DESIGN K13).  Returns ``(x, f, passes, accepted, status)``: the refined [B, D] (the
         start, bit for bit, where no step was accepted), sqrt(s/N) there [B], the passes of the normal equations,
-        the accepted steps and the ``REFINE_*`` status [B]."""
-        x, lb, ub = check_refine_args(x, lb, ub, max_iter, xtol, self.B, self.N, self.P)
+        the accepted steps and the ``REFINE_*`` status [B].
+
+        ``ties`` = ``(master, scale, offset)``, each [D] or [B, D] (``utils.Ties.arrays()``), refines the free
+        parameters of the tied model instead (``nmrfit_ctx_refine_tied``, DESIGN K15): fixed and linked parameters
+        follow from them, the start's free entries are clipped into the reduced box and the returned x is expanded."""
+        if ties is None:
+            x, lb, ub = check_refine_args(x, lb, ub, max_iter, xtol, self.B, self.N, self.P)
+        else:
+            x, lb, ub = check_refine_args(x, lb, ub, max_iter, xtol, self.B, self.N, self.P, box=False)
+            master, scale, offset = check_ties(*ties, lb, ub, self.B, self.N, self.P)
         f = np.empty(self.B)
         passes, accepted, status = (np.empty(self.B, dtype=np.int32) for _ in range(3))
-        check(lib().nmrfit_ctx_refine(self._h, ptr(x), ptr(lb), ptr(ub), int(max_iter), float(xtol), ptr(f),
-                                      ptr(passes), ptr(accepted), ptr(status), ptr(stream)))
+        if ties is None:
+            check(lib().nmrfit_ctx_refine(self._h, ptr(x), ptr(lb), ptr(ub), int(max_iter), float(xtol), ptr(f),
+                                          ptr(passes), ptr(accepted), ptr(status), ptr(stream)))
+        else:
+            check(lib().nmrfit_ctx_refine_tied(self._h, ptr(x), ptr(lb), ptr(ub), ptr(master), ptr(scale),
+                                               ptr(offset), int(max_iter), float(xtol), ptr(f), ptr(passes),
+                                               ptr(accepted), ptr(status), ptr(stream)))
         return x, f, passes, accepted, status
 
     def residual_acf(self, x, max_lag, stream=None):

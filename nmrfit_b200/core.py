@@ -34,7 +34,8 @@ def fit_batch(datas, lowers, uppers, expon=0.5, dynamic_weighting=True, fit_im=F
     advance together, one launch per generation.  With options['rng'] == 'host' and
     options['seeds'] = [k_0, k_1, ...], spectrum b reproduces the reference fit run
     after ``np.random.seed(k_b)``.  With options['refine'] every fit is then refined (``utils.refine_batch``) in the
-    same context, where the spectra and weights already are.  Returns a list of ``FitUtility``.
+    same context, where the spectra and weights already are, with options['ties'] (one ``utils.Ties`` for every
+    spectrum or a list of them) if given.  Returns a list of ``FitUtility``.
     """
     fits = [utils.FitUtility(d, lo, up, expon, dynamic_weighting, fit_im, 1, summary, options)
             for d, lo, up in zip(datas, lowers, uppers)]
@@ -42,6 +43,8 @@ def fit_batch(datas, lowers, uppers, expon=0.5, dynamic_weighting=True, fit_im=F
     refine = opt.get('refine', False)
     if refine and fits:
         utils._check_refinable(fits[0])
+    if not refine and opt.get('ties') is not None:
+        raise ValueError(utils.TIES_NEED_REFINE)
     B = len(fits)
     lb = np.array(lowers, dtype=np.float64)
     n_peaks = (lb.shape[1] - 4) // 3
@@ -70,7 +73,8 @@ def fit_batch(datas, lowers, uppers, expon=0.5, dynamic_weighting=True, fit_im=F
             f.error = float(fbest[b])
             f.fit_info = dict(generations=int(it[b]), stop=int(stop[b]))
         if refine:
-            utils.apply_refinement(fits, *ctx.refine(x, lowers, uppers))
+            per, arrays = utils.batch_ties(opt.get('ties'), B, n_peaks)
+            utils.apply_refinement(fits, *ctx.refine(x, lowers, uppers, ties=arrays), ties=per)
     for f in fits:
         if summary is True:
             f._print_summary()

@@ -144,6 +144,8 @@ struct nmrfit_ctx {
     DevBuf<double> rf_x, rf_cur;       // refinement: current, trial, lb, ub [4][B][D]; H | g | s at the current point
     DevBuf<RefineState> rf_state;
     DevBuf<int> rf_active;             // spectra still running after the last polled step
+    DevBuf<int> rf_tie_i;              // tied refinement: the tie map of each spectrum (RefineTies)
+    DevBuf<double> rf_tie_d;
     Stream pipe[2];                    // nmrfit_objective_batch_host: slices of a large particle set
     PinnedBuf<double> h_f;             // ... and staging of their values
     int far_cells = 0;                 // far-field cells per region: 0 = far_cells_per_region(N, R), else 1 | 2 | 4
@@ -787,31 +789,24 @@ int nmrfit_lagged_plan(int n_points, int n_peaks, int max_lag, int* out) {
 
 constexpr int kRefinePoll = 8;   // refinement iterations queued between host reads of the running count
 
-int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* ub, int max_iter, double xtol,
-                      double* f_out, int* passes_out, int* accepted_out, int* status_out, void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
+// the checks both refinement entry points make past the NULL pointers
+// (the tied refinement needs more points than free parameters only: build_ties checks that)
+static int refine_check(const nmrfit_ctx* c, int max_iter, double xtol, bool tied) {
     if (c->P > 64)
         return fail(NMRFIT_ERR_ARG, "refinement supports at most 64 peaks (D <= 196), the context has " +
                                         std::to_string(c->P));
-    if (c->N <= c->D) return fail(NMRFIT_ERR_ARG, "refinement needs more points than parameters");
+    if (!tied && c->N <= c->D) return fail(NMRFIT_ERR_ARG, "refinement needs more points than parameters");
     if (max_iter < 1) return fail(NMRFIT_ERR_ARG, "max_iter must be >= 1");
     if (!(xtol > 0.0)) return fail(NMRFIT_ERR_ARG, "xtol must be > 0");
-    if (int r = require_spectra(c, "it is refined")) return r;
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
+    return NMRFIT_OK;
+}
+
+// The refinement loop of both entry points: h = [x | x | lb | ub] (the start is the first current point and the first
+// trial; for tied parameters lb, ub hold the reduced box), ties null or on the device.
+static int refine_run(nmrfit_ctx* c, const std::vector<double>& h, const RefineTies* ties, int max_iter, double xtol,
+                      double* x, double* f_out, int* passes_out, int* accepted_out, int* status_out,
+                      cudaStream_t st) {
     const size_t B = (size_t)c->B, D = (size_t)c->D, BD = B * D;
-    // [x | x | lb | ub]: the start is the first current point and the first trial
-    std::vector<double> h(4 * BD);
-    CK(cudaMemcpy(h.data(), x, sizeof(double) * BD, cudaMemcpyDefault));
-    CK(cudaMemcpy(h.data() + 2 * BD, lb, sizeof(double) * BD, cudaMemcpyDefault));
-    CK(cudaMemcpy(h.data() + 3 * BD, ub, sizeof(double) * BD, cudaMemcpyDefault));
-    std::copy(h.begin(), h.begin() + BD, h.begin() + BD);
-    for (size_t i = 0; i < BD; ++i) {
-        const double xi = h[i], lo = h[2 * BD + i], hi = h[3 * BD + i];
-        if (!(hi > lo)) return fail(NMRFIT_ERR_ARG, "every lower bound must be below its upper bound");
-        if (!(xi >= lo && xi <= hi)) return fail(NMRFIT_ERR_ARG, "the start must lie inside its box");
-    }
     const NormalEqPlan p = normal_eq_plan(c->N, c->P);
     CK(c->ne_part.reserve(normal_eq_scratch_doubles(p, c->B)));
     CK(c->ne_out.reserve(B * (2 * D * D + D + 2)));
@@ -829,7 +824,7 @@ int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* 
         const bool poll = (it + 1) % kRefinePoll == 0 && it + 1 < max_iter;
         if (poll) CK(cudaMemsetAsync(c->rf_active.ptr, 0, sizeof(int), st));
         e = launch_refine_step(c->ne_out.ptr, c->rf_cur.ptr, c->rf_state.ptr, xc, xt, lbd, ubd, c->B, c->N, c->D,
-                               max_iter, xtol, poll ? c->rf_active.ptr : nullptr, st);
+                               max_iter, xtol, poll ? c->rf_active.ptr : nullptr, ties, st);
         if (e != cudaSuccess) return fail_cuda(e, "refinement step launch");
         if (poll) {
             CK(cudaMemcpyAsync(c->h_flags.ptr, c->rf_active.ptr, sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -847,6 +842,136 @@ int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* 
         if (outs[k]) CK(cudaMemcpy2DAsync(outs[k], sizeof(int), srcs[k], pitch, sizeof(int), B, cudaMemcpyDefault, st));
     CK(cudaStreamSynchronize(st));                         // the staged starts and the outputs may be pageable memory
     return NMRFIT_OK;
+}
+
+int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* ub, int max_iter, double xtol,
+                      double* f_out, int* passes_out, int* accepted_out, int* status_out, void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
+    if (int r = refine_check(c, max_iter, xtol, false)) return r;
+    if (int r = require_spectra(c, "it is refined")) return r;
+    CK(cudaSetDevice(c->device));
+    const size_t BD = (size_t)c->B * c->D;
+    std::vector<double> h(4 * BD);
+    CK(cudaMemcpy(h.data(), x, sizeof(double) * BD, cudaMemcpyDefault));
+    CK(cudaMemcpy(h.data() + 2 * BD, lb, sizeof(double) * BD, cudaMemcpyDefault));
+    CK(cudaMemcpy(h.data() + 3 * BD, ub, sizeof(double) * BD, cudaMemcpyDefault));
+    std::copy(h.begin(), h.begin() + BD, h.begin() + BD);
+    for (size_t i = 0; i < BD; ++i) {
+        const double xi = h[i], lo = h[2 * BD + i], hi = h[3 * BD + i];
+        if (!(hi > lo)) return fail(NMRFIT_ERR_ARG, "every lower bound must be below its upper bound");
+        if (!(xi >= lo && xi <= hi)) return fail(NMRFIT_ERR_ARG, "the start must lie inside its box");
+    }
+    return refine_run(c, h, nullptr, max_iter, xtol, x, f_out, passes_out, accepted_out, status_out,
+                      (cudaStream_t)stream);
+}
+
+// One spectrum's tie map checked, with its start and box, and turned into the kernel's layout: ti [3D + 2] and
+// td [2D] (RefineTies), the reduced box in lo, hi [D] (first d entries), the start expanded in place in x [D].
+static int build_ties(int b, int D, int N, const int* master, const double* scale, const double* offset, double* x,
+                      const double* lb, const double* ub, int* ti, double* td, double* lo, double* hi) {
+    const std::string at = "spectrum " + std::to_string(b) + ", parameter ";
+    for (int j = 0; j < D; ++j) {
+        const int m = master[j];
+        if (m < -1 || m >= D)
+            return fail(NMRFIT_ERR_ARG, at + std::to_string(j) + ": master " + std::to_string(m) +
+                                            " is out of range (-1 fixed, j free, else a free parameter below " +
+                                            std::to_string(D) + ")");
+        if (m == j) continue;
+        if (!std::isfinite(offset[j])) return fail(NMRFIT_ERR_ARG, at + std::to_string(j) + ": offset is not finite");
+        if (m == -1) continue;
+        if (!std::isfinite(scale[j]) || scale[j] == 0.0)
+            return fail(NMRFIT_ERR_ARG, at + std::to_string(j) + ": scale must be finite and non-zero (fix the "
+                                            "parameter instead of a zero scale)");
+        if (master[m] == -1)
+            return fail(NMRFIT_ERR_ARG, at + std::to_string(j) + ": its master " + std::to_string(m) + " is fixed");
+        if (master[m] != m)
+            return fail(NMRFIT_ERR_ARG, at + std::to_string(j) + ": its master " + std::to_string(m) +
+                                            " is itself linked (no chains)");
+    }
+    int* off = ti + 1;
+    int* mem = ti + D + 2;
+    int* fm = ti + 2 * D + 2;
+    double* a = td;
+    double* c = td + D;
+    int d = 0, k = 0;
+    for (int j = 0; j < D; ++j) {
+        if (master[j] != j) continue;
+        // the reduced box of theta_d: the master's own box intersected with each dependent's, mapped through it
+        double l = lb[j], u = ub[j];
+        if (!(u > l))
+            return fail(NMRFIT_ERR_ARG, at + std::to_string(j) + " (a master or free): its box is empty or a single "
+                                            "point");
+        off[d] = k;
+        fm[d] = j;
+        for (int i = 0; i < D; ++i) {
+            if (i != j && master[i] != j) continue;
+            mem[k] = i;
+            a[k] = i == j ? 1.0 : scale[i];
+            c[k] = i == j ? 0.0 : offset[i];
+            ++k;
+            if (i == j) continue;
+            double li = (lb[i] - offset[i]) / scale[i], ui = (ub[i] - offset[i]) / scale[i];
+            if (scale[i] < 0.0) std::swap(li, ui);
+            l = std::max(l, li);
+            u = std::min(u, ui);
+            if (!(u > l) || std::isnan(li) || std::isnan(ui))
+                return fail(NMRFIT_ERR_ARG, at + std::to_string(i) + " and its master " + std::to_string(j) +
+                                                ": the reduced box is empty or a single point");
+        }
+        lo[d] = l;
+        hi[d] = u;
+        x[j] = std::fmin(std::fmax(x[j], l), u);
+        ++d;
+    }
+    off[d] = k;
+    ti[0] = d;
+    if (N <= d)
+        return fail(NMRFIT_ERR_ARG, "spectrum " + std::to_string(b) + ": refinement needs more points than free "
+                                    "parameters");
+    for (int m = 0; m < d; ++m)                            // the expansion, as the step kernel makes it (no FMA)
+        for (int q = off[m]; q < off[m + 1]; ++q)
+            if (mem[q] != fm[m]) {
+                volatile double t = a[q] * x[fm[m]];
+                x[mem[q]] = t + c[q];
+            }
+    for (int j = 0; j < D; ++j)
+        if (master[j] == -1) x[j] = offset[j];
+    return NMRFIT_OK;
+}
+
+int nmrfit_ctx_refine_tied(nmrfit_ctx* c, double* x, const double* lb, const double* ub, const int* tie_master,
+                           const double* tie_scale, const double* tie_offset, int max_iter, double xtol, double* f_out,
+                           int* passes_out, int* accepted_out, int* status_out, void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !lb || !ub || !tie_master || !tie_scale || !tie_offset)
+        return fail(NMRFIT_ERR_ARG, "x, lb, ub, tie_master, tie_scale and tie_offset must be non-NULL");
+    if (int r = refine_check(c, max_iter, xtol, true)) return r;
+    if (int r = require_spectra(c, "it is refined")) return r;
+    CK(cudaSetDevice(c->device));
+    const size_t B = (size_t)c->B, D = (size_t)c->D, BD = B * D;
+    std::vector<double> h(4 * BD, 0.0), box(2 * BD), sc(BD), of(BD), td(2 * BD, 0.0);
+    std::vector<int> ms(BD), ti(B * (3 * D + 2), 0);
+    CK(cudaMemcpy(h.data(), x, sizeof(double) * BD, cudaMemcpyDefault));
+    CK(cudaMemcpy(box.data(), lb, sizeof(double) * BD, cudaMemcpyDefault));
+    CK(cudaMemcpy(box.data() + BD, ub, sizeof(double) * BD, cudaMemcpyDefault));
+    CK(cudaMemcpy(ms.data(), tie_master, sizeof(int) * BD, cudaMemcpyDefault));
+    CK(cudaMemcpy(sc.data(), tie_scale, sizeof(double) * BD, cudaMemcpyDefault));
+    CK(cudaMemcpy(of.data(), tie_offset, sizeof(double) * BD, cudaMemcpyDefault));
+    for (size_t b = 0; b < B; ++b)
+        if (int r = build_ties((int)b, (int)D, c->N, ms.data() + b * D, sc.data() + b * D, of.data() + b * D,
+                               h.data() + b * D, box.data() + b * D, box.data() + BD + b * D,
+                               ti.data() + b * (3 * D + 2), td.data() + b * 2 * D, h.data() + 2 * BD + b * D,
+                               h.data() + 3 * BD + b * D))
+            return r;
+    std::copy(h.begin(), h.begin() + BD, h.begin() + BD);
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(c->rf_tie_i.reserve(ti.size()));
+    CK(c->rf_tie_d.reserve(td.size()));
+    CK(cudaMemcpyAsync(c->rf_tie_i.ptr, ti.data(), sizeof(int) * ti.size(), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(c->rf_tie_d.ptr, td.data(), sizeof(double) * td.size(), cudaMemcpyHostToDevice, st));
+    const RefineTies ties{c->rf_tie_i.ptr, c->rf_tie_d.ptr};
+    return refine_run(c, h, &ties, max_iter, xtol, x, f_out, passes_out, accepted_out, status_out, st);
 }
 
 int nmrfit_normal_eq_plan(int n_points, int n_peaks, int* out) {

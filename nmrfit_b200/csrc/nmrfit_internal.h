@@ -255,12 +255,19 @@ struct RefineState {
     double lam, f;              // damping of the next trial; sqrt(s/N) at the current point
     int status, passes, accepted, pad;
 };
+// K15 tie map of a batch (built by nmrfit_ctx_refine_tied): per spectrum the d free parameters theta in index order,
+// each with its group G(m) = its master plus its dependents in ascending index.
+struct RefineTies {
+    const int* ints;        // [B][3D + 2]: d | off [D+1] (G(m) = members off[m] .. off[m+1]) | members [D] | master [D]
+    const double* dbls;     // [B][2D]: scale | offset of each member slot (1 | 0 for the master)
+};
 size_t refine_step_smem(int D);
 // trial [B][2*D*D + D + 2] is launch_normal_eq's output at xt; cur [B][D*D + D + 1] holds H | g | s at xc.
-// `active` (or null) gains one per spectrum still running after the step.
+// `active` (or null) gains one per spectrum still running after the step.  ties == null: x itself is refined within
+// [lb, ub]; else theta within the reduced box [lb, ub] ([B][D], the first d entries of a spectrum's row).
 cudaError_t launch_refine_step(const double* trial, double* cur, RefineState* state, double* xc, double* xt,
                                const double* lb, const double* ub, int B, int N, int D, int max_iter, double xtol,
-                               int* active, cudaStream_t st);
+                               int* active, const RefineTies* ties, cudaStream_t st);
 
 // ---- probes -------------------------------------------------------------------
 cudaError_t fp64_peak_probe(int iters, int repeats, double* tflops, double* sustained, cudaStream_t st);

@@ -107,6 +107,32 @@ def multiplet(n_points, n_peaks=6, seed=0, noise=1e-4, jitter=None):
     return data, np.array(true)
 
 
+# each main line's 13C satellites, (main, lower satellite, upper satellite) by position within a group: the pairs
+# sit at -/+ J/2 = -/+ 0.1 (per group) around their main line
+_SATELLITES = ((2, 0, 4), (3, 1, 5))
+
+
+def satellite_ties(n_peaks):
+    """The natural ties of ``multiplet``'s propcar-like groups (``utils.Ties``): for each main line m with satellites
+    s- and s+, width(s-) = width(s+) = width(m), area(s+) = area(s-) and loc(s-/+) = loc(m) -/+ J/2, with J/2 the
+    offset ``_OFFS`` puts between them (scaled by the number of groups, as ``multiplet`` scales it).  The true vector
+    of ``multiplet(..., jitter=False)`` satisfies them; jittered centres leave the satellites' boxes off the tie."""
+    from .utils import Ties
+    if n_peaks % 6:
+        raise ValueError('n_peaks must be a multiple of 6')
+    groups = n_peaks // 6
+    t = Ties(n_peaks)
+    for g in range(groups):
+        for m, lo, hi in _SATELLITES:
+            assert _IS_MAIN[m] and not _IS_MAIN[lo] and not _IS_MAIN[hi]
+            km, kl, kh = 6 * g + m, 6 * g + lo, 6 * g + hi
+            for s in (kl, kh):
+                t.link(('width', s), ('width', km))
+                t.link(('loc', s), ('loc', km), offset=(_OFFS[s % 6] - _OFFS[m]) / groups)
+            t.link(('area', kh), ('area', kl))
+    return t
+
+
 def processed_noise(n_points, sigma, broadening=3.0, zero_fill=2, n_realisations=1, seed=0):
     """Noise of a processed spectrum, for ``u`` and ``v``: white complex noise on an FID of n_points / zero_fill
     samples, exponential line broadening of ``broadening`` spectral points (the FWHM it gives a Lorentzian line;

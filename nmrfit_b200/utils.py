@@ -99,6 +99,8 @@ class FitUtility:
                     cooperative launch (bit-identical to the per-step kernels).
       ``device``    CUDA device index.
       ``refine``    True: ``refine()`` after the swarm (default False).
+      ``ties``      a ``Ties`` the refinement holds (``refine(ties=...)``; needs ``refine``: the swarm does not
+                    honour ties).  ``fit_batch`` takes one ``Ties`` for every spectrum or a list of them.
     ``processes`` is accepted and ignored (the GPU evaluates every particle at once).
     """
 
@@ -119,6 +121,8 @@ class FitUtility:
         ``options['refine']``)."""
         if self.options.get('refine', False):
             _check_refinable(self)
+        elif self.options.get('ties') is not None:
+            raise ValueError(TIES_NEED_REFINE)
         self.weights = self._compute_weights()
         if self.dynamic_weighting is False:
             self.weights = np.ones_like(self.weights)
@@ -137,7 +141,7 @@ class FitUtility:
         self.error = fopt
         self.fit_info = info
         if opt.get('refine', False):
-            self.refine()
+            self.refine(ties=opt.get('ties'))
 
         if self.summary is True:
             self._print_summary()
@@ -190,15 +194,20 @@ class FitUtility:
         """Fitted areas: every third parameter from index 6 (utils.py:322)."""
         return np.array([self.params[i] for i in range(6, len(self.params), 3)])
 
-    def refine(self, max_iter=50, xtol=1e-6):
+    def refine(self, max_iter=50, xtol=1e-6, ties=None):
         """Refine the swarm's ``params`` to the least-squares optimum of the weighted residual within the box, by
         bounded Levenberg-Marquardt on the GPU (see ``refine_batch``).  Replaces ``params`` and ``error`` (which
         becomes sqrt(s/N) from the normal equations at the new point; both stay bit for bit as they were if no step
         was accepted) and sets ``refine_info`` = dict(start_params, start_error, passes, accepted, status), status one
         of ``_cabi.REFINE_CONVERGED``, ``_STALLED``, ``_MAX_ITER``, ``_NONFINITE``.
 
+        ``ties`` (a ``Ties``) refines the constrained model: fixed parameters keep their values, linked ones follow
+        their masters, and the free ones are refined within the reduced box (DESIGN K15).  The ties used are kept
+        as ``self.ties``, so that ``compute_uncertainties()`` and ``area_fraction_stderr()`` give the errors of that
+        model.
+
         Raises RuntimeError before ``fit()`` and NotImplementedError with ``fit_im``."""
-        refine_batch([self], max_iter, xtol)
+        refine_batch([self], max_iter, xtol, ties=None if ties is None else [ties])
         return self.params
 
     def compute_uncertainties(self, noise='white', max_lag=32, noise_acf=None):
@@ -209,6 +218,9 @@ class FitUtility:
         The errors assume that ``params`` is the least-squares optimum; the swarm stops short of it, and ``refine()``
         takes ``params`` there first.  ``noise='correlated'`` accounts for noise that is correlated from point to point,
         as line broadening makes it (see ``compute_uncertainties_batch`` for it and for ``max_lag`` and ``noise_acf``).
+
+        After ``refine(ties=...)`` the errors are those of the tied model (``self.ties``, see
+        ``covariance_from_normal``): 0 for a fixed parameter, |scale| times its master's for a linked one.
 
         Raises RuntimeError before ``fit()``, NotImplementedError with ``fit_im`` (that objective is a sum of two
         RMSEs, not a least-squares problem) and ValueError when the spectrum has no more points than parameters or
@@ -245,7 +257,7 @@ class FitUtility:
 
 
 # ---- parameter uncertainties (not in the reference) ---------------------------------------------------------------
-def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper):
+def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper, ties=None):
     """Sandwich covariance of the weighted least-squares estimate from the normal equations of one spectrum
     (``Context.normal_equations``): ``C = s^2 H^-1 M H^-1`` with ``s^2 = sum res^2 / (N - D)``.
 
@@ -260,7 +272,15 @@ def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper):
     of a peak of area 0), ``C`` is all NaN and ``info['singular']`` is True.
 
     Returns ``(C [D, D], info)``, info = dict(sigma, dof, gradient=g, at_bound, singular); ``at_bound[j]`` flags a
-    parameter within 1e-9 of its box width of a bound, where the linearisation says little."""
+    parameter within 1e-9 of its box width of a bound, where the linearisation says little.
+
+    ``ties`` (a ``Ties``): the covariance of the tied model x = T theta + c (DESIGN K15).  H, M and g are projected
+    onto the d free parameters (H_theta = T^T H T, summed member by member as the refinement does, so the identity
+    map gives this function's untied result bit for bit), s^2 = sum res^2 / (N - d), and ``C = T C_theta T^T``: a
+    fixed parameter has error 0 and a linked one |scale| times its master's.  ``dof`` is N - d; ``at_bound`` is judged
+    on the reduced box and a linked parameter carries its master's flag."""
+    if ties is not None:
+        return _tied_covariance(H, M, g, ssr, n_points, params, lower, upper, ties)
     H, M, g = np.asarray(H, dtype=np.float64), np.asarray(M, dtype=np.float64), np.asarray(g, dtype=np.float64)
     x, lb, ub = (np.asarray(a, dtype=np.float64) for a in (params, lower, upper))
     D = H.shape[0]
@@ -283,6 +303,165 @@ def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper):
     Hinv = s[:, None] * (Linv.T @ Linv) * s[None, :]
     C = sigma2 * (Hinv @ M @ Hinv)
     return 0.5 * (C + C.T), info
+
+
+def _tied_covariance(H, M, g, ssr, n_points, params, lower, upper, ties):
+    """``covariance_from_normal`` with ``ties``: the untied computation on the free parameters, then expanded."""
+    x, lb, ub = (np.asarray(a, dtype=np.float64) for a in (params, lower, upper))
+    master, scale, offset = ties.arrays()
+    free, lo, hi = _cabi.reduced_box(master, scale, offset, lb, ub)
+    Ht, Mt, gt = ties.project(H, M, g)
+    Ct, info = covariance_from_normal(Ht, Mt, gt, ssr, n_points, x[free], lo, hi)
+    group, a = ties.groups()
+    D = len(master)
+    tied = group >= 0
+    C = np.zeros((D, D))
+    C[np.ix_(tied, tied)] = (a[tied, None] * a[None, tied]) * Ct[np.ix_(group[tied], group[tied])]
+    at_bound = np.zeros(D, dtype=bool)
+    at_bound[tied] = info['at_bound'][group[tied]]
+    info.update(gradient=np.asarray(g, dtype=np.float64).copy(), at_bound=at_bound)
+    return C, info
+
+
+class Ties:
+    """Fixed and linked parameters of a model of ``n_peaks`` peaks (D = 4 + 3 n_peaks), for the refinement and the
+    standard errors (DESIGN K15).  Every parameter starts free; ``fix(j, value)`` holds x_j = value, and
+    ``link(j, master, scale, offset)`` makes x_j = scale * x_master + offset, where the master must stay free (one
+    master per dependent, no chains).  Indices come from ``index``.  The free parameters theta, in index order, are
+    what the refinement moves: x = T theta + c (``matrix``, ``expand``).  Malformed ties raise ValueError at once."""
+
+    GLOBALS = ('p0', 'p1', 'r', 'yoff')
+    PEAK = ('width', 'loc', 'area')
+
+    def __init__(self, n_peaks):
+        self.n_peaks = int(n_peaks)
+        self.D = 4 + 3 * self.n_peaks
+        self.master = np.arange(self.D, dtype=np.int32)
+        self.scale = np.ones(self.D)
+        self.offset = np.zeros(self.D)
+
+    def index(self, name, peak=None):
+        """Index of ``'p0'``, ``'p1'``, ``'r'``, ``'yoff'``, or of ``'width'``, ``'loc'``, ``'area'`` of ``peak``
+        (also given as ``(name, peak)``)."""
+        if isinstance(name, tuple):
+            name, peak = name
+        if name in self.GLOBALS:
+            if peak is not None:
+                raise ValueError('%r is a global parameter: it takes no peak' % name)
+            return self.GLOBALS.index(name)
+        if name not in self.PEAK:
+            raise ValueError('unknown parameter %r: one of %s' % (name, ', '.join(self.GLOBALS + self.PEAK)))
+        if isinstance(peak, bool) or not isinstance(peak, (int, np.integer)) or not 0 <= peak < self.n_peaks:
+            raise ValueError('peak must be an integer in [0, %d), got %r' % (self.n_peaks, peak))
+        return 4 + 3 * int(peak) + self.PEAK.index(name)
+
+    def _param(self, j):
+        if isinstance(j, (str, tuple)):
+            return self.index(j)
+        if isinstance(j, bool) or not isinstance(j, (int, np.integer)) or not 0 <= j < self.D:
+            raise ValueError('parameter index must be an integer in [0, %d), got %r' % (self.D, j))
+        return int(j)
+
+    def _dependents(self, j):
+        return [i for i in range(self.D) if i != j and self.master[i] == j]
+
+    def fix(self, j, value):
+        """Hold parameter ``j`` at ``value`` (finite)."""
+        j = self._param(j)
+        if not np.isfinite(value):
+            raise ValueError('parameter %d: offset is not finite' % j)
+        if self._dependents(j):
+            raise ValueError('parameter %d: it is the master of %s and cannot be fixed' % (j, self._dependents(j)))
+        self.master[j], self.scale[j], self.offset[j] = -1, 1.0, float(value)
+        return self
+
+    def link(self, j, master, scale=1.0, offset=0.0):
+        """x_j = ``scale`` * x_master + ``offset``; ``scale`` finite and non-zero (for zero, use ``fix``), ``offset``
+        finite, ``master`` a free parameter other than j."""
+        j, m = self._param(j), self._param(master)
+        if m == j:
+            raise ValueError('parameter %d cannot be linked to itself' % j)
+        if not np.isfinite(scale) or scale == 0:
+            raise ValueError('parameter %d: scale must be finite and non-zero (fix the parameter instead of a zero '
+                             'scale)' % j)
+        if not np.isfinite(offset):
+            raise ValueError('parameter %d: offset is not finite' % j)
+        if self.master[m] == -1:
+            raise ValueError('parameter %d: its master %d is fixed' % (j, m))
+        if self.master[m] != m:
+            raise ValueError('parameter %d: its master %d is itself linked (no chains)' % (j, m))
+        if self._dependents(j):
+            raise ValueError('parameter %d: it is the master of %s and cannot be linked (no chains)'
+                             % (j, self._dependents(j)))
+        self.master[j], self.scale[j], self.offset[j] = m, float(scale), float(offset)
+        return self
+
+    def arrays(self):
+        """``(master [D] int32, scale [D], offset [D])`` as ``Context.refine(ties=...)`` and the C ABI take them."""
+        return self.master.copy(), self.scale.copy(), self.offset.copy()
+
+    def free(self):
+        """Indices of the free parameters theta, ascending."""
+        return np.flatnonzero(self.master == np.arange(self.D))
+
+    def groups(self):
+        """``(group [D], a [D])``: the index into theta of each parameter's master (-1 for a fixed parameter) and its
+        scale (1 for a free one, 0 for a fixed one)."""
+        free = self.free()
+        pos = np.full(self.D, -1)
+        pos[free] = np.arange(free.size)
+        group = np.where(self.master >= 0, pos[np.maximum(self.master, 0)], -1)
+        a = np.where(self.master == np.arange(self.D), 1.0, np.where(self.master < 0, 0.0, self.scale))
+        return group, a
+
+    def matrix(self):
+        """``(T [D, d], c [D])`` with x = T theta + c."""
+        group, a = self.groups()
+        T = np.zeros((self.D, self.free().size))
+        tied = group >= 0
+        T[np.flatnonzero(tied), group[tied]] = a[tied]
+        c = np.where(self.master == np.arange(self.D), 0.0, self.offset)
+        return T, c
+
+    def expand(self, theta):
+        """x [D] from the free parameters ``theta`` [d]: x_j = scale_j * theta + offset_j for a linked parameter (as
+        numpy's ``a * t + c``, which the refinement's expansion reproduces bit for bit), the value for a fixed one."""
+        theta = np.asarray(theta, dtype=np.float64)
+        free = self.free()
+        if theta.shape != (free.size,):
+            raise ValueError('theta must have shape (%d,), got %s' % (free.size, theta.shape))
+        group, a = self.groups()
+        x = self.offset.copy()
+        x[free] = theta
+        linked = (self.master >= 0) & (self.master != np.arange(self.D))
+        x[linked] = self.scale[linked] * theta[group[linked]] + self.offset[linked]
+        return x
+
+    def project(self, H, M, g):
+        """``(T^T H T, T^T M T, T^T g)`` summed as the refinement sums them: over each group's members in ascending
+        index (the master with scale 1), starting from the first term, so that the identity map returns H, M and g
+        exactly."""
+        H, M, g = (np.asarray(v, dtype=np.float64) for v in (H, M, g))
+        free = self.free()
+        members = [np.flatnonzero((self.master == j)) for j in free]   # the master is its own member
+        a = [np.where(mem == j, 1.0, self.scale[mem]) for mem, j in zip(members, free)]
+        d, width = free.size, max(len(m) for m in members)
+        mem = np.array([np.r_[m, np.full(width - len(m), -1)] for m in members])
+        sc = np.array([np.r_[s, np.zeros(width - len(s))] for s in a])
+        out = []
+        for X in (H, M):
+            Xt = None
+            for p in range(width):
+                for q in range(width):
+                    ok = (mem[:, p] >= 0)[:, None] & (mem[:, q] >= 0)[None, :]
+                    t = (sc[:, p][:, None] * sc[:, q][None, :]) * X[np.ix_(np.maximum(mem[:, p], 0),
+                                                                           np.maximum(mem[:, q], 0))]
+                    Xt = t if Xt is None else np.where(ok, Xt + t, Xt)
+            out.append(Xt)
+        gt = sc[:, 0] * g[mem[:, 0]]
+        for p in range(1, width):
+            gt = np.where(mem[:, p] >= 0, gt + sc[:, p] * g[np.maximum(mem[:, p], 0)], gt)
+        return out[0], out[1], gt
 
 
 def bartlett_taper(rho):
@@ -350,8 +529,10 @@ def compute_uncertainties_batch(fits, noise='white', max_lag=32, noise_acf=None)
     for f in fits:
         if len(f.data.w) != N or len(f.params) != D:
             raise ValueError('every fit of a batch must have the same number of points and peaks')
-    if N <= D:
-        raise ValueError('the spectrum has %d points for %d parameters: no residual degrees of freedom' % (N, D))
+    ties = [getattr(f, 'ties', None) for f in fits]
+    d = max(D if t is None else t.free().size for t in ties)
+    if N <= d:
+        raise ValueError('the spectrum has %d points for %d parameters: no residual degrees of freedom' % (N, d))
     B, P = len(fits), (D - 4) // 3
     L, rho = _check_noise_args(noise, max_lag, noise_acf, B, N, P)
     W, U, V, weights = (np.stack([_cabi.as_f64(a) for a in arrs])
@@ -368,15 +549,18 @@ def compute_uncertainties_batch(fits, noise='white', max_lag=32, noise_acf=None)
             M_rho = ctx.normal_m_lagged(X, rho)
     for b, f in enumerate(fits):
         f.covariance, f.uncertainty_info = covariance_from_normal(H[b], M[b], g[b], ssr[b], N, f.params, f.lower,
-                                                                  f.upper)
+                                                                  f.upper, ties=ties[b])
         f.stderr = np.sqrt(np.diag(f.covariance))
         inflation = np.ones(D)
         if noise == 'correlated':
             white = f.stderr
             f.covariance, f.uncertainty_info = covariance_from_normal(H[b], M_rho[b], g[b], ssr[b], N, f.params,
-                                                                      f.lower, f.upper)
+                                                                      f.lower, f.upper, ties=ties[b])
             f.stderr = np.sqrt(np.diag(f.covariance))
-            inflation = f.stderr / white
+            with np.errstate(divide='ignore', invalid='ignore'):
+                inflation = f.stderr / white
+            if ties[b] is not None:
+                inflation[ties[b].master == -1] = 1.0             # a fixed parameter: 0 / 0
         f.uncertainty_info.update(noise=noise, noise_acf=np.ones(1) if rho is None else rho[b].copy(), max_lag=L,
                                   inflation=inflation)
     return [f.stderr for f in fits]
@@ -390,9 +574,11 @@ def _check_refinable(f, fitted=False):
                                   'not a least-squares problem')
 
 
-def apply_refinement(fits, x, fval, passes, accepted, status):
-    """Store the result of ``Context.refine`` on the fits it refined (see ``FitUtility.refine``)."""
+def apply_refinement(fits, x, fval, passes, accepted, status, ties=None):
+    """Store the result of ``Context.refine`` on the fits it refined (see ``FitUtility.refine``), with the ``ties``
+    of each (a list, or None for none)."""
     for b, f in enumerate(fits):
+        f.ties = None if ties is None else ties[b]
         f.refine_info = dict(start_params=np.array(f.params, dtype=np.float64), start_error=f.error,
                              passes=int(passes[b]), accepted=int(accepted[b]), status=int(status[b]))
         if accepted[b] > 0:
@@ -400,10 +586,31 @@ def apply_refinement(fits, x, fval, passes, accepted, status):
             f.error = float(fval[b])
 
 
-def refine_batch(fits, max_iter=50, xtol=1e-6):
+TIES_NEED_REFINE = "options['ties'] needs options['refine'] = True: the swarm does not honour ties"
+
+
+def batch_ties(ties, B, P):
+    """``ties`` as ``refine_batch`` takes it (None, one ``Ties`` for every spectrum, or a list of ``Ties`` or None)
+    -> ``(list of B Ties or None, (master, scale, offset) [B, D] or None)``.  None entries of a list are untied
+    (the identity map)."""
+    if ties is None:
+        return [None] * B, None
+    per = list(ties) if isinstance(ties, (list, tuple)) else [ties] * B
+    if len(per) != B:
+        raise ValueError('ties must be one Ties or a list of %d, got %d' % (B, len(per)))
+    full = [Ties(P) if t is None else t for t in per]
+    for t in full:
+        if not isinstance(t, Ties) or t.n_peaks != P:
+            raise ValueError('every tie set must be a Ties of %d peaks' % P)
+    return per, tuple(np.stack(a) for a in zip(*[t.arrays() for t in full]))
+
+
+def refine_batch(fits, max_iter=50, xtol=1e-6, ties=None):
     """``refine()`` for many fits of equal length and peak count (what ``fit_batch`` returns) in one device call:
     the spectra and each fit's ``weights`` go to a pooled context, and every spectrum runs bounded Levenberg-Marquardt
-    (``Context.refine``, DESIGN K13) from its ``params`` within its box.  Returns the list of refined ``params``."""
+    (``Context.refine``, DESIGN K13) from its ``params`` within its box.  ``ties``: one ``Ties`` for every fit, or a
+    list with one ``Ties`` (or None) per fit (DESIGN K15); each fit keeps its own as ``ties``.  Returns the list of
+    refined ``params``."""
     fits = list(fits)
     if not fits:
         return []
@@ -413,14 +620,19 @@ def refine_batch(fits, max_iter=50, xtol=1e-6):
     for f in fits:
         if len(f.data.w) != N or len(f.params) != D:
             raise ValueError('every fit of a batch must have the same number of points and peaks')
+    per, arrays = batch_ties(ties, len(fits), (D - 4) // 3)
     W, U, V, weights = (np.stack([_cabi.as_f64(a) for a in arrs])
                         for arrs in zip(*[(f.data.w, f.data.u, f.data.v, f.weights) for f in fits]))
     X, LB, UB = (np.stack([_cabi.as_f64(getattr(f, k)) for f in fits]) for k in ('params', 'lower', 'upper'))
-    _cabi.check_refine_args(X, LB, UB, max_iter, xtol, len(fits), N, (D - 4) // 3)
+    if arrays is None:
+        _cabi.check_refine_args(X, LB, UB, max_iter, xtol, len(fits), N, (D - 4) // 3)
+    else:
+        _cabi.check_refine_args(X, LB, UB, max_iter, xtol, len(fits), N, (D - 4) // 3, box=False)
+        _cabi.check_ties(*arrays, LB, UB, len(fits), N, (D - 4) // 3)
     with _cabi.pooled_context(len(fits), N, (D - 4) // 3, device=fits[0].options.get('device')) as ctx:
         ctx.set_spectra(W, U, V, weights)
-        out = ctx.refine(X, LB, UB, max_iter, xtol)
-    apply_refinement(fits, *out)
+        out = ctx.refine(X, LB, UB, max_iter, xtol, ties=arrays)
+    apply_refinement(fits, *out, ties=per)
     return [f.params for f in fits]
 
 
