@@ -173,6 +173,50 @@ int nmrfit_ctx_refine_tied(nmrfit_ctx* ctx, double* x_inout, const double* lb, c
                            const double* tie_scale, const double* tie_offset, int max_iter, double xtol, double* f_out,
                            int* passes_out, int* accepted_out, int* status_out, void* stream);
 
+/* Robust losses of the refinement (DESIGN K16), in scipy.optimize.least_squares' convention: with the unweighted
+ * residual res_i, the scale c = f_scale > 0 of its spectrum (units of the data u) and z_i = (res_i / c)^2,
+ *   LINEAR  rho(z) = z                       (least squares: the paths above, bit for bit)
+ *   HUBER   rho(z) = z for z <= 1, else 2 sqrt(z) - 1
+ *   SOFT_L1 rho(z) = 2 (sqrt(1 + z) - 1)
+ *   CAUCHY  rho(z) = ln(1 + z)
+ * The loss is per call; the scale is per spectrum, since the spectra of one batch have different noise levels. */
+#define NMRFIT_LOSS_LINEAR 0
+#define NMRFIT_LOSS_HUBER 1
+#define NMRFIT_LOSS_SOFT_L1 2
+#define NMRFIT_LOSS_CAUCHY 3
+
+/* Robust normal equations at one x [n_spectra][D] per spectrum, with res_i, A_i and w_i as in
+ * nmrfit_ctx_normal_equations and rho' = d rho / dz > 0:
+ *   H [n_spectra][D][D] = sum w_i^2 rho'(z_i) A_i^T A_i   (the Gauss-Newton matrix of iteratively reweighted LS)
+ *   g [n_spectra][D]    = sum w_i^2 rho'(z_i) res_i A_i   (the gradient of cost / 2)
+ *   cost [n_spectra]    = sum w_i^2 c^2 rho(z_i)
+ * One pass of K12's launch plan, each point's row of H_ext scaled by sqrt(rho'); any output may be NULL.  With
+ * NMRFIT_LOSS_LINEAR the outputs are nmrfit_ctx_normal_equations' H, g and ssr[0] bit for bit and f_scale is not read.
+ * Host or device pointers; returns when the outputs are written; fixed summation order (as K12).  NMRFIT_ERR_ARG for a
+ * NULL x, an unknown loss, more than 64 peaks, and for a non-linear loss a NULL f_scale or one that is not finite and
+ * > 0 (the message names the spectrum). */
+int nmrfit_ctx_normal_equations_loss(nmrfit_ctx* ctx, const double* x, int loss, const double* f_scale, double* H,
+                                     double* g, double* cost, void* stream);
+/* The moments of the loss at one x [n_spectra][D] per spectrum, out [n_spectra][5] =
+ *   (cost = sum w_i^2 c^2 rho(z_i),  sum w_i^2 res_i^2,  sum psi_i^2,  sum psi'_i,  sum psi'_i^2)
+ * with psi_i = rho'(z_i) res_i and psi'_i = rho'(z_i) + 2 z_i rho''(z_i) (unweighted: they give the M-estimator's scale
+ * factor of the sandwich covariance, DESIGN K16).  For LINEAR psi = res, psi' = 1 and f_scale is not read.  Chunk
+ * partials added in a fixed order: bit-reproducible, the same alone or in a batch.  Refusals as
+ * nmrfit_ctx_normal_equations_loss, and a NULL out. */
+int nmrfit_ctx_loss_moments(nmrfit_ctx* ctx, const double* x, int loss, const double* f_scale, double* out,
+                            void* stream);
+/* nmrfit_ctx_refine (tie arrays NULL) or nmrfit_ctx_refine_tied (all three given) on the robust cost: every pass is
+ * nmrfit_ctx_normal_equations_loss at the trial, and the step kernel runs its rules unchanged on (H, g, cost) of the
+ * loss: acceptance on the cost, damping, frozen set, statuses, and convergence max |dx_j| sqrt(H_jj (N - d)/cost) <= xtol.
+ * f_out = sqrt(cost / N) at the returned point.  With NMRFIT_LOSS_LINEAR the outputs are those of nmrfit_ctx_refine /
+ * nmrfit_ctx_refine_tied bit for bit and f_scale is not read.  NMRFIT_ERR_ARG for what those refuse, an unknown loss,
+ * tie arrays given only in part, and for a non-linear loss a NULL f_scale or one not finite and > 0 (naming the
+ * spectrum). */
+int nmrfit_ctx_refine_loss(nmrfit_ctx* ctx, double* x_inout, const double* lb, const double* ub, const int* tie_master,
+                           const double* tie_scale, const double* tie_offset, int loss, const double* f_scale,
+                           int max_iter, double xtol, double* f_out, int* passes_out, int* accepted_out,
+                           int* status_out, void* stream);
+
 /* Which objective kernel runs (default NMRFIT_ALGO_AUTO), and which one a launch with this fit_im would use.
  * Both kernels evaluate equations.objective (equations.py:152-212); the uniform-axis one exploits
  * w_i = w_0 + i*h (what core.load builds, core.py:58-60) to replace most exponentials by a recurrence. */

@@ -19,6 +19,8 @@ ALGO_AUTO, ALGO_GENERAL, ALGO_UNIFORM = 0, 1, 2
 FUSED_AUTO, FUSED_OFF, FUSED_REQUIRE = 0, 1, 2
 RUNNING, STOP_MINFUNC, STOP_MINSTEP, STOP_MAXITER, STOP_PEER_LOST = 0, 1, 2, 3, 4
 REFINE_CONVERGED, REFINE_STALLED, REFINE_MAX_ITER, REFINE_NONFINITE = 1, 2, 3, 4
+LOSS_LINEAR, LOSS_HUBER, LOSS_SOFT_L1, LOSS_CAUCHY = 0, 1, 2, 3
+LOSSES = {'linear': LOSS_LINEAR, 'huber': LOSS_HUBER, 'soft_l1': LOSS_SOFT_L1, 'cauchy': LOSS_CAUCHY}
 
 c_double_p = ctypes.POINTER(ctypes.c_double)
 c_int_p = ctypes.POINTER(ctypes.c_int)
@@ -56,6 +58,9 @@ SIGNATURES = {
     'nmrfit_normal_eq_plan': (_i, [_i, _i, c_int_p]),
     'nmrfit_ctx_refine': (_i, [_vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
     'nmrfit_ctx_refine_tied': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
+    'nmrfit_ctx_normal_equations_loss': (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
+    'nmrfit_ctx_loss_moments': (_i, [_vp, _vp, _i, _vp, _vp, _vp]),
+    'nmrfit_ctx_refine_loss': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
     'nmrfit_ctx_residual_acf': (_i, [_vp, _vp, _i, _vp, _vp]),
     'nmrfit_ctx_normal_m_lagged': (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     'nmrfit_lagged_plan': (_i, [_i, _i, _i, c_int_p]),
@@ -343,6 +348,30 @@ def check_ties(master, scale, offset, lb, ub, B, N, P):
     return master, np.ascontiguousarray(scale), np.ascontiguousarray(offset)
 
 
+def check_loss(loss, f_scale, B):
+    """The loss checks of the robust entry points (the library makes them again): ``loss`` a ``LOSS_*`` code or one of
+    ``LOSSES``' names, ``f_scale`` a scalar or [B], finite and > 0, for a robust loss (not read for linear).  Returns
+    ``(code, f_scale as a fresh [B] float64 array, or None for linear)``, else ValueError naming the spectrum."""
+    if isinstance(loss, str):
+        if loss not in LOSSES:
+            raise ValueError('unknown loss %r: one of %s' % (loss, ', '.join(LOSSES)))
+        loss = LOSSES[loss]
+    if isinstance(loss, bool) or not isinstance(loss, (int, np.integer)) or loss not in LOSSES.values():
+        raise ValueError('unknown loss %r: one of %s or their LOSS_* codes' % (loss, ', '.join(LOSSES)))
+    if loss == LOSS_LINEAR:
+        return LOSS_LINEAR, None
+    if f_scale is None:
+        raise ValueError('a robust loss needs f_scale, the scale c of the residual in units of the data')
+    try:
+        fs = np.array(np.broadcast_to(np.asarray(f_scale, dtype=np.float64), (B,)), dtype=np.float64)
+    except (TypeError, ValueError):
+        raise ValueError('f_scale must be a scalar or have shape (%d,)' % B) from None
+    bad = np.flatnonzero(~(np.isfinite(fs) & (fs > 0)))
+    if bad.size:
+        raise ValueError('spectrum %d: f_scale must be finite and > 0, got %r' % (bad[0], fs[bad[0]]))
+    return int(loss), fs
+
+
 def default_device():
     """LOCAL_RANK under torchrun, else NMRFIT_DEVICE, else 0."""
     for key in ('NMRFIT_DEVICE', 'LOCAL_RANK'):
@@ -429,7 +458,34 @@ class Context(_Handle):
         check(lib().nmrfit_ctx_normal_equations(self._h, ptr(x), ptr(H), ptr(M), ptr(g), ptr(ssr), ptr(stream)))
         return H, M, g, ssr
 
-    def refine(self, x, lb, ub, max_iter=50, xtol=1e-6, stream=None, ties=None):
+    def normal_equations_loss(self, x, loss, f_scale=None, stream=None):
+        """Robust normal equations at ``x`` [B, D] (DESIGN K16): returns host arrays ``H`` [B, D, D] =
+        sum w^2 rho' A^T A, ``g`` [B, D] = sum w^2 rho' res A and ``cost`` [B] = sum w^2 c^2 rho, with z = (res/c)^2,
+        c = ``f_scale`` (scalar or [B]) and ``loss`` a ``LOSS_*`` code or name.  For linear they are
+        ``normal_equations``' H, g and ssr[:, 0] bit for bit."""
+        loss, fs = check_loss(loss, f_scale, self.B)
+        x = as_f64(x)
+        if x.shape != (self.B, self.D):
+            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        H = np.empty((self.B, self.D, self.D))
+        g = np.empty((self.B, self.D))
+        cost = np.empty(self.B)
+        check(lib().nmrfit_ctx_normal_equations_loss(self._h, ptr(x), loss, ptr(fs), ptr(H), ptr(g), ptr(cost),
+                                                     ptr(stream)))
+        return H, g, cost
+
+    def loss_moments(self, x, loss, f_scale=None, stream=None):
+        """Moments of the loss at ``x`` [B, D] (DESIGN K16): [B, 5] = (cost, sum w^2 res^2, sum psi^2, sum psi',
+        sum psi'^2), psi = rho'(z) res and psi' = rho' + 2 z rho'' unweighted.  Arguments as ``normal_equations_loss``."""
+        loss, fs = check_loss(loss, f_scale, self.B)
+        x = as_f64(x)
+        if x.shape != (self.B, self.D):
+            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        out = np.empty((self.B, 5))
+        check(lib().nmrfit_ctx_loss_moments(self._h, ptr(x), loss, ptr(fs), ptr(out), ptr(stream)))
+        return out
+
+    def refine(self, x, lb, ub, max_iter=50, xtol=1e-6, stream=None, ties=None, loss=LOSS_LINEAR, f_scale=None):
         """Bounded Levenberg-Marquardt refinement of ``x`` [B, D] (one start per spectrum) to the least-squares optimum
         of the weighted residual within [``lb``, ``ub``] ([B, D], or [D] for every spectrum), looping on the device
         (include/nmrfit_b200.h, DESIGN K13).  Returns ``(x, f, passes, accepted, status)``: the refined [B, D] (the
@@ -438,7 +494,12 @@ class Context(_Handle):
 
         ``ties`` = ``(master, scale, offset)``, each [D] or [B, D] (``utils.Ties.arrays()``), refines the free
         parameters of the tied model instead (``nmrfit_ctx_refine_tied``, DESIGN K15): fixed and linked parameters
-        follow from them, the start's free entries are clipped into the reduced box and the returned x is expanded."""
+        follow from them, the start's free entries are clipped into the reduced box and the returned x is expanded.
+
+        ``loss`` (a ``LOSS_*`` code or name) with ``f_scale`` (scalar or [B]) minimises the robust cost
+        sum w^2 c^2 rho((res/c)^2) instead (``nmrfit_ctx_refine_loss``, DESIGN K16); f is then sqrt(cost/N).  Linear is
+        the least-squares refinement bit for bit."""
+        loss, fs = check_loss(loss, f_scale, self.B)
         if ties is None:
             x, lb, ub = check_refine_args(x, lb, ub, max_iter, xtol, self.B, self.N, self.P)
         else:
@@ -446,7 +507,12 @@ class Context(_Handle):
             master, scale, offset = check_ties(*ties, lb, ub, self.B, self.N, self.P)
         f = np.empty(self.B)
         passes, accepted, status = (np.empty(self.B, dtype=np.int32) for _ in range(3))
-        if ties is None:
+        if loss != LOSS_LINEAR:
+            tie_ptrs = (None, None, None) if ties is None else (ptr(master), ptr(scale), ptr(offset))
+            check(lib().nmrfit_ctx_refine_loss(self._h, ptr(x), ptr(lb), ptr(ub), *tie_ptrs, loss, ptr(fs),
+                                               int(max_iter), float(xtol), ptr(f), ptr(passes), ptr(accepted),
+                                               ptr(status), ptr(stream)))
+        elif ties is None:
             check(lib().nmrfit_ctx_refine(self._h, ptr(x), ptr(lb), ptr(ub), int(max_iter), float(xtol), ptr(f),
                                           ptr(passes), ptr(accepted), ptr(status), ptr(stream)))
         else:

@@ -35,17 +35,19 @@ def fit_batch(datas, lowers, uppers, expon=0.5, dynamic_weighting=True, fit_im=F
     options['seeds'] = [k_0, k_1, ...], spectrum b reproduces the reference fit run
     after ``np.random.seed(k_b)``.  With options['refine'] every fit is then refined (``utils.refine_batch``) in the
     same context, where the spectra and weights already are, with options['ties'] (one ``utils.Ties`` for every
-    spectrum or a list of them) if given.  Returns a list of ``FitUtility``.
+    spectrum or a list of them) and options['loss'] / options['f_scale'] (one scale for every spectrum or one per
+    spectrum) if given.  Returns a list of ``FitUtility``.
     """
     fits = [utils.FitUtility(d, lo, up, expon, dynamic_weighting, fit_im, 1, summary, options)
             for d, lo, up in zip(datas, lowers, uppers)]
     opt = options
     refine = opt.get('refine', False)
+    B = len(fits)
     if refine and fits:
         utils._check_refinable(fits[0])
-    if not refine and opt.get('ties') is not None:
-        raise ValueError(utils.TIES_NEED_REFINE)
-    B = len(fits)
+        _cabi.check_loss(opt.get('loss', 'linear'), opt.get('f_scale'), B)
+    if not refine:
+        utils.check_unrefined_options(opt)
     lb = np.array(lowers, dtype=np.float64)
     n_peaks = (lb.shape[1] - 4) // 3
     W, U, V = (np.stack([_cabi.as_f64(getattr(f.data, k)) for f in fits]) for k in ('w', 'u', 'v'))
@@ -74,7 +76,8 @@ def fit_batch(datas, lowers, uppers, expon=0.5, dynamic_weighting=True, fit_im=F
             f.fit_info = dict(generations=int(it[b]), stop=int(stop[b]))
         if refine:
             per, arrays = utils.batch_ties(opt.get('ties'), B, n_peaks)
-            utils.apply_refinement(fits, *ctx.refine(x, lowers, uppers, ties=arrays), ties=per)
+            utils.refine_with_loss(ctx, fits, x, lowers, uppers, ties=arrays, ties_per=per,
+                                   loss=opt.get('loss', 'linear'), f_scale=opt.get('f_scale'))
     for f in fits:
         if summary is True:
             f._print_summary()

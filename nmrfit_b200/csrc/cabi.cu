@@ -146,6 +146,7 @@ struct nmrfit_ctx {
     DevBuf<int> rf_active;             // spectra still running after the last polled step
     DevBuf<int> rf_tie_i;              // tied refinement: the tie map of each spectrum (RefineTies)
     DevBuf<double> rf_tie_d;
+    DevBuf<double> rb_scale, rb_part, rb_out;   // robust losses: f_scale [B], moments chunk partials, moments [B][5]
     Stream pipe[2];                    // nmrfit_objective_batch_host: slices of a large particle set
     PinnedBuf<double> h_f;             // ... and staging of their values
     int far_cells = 0;                 // far-field cells per region: 0 = far_cells_per_region(N, R), else 1 | 2 | 4
@@ -709,6 +710,83 @@ int nmrfit_ctx_normal_equations(nmrfit_ctx* c, const double* x, double* H, doubl
     return NMRFIT_OK;
 }
 
+// The loss checks of the robust entry points: an unknown loss, and for a robust one f_scale [B] (host or device) read,
+// checked and staged on the device.  *dev stays null for LINEAR, whose f_scale is not read.
+static int stage_loss(nmrfit_ctx* c, int loss, const double* f_scale, cudaStream_t st, const double** dev) {
+    *dev = nullptr;
+    if (loss < NMRFIT_LOSS_LINEAR || loss > NMRFIT_LOSS_CAUCHY)
+        return fail(NMRFIT_ERR_ARG, "unknown loss " + std::to_string(loss) + " (NMRFIT_LOSS_LINEAR, _HUBER, _SOFT_L1 "
+                                    "or _CAUCHY)");
+    if (loss == NMRFIT_LOSS_LINEAR) return NMRFIT_OK;
+    if (!f_scale) return fail(NMRFIT_ERR_ARG, "f_scale must be non-NULL for a robust loss");
+    std::vector<double> h(c->B);
+    CK(cudaMemcpy(h.data(), f_scale, sizeof(double) * c->B, cudaMemcpyDefault));
+    for (int b = 0; b < c->B; ++b)
+        if (!(std::isfinite(h[b]) && h[b] > 0.0))
+            return fail(NMRFIT_ERR_ARG, "spectrum " + std::to_string(b) + ": f_scale must be finite and > 0");
+    CK(c->rb_scale.reserve(c->B));
+    CK(cudaMemcpyAsync(c->rb_scale.ptr, h.data(), sizeof(double) * c->B, cudaMemcpyHostToDevice, st));
+    *dev = c->rb_scale.ptr;
+    return NMRFIT_OK;
+}
+
+// the checks of both robust passes past the NULL pointers, and f_scale staged
+static int loss_pass_check(nmrfit_ctx* c, int loss, const double* f_scale, const char* what, cudaStream_t st,
+                           const double** fs) {
+    if (loss < NMRFIT_LOSS_LINEAR || loss > NMRFIT_LOSS_CAUCHY) return stage_loss(c, loss, f_scale, st, fs);
+    if (c->P > 64)
+        return fail(NMRFIT_ERR_ARG, std::string(what) + " support at most 64 peaks (D <= 196), the context has " +
+                                        std::to_string(c->P));
+    if (int r = require_spectra(c, "a robust pass runs")) return r;
+    CK(cudaSetDevice(c->device));
+    return stage_loss(c, loss, f_scale, st, fs);
+}
+
+int nmrfit_ctx_normal_equations_loss(nmrfit_ctx* c, const double* x, int loss, const double* f_scale, double* H,
+                                     double* g, double* cost, void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x) return fail(NMRFIT_ERR_ARG, "x must be non-NULL");
+    cudaStream_t st = (cudaStream_t)stream;
+    const double* fs = nullptr;
+    if (int r = loss_pass_check(c, loss, f_scale, "robust normal equations", st, &fs)) return r;
+    const size_t B = (size_t)c->B, D = (size_t)c->D, DD = D * D, per = 2 * DD + D + 2;
+    const NormalEqPlan p = normal_eq_plan(c->N, c->P);
+    const double* xd = nullptr;
+    if (int r = stage(x, B * D, c->ne_x, st, &xd)) return r;
+    CK(c->ne_part.reserve(normal_eq_scratch_doubles(p, c->B)));
+    CK(c->ne_out.reserve(B * per));
+    cudaError_t e = launch_normal_eq_loss(c->spec.ptr, xd, loss, fs, p, c->B, c->ne_part.ptr, c->ne_out.ptr, st);
+    if (e != cudaSuccess) return fail_cuda(e, "robust normal equations launch");
+    // per spectrum the device block is H_rho [D][D] | M [D][D] | g_rho [D] | (cost, sum w^2 rho' res^2)
+    const size_t offs[3] = {0, 2 * DD, 2 * DD + D}, lens[3] = {DD, D, 1};
+    double* dst[3] = {H, g, cost};
+    for (int k = 0; k < 3; ++k)
+        if (dst[k])
+            CK(cudaMemcpy2DAsync(dst[k], sizeof(double) * lens[k], c->ne_out.ptr + offs[k], sizeof(double) * per,
+                                 sizeof(double) * lens[k], B, cudaMemcpyDefault, st));
+    CK(cudaStreamSynchronize(st));                         // x and the outputs may be pageable host memory
+    return NMRFIT_OK;
+}
+
+int nmrfit_ctx_loss_moments(nmrfit_ctx* c, const double* x, int loss, const double* f_scale, double* out,
+                            void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !out) return fail(NMRFIT_ERR_ARG, "x and out must be non-NULL");
+    cudaStream_t st = (cudaStream_t)stream;
+    const double* fs = nullptr;
+    if (int r = loss_pass_check(c, loss, f_scale, "loss moments", st, &fs)) return r;
+    const size_t B = (size_t)c->B;
+    const double* xd = nullptr;
+    if (int r = stage(x, B * c->D, c->ne_x, st, &xd)) return r;
+    CK(c->rb_part.reserve(loss_moments_scratch_doubles(c->B, c->N)));
+    CK(c->rb_out.reserve(B * 5));
+    cudaError_t e = launch_loss_moments(c->spec.ptr, xd, loss, fs, c->B, c->N, c->P, c->rb_part.ptr, c->rb_out.ptr, st);
+    if (e != cudaSuccess) return fail_cuda(e, "loss moments launch");
+    CK(cudaMemcpyAsync(out, c->rb_out.ptr, sizeof(double) * B * 5, cudaMemcpyDefault, st));
+    CK(cudaStreamSynchronize(st));                         // x and out may be pageable host memory
+    return NMRFIT_OK;
+}
+
 // the checks of both lagged passes past the NULL pointers; fills the plan
 static int lagged_check(const nmrfit_ctx* c, int max_lag, LaggedPlan* plan) {
     if (c->P > 64)
@@ -803,9 +881,10 @@ static int refine_check(const nmrfit_ctx* c, int max_iter, double xtol, bool tie
 
 // The refinement loop of both entry points: h = [x | x | lb | ub] (the start is the first current point and the first
 // trial; for tied parameters lb, ub hold the reduced box), ties null or on the device.
-static int refine_run(nmrfit_ctx* c, const std::vector<double>& h, const RefineTies* ties, int max_iter, double xtol,
-                      double* x, double* f_out, int* passes_out, int* accepted_out, int* status_out,
-                      cudaStream_t st) {
+// `loss` and `fscale` (on the device, null for LINEAR) choose the pass (launch_normal_eq_loss).
+static int refine_run(nmrfit_ctx* c, const std::vector<double>& h, const RefineTies* ties, int loss,
+                      const double* fscale, int max_iter, double xtol, double* x, double* f_out, int* passes_out,
+                      int* accepted_out, int* status_out, cudaStream_t st) {
     const size_t B = (size_t)c->B, D = (size_t)c->D, BD = B * D;
     const NormalEqPlan p = normal_eq_plan(c->N, c->P);
     CK(c->ne_part.reserve(normal_eq_scratch_doubles(p, c->B)));
@@ -819,7 +898,7 @@ static int refine_run(nmrfit_ctx* c, const std::vector<double>& h, const RefineT
     CK(cudaMemsetAsync(c->rf_state.ptr, 0, sizeof(RefineState) * B, st));
     // every running spectrum has had the same number of passes, so max_iter iterations finish them all
     for (int it = 0; it < max_iter; ++it) {
-        cudaError_t e = launch_normal_eq(c->spec.ptr, xt, p, c->B, c->ne_part.ptr, c->ne_out.ptr, st);
+        cudaError_t e = launch_normal_eq_loss(c->spec.ptr, xt, loss, fscale, p, c->B, c->ne_part.ptr, c->ne_out.ptr, st);
         if (e != cudaSuccess) return fail_cuda(e, "refinement: normal equations launch");
         const bool poll = (it + 1) % kRefinePoll == 0 && it + 1 < max_iter;
         if (poll) CK(cudaMemsetAsync(c->rf_active.ptr, 0, sizeof(int), st));
@@ -844,13 +923,10 @@ static int refine_run(nmrfit_ctx* c, const std::vector<double>& h, const RefineT
     return NMRFIT_OK;
 }
 
-int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* ub, int max_iter, double xtol,
-                      double* f_out, int* passes_out, int* accepted_out, int* status_out, void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
-    if (int r = refine_check(c, max_iter, xtol, false)) return r;
-    if (int r = require_spectra(c, "it is refined")) return r;
-    CK(cudaSetDevice(c->device));
+// the untied refinement past the checks of refine_check and require_spectra, the device current
+static int refine_untied(nmrfit_ctx* c, double* x, const double* lb, const double* ub, int loss, const double* fscale,
+                         int max_iter, double xtol, double* f_out, int* passes_out, int* accepted_out, int* status_out,
+                         cudaStream_t st) {
     const size_t BD = (size_t)c->B * c->D;
     std::vector<double> h(4 * BD);
     CK(cudaMemcpy(h.data(), x, sizeof(double) * BD, cudaMemcpyDefault));
@@ -862,8 +938,18 @@ int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* 
         if (!(hi > lo)) return fail(NMRFIT_ERR_ARG, "every lower bound must be below its upper bound");
         if (!(xi >= lo && xi <= hi)) return fail(NMRFIT_ERR_ARG, "the start must lie inside its box");
     }
-    return refine_run(c, h, nullptr, max_iter, xtol, x, f_out, passes_out, accepted_out, status_out,
-                      (cudaStream_t)stream);
+    return refine_run(c, h, nullptr, loss, fscale, max_iter, xtol, x, f_out, passes_out, accepted_out, status_out, st);
+}
+
+int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* ub, int max_iter, double xtol,
+                      double* f_out, int* passes_out, int* accepted_out, int* status_out, void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
+    if (int r = refine_check(c, max_iter, xtol, false)) return r;
+    if (int r = require_spectra(c, "it is refined")) return r;
+    CK(cudaSetDevice(c->device));
+    return refine_untied(c, x, lb, ub, NMRFIT_LOSS_LINEAR, nullptr, max_iter, xtol, f_out, passes_out, accepted_out,
+                         status_out, (cudaStream_t)stream);
 }
 
 // One spectrum's tie map checked, with its start and box, and turned into the kernel's layout: ti [3D + 2] and
@@ -940,15 +1026,11 @@ static int build_ties(int b, int D, int N, const int* master, const double* scal
     return NMRFIT_OK;
 }
 
-int nmrfit_ctx_refine_tied(nmrfit_ctx* c, double* x, const double* lb, const double* ub, const int* tie_master,
-                           const double* tie_scale, const double* tie_offset, int max_iter, double xtol, double* f_out,
-                           int* passes_out, int* accepted_out, int* status_out, void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x || !lb || !ub || !tie_master || !tie_scale || !tie_offset)
-        return fail(NMRFIT_ERR_ARG, "x, lb, ub, tie_master, tie_scale and tie_offset must be non-NULL");
-    if (int r = refine_check(c, max_iter, xtol, true)) return r;
-    if (int r = require_spectra(c, "it is refined")) return r;
-    CK(cudaSetDevice(c->device));
+// the tied refinement past the checks of refine_check and require_spectra, the device current
+static int refine_tied(nmrfit_ctx* c, double* x, const double* lb, const double* ub, const int* tie_master,
+                       const double* tie_scale, const double* tie_offset, int loss, const double* fscale, int max_iter,
+                       double xtol, double* f_out, int* passes_out, int* accepted_out, int* status_out,
+                       cudaStream_t st) {
     const size_t B = (size_t)c->B, D = (size_t)c->D, BD = B * D;
     std::vector<double> h(4 * BD, 0.0), box(2 * BD), sc(BD), of(BD), td(2 * BD, 0.0);
     std::vector<int> ms(BD), ti(B * (3 * D + 2), 0);
@@ -965,13 +1047,48 @@ int nmrfit_ctx_refine_tied(nmrfit_ctx* c, double* x, const double* lb, const dou
                                h.data() + 3 * BD + b * D))
             return r;
     std::copy(h.begin(), h.begin() + BD, h.begin() + BD);
-    cudaStream_t st = (cudaStream_t)stream;
     CK(c->rf_tie_i.reserve(ti.size()));
     CK(c->rf_tie_d.reserve(td.size()));
     CK(cudaMemcpyAsync(c->rf_tie_i.ptr, ti.data(), sizeof(int) * ti.size(), cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(c->rf_tie_d.ptr, td.data(), sizeof(double) * td.size(), cudaMemcpyHostToDevice, st));
     const RefineTies ties{c->rf_tie_i.ptr, c->rf_tie_d.ptr};
-    return refine_run(c, h, &ties, max_iter, xtol, x, f_out, passes_out, accepted_out, status_out, st);
+    return refine_run(c, h, &ties, loss, fscale, max_iter, xtol, x, f_out, passes_out, accepted_out, status_out, st);
+}
+
+int nmrfit_ctx_refine_tied(nmrfit_ctx* c, double* x, const double* lb, const double* ub, const int* tie_master,
+                           const double* tie_scale, const double* tie_offset, int max_iter, double xtol, double* f_out,
+                           int* passes_out, int* accepted_out, int* status_out, void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !lb || !ub || !tie_master || !tie_scale || !tie_offset)
+        return fail(NMRFIT_ERR_ARG, "x, lb, ub, tie_master, tie_scale and tie_offset must be non-NULL");
+    if (int r = refine_check(c, max_iter, xtol, true)) return r;
+    if (int r = require_spectra(c, "it is refined")) return r;
+    CK(cudaSetDevice(c->device));
+    return refine_tied(c, x, lb, ub, tie_master, tie_scale, tie_offset, NMRFIT_LOSS_LINEAR, nullptr, max_iter, xtol,
+                       f_out, passes_out, accepted_out, status_out, (cudaStream_t)stream);
+}
+
+int nmrfit_ctx_refine_loss(nmrfit_ctx* c, double* x, const double* lb, const double* ub, const int* tie_master,
+                           const double* tie_scale, const double* tie_offset, int loss, const double* f_scale,
+                           int max_iter, double xtol, double* f_out, int* passes_out, int* accepted_out,
+                           int* status_out, void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
+    const int n_tie = (tie_master != nullptr) + (tie_scale != nullptr) + (tie_offset != nullptr);
+    if (n_tie != 0 && n_tie != 3)
+        return fail(NMRFIT_ERR_ARG, "tie_master, tie_scale and tie_offset must be all NULL (untied) or all non-NULL");
+    const bool tied = n_tie == 3;
+    cudaStream_t st = (cudaStream_t)stream;
+    const double* fs = nullptr;
+    if (loss < NMRFIT_LOSS_LINEAR || loss > NMRFIT_LOSS_CAUCHY) return stage_loss(c, loss, f_scale, st, &fs);
+    if (int r = refine_check(c, max_iter, xtol, tied)) return r;
+    if (int r = require_spectra(c, "it is refined")) return r;
+    CK(cudaSetDevice(c->device));
+    if (int r = stage_loss(c, loss, f_scale, st, &fs)) return r;
+    if (tied)
+        return refine_tied(c, x, lb, ub, tie_master, tie_scale, tie_offset, loss, fs, max_iter, xtol, f_out,
+                           passes_out, accepted_out, status_out, st);
+    return refine_untied(c, x, lb, ub, loss, fs, max_iter, xtol, f_out, passes_out, accepted_out, status_out, st);
 }
 
 int nmrfit_normal_eq_plan(int n_points, int n_peaks, int* out) {

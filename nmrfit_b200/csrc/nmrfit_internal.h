@@ -226,6 +226,14 @@ size_t normal_eq_scratch_doubles(const NormalEqPlan& p, int B);
 // x [B][D] -> out [B][2*D*D + D + 2] (H, M, g, ssr per spectrum); `part` holds normal_eq_scratch_doubles doubles
 cudaError_t launch_normal_eq(const double* spec, const double* x, const NormalEqPlan& p, int B, double* part,
                              double* out, cudaStream_t st);
+// K16: the same pass for a robust loss (NMRFIT_LOSS_*; LINEAR is launch_normal_eq), fscale [B] on the device.  Out
+// block as launch_normal_eq's with H_rho | M | g_rho | (s_rho, sum w^2 rho' res^2) (normal_eq.cu)
+cudaError_t launch_normal_eq_loss(const double* spec, const double* x, int loss, const double* fscale,
+                                  const NormalEqPlan& p, int B, double* part, double* out, cudaStream_t st);
+// K16 moments of the loss (robust.cu): x [B][D] -> out [B][5]; `part` holds loss_moments_scratch_doubles doubles
+size_t loss_moments_scratch_doubles(int B, int N);
+cudaError_t launch_loss_moments(const double* spec, const double* x, int loss, const double* fscale, int B, int N,
+                                int P, double* part, double* out, cudaStream_t st);
 
 // ---- K14 residual autocorrelation and lag-weighted M (lagged.cu) --------------------
 // Tiling of both passes: a function of N, P and the largest lag L only.

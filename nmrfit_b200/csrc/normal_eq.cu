@@ -11,10 +11,17 @@
 //   (a symmetric rank-tp update per tile: RB^2 DFMA per 2*RB shared loads).  When the blocks are fewer than the
 //   threads, `ng` point groups split the tile's points and are added in group order at the end of the chunk.
 //   Chunk partials [B][n_chunks][tasks][RB*RB] are added in chunk order by the second launch.  No atomics.
+//
+// K16, robust losses (robust_loss.cuh, DESIGN K16): the same pass with every H_ext row scaled by sqrt(rho'(z_i)),
+// z_i = (res_i / c)^2, so that H holds H_rho = sum w^2 rho' A^T A and g holds g_rho = sum w^2 rho' res A, and the last
+// column of the M_ext row set to q_i = w_i c sqrt(rho(z_i)), whose corner is the cost s_rho = sum w^2 c^2 rho.  The
+// plan is K12's.  Out block: H_rho | M (K12's) | g_rho | ssr = (s_rho, sum w^2 rho' res^2): the two corners swap
+// places, so the step kernel finds the cost where it finds s.  Loss = LossLinear is K12 (same SASS).
 #include <cuda_runtime.h>
 #include <algorithm>
 #include "nmrfit_internal.h"
 #include "normal_eq_rows.cuh"
+#include "robust_loss.cuh"
 
 namespace nmrfit {
 
@@ -30,9 +37,12 @@ __device__ __forceinline__ void tri_block(int q, int nb, int* bi, int* bj) {
     *bj = i + q;
 }
 
+// fscale [B]: the loss's scale c of each spectrum (not read by LossLinear)
+template <typename Loss>
 __global__ void __launch_bounds__(512) normal_eq_partial_kernel(const double* __restrict__ spec,
                                                                 const double* __restrict__ xs, NormalEqPlan p,
-                                                                double* __restrict__ part) {
+                                                                double* __restrict__ part,
+                                                                const double* __restrict__ fscale) {
     extern __shared__ __align__(16) double smem[];
     const int b = blockIdx.z, chunk = blockIdx.x, slice = blockIdx.y;
     const int tid = threadIdx.x, nt = blockDim.x;
@@ -109,13 +119,29 @@ __global__ void __launch_bounds__(512) normal_eq_partial_kernel(const double* __
             double a[4], wt, res;
             ne_point_terms(p0, p1, pt, N, rN, sw, fit, dr, P, a, &wt, &res);
             const double wt2 = wt * wt;
+            if constexpr (Loss::kRobust) {
+                // the IRLS weight is known only now: the peak columns written above are scaled here too
+                const double c = fscale[b], zr = res / c;
+                double rho, d1, dpsi;
+                Loss::eval(zr * zr, &rho, &d1, &dpsi);
+                const double sr = sqrt(d1);
+                for (int j = 4; j < D; ++j) rh[j] *= sr;
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                rh[j] = wt * a[j];
-                rm[j] = wt2 * a[j];
+                for (int j = 0; j < 4; ++j) {
+                    rh[j] = (wt * a[j]) * sr;
+                    rm[j] = wt2 * a[j];
+                }
+                rh[D] = (wt * res) * sr;
+                rm[D] = wt * c * sqrt(rho);
+            } else {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    rh[j] = wt * a[j];
+                    rm[j] = wt2 * a[j];
+                }
+                rh[D] = wt * res;
+                rm[D] = res;
             }
-            rh[D] = wt * res;
-            rm[D] = res;
         }
         __syncthreads();
         if (active) {
@@ -157,6 +183,8 @@ __global__ void __launch_bounds__(512) normal_eq_partial_kernel(const double* __
 }
 
 // fixed-order sum over chunks; one thread per (spectrum, matrix, j, k) of the E x E square, both triangles
+// (kRobust: the corner of M_ext, the cost, goes to ssr[0] and that of H_ext to ssr[1])
+template <bool kRobust>
 __global__ void normal_eq_reduce_kernel(const double* __restrict__ part, NormalEqPlan p, int n_chunks, int B,
                                         double* __restrict__ out) {
     const int D = 4 + 3 * p.P, E = D + 1;
@@ -178,7 +206,7 @@ __global__ void normal_eq_reduce_kernel(const double* __restrict__ part, NormalE
     double* o = out + (size_t)b * (2 * DD + D + 2);
     if (j0 < D && k0 < D) o[mat * DD + (size_t)j0 * D + k0] = s;
     else if (mat == 0 && j0 < D) o[2 * DD + j0] = s;     // (j0, D) of H_ext: g
-    else if (j0 == D && k0 == D) o[2 * DD + D + mat] = s;
+    else if (j0 == D && k0 == D) o[2 * DD + D + (kRobust ? 1 - mat : mat)] = s;
 }
 
 }  // namespace
@@ -221,26 +249,47 @@ size_t normal_eq_scratch_doubles(const NormalEqPlan& p, int B) {
     return (size_t)B * p.n_chunks * p.tasks * RB * RB;
 }
 
-cudaError_t launch_normal_eq(const double* spec, const double* x, const NormalEqPlan& p, int B, double* part,
-                             double* out, cudaStream_t st) {
+namespace {
+
+template <typename Loss>
+cudaError_t launch_pass(const double* spec, const double* x, const double* fscale, const NormalEqPlan& p, int B,
+                        double* part, double* out, cudaStream_t st) {
     static bool attr_set[NMRFIT_MAX_DEVICES] = {};
     int dev = 0;
     cudaGetDevice(&dev);
     if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-        cudaError_t e = cudaFuncSetAttribute(normal_eq_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             200 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(normal_eq_partial_kernel<Loss>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (e != cudaSuccess) return e;
         attr_set[dev % NMRFIT_MAX_DEVICES] = true;
     }
     dim3 grid(p.n_chunks, p.slices, B);
-    normal_eq_partial_kernel<<<grid, p.threads, p.smem, st>>>(spec, x, p, part);
+    normal_eq_partial_kernel<Loss><<<grid, p.threads, p.smem, st>>>(spec, x, p, part, fscale);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int E = 5 + 3 * p.P;
     const long long total = (long long)B * 2 * E * E;
-    normal_eq_reduce_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(part, p, p.n_chunks, B, out);
+    normal_eq_reduce_kernel<Loss::kRobust><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(part, p, p.n_chunks, B,
+                                                                                            out);
     count_launches(2);
     return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t launch_normal_eq(const double* spec, const double* x, const NormalEqPlan& p, int B, double* part,
+                             double* out, cudaStream_t st) {
+    return launch_pass<LossLinear>(spec, x, nullptr, p, B, part, out, st);
+}
+
+cudaError_t launch_normal_eq_loss(const double* spec, const double* x, int loss, const double* fscale,
+                                  const NormalEqPlan& p, int B, double* part, double* out, cudaStream_t st) {
+    switch (loss) {
+    case NMRFIT_LOSS_HUBER: return launch_pass<LossHuber>(spec, x, fscale, p, B, part, out, st);
+    case NMRFIT_LOSS_SOFT_L1: return launch_pass<LossSoftL1>(spec, x, fscale, p, B, part, out, st);
+    case NMRFIT_LOSS_CAUCHY: return launch_pass<LossCauchy>(spec, x, fscale, p, B, part, out, st);
+    default: return launch_normal_eq(spec, x, p, B, part, out, st);
+    }
 }
 
 }  // namespace nmrfit

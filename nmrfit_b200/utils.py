@@ -101,6 +101,9 @@ class FitUtility:
       ``refine``    True: ``refine()`` after the swarm (default False).
       ``ties``      a ``Ties`` the refinement holds (``refine(ties=...)``; needs ``refine``: the swarm does not
                     honour ties).  ``fit_batch`` takes one ``Ties`` for every spectrum or a list of them.
+      ``loss``, ``f_scale``   a robust loss the refinement minimises (``refine(loss=..., f_scale=...)``; needs
+                    ``refine``: the swarm keeps the reference's objective).  ``fit_batch`` takes one f_scale for every
+                    spectrum or one per spectrum.
     ``processes`` is accepted and ignored (the GPU evaluates every particle at once).
     """
 
@@ -121,8 +124,9 @@ class FitUtility:
         ``options['refine']``)."""
         if self.options.get('refine', False):
             _check_refinable(self)
-        elif self.options.get('ties') is not None:
-            raise ValueError(TIES_NEED_REFINE)
+            _cabi.check_loss(self.options.get('loss', 'linear'), self.options.get('f_scale'), 1)
+        else:
+            check_unrefined_options(self.options)
         self.weights = self._compute_weights()
         if self.dynamic_weighting is False:
             self.weights = np.ones_like(self.weights)
@@ -141,7 +145,7 @@ class FitUtility:
         self.error = fopt
         self.fit_info = info
         if opt.get('refine', False):
-            self.refine(ties=opt.get('ties'))
+            self.refine(ties=opt.get('ties'), loss=opt.get('loss', 'linear'), f_scale=opt.get('f_scale'))
 
         if self.summary is True:
             self._print_summary()
@@ -194,7 +198,7 @@ class FitUtility:
         """Fitted areas: every third parameter from index 6 (utils.py:322)."""
         return np.array([self.params[i] for i in range(6, len(self.params), 3)])
 
-    def refine(self, max_iter=50, xtol=1e-6, ties=None):
+    def refine(self, max_iter=None, xtol=1e-6, ties=None, loss='linear', f_scale=None):
         """Refine the swarm's ``params`` to the least-squares optimum of the weighted residual within the box, by
         bounded Levenberg-Marquardt on the GPU (see ``refine_batch``).  Replaces ``params`` and ``error`` (which
         becomes sqrt(s/N) from the normal equations at the new point; both stay bit for bit as they were if no step
@@ -206,8 +210,19 @@ class FitUtility:
         as ``self.ties``, so that ``compute_uncertainties()`` and ``area_fraction_stderr()`` give the errors of that
         model.
 
+        ``loss`` ('linear', 'huber', 'soft_l1' or 'cauchy', scipy's convention) with ``f_scale`` c > 0, in units of the
+        data, minimises the robust cost sum w^2 c^2 rho((res/c)^2) instead (DESIGN K16): a point whose unweighted
+        residual is far beyond c, such as an unmodelled impurity line, then has bounded influence.  c = 1.345 sigma for
+        'huber' and 2.385 sigma for 'cauchy' keep 95 % efficiency on Gaussian noise of level sigma.  The loss is kept as
+        ``self.loss`` = dict(name, f_scale) (None for linear), so that ``compute_uncertainties()`` gives the robust
+        covariance; ``error`` stays the weighted RMSE sqrt(sum w^2 res^2 / N) at the new point, and ``refine_info``
+        gains ``loss``, ``f_scale`` and ``cost`` (the robust cost at the returned point; N error^2 for linear).
+        Iteratively reweighted steps converge linearly while points lie beyond c, so a robust refinement takes more
+        passes than least squares (DESIGN K16): ``max_iter`` None is 50 for linear and ``ROBUST_MAX_ITER`` = 200 for a
+        robust loss.  The loop stops as soon as every spectrum has finished, so the larger cap costs nothing then.
+
         Raises RuntimeError before ``fit()`` and NotImplementedError with ``fit_im``."""
-        refine_batch([self], max_iter, xtol, ties=None if ties is None else [ties])
+        refine_batch([self], max_iter, xtol, ties=None if ties is None else [ties], loss=loss, f_scale=f_scale)
         return self.params
 
     def compute_uncertainties(self, noise='white', max_lag=32, noise_acf=None):
@@ -220,7 +235,9 @@ class FitUtility:
         as line broadening makes it (see ``compute_uncertainties_batch`` for it and for ``max_lag`` and ``noise_acf``).
 
         After ``refine(ties=...)`` the errors are those of the tied model (``self.ties``, see
-        ``covariance_from_normal``): 0 for a fixed parameter, |scale| times its master's for a linked one.
+        ``covariance_from_normal``): 0 for a fixed parameter, |scale| times its master's for a linked one.  After a
+        robust ``refine(loss=...)`` they are Huber's M-estimator covariance (``covariance_from_normal(moments=...)``);
+        ``noise='correlated'`` is then refused with NotImplementedError.
 
         Raises RuntimeError before ``fit()``, NotImplementedError with ``fit_im`` (that objective is a sum of two
         RMSEs, not a least-squares problem) and ValueError when the spectrum has no more points than parameters or
@@ -257,7 +274,7 @@ class FitUtility:
 
 
 # ---- parameter uncertainties (not in the reference) ---------------------------------------------------------------
-def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper, ties=None):
+def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper, ties=None, moments=None):
     """Sandwich covariance of the weighted least-squares estimate from the normal equations of one spectrum
     (``Context.normal_equations``): ``C = s^2 H^-1 M H^-1`` with ``s^2 = sum res^2 / (N - D)``.
 
@@ -278,9 +295,15 @@ def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper, ties=No
     onto the d free parameters (H_theta = T^T H T, summed member by member as the refinement does, so the identity
     map gives this function's untied result bit for bit), s^2 = sum res^2 / (N - d), and ``C = T C_theta T^T``: a
     fixed parameter has error 0 and a linked one |scale| times its master's.  ``dof`` is N - d; ``at_bound`` is judged
-    on the reduced box and a linked parameter carries its master's flag."""
+    on the reduced box and a linked parameter carries its master's flag.
+
+    ``moments`` (``Context.loss_moments`` at ``params``: cost, sum w^2 res^2, sum psi^2, sum psi', sum psi'^2): the
+    covariance of a robust fit (DESIGN K16, Huber 1981 section 7.6), s^2 replaced by
+    K^2 [sum psi^2 / (N - D)] / [sum psi' / N]^2 with K = 1 + (D/N) Var(psi') / E[psi']^2; H and M stay those of K12.
+    ``info`` then gains ``robust_factor``, that scalar over s^2 (``sigma`` stays s).  sum psi' <= 0 (a Cauchy fit with
+    gross misfit) makes ``C`` all NaN and ``singular`` True.  None is the least-squares computation, bit for bit."""
     if ties is not None:
-        return _tied_covariance(H, M, g, ssr, n_points, params, lower, upper, ties)
+        return _tied_covariance(H, M, g, ssr, n_points, params, lower, upper, ties, moments)
     H, M, g = np.asarray(H, dtype=np.float64), np.asarray(M, dtype=np.float64), np.asarray(g, dtype=np.float64)
     x, lb, ub = (np.asarray(a, dtype=np.float64) for a in (params, lower, upper))
     D = H.shape[0]
@@ -289,6 +312,13 @@ def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper, ties=No
     tol = 1e-9 * (ub - lb)
     info = dict(sigma=float(np.sqrt(sigma2)), dof=dof, gradient=g.copy(),
                 at_bound=(np.abs(x - lb) <= tol) | (np.abs(ub - x) <= tol), singular=False)
+    if moments is not None:
+        scalar = robust_scale(moments, n_points, D)
+        info['robust_factor'] = scalar / sigma2
+        if not np.isfinite(scalar):
+            info['singular'] = True
+            return np.full((D, D), np.nan), info
+        sigma2 = scalar
     diag = np.diag(H)
     if not np.all(np.isfinite(H)) or np.any(diag <= 0):
         info['singular'] = True
@@ -305,13 +335,26 @@ def covariance_from_normal(H, M, g, ssr, n_points, params, lower, upper, ties=No
     return 0.5 * (C + C.T), info
 
 
-def _tied_covariance(H, M, g, ssr, n_points, params, lower, upper, ties):
+def robust_scale(moments, n_points, d):
+    """Huber's scale of the sandwich for an M-estimator with d free parameters from ``moments`` (cost, sum w^2 res^2,
+    sum psi^2, sum psi', sum psi'^2): K^2 [sum psi^2 / (N - d)] / [sum psi' / N]^2, K = 1 + (d/N) Var(psi') / E[psi']^2.
+    NaN when sum psi' <= 0.  For the linear loss (psi = res, psi' = 1) it is sum res^2 / (N - d)."""
+    m = np.asarray(moments, dtype=np.float64)
+    N = float(n_points)
+    if not m[3] > 0:
+        return float('nan')
+    mean = m[3] / N
+    K = 1.0 + (d / N) * (m[4] / N - mean * mean) / (mean * mean)
+    return float(K * K * (m[2] / (N - d)) / (mean * mean))
+
+
+def _tied_covariance(H, M, g, ssr, n_points, params, lower, upper, ties, moments=None):
     """``covariance_from_normal`` with ``ties``: the untied computation on the free parameters, then expanded."""
     x, lb, ub = (np.asarray(a, dtype=np.float64) for a in (params, lower, upper))
     master, scale, offset = ties.arrays()
     free, lo, hi = _cabi.reduced_box(master, scale, offset, lb, ub)
     Ht, Mt, gt = ties.project(H, M, g)
-    Ct, info = covariance_from_normal(Ht, Mt, gt, ssr, n_points, x[free], lo, hi)
+    Ct, info = covariance_from_normal(Ht, Mt, gt, ssr, n_points, x[free], lo, hi, moments=moments)
     group, a = ties.groups()
     D = len(master)
     tied = group >= 0
@@ -530,6 +573,10 @@ def compute_uncertainties_batch(fits, noise='white', max_lag=32, noise_acf=None)
         if len(f.data.w) != N or len(f.params) != D:
             raise ValueError('every fit of a batch must have the same number of points and peaks')
     ties = [getattr(f, 'ties', None) for f in fits]
+    losses = [getattr(f, 'loss', None) for f in fits]
+    if noise == 'correlated' and any(lo is not None for lo in losses):
+        raise NotImplementedError("noise='correlated' is not available after a robust refinement: the lag-weighted "
+                                  "meat of psi is a separate derivation")
     d = max(D if t is None else t.free().size for t in ties)
     if N <= d:
         raise ValueError('the spectrum has %d points for %d parameters: no residual degrees of freedom' % (N, d))
@@ -541,6 +588,12 @@ def compute_uncertainties_batch(fits, noise='white', max_lag=32, noise_acf=None)
     with _cabi.pooled_context(B, N, P, device=fits[0].options.get('device')) as ctx:
         ctx.set_spectra(W, U, V, weights)
         H, M, g, ssr = ctx.normal_equations(X)
+        moments = [None] * B
+        for name in sorted({lo['name'] for lo in losses if lo is not None}):
+            use = [lo is not None and lo['name'] == name for lo in losses]
+            m = ctx.loss_moments(X, name, [lo['f_scale'] if u else 1.0 for lo, u in zip(losses, use)])
+            for b in np.flatnonzero(use):
+                moments[b] = m[b]
         if noise == 'correlated':
             if rho is None:
                 r = ctx.residual_acf(X, L)
@@ -549,8 +602,11 @@ def compute_uncertainties_batch(fits, noise='white', max_lag=32, noise_acf=None)
             M_rho = ctx.normal_m_lagged(X, rho)
     for b, f in enumerate(fits):
         f.covariance, f.uncertainty_info = covariance_from_normal(H[b], M[b], g[b], ssr[b], N, f.params, f.lower,
-                                                                  f.upper, ties=ties[b])
+                                                                  f.upper, ties=ties[b], moments=moments[b])
         f.stderr = np.sqrt(np.diag(f.covariance))
+        lo = losses[b]
+        f.uncertainty_info.update(loss='linear' if lo is None else lo['name'], f_scale=None if lo is None else
+                                  lo['f_scale'], robust_factor=f.uncertainty_info.get('robust_factor', 1.0))
         inflation = np.ones(D)
         if noise == 'correlated':
             white = f.stderr
@@ -574,19 +630,60 @@ def _check_refinable(f, fitted=False):
                                   'not a least-squares problem')
 
 
-def apply_refinement(fits, x, fval, passes, accepted, status, ties=None):
+def apply_refinement(fits, x, fval, passes, accepted, status, ties=None, loss='linear', f_scale=None, moments=None):
     """Store the result of ``Context.refine`` on the fits it refined (see ``FitUtility.refine``), with the ``ties``
-    of each (a list, or None for none)."""
+    of each (a list, or None for none).  For a robust ``loss`` (a name), ``f_scale`` [B] and ``moments``
+    (``Context.loss_moments`` at the returned x) are required: ``error`` then comes from moments[:, 1] and the cost from
+    moments[:, 0]."""
+    robust = loss != 'linear'
+    N = len(fits[0].data.w) if fits else 0
     for b, f in enumerate(fits):
         f.ties = None if ties is None else ties[b]
+        f.loss = dict(name=loss, f_scale=float(f_scale[b])) if robust else None
         f.refine_info = dict(start_params=np.array(f.params, dtype=np.float64), start_error=f.error,
-                             passes=int(passes[b]), accepted=int(accepted[b]), status=int(status[b]))
+                             passes=int(passes[b]), accepted=int(accepted[b]), status=int(status[b]), loss=loss,
+                             f_scale=float(f_scale[b]) if robust else None,
+                             cost=float(moments[b, 0]) if robust else N * float(fval[b]) ** 2)
         if accepted[b] > 0:
             f.params = x[b].copy()
-            f.error = float(fval[b])
+            f.error = float(np.sqrt(moments[b, 1] / N)) if robust else float(fval[b])
+
+
+ROBUST_MAX_ITER = 200
+
+
+def default_max_iter(max_iter, loss):
+    """``max_iter`` of the refinement: as given, else 50 for the linear loss and ``ROBUST_MAX_ITER`` for a robust one
+    (``loss`` a name or ``_cabi.LOSS_*`` code)."""
+    if max_iter is not None:
+        return max_iter
+    return 50 if loss in ('linear', _cabi.LOSS_LINEAR) else ROBUST_MAX_ITER
+
+
+def refine_with_loss(ctx, fits, x, lb, ub, ties=None, ties_per=None, loss='linear', f_scale=None, max_iter=None,
+                     xtol=1e-6):
+    """``ctx.refine`` (its spectra and weights set) and ``apply_refinement``, with the moments pass at the result for a
+    robust loss.  ``loss`` and ``f_scale`` must have passed ``_cabi.check_loss``; ``max_iter`` None is
+    ``default_max_iter``."""
+    out = ctx.refine(x, lb, ub, ties=ties, loss=loss, f_scale=f_scale, max_iter=default_max_iter(max_iter, loss),
+                     xtol=xtol)
+    code, fs = _cabi.check_loss(loss, f_scale, len(fits))
+    moments = None if code == _cabi.LOSS_LINEAR else ctx.loss_moments(out[0], code, fs)
+    name = [k for k, v in _cabi.LOSSES.items() if v == code][0]
+    apply_refinement(fits, *out, ties=ties_per, loss=name, f_scale=fs, moments=moments)
 
 
 TIES_NEED_REFINE = "options['ties'] needs options['refine'] = True: the swarm does not honour ties"
+LOSS_NEEDS_REFINE = ("options['loss'] and options['f_scale'] need options['refine'] = True: the swarm keeps the "
+                     "reference's objective")
+
+
+def check_unrefined_options(opt):
+    """ValueError for options that only the refinement honours, given without options['refine']."""
+    if opt.get('ties') is not None:
+        raise ValueError(TIES_NEED_REFINE)
+    if opt.get('loss') is not None or opt.get('f_scale') is not None:
+        raise ValueError(LOSS_NEEDS_REFINE)
 
 
 def batch_ties(ties, B, P):
@@ -605,12 +702,13 @@ def batch_ties(ties, B, P):
     return per, tuple(np.stack(a) for a in zip(*[t.arrays() for t in full]))
 
 
-def refine_batch(fits, max_iter=50, xtol=1e-6, ties=None):
+def refine_batch(fits, max_iter=None, xtol=1e-6, ties=None, loss='linear', f_scale=None):
     """``refine()`` for many fits of equal length and peak count (what ``fit_batch`` returns) in one device call:
     the spectra and each fit's ``weights`` go to a pooled context, and every spectrum runs bounded Levenberg-Marquardt
     (``Context.refine``, DESIGN K13) from its ``params`` within its box.  ``ties``: one ``Ties`` for every fit, or a
-    list with one ``Ties`` (or None) per fit (DESIGN K15); each fit keeps its own as ``ties``.  Returns the list of
-    refined ``params``."""
+    list with one ``Ties`` (or None) per fit (DESIGN K15); each fit keeps its own as ``ties``.  ``loss`` and
+    ``f_scale`` (a scalar or one per fit) and ``max_iter`` (None: ``default_max_iter``) as ``FitUtility.refine``
+    (DESIGN K16).  Returns the list of refined ``params``."""
     fits = list(fits)
     if not fits:
         return []
@@ -621,6 +719,8 @@ def refine_batch(fits, max_iter=50, xtol=1e-6, ties=None):
         if len(f.data.w) != N or len(f.params) != D:
             raise ValueError('every fit of a batch must have the same number of points and peaks')
     per, arrays = batch_ties(ties, len(fits), (D - 4) // 3)
+    _cabi.check_loss(loss, f_scale, len(fits))
+    max_iter = default_max_iter(max_iter, loss)
     W, U, V, weights = (np.stack([_cabi.as_f64(a) for a in arrs])
                         for arrs in zip(*[(f.data.w, f.data.u, f.data.v, f.weights) for f in fits]))
     X, LB, UB = (np.stack([_cabi.as_f64(getattr(f, k)) for f in fits]) for k in ('params', 'lower', 'upper'))
@@ -631,8 +731,8 @@ def refine_batch(fits, max_iter=50, xtol=1e-6, ties=None):
         _cabi.check_ties(*arrays, LB, UB, len(fits), N, (D - 4) // 3)
     with _cabi.pooled_context(len(fits), N, (D - 4) // 3, device=fits[0].options.get('device')) as ctx:
         ctx.set_spectra(W, U, V, weights)
-        out = ctx.refine(X, LB, UB, max_iter, xtol, ties=arrays)
-    apply_refinement(fits, *out, ties=per)
+        refine_with_loss(ctx, fits, X, LB, UB, ties=arrays, ties_per=per, loss=loss, f_scale=f_scale,
+                         max_iter=max_iter, xtol=xtol)
     return [f.params for f in fits]
 
 
