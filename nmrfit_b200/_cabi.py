@@ -443,14 +443,19 @@ class Context(_Handle):
                                                ptr(out), ptr(stream)))
         return out
 
+    def _params(self, x):
+        """One parameter vector per spectrum, ``x`` [B, D], as float64 for the post-fit passes."""
+        x = as_f64(x)
+        if x.shape != (self.B, self.D):
+            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        return x
+
     def normal_equations(self, x, stream=None):
         """Normal equations of the objective at ``x`` [B, D] (one parameter vector per spectrum) over the spectra and
         weights the context holds: returns host arrays ``H`` [B, D, D] = sum w^2 A^T A, ``M`` [B, D, D] = sum w^4 A^T A,
         ``g`` [B, D] = sum w^2 res A and ``ssr`` [B, 2] = (sum w^2 res^2, sum res^2), with res = Vdata - Vfit and
         A = d res / dx (include/nmrfit_b200.h)."""
-        x = as_f64(x)
-        if x.shape != (self.B, self.D):
-            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        x = self._params(x)
         H = np.empty((self.B, self.D, self.D))
         M = np.empty((self.B, self.D, self.D))
         g = np.empty((self.B, self.D))
@@ -464,9 +469,7 @@ class Context(_Handle):
         c = ``f_scale`` (scalar or [B]) and ``loss`` a ``LOSS_*`` code or name.  For linear they are
         ``normal_equations``' H, g and ssr[:, 0] bit for bit."""
         loss, fs = check_loss(loss, f_scale, self.B)
-        x = as_f64(x)
-        if x.shape != (self.B, self.D):
-            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        x = self._params(x)
         H = np.empty((self.B, self.D, self.D))
         g = np.empty((self.B, self.D))
         cost = np.empty(self.B)
@@ -478,9 +481,7 @@ class Context(_Handle):
         """Moments of the loss at ``x`` [B, D] (DESIGN K16): [B, 5] = (cost, sum w^2 res^2, sum psi^2, sum psi',
         sum psi'^2), psi = rho'(z) res and psi' = rho' + 2 z rho'' unweighted.  Arguments as ``normal_equations_loss``."""
         loss, fs = check_loss(loss, f_scale, self.B)
-        x = as_f64(x)
-        if x.shape != (self.B, self.D):
-            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        x = self._params(x)
         out = np.empty((self.B, 5))
         check(lib().nmrfit_ctx_loss_moments(self._h, ptr(x), loss, ptr(fs), ptr(out), ptr(stream)))
         return out
@@ -493,7 +494,7 @@ class Context(_Handle):
         the accepted steps and the ``REFINE_*`` status [B].
 
         ``ties`` = ``(master, scale, offset)``, each [D] or [B, D] (``utils.Ties.arrays()``), refines the free
-        parameters of the tied model instead (``nmrfit_ctx_refine_tied``, DESIGN K15): fixed and linked parameters
+        parameters of the tied model instead (DESIGN K15): fixed and linked parameters
         follow from them, the start's free entries are clipped into the reduced box and the returned x is expanded.
 
         ``loss`` (a ``LOSS_*`` code or name) with ``f_scale`` (scalar or [B]) minimises the robust cost
@@ -507,18 +508,9 @@ class Context(_Handle):
             master, scale, offset = check_ties(*ties, lb, ub, self.B, self.N, self.P)
         f = np.empty(self.B)
         passes, accepted, status = (np.empty(self.B, dtype=np.int32) for _ in range(3))
-        if loss != LOSS_LINEAR:
-            tie_ptrs = (None, None, None) if ties is None else (ptr(master), ptr(scale), ptr(offset))
-            check(lib().nmrfit_ctx_refine_loss(self._h, ptr(x), ptr(lb), ptr(ub), *tie_ptrs, loss, ptr(fs),
-                                               int(max_iter), float(xtol), ptr(f), ptr(passes), ptr(accepted),
-                                               ptr(status), ptr(stream)))
-        elif ties is None:
-            check(lib().nmrfit_ctx_refine(self._h, ptr(x), ptr(lb), ptr(ub), int(max_iter), float(xtol), ptr(f),
-                                          ptr(passes), ptr(accepted), ptr(status), ptr(stream)))
-        else:
-            check(lib().nmrfit_ctx_refine_tied(self._h, ptr(x), ptr(lb), ptr(ub), ptr(master), ptr(scale),
-                                               ptr(offset), int(max_iter), float(xtol), ptr(f), ptr(passes),
-                                               ptr(accepted), ptr(status), ptr(stream)))
+        tie_ptrs = (None, None, None) if ties is None else (ptr(master), ptr(scale), ptr(offset))
+        check(lib().nmrfit_ctx_refine_loss(self._h, ptr(x), ptr(lb), ptr(ub), *tie_ptrs, loss, ptr(fs), int(max_iter),
+                                           float(xtol), ptr(f), ptr(passes), ptr(accepted), ptr(status), ptr(stream)))
         return x, f, passes, accepted, status
 
     def residual_acf(self, x, max_lag, stream=None):
@@ -526,9 +518,7 @@ class Context(_Handle):
         host, r_k = sum_{i < N-k} res_i res_{i+k} (the biased form; r_0 is ``normal_equations``' ssr[:, 1]).
         ``max_lag`` = L, 0 <= L < N and at most ``lagged_plan(N, P)['max_lag']``."""
         L = check_lag(max_lag, self.N, self.P)
-        x = as_f64(x)
-        if x.shape != (self.B, self.D):
-            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        x = self._params(x)
         r = np.empty((self.B, L + 1))
         check(lib().nmrfit_ctx_residual_acf(self._h, ptr(x), L, ptr(r), ptr(stream)))
         return r
@@ -538,9 +528,7 @@ class Context(_Handle):
         (rows outside the spectrum are zero), from ``rho`` [L+1] or [B, L+1].  With rho = [1] it is ``normal_equations``'
         M.  The result is exactly symmetric."""
         rho = check_rho(rho, self.B, self.N, self.P)
-        x = as_f64(x)
-        if x.shape != (self.B, self.D):
-            raise ValueError('x must have shape (%d, %d), got %s' % (self.B, self.D, x.shape))
+        x = self._params(x)
         M = np.empty((self.B, self.D, self.D))
         check(lib().nmrfit_ctx_normal_m_lagged(self._h, ptr(x), ptr(rho), rho.shape[1] - 1, ptr(M), ptr(stream)))
         return M

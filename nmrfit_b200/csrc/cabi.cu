@@ -417,6 +417,26 @@ int stage(const double* src, size_t n, DevBuf<double>& buf, cudaStream_t st, con
     return NMRFIT_OK;
 }
 
+// The prologue of the post-fit entry points, in the order of their refusals: the context; `args`, the entry point's
+// checks of its own arguments (NULL pointers first); at most 64 peaks (`peaks` opens that message); `plan_args`, its
+// checks against the pass's plan; every spectrum set (`when` ends that message).  Then the device is made current and
+// x [B][D] staged in *xd (x null stages nothing).
+template <typename Args, typename PlanArgs>
+int post_fit_begin(nmrfit_ctx* c, Args&& args, const char* peaks, PlanArgs&& plan_args, const char* when,
+                   const double* x, cudaStream_t st, const double** xd) {
+    if (int r = check_ctx(c)) return r;
+    if (int r = args()) return r;
+    if (c->P > 64)
+        return fail(NMRFIT_ERR_ARG, std::string(peaks) + " at most 64 peaks (D <= 196), the context has " +
+                                        std::to_string(c->P));
+    if (int r = plan_args()) return r;
+    if (int r = require_spectra(c, when)) return r;
+    CK(cudaSetDevice(c->device));
+    return stage(x, (size_t)c->B * c->D, c->ne_x, st, xd);
+}
+
+int no_checks() { return NMRFIT_OK; }
+
 // Fill the fused kernel's arguments for `n_gen` generations and decide whether it can run (FP64, uniform axis,
 // real-only fit, default exp table, and every CTA co-resident).
 int fused_setup(nmrfit_ctx* c, int n_gen, const double* rp_d, const double* rg_d, FusedArgs* a, FusedPlan* plan) {
@@ -681,42 +701,17 @@ int nmrfit_ctx_compute_weights(nmrfit_ctx* c, const double* peak_bounds, const d
     return NMRFIT_OK;
 }
 
-int nmrfit_ctx_normal_equations(nmrfit_ctx* c, const double* x, double* H, double* M, double* g, double* ssr,
-                                void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x) return fail(NMRFIT_ERR_ARG, "x must be non-NULL");
-    if (c->P > 64)
-        return fail(NMRFIT_ERR_ARG, "normal equations support at most 64 peaks (D <= 196), the context has " +
-                                        std::to_string(c->P));
-    if (int r = require_spectra(c, "its normal equations are computed")) return r;
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    const size_t B = (size_t)c->B, D = (size_t)c->D, DD = D * D, per = 2 * DD + D + 2;
-    const NormalEqPlan p = normal_eq_plan(c->N, c->P);
-    const double* xd = nullptr;
-    if (int r = stage(x, B * D, c->ne_x, st, &xd)) return r;
-    CK(c->ne_part.reserve(normal_eq_scratch_doubles(p, c->B)));
-    CK(c->ne_out.reserve(B * per));
-    cudaError_t e = launch_normal_eq(c->spec.ptr, xd, p, c->B, c->ne_part.ptr, c->ne_out.ptr, st);
-    if (e != cudaSuccess) return fail_cuda(e, "normal equations launch");
-    // per spectrum the device block is H [D][D] | M [D][D] | g [D] | ssr [2]
-    const size_t offs[4] = {0, DD, 2 * DD, 2 * DD + D}, lens[4] = {DD, DD, D, 2};
-    double* dst[4] = {H, M, g, ssr};
-    for (int k = 0; k < 4; ++k)
-        if (dst[k])
-            CK(cudaMemcpy2DAsync(dst[k], sizeof(double) * lens[k], c->ne_out.ptr + offs[k], sizeof(double) * per,
-                                 sizeof(double) * lens[k], B, cudaMemcpyDefault, st));
-    CK(cudaStreamSynchronize(st));                         // x and the outputs may be pageable host memory
-    return NMRFIT_OK;
-}
-
-// The loss checks of the robust entry points: an unknown loss, and for a robust one f_scale [B] (host or device) read,
-// checked and staged on the device.  *dev stays null for LINEAR, whose f_scale is not read.
-static int stage_loss(nmrfit_ctx* c, int loss, const double* f_scale, cudaStream_t st, const double** dev) {
-    *dev = nullptr;
+static int check_loss(int loss) {
     if (loss < NMRFIT_LOSS_LINEAR || loss > NMRFIT_LOSS_CAUCHY)
         return fail(NMRFIT_ERR_ARG, "unknown loss " + std::to_string(loss) + " (NMRFIT_LOSS_LINEAR, _HUBER, _SOFT_L1 "
                                     "or _CAUCHY)");
+    return NMRFIT_OK;
+}
+
+// A robust loss's f_scale [B] (host or device) read, checked and staged on the device in *dev.  *dev stays null for
+// LINEAR, whose f_scale is not read.
+static int stage_loss(nmrfit_ctx* c, int loss, const double* f_scale, cudaStream_t st, const double** dev) {
+    *dev = nullptr;
     if (loss == NMRFIT_LOSS_LINEAR) return NMRFIT_OK;
     if (!f_scale) return fail(NMRFIT_ERR_ARG, "f_scale must be non-NULL for a robust loss");
     std::vector<double> h(c->B);
@@ -730,37 +725,26 @@ static int stage_loss(nmrfit_ctx* c, int loss, const double* f_scale, cudaStream
     return NMRFIT_OK;
 }
 
-// the checks of both robust passes past the NULL pointers, and f_scale staged
-static int loss_pass_check(nmrfit_ctx* c, int loss, const double* f_scale, const char* what, cudaStream_t st,
-                           const double** fs) {
-    if (loss < NMRFIT_LOSS_LINEAR || loss > NMRFIT_LOSS_CAUCHY) return stage_loss(c, loss, f_scale, st, fs);
-    if (c->P > 64)
-        return fail(NMRFIT_ERR_ARG, std::string(what) + " support at most 64 peaks (D <= 196), the context has " +
-                                        std::to_string(c->P));
-    if (int r = require_spectra(c, "a robust pass runs")) return r;
-    CK(cudaSetDevice(c->device));
-    return stage_loss(c, loss, f_scale, st, fs);
-}
-
-int nmrfit_ctx_normal_equations_loss(nmrfit_ctx* c, const double* x, int loss, const double* f_scale, double* H,
-                                     double* g, double* cost, void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x) return fail(NMRFIT_ERR_ARG, "x must be non-NULL");
-    cudaStream_t st = (cudaStream_t)stream;
+// Both normal-equations entry points: the pass of `loss` (launch_normal_eq_loss, LINEAR is K12), then the blocks
+// dst[k] that are non-null copied out of each spectrum's H [D][D] | M [D][D] | g [D] | ssr [2], n_ssr entries of ssr.
+// `pass` names the pass in the messages.
+static int normal_eq_pass(nmrfit_ctx* c, const double* x, int loss, const double* f_scale, const char* pass,
+                          const char* when, double* const dst[4], size_t n_ssr, cudaStream_t st) {
+    const double* xd = nullptr;
+    if (int r = post_fit_begin(
+            c, [&] { return x ? check_loss(loss) : fail(NMRFIT_ERR_ARG, "x must be non-NULL"); },
+            (std::string(pass) + " support").c_str(), no_checks, when, x, st, &xd))
+        return r;
     const double* fs = nullptr;
-    if (int r = loss_pass_check(c, loss, f_scale, "robust normal equations", st, &fs)) return r;
+    if (int r = stage_loss(c, loss, f_scale, st, &fs)) return r;
     const size_t B = (size_t)c->B, D = (size_t)c->D, DD = D * D, per = 2 * DD + D + 2;
     const NormalEqPlan p = normal_eq_plan(c->N, c->P);
-    const double* xd = nullptr;
-    if (int r = stage(x, B * D, c->ne_x, st, &xd)) return r;
     CK(c->ne_part.reserve(normal_eq_scratch_doubles(p, c->B)));
     CK(c->ne_out.reserve(B * per));
     cudaError_t e = launch_normal_eq_loss(c->spec.ptr, xd, loss, fs, p, c->B, c->ne_part.ptr, c->ne_out.ptr, st);
-    if (e != cudaSuccess) return fail_cuda(e, "robust normal equations launch");
-    // per spectrum the device block is H_rho [D][D] | M [D][D] | g_rho [D] | (cost, sum w^2 rho' res^2)
-    const size_t offs[3] = {0, 2 * DD, 2 * DD + D}, lens[3] = {DD, D, 1};
-    double* dst[3] = {H, g, cost};
-    for (int k = 0; k < 3; ++k)
+    if (e != cudaSuccess) return fail_cuda(e, (std::string(pass) + " launch").c_str());
+    const size_t offs[4] = {0, DD, 2 * DD, 2 * DD + D}, lens[4] = {DD, DD, D, n_ssr};
+    for (int k = 0; k < 4; ++k)
         if (dst[k])
             CK(cudaMemcpy2DAsync(dst[k], sizeof(double) * lens[k], c->ne_out.ptr + offs[k], sizeof(double) * per,
                                  sizeof(double) * lens[k], B, cudaMemcpyDefault, st));
@@ -768,16 +752,32 @@ int nmrfit_ctx_normal_equations_loss(nmrfit_ctx* c, const double* x, int loss, c
     return NMRFIT_OK;
 }
 
+int nmrfit_ctx_normal_equations(nmrfit_ctx* c, const double* x, double* H, double* M, double* g, double* ssr,
+                                void* stream) {
+    double* const dst[4] = {H, M, g, ssr};
+    return normal_eq_pass(c, x, NMRFIT_LOSS_LINEAR, nullptr, "normal equations", "its normal equations are computed",
+                          dst, 2, (cudaStream_t)stream);
+}
+
+// the robust pass's block is H_rho | M | g_rho | (cost, sum w^2 rho' res^2): H, g and the cost are copied out
+int nmrfit_ctx_normal_equations_loss(nmrfit_ctx* c, const double* x, int loss, const double* f_scale, double* H,
+                                     double* g, double* cost, void* stream) {
+    double* const dst[4] = {H, nullptr, g, cost};
+    return normal_eq_pass(c, x, loss, f_scale, "robust normal equations", "a robust pass runs", dst, 1,
+                          (cudaStream_t)stream);
+}
+
 int nmrfit_ctx_loss_moments(nmrfit_ctx* c, const double* x, int loss, const double* f_scale, double* out,
                             void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x || !out) return fail(NMRFIT_ERR_ARG, "x and out must be non-NULL");
     cudaStream_t st = (cudaStream_t)stream;
-    const double* fs = nullptr;
-    if (int r = loss_pass_check(c, loss, f_scale, "loss moments", st, &fs)) return r;
-    const size_t B = (size_t)c->B;
     const double* xd = nullptr;
-    if (int r = stage(x, B * c->D, c->ne_x, st, &xd)) return r;
+    if (int r = post_fit_begin(
+            c, [&] { return x && out ? check_loss(loss) : fail(NMRFIT_ERR_ARG, "x and out must be non-NULL"); },
+            "loss moments support", no_checks, "a robust pass runs", x, st, &xd))
+        return r;
+    const double* fs = nullptr;
+    if (int r = stage_loss(c, loss, f_scale, st, &fs)) return r;
+    const size_t B = (size_t)c->B;
     CK(c->rb_part.reserve(loss_moments_scratch_doubles(c->B, c->N)));
     CK(c->rb_out.reserve(B * 5));
     cudaError_t e = launch_loss_moments(c->spec.ptr, xd, loss, fs, c->B, c->N, c->P, c->rb_part.ptr, c->rb_out.ptr, st);
@@ -787,11 +787,8 @@ int nmrfit_ctx_loss_moments(nmrfit_ctx* c, const double* x, int loss, const doub
     return NMRFIT_OK;
 }
 
-// the checks of both lagged passes past the NULL pointers; fills the plan
+// the lag checks of both lagged passes; fills the plan
 static int lagged_check(const nmrfit_ctx* c, int max_lag, LaggedPlan* plan) {
-    if (c->P > 64)
-        return fail(NMRFIT_ERR_ARG, "the lagged passes support at most 64 peaks (D <= 196), the context has " +
-                                        std::to_string(c->P));
     if (max_lag < 0) return fail(NMRFIT_ERR_ARG, "max_lag must be >= 0");
     if (max_lag >= c->N)
         return fail(NMRFIT_ERR_ARG, "max_lag must be below the number of points, " + std::to_string(c->N));
@@ -803,16 +800,15 @@ static int lagged_check(const nmrfit_ctx* c, int max_lag, LaggedPlan* plan) {
 }
 
 int nmrfit_ctx_residual_acf(nmrfit_ctx* c, const double* x, int max_lag, double* r_out, void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x || !r_out) return fail(NMRFIT_ERR_ARG, "x and r_out must be non-NULL");
-    LaggedPlan p;
-    if (int r = lagged_check(c, max_lag, &p)) return r;
-    if (int r = require_spectra(c, "its residual autocorrelation is computed")) return r;
-    CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t B = (size_t)c->B, K = (size_t)max_lag + 1;
+    LaggedPlan p;
     const double* xd = nullptr;
-    if (int r = stage(x, B * c->D, c->ne_x, st, &xd)) return r;
+    if (int r = post_fit_begin(
+            c, [&] { return x && r_out ? NMRFIT_OK : fail(NMRFIT_ERR_ARG, "x and r_out must be non-NULL"); },
+            "the lagged passes support", [&] { return lagged_check(c, max_lag, &p); },
+            "its residual autocorrelation is computed", x, st, &xd))
+        return r;
+    const size_t B = (size_t)c->B, K = (size_t)max_lag + 1;
     CK(c->lg_part.reserve(residual_acf_scratch_doubles(p, c->B)));
     CK(c->lg_out.reserve(B * K));
     cudaError_t e = launch_residual_acf(c->spec.ptr, xd, p, c->B, c->lg_part.ptr, c->lg_out.ptr, st);
@@ -824,22 +820,28 @@ int nmrfit_ctx_residual_acf(nmrfit_ctx* c, const double* x, int max_lag, double*
 
 int nmrfit_ctx_normal_m_lagged(nmrfit_ctx* c, const double* x, const double* rho, int max_lag, double* M_out,
                                void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x || !rho || !M_out) return fail(NMRFIT_ERR_ARG, "x, rho and M_out must be non-NULL");
-    LaggedPlan p;
-    if (int r = lagged_check(c, max_lag, &p)) return r;
-    CK(cudaSetDevice(c->device));
-    const size_t B = (size_t)c->B, K = (size_t)max_lag + 1, D = (size_t)c->D;
-    std::vector<double> h(B * K);
-    CK(cudaMemcpy(h.data(), rho, sizeof(double) * B * K, cudaMemcpyDefault));
-    for (double v : h)
-        if (!std::isfinite(v)) return fail(NMRFIT_ERR_ARG, "every rho must be finite");
-    if (int r = require_spectra(c, "its lagged M is computed")) return r;
     cudaStream_t st = (cudaStream_t)stream;
+    LaggedPlan p;
+    std::vector<double> h;
+    // rho is read and checked before the spectra are: it may be device memory, so with the device current
+    auto rho_check = [&] {
+        if (int r = lagged_check(c, max_lag, &p)) return r;
+        CK(cudaSetDevice(c->device));
+        h.resize((size_t)c->B * (max_lag + 1));
+        CK(cudaMemcpy(h.data(), rho, sizeof(double) * h.size(), cudaMemcpyDefault));
+        for (double v : h)
+            if (!std::isfinite(v)) return fail(NMRFIT_ERR_ARG, "every rho must be finite");
+        return NMRFIT_OK;
+    };
+    auto args = [&] {
+        return x && rho && M_out ? NMRFIT_OK : fail(NMRFIT_ERR_ARG, "x, rho and M_out must be non-NULL");
+    };
     const double* xd = nullptr;
-    if (int r = stage(x, B * D, c->ne_x, st, &xd)) return r;
-    CK(c->lg_rho.reserve(B * K));
-    CK(cudaMemcpyAsync(c->lg_rho.ptr, h.data(), sizeof(double) * B * K, cudaMemcpyHostToDevice, st));
+    if (int r = post_fit_begin(c, args, "the lagged passes support", rho_check, "its lagged M is computed", x, st, &xd))
+        return r;
+    const size_t B = (size_t)c->B, D = (size_t)c->D;
+    CK(c->lg_rho.reserve(h.size()));
+    CK(cudaMemcpyAsync(c->lg_rho.ptr, h.data(), sizeof(double) * h.size(), cudaMemcpyHostToDevice, st));
     CK(c->lg_part.reserve(lagged_m_scratch_doubles(p, c->B)));
     CK(c->lg_out.reserve(B * D * D));
     cudaError_t e = launch_lagged_m(c->spec.ptr, xd, c->lg_rho.ptr, p, c->B, c->lg_part.ptr, c->lg_out.ptr, st);
@@ -867,12 +869,9 @@ int nmrfit_lagged_plan(int n_points, int n_peaks, int max_lag, int* out) {
 
 constexpr int kRefinePoll = 8;   // refinement iterations queued between host reads of the running count
 
-// the checks both refinement entry points make past the NULL pointers
+// the refinement's checks past the peak count
 // (the tied refinement needs more points than free parameters only: build_ties checks that)
 static int refine_check(const nmrfit_ctx* c, int max_iter, double xtol, bool tied) {
-    if (c->P > 64)
-        return fail(NMRFIT_ERR_ARG, "refinement supports at most 64 peaks (D <= 196), the context has " +
-                                        std::to_string(c->P));
     if (!tied && c->N <= c->D) return fail(NMRFIT_ERR_ARG, "refinement needs more points than parameters");
     if (max_iter < 1) return fail(NMRFIT_ERR_ARG, "max_iter must be >= 1");
     if (!(xtol > 0.0)) return fail(NMRFIT_ERR_ARG, "xtol must be > 0");
@@ -923,7 +922,7 @@ static int refine_run(nmrfit_ctx* c, const std::vector<double>& h, const RefineT
     return NMRFIT_OK;
 }
 
-// the untied refinement past the checks of refine_check and require_spectra, the device current
+// the untied refinement past the prologue of nmrfit_ctx_refine_loss
 static int refine_untied(nmrfit_ctx* c, double* x, const double* lb, const double* ub, int loss, const double* fscale,
                          int max_iter, double xtol, double* f_out, int* passes_out, int* accepted_out, int* status_out,
                          cudaStream_t st) {
@@ -939,17 +938,6 @@ static int refine_untied(nmrfit_ctx* c, double* x, const double* lb, const doubl
         if (!(xi >= lo && xi <= hi)) return fail(NMRFIT_ERR_ARG, "the start must lie inside its box");
     }
     return refine_run(c, h, nullptr, loss, fscale, max_iter, xtol, x, f_out, passes_out, accepted_out, status_out, st);
-}
-
-int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* ub, int max_iter, double xtol,
-                      double* f_out, int* passes_out, int* accepted_out, int* status_out, void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
-    if (int r = refine_check(c, max_iter, xtol, false)) return r;
-    if (int r = require_spectra(c, "it is refined")) return r;
-    CK(cudaSetDevice(c->device));
-    return refine_untied(c, x, lb, ub, NMRFIT_LOSS_LINEAR, nullptr, max_iter, xtol, f_out, passes_out, accepted_out,
-                         status_out, (cudaStream_t)stream);
 }
 
 // One spectrum's tie map checked, with its start and box, and turned into the kernel's layout: ti [3D + 2] and
@@ -1026,7 +1014,7 @@ static int build_ties(int b, int D, int N, const int* master, const double* scal
     return NMRFIT_OK;
 }
 
-// the tied refinement past the checks of refine_check and require_spectra, the device current
+// the tied refinement past the prologue of nmrfit_ctx_refine_loss
 static int refine_tied(nmrfit_ctx* c, double* x, const double* lb, const double* ub, const int* tie_master,
                        const double* tie_scale, const double* tie_offset, int loss, const double* fscale, int max_iter,
                        double xtol, double* f_out, int* passes_out, int* accepted_out, int* status_out,
@@ -1055,40 +1043,51 @@ static int refine_tied(nmrfit_ctx* c, double* x, const double* lb, const double*
     return refine_run(c, h, &ties, loss, fscale, max_iter, xtol, x, f_out, passes_out, accepted_out, status_out, st);
 }
 
+int nmrfit_ctx_refine_loss(nmrfit_ctx* c, double* x, const double* lb, const double* ub, const int* tie_master,
+                           const double* tie_scale, const double* tie_offset, int loss, const double* f_scale,
+                           int max_iter, double xtol, double* f_out, int* passes_out, int* accepted_out,
+                           int* status_out, void* stream) {
+    const int n_tie = (tie_master != nullptr) + (tie_scale != nullptr) + (tie_offset != nullptr);
+    const bool tied = n_tie == 3;
+    cudaStream_t st = (cudaStream_t)stream;
+    const double* unused = nullptr;
+    if (int r = post_fit_begin(
+            c,
+            [&] {
+                if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
+                if (n_tie != 0 && n_tie != 3)
+                    return fail(NMRFIT_ERR_ARG, "tie_master, tie_scale and tie_offset must be all NULL (untied) or "
+                                                "all non-NULL");
+                return check_loss(loss);
+            },
+            "refinement supports", [&] { return refine_check(c, max_iter, xtol, tied); }, "it is refined", nullptr, st,
+            &unused))
+        return r;
+    const double* fs = nullptr;
+    if (int r = stage_loss(c, loss, f_scale, st, &fs)) return r;
+    if (tied)
+        return refine_tied(c, x, lb, ub, tie_master, tie_scale, tie_offset, loss, fs, max_iter, xtol, f_out,
+                           passes_out, accepted_out, status_out, st);
+    return refine_untied(c, x, lb, ub, loss, fs, max_iter, xtol, f_out, passes_out, accepted_out, status_out, st);
+}
+
+// the least-squares refinements: nmrfit_ctx_refine_loss with LINEAR, past their own NULL checks
+int nmrfit_ctx_refine(nmrfit_ctx* c, double* x, const double* lb, const double* ub, int max_iter, double xtol,
+                      double* f_out, int* passes_out, int* accepted_out, int* status_out, void* stream) {
+    if (int r = check_ctx(c)) return r;
+    if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
+    return nmrfit_ctx_refine_loss(c, x, lb, ub, nullptr, nullptr, nullptr, NMRFIT_LOSS_LINEAR, nullptr, max_iter, xtol,
+                                  f_out, passes_out, accepted_out, status_out, stream);
+}
+
 int nmrfit_ctx_refine_tied(nmrfit_ctx* c, double* x, const double* lb, const double* ub, const int* tie_master,
                            const double* tie_scale, const double* tie_offset, int max_iter, double xtol, double* f_out,
                            int* passes_out, int* accepted_out, int* status_out, void* stream) {
     if (int r = check_ctx(c)) return r;
     if (!x || !lb || !ub || !tie_master || !tie_scale || !tie_offset)
         return fail(NMRFIT_ERR_ARG, "x, lb, ub, tie_master, tie_scale and tie_offset must be non-NULL");
-    if (int r = refine_check(c, max_iter, xtol, true)) return r;
-    if (int r = require_spectra(c, "it is refined")) return r;
-    CK(cudaSetDevice(c->device));
-    return refine_tied(c, x, lb, ub, tie_master, tie_scale, tie_offset, NMRFIT_LOSS_LINEAR, nullptr, max_iter, xtol,
-                       f_out, passes_out, accepted_out, status_out, (cudaStream_t)stream);
-}
-
-int nmrfit_ctx_refine_loss(nmrfit_ctx* c, double* x, const double* lb, const double* ub, const int* tie_master,
-                           const double* tie_scale, const double* tie_offset, int loss, const double* f_scale,
-                           int max_iter, double xtol, double* f_out, int* passes_out, int* accepted_out,
-                           int* status_out, void* stream) {
-    if (int r = check_ctx(c)) return r;
-    if (!x || !lb || !ub) return fail(NMRFIT_ERR_ARG, "x, lb and ub must be non-NULL");
-    const int n_tie = (tie_master != nullptr) + (tie_scale != nullptr) + (tie_offset != nullptr);
-    if (n_tie != 0 && n_tie != 3)
-        return fail(NMRFIT_ERR_ARG, "tie_master, tie_scale and tie_offset must be all NULL (untied) or all non-NULL");
-    const bool tied = n_tie == 3;
-    cudaStream_t st = (cudaStream_t)stream;
-    const double* fs = nullptr;
-    if (loss < NMRFIT_LOSS_LINEAR || loss > NMRFIT_LOSS_CAUCHY) return stage_loss(c, loss, f_scale, st, &fs);
-    if (int r = refine_check(c, max_iter, xtol, tied)) return r;
-    if (int r = require_spectra(c, "it is refined")) return r;
-    CK(cudaSetDevice(c->device));
-    if (int r = stage_loss(c, loss, f_scale, st, &fs)) return r;
-    if (tied)
-        return refine_tied(c, x, lb, ub, tie_master, tie_scale, tie_offset, loss, fs, max_iter, xtol, f_out,
-                           passes_out, accepted_out, status_out, st);
-    return refine_untied(c, x, lb, ub, loss, fs, max_iter, xtol, f_out, passes_out, accepted_out, status_out, st);
+    return nmrfit_ctx_refine_loss(c, x, lb, ub, tie_master, tie_scale, tie_offset, NMRFIT_LOSS_LINEAR, nullptr,
+                                  max_iter, xtol, f_out, passes_out, accepted_out, status_out, stream);
 }
 
 int nmrfit_normal_eq_plan(int n_points, int n_peaks, int* out) {

@@ -18,24 +18,17 @@
 #include <cuda_runtime.h>
 #include <algorithm>
 #include "nmrfit_internal.h"
+#include "gram_blocks.cuh"
 #include "normal_eq_rows.cuh"
 
 namespace nmrfit {
 
 namespace {
 
-constexpr int RB = 4;                       // register block edge
 constexpr int kSmemCap = 200 * 1024 / 8;    // doubles of dynamic shared memory the M kernel opts into
 constexpr int kTileTarget = 96 * 1024 / 8;  // staged rows aimed at per CTA: two CTAs per SM
 constexpr int kAcfChunk = 512;
 constexpr int kAcfThreads = 256;
-
-__device__ __forceinline__ void tri_block(int q, int nb, int* bi, int* bj) {
-    int i = 0;
-    while (q >= nb - i) { q -= nb - i; ++i; }
-    *bi = i;
-    *bj = i + q;
-}
 
 __device__ __forceinline__ void load_peaks(const double* x, int P, PeakK* pk) {
     for (int k = threadIdx.x; k < P; k += blockDim.x) {
@@ -64,15 +57,8 @@ __global__ void __launch_bounds__(kAcfThreads) residual_acf_partial_kernel(const
     for (int i = tid; i < CH + L; i += nt) {
         const int pt = c0 + i;
         if (pt >= N) { res[i] = 0.0; continue; }
-        double fit = 0.0, dr = 0.0;
-        for (int k = 0; k < P; ++k) {                          // peaks in index order, as K12 sums them
-            double f, d;
-            ne_peak_terms(pk[k], sw[pt], r, yoff, [](double, double, double) {}, &f, &d);
-            fit += f;
-            dr += d;
-        }
-        double a[4], wt, rs;
-        ne_point_terms(p0, p1, pt, N, rN, sw, fit, dr, P, a, &wt, &rs);
+        double wt, rs;
+        ne_residual(pk, P, p0, p1, r, yoff, pt, N, rN, sw, &wt, &rs);
         res[i] = rs;
     }
     __syncthreads();
@@ -127,17 +113,13 @@ __global__ void __launch_bounds__(512) lagged_m_partial_kernel(const double* __r
     for (int k = tid; k <= L; k += nt) rk[k] = rho[(size_t)b * (L + 1) + k];
     for (int idx = tid; idx < (R + TP) * EP; idx += nt) rows[idx] = 0.0;    // padding columns stay zero
 
-    const int task0 = slice * p.tasks_per_slice;
-    const int grp = p.ng > 1 ? tid / p.tasks : 0;
-    const int task = task0 + (p.ng > 1 ? tid - grp * p.tasks : tid);
-    const bool active = grp < p.ng && task < p.tasks && (p.ng > 1 || tid < p.tasks_per_slice);
+    int grp, task;
+    bool active;
+    gram_task(p, slice, tid, &grp, &task, &active);
     int bi = 0, bj = 0;
     if (active) tri_block(task, p.nb, &bi, &bj);
     double acc[RB][RB];
-#pragma unroll
-    for (int i = 0; i < RB; ++i)
-#pragma unroll
-        for (int j = 0; j < RB; ++j) acc[i][j] = 0.0;
+    gram_zero(acc);
 
     const int c0 = chunk * p.chunk, c1 = min(c0 + p.chunk, N);
     const double rN = (double)N;
@@ -201,27 +183,7 @@ __global__ void __launch_bounds__(512) lagged_m_partial_kernel(const double* __r
             }
         }
     }
-    double* out = part + (((size_t)b * gridDim.x + chunk) * p.tasks) * (RB * RB);
-    if (p.ng > 1) {
-        __syncthreads();
-        if (active)
-#pragma unroll
-            for (int u = 0; u < RB; ++u)
-#pragma unroll
-                for (int v = 0; v < RB; ++v) red[tid * RB * RB + u * RB + v] = acc[u][v];
-        __syncthreads();
-        for (int idx = tid; idx < p.tasks * RB * RB; idx += nt) {
-            const int tk = idx / (RB * RB), e = idx - tk * (RB * RB);
-            double s = 0.0;
-            for (int gi = 0; gi < p.ng; ++gi) s += red[(gi * p.tasks + tk) * RB * RB + e];
-            out[idx] = s;
-        }
-    } else if (active) {
-#pragma unroll
-        for (int u = 0; u < RB; ++u)
-#pragma unroll
-            for (int v = 0; v < RB; ++v) out[(size_t)task * RB * RB + u * RB + v] = acc[u][v];
-    }
+    gram_store(p, acc, active, task, tid, nt, red, part + (((size_t)b * gridDim.x + chunk) * p.tasks) * (RB * RB));
 }
 
 // fixed-order sum over chunks; one thread per (spectrum, j, k) of the D x D square, both triangles from (min, max)
@@ -233,9 +195,8 @@ __global__ void lagged_m_reduce_kernel(const double* __restrict__ part, LaggedPl
     const int rem = (int)(idx - (long long)b * D * D);
     const int j0 = rem / D, k0 = rem % D;
     const int j = min(j0, k0), k = max(j0, k0);
-    const int bi = j / RB, bj = k / RB;
-    const int q = bi * p.nb - bi * (bi - 1) / 2 + (bj - bi);
-    const double* src = part + ((size_t)b * p.n_chunks * p.tasks + q) * (RB * RB) + (j % RB) * RB + (k % RB);
+    const double* src =
+        part + ((size_t)b * p.n_chunks * p.tasks + tri_index(j, k, p.nb)) * (RB * RB) + (j % RB) * RB + (k % RB);
     double s = 0.0;
     for (int c = 0; c < p.n_chunks; ++c) s += src[(size_t)c * p.tasks * RB * RB];
     M[idx] = s;
@@ -252,33 +213,15 @@ LaggedPlan lagged_plan(int N, int P, int L) {
     LaggedPlan p{};
     p.N = N; p.P = P; p.L = L;
     const int D = 4 + 3 * P;
-    p.nb = (D + RB - 1) / RB;
-    p.ep = p.nb * RB;
-    p.tasks = p.nb * (p.nb + 1) / 2;
-    if (p.tasks <= 128) {                                 // few blocks: point groups share the tile
-        p.ng = 256 / p.tasks;
-        p.slices = 1;
-        p.tasks_per_slice = p.tasks;
-        p.threads = (p.ng * p.tasks + 31) / 32 * 32;
-    } else {                                              // many blocks: up to 512 per CTA, the rest in further slices
-        p.ng = 1;
-        p.slices = (p.tasks + 511) / 512;
-        p.tasks_per_slice = (p.tasks + p.slices - 1) / p.slices;
-        p.threads = (p.tasks_per_slice + 31) / 32 * 32;
-    }
+    gram_layout(p, D, 1);
     // the largest L whose 16-point tile fits the shared memory the kernel opts into
     const long long fixed = (long long)32 * p.ep + 16LL * P + (long long)P * (sizeof(PeakK) / sizeof(double)) + 1;
     p.max_lag = (int)std::max(0LL, ((long long)kSmemCap - fixed) / (2LL * p.ep + 1));
     int tp = 128;                                         // staged rows and halo: about 96 KB
     while (tp > 16 && m_stage(tp, L, p.ep, P) > (size_t)kTileTarget) tp /= 2;
     p.tp = tp;
-    // chunk: about 2^22 Gram FMAs, between 256 points and N/128 rounded up (as K12)
-    const long long target = (1LL << 22) / ((long long)D * D);
-    int ch = 256;
-    while ((long long)ch * 2 <= target && ch < 16384) ch *= 2;
-    while ((long long)ch * 128 < N) ch *= 2;
-    p.chunk = ch;
-    p.n_chunks = (N + ch - 1) / ch;
+    p.chunk = gram_chunk(N, D);
+    p.n_chunks = (N + p.chunk - 1) / p.chunk;
     p.smem = sizeof(double) * std::max(m_stage(tp, L, p.ep, P), (size_t)p.threads * RB * RB);
     p.acf_chunk = kAcfChunk;
     p.acf_n_chunks = (N + kAcfChunk - 1) / kAcfChunk;
@@ -308,17 +251,10 @@ cudaError_t launch_residual_acf(const double* spec, const double* x, const Lagge
 
 cudaError_t launch_lagged_m(const double* spec, const double* x, const double* rho, const LaggedPlan& p, int B,
                             double* part, double* M, cudaStream_t st) {
-    static bool attr_set[NMRFIT_MAX_DEVICES] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-        cudaError_t e = cudaFuncSetAttribute(lagged_m_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             kSmemCap * 8);
-        if (e != cudaSuccess) return e;
-        attr_set[dev % NMRFIT_MAX_DEVICES] = true;
-    }
+    cudaError_t e = opt_in_smem<lagged_m_partial_kernel>(kSmemCap * 8);
+    if (e != cudaSuccess) return e;
     lagged_m_partial_kernel<<<dim3(p.n_chunks, p.slices, B), p.threads, p.smem, st>>>(spec, x, rho, p, part);
-    cudaError_t e = cudaGetLastError();
+    e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int D = 4 + 3 * p.P;
     const long long total = (long long)B * D * D;

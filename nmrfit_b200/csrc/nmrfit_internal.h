@@ -10,6 +10,19 @@ namespace nmrfit {
 
 void count_launches(int n);   // bookkeeping for nmrfit_launch_count()
 
+// Opts `Kernel` into `bytes` of dynamic shared memory on the current device.  The attribute is per device, so it is
+// set once per device and kernel (each instantiation of this template keeps its own record).
+template <auto Kernel>
+cudaError_t opt_in_smem(int bytes) {
+    static bool done[NMRFIT_MAX_DEVICES] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (done[dev % NMRFIT_MAX_DEVICES]) return cudaSuccess;
+    cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess) done[dev % NMRFIT_MAX_DEVICES] = true;
+    return e;
+}
+
 // ---- K1 objective -------------------------------------------------------------
 struct ObjArgs {
     const double* spec;     // [B][4][N]: w, u, v, weights

@@ -20,22 +20,13 @@
 #include <cuda_runtime.h>
 #include <algorithm>
 #include "nmrfit_internal.h"
+#include "gram_blocks.cuh"
 #include "normal_eq_rows.cuh"
 #include "robust_loss.cuh"
 
 namespace nmrfit {
 
 namespace {
-
-constexpr int RB = 4;                  // register block edge
-
-// upper-triangle block q of an nb x nb block grid -> (row block, column block), row-major over bi <= bj
-__device__ __forceinline__ void tri_block(int q, int nb, int* bi, int* bj) {
-    int i = 0;
-    while (q >= nb - i) { q -= nb - i; ++i; }
-    *bi = i;
-    *bj = i + q;
-}
 
 // fscale [B]: the loss's scale c of each spectrum (not read by LossLinear)
 template <typename Loss>
@@ -65,20 +56,16 @@ __global__ void __launch_bounds__(512) normal_eq_partial_kernel(const double* __
     for (int idx = tid; idx < 2 * TP * EP; idx += nt) rows[idx] = 0.0;    // padding columns stay zero
 
     // this thread's block of the Gram matrices
-    const int task0 = slice * p.tasks_per_slice;
-    const int grp = p.ng > 1 ? tid / p.tasks : 0;
-    const int task = task0 + (p.ng > 1 ? tid - grp * p.tasks : tid);
-    const bool active = grp < p.ng && task < p.tasks && (p.ng > 1 || tid < p.tasks_per_slice);
+    int grp, task;
+    bool active;
+    gram_task(p, slice, tid, &grp, &task, &active);
     int mat = 0, bi = 0, bj = 0;
     if (active) {
         mat = task / p.tri;
         tri_block(task - mat * p.tri, p.nb, &bi, &bj);
     }
     double acc[RB][RB];
-#pragma unroll
-    for (int i = 0; i < RB; ++i)
-#pragma unroll
-        for (int j = 0; j < RB; ++j) acc[i][j] = 0.0;
+    gram_zero(acc);
 
     const int c0 = chunk * p.chunk, c1 = min(c0 + p.chunk, N);
     const double rN = (double)N;
@@ -159,27 +146,7 @@ __global__ void __launch_bounds__(512) normal_eq_partial_kernel(const double* __
         }
     }
     // point groups added in group order, then one block per task to the chunk's partials
-    double* out = part + (((size_t)b * gridDim.x + chunk) * p.tasks) * (RB * RB);
-    if (p.ng > 1) {
-        __syncthreads();
-        if (active)
-#pragma unroll
-            for (int u = 0; u < RB; ++u)
-#pragma unroll
-                for (int v = 0; v < RB; ++v) red[tid * RB * RB + u * RB + v] = acc[u][v];
-        __syncthreads();
-        for (int idx = tid; idx < p.tasks * RB * RB; idx += nt) {
-            const int tk = idx / (RB * RB), e = idx - tk * (RB * RB);
-            double s = 0.0;
-            for (int gi = 0; gi < p.ng; ++gi) s += red[(gi * p.tasks + tk) * RB * RB + e];
-            out[idx] = s;
-        }
-    } else if (active) {
-#pragma unroll
-        for (int u = 0; u < RB; ++u)
-#pragma unroll
-            for (int v = 0; v < RB; ++v) out[(size_t)task * RB * RB + u * RB + v] = acc[u][v];
-    }
+    gram_store(p, acc, active, task, tid, nt, red, part + (((size_t)b * gridDim.x + chunk) * p.tasks) * (RB * RB));
 }
 
 // fixed-order sum over chunks; one thread per (spectrum, matrix, j, k) of the E x E square, both triangles
@@ -195,9 +162,7 @@ __global__ void normal_eq_reduce_kernel(const double* __restrict__ part, NormalE
     const int mat = rem / (E * E), j0 = (rem / E) % E, k0 = rem % E;
     if (mat == 1 && (j0 == D) != (k0 == D)) return;      // M_ext's last column repeats g
     const int j = min(j0, k0), k = max(j0, k0);
-    const int bi = j / RB, bj = k / RB;
-    const int q = bi * p.nb - bi * (bi - 1) / 2 + (bj - bi);
-    const int task = mat * p.tri + q, e = (j % RB) * RB + (k % RB);
+    const int task = mat * p.tri + tri_index(j, k, p.nb), e = (j % RB) * RB + (k % RB);
     const double* src = part + ((size_t)b * n_chunks * p.tasks + task) * (RB * RB) + e;
     double s = 0.0;
     for (int c = 0; c < n_chunks; ++c) s += src[(size_t)c * p.tasks * RB * RB];
@@ -215,31 +180,12 @@ NormalEqPlan normal_eq_plan(int N, int P) {
     NormalEqPlan p{};
     p.N = N; p.P = P;
     const int D = 4 + 3 * P, E = D + 1;
-    p.nb = (E + RB - 1) / RB;
-    p.ep = p.nb * RB;
-    p.tri = p.nb * (p.nb + 1) / 2;
-    p.tasks = 2 * p.tri;
-    if (p.tasks <= 128) {                                 // few blocks: point groups share the tile
-        p.ng = 256 / p.tasks;
-        p.slices = 1;
-        p.tasks_per_slice = p.tasks;
-        p.threads = (p.ng * p.tasks + 31) / 32 * 32;
-    } else {                                              // many blocks: up to 512 per CTA, the rest in further slices
-        p.ng = 1;
-        p.slices = (p.tasks + 511) / 512;
-        p.tasks_per_slice = (p.tasks + p.slices - 1) / p.slices;
-        p.threads = (p.tasks_per_slice + 31) / 32 * 32;
-    }
+    p.tri = gram_layout(p, E, 2);
     int tp = 128;                                         // staged rows of both matrices: about 48 KB
     while (tp > 16 && 2 * tp * p.ep > 6144) tp /= 2;
     p.tp = tp;
-    // chunk: about 2^22 Gram FMAs per matrix, between 256 points and N/128 rounded up
-    const long long target = (1LL << 22) / ((long long)E * E);
-    int ch = 256;
-    while ((long long)ch * 2 <= target && ch < 16384) ch *= 2;
-    while ((long long)ch * 128 < N) ch *= 2;
-    p.chunk = ch;
-    p.n_chunks = (N + ch - 1) / ch;
+    p.chunk = gram_chunk(N, E);
+    p.n_chunks = (N + p.chunk - 1) / p.chunk;
     const size_t stage = (size_t)2 * tp * p.ep + (size_t)2 * tp * P + (size_t)P * (sizeof(PeakK) / sizeof(double));
     p.smem = sizeof(double) * std::max(stage, (size_t)p.threads * RB * RB);
     return p;
@@ -254,18 +200,11 @@ namespace {
 template <typename Loss>
 cudaError_t launch_pass(const double* spec, const double* x, const double* fscale, const NormalEqPlan& p, int B,
                         double* part, double* out, cudaStream_t st) {
-    static bool attr_set[NMRFIT_MAX_DEVICES] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-        cudaError_t e = cudaFuncSetAttribute(normal_eq_partial_kernel<Loss>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev % NMRFIT_MAX_DEVICES] = true;
-    }
+    cudaError_t e = opt_in_smem<normal_eq_partial_kernel<Loss>>(200 * 1024);
+    if (e != cudaSuccess) return e;
     dim3 grid(p.n_chunks, p.slices, B);
     normal_eq_partial_kernel<Loss><<<grid, p.threads, p.smem, st>>>(spec, x, p, part, fscale);
-    cudaError_t e = cudaGetLastError();
+    e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const int E = 5 + 3 * p.P;
     const long long total = (long long)B * 2 * E * E;

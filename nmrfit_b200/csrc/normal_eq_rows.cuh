@@ -4,7 +4,8 @@
 // With res_i = Vdata_i(p0, p1) - Vfit_i(x) and A_i = d res_i / dx (D = 4 + 3P columns):
 //   per (point, peak): the peak's three columns of A, its model value and its d/dr term   (ne_peak_terms)
 //   per point:         the phase, the residual and the four global columns                 (ne_point_terms)
-// The model value and the d/dr term are summed over the peaks in index order by the caller.
+// The model value and the d/dr term are summed over the peaks in index order by the caller, or by ne_residual for the
+// passes that need the residual only (K14's residual pass, K16's moments in robust.cu).
 // The statement order here (columns handed to the caller before the model value is formed, the weight loaded after the
 // phase) is the order K12 had before it was factored out: its SASS is byte-identical to that version.
 #pragma once
@@ -61,6 +62,21 @@ __device__ __forceinline__ void ne_point_terms(double p0, double p1, int pt, int
     a[3] = -(double)P;
     *wt = sw[3 * N + pt];
     *res = vd - fit;
+}
+
+// the residual walk of point pt for the passes that need no Jacobian row: the model and its d/dr summed over the
+// peaks pk [P] in index order, as K12 sums them, then ne_point_terms -> the point's weight and residual
+__device__ __forceinline__ void ne_residual(const PeakK* pk, int P, double p0, double p1, double r, double yoff, int pt,
+                                            int N, double rN, const double* sw, double* wt, double* res) {
+    double fit = 0.0, dr = 0.0;
+    for (int k = 0; k < P; ++k) {
+        double f, d;
+        ne_peak_terms(pk[k], sw[pt], r, yoff, [](double, double, double) {}, &f, &d);
+        fit += f;
+        dr += d;
+    }
+    double a[4];
+    ne_point_terms(p0, p1, pt, N, rN, sw, fit, dr, P, a, wt, res);
 }
 
 }  // namespace nmrfit

@@ -235,17 +235,10 @@ __global__ void objective_finalize_kernel(const double* __restrict__ partials, i
 // ---- launcher -----------------------------------------------------------------
 template <int THREADS, int R, int TB, int KK>
 static cudaError_t launch_one(const ObjArgs& a, dim3 grid, cudaStream_t st) {
-    static bool attr_set[NMRFIT_MAX_DEVICES] = {};
     ObjSmem L(a.sp, a.P, THREADS / 32, R, TB, KK ? 2 : 1);
     size_t bytes = (size_t)L.total * sizeof(double);
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-        cudaError_t e = cudaFuncSetAttribute(objective_kernel<THREADS, R, TB, KK>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev % NMRFIT_MAX_DEVICES] = true;
-    }
+    cudaError_t e = opt_in_smem<objective_kernel<THREADS, R, TB, KK>>(200 * 1024);
+    if (e != cudaSuccess) return e;
     objective_kernel<THREADS, R, TB, KK><<<grid, THREADS, bytes, st>>>(a);
     return cudaGetLastError();
 }

@@ -326,16 +326,9 @@ size_t objective_f32_smem_bytes(int P, const ObjTune& t) {
 
 template <int THREADS, int R>
 static cudaError_t launch_uniform_f32(const ObjArgs& a, int B, cudaStream_t st) {
-    static bool attr_set[NMRFIT_MAX_DEVICES] = {};
     const size_t bytes = (size_t)F32Smem(a.sp, a.P, THREADS, R).total * sizeof(double);
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-        cudaError_t e = cudaFuncSetAttribute(objective_uniform_f32_kernel<THREADS, R>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev % NMRFIT_MAX_DEVICES] = true;
-    }
+    cudaError_t e = opt_in_smem<objective_uniform_f32_kernel<THREADS, R>>(200 * 1024);
+    if (e != cudaSuccess) return e;
     dim3 grid((a.S + a.sp - 1) / a.sp, a.n_tiles, B);
     objective_uniform_f32_kernel<THREADS, R><<<grid, THREADS, bytes, st>>>(a);
     return cudaGetLastError();
@@ -360,14 +353,8 @@ cudaError_t launch_objective_f32(ObjArgs a, const ObjTune& t, int B, double* f, 
         n_tiles = a.n_tiles;
         count_launches(1);
     } else {
-        static bool attr_set[NMRFIT_MAX_DEVICES] = {};
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-            e = cudaFuncSetAttribute(objective_general_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-            if (e != cudaSuccess) return e;
-            attr_set[dev % NMRFIT_MAX_DEVICES] = true;
-        }
+        e = opt_in_smem<objective_general_f32_kernel>(200 * 1024);
+        if (e != cudaSuccess) return e;
         a.sp = t.sp;
         n_tiles = (a.N + kGenThreads32 * kGenR32 - 1) / (kGenThreads32 * kGenR32);
         const size_t bytes = ((size_t)a.sp * a.P * 3 + (size_t)a.sp * (kGenThreads32 / 32)) * sizeof(double);

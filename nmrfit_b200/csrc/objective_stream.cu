@@ -225,17 +225,10 @@ objective_stream_kernel(ObjArgs a) {
 
 template <int THREADS, int R, int TB, int KK, int OCC, int SUB>
 cudaError_t launch_sub(const ObjArgs& a, int B, cudaStream_t st) {
-    static bool attr_set[NMRFIT_MAX_DEVICES] = {};
     StreamSmem L(a.sp, a.stages, a.P, THREADS, R, TB, a.sub);
     const size_t bytes = (size_t)L.total * sizeof(double);
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-        cudaError_t e = cudaFuncSetAttribute(objective_stream_kernel<THREADS, R, TB, KK, OCC, SUB>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev % NMRFIT_MAX_DEVICES] = true;
-    }
+    cudaError_t e = opt_in_smem<objective_stream_kernel<THREADS, R, TB, KK, OCC, SUB>>(200 * 1024);
+    if (e != cudaSuccess) return e;
     const int n_groups = (a.S + a.sp - 1) / a.sp;
     dim3 grid((n_groups + a.gpc - 1) / a.gpc, a.n_tiles, B);
     objective_stream_kernel<THREADS, R, TB, KK, OCC, SUB><<<grid, THREADS, bytes, st>>>(a);

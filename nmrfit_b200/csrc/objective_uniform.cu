@@ -304,17 +304,10 @@ objective_uniform_kernel(ObjArgs a) {
 // ---- launcher -----------------------------------------------------------------
 template <int THREADS, int R, int TB, int KK>
 static cudaError_t launch_one(const ObjArgs& a, int B, cudaStream_t st) {
-    static bool attr_set[NMRFIT_MAX_DEVICES] = {};
     UniSmem L(a.sp, a.P, THREADS, R, TB, KK ? 2 : 1, a.sub);
     const size_t bytes = (size_t)L.total * sizeof(double);
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-        cudaError_t e = cudaFuncSetAttribute(objective_uniform_kernel<THREADS, R, TB, KK>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev % NMRFIT_MAX_DEVICES] = true;
-    }
+    cudaError_t e = opt_in_smem<objective_uniform_kernel<THREADS, R, TB, KK>>(200 * 1024);
+    if (e != cudaSuccess) return e;
     dim3 grid((a.S + a.sp - 1) / a.sp, a.n_tiles, B);
     objective_uniform_kernel<THREADS, R, TB, KK><<<grid, THREADS, bytes, st>>>(a);
     return cudaGetLastError();

@@ -250,15 +250,8 @@ template <bool kTied>
 cudaError_t launch_step(const double* trial, double* cur, RefineState* state, double* xc, double* xt, const double* lb,
                         const double* ub, int B, int N, int D, int max_iter, double xtol, int* active,
                         const RefineTies& ties, cudaStream_t st) {
-    static bool attr_set[NMRFIT_MAX_DEVICES] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-        cudaError_t e = cudaFuncSetAttribute(refine_step_kernel<kTied>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             200 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev % NMRFIT_MAX_DEVICES] = true;
-    }
+    cudaError_t e = opt_in_smem<refine_step_kernel<kTied>>(200 * 1024);
+    if (e != cudaSuccess) return e;
     const int threads = std::min(256, (D + 31) / 32 * 32);   // one row of the factor per thread
     refine_step_kernel<kTied><<<B, threads, refine_step_smem(D), st>>>(trial, cur, state, xc, xt, lb, ub, N, D,
                                                                        max_iter, xtol, active, ties);

@@ -44,15 +44,8 @@ __global__ void __launch_bounds__(kThreads) loss_moments_partial_kernel(const do
     const double rN = (double)N;
     double m[kMoments] = {0.0, 0.0, 0.0, 0.0, 0.0};
     for (int pt = c0 + tid; pt < c1; pt += nt) {
-        double fit = 0.0, dr = 0.0;
-        for (int k = 0; k < P; ++k) {                                  // peaks in index order, as K12 sums them
-            double f, d;
-            ne_peak_terms(pk[k], sw[pt], r, yoff, [](double, double, double) {}, &f, &d);
-            fit += f;
-            dr += d;
-        }
-        double a[4], wt, res;
-        ne_point_terms(p0, p1, pt, N, rN, sw, fit, dr, P, a, &wt, &res);
+        double wt, res;
+        ne_residual(pk, P, p0, p1, r, yoff, pt, N, rN, sw, &wt, &res);
         const double wr = wt * res;
         double q = wr, psi = res, dpsi = 1.0;
         if constexpr (Loss::kRobust) {

@@ -89,14 +89,8 @@ cudaError_t launch_weights(double* spec, double* scratch, const double* bounds_d
                            int N, int n_windows, int sweeps, double omega, cudaStream_t st) {
     const size_t smem = sizeof(int) * 2 * ((n_windows + 1) & ~1) + sizeof(double) * n_windows;
     if (smem > 48 * 1024) {                                // up to 4,096 windows (64 KB): beyond the default limit
-        static bool attr_set[NMRFIT_MAX_DEVICES] = {};
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (!attr_set[dev % NMRFIT_MAX_DEVICES]) {
-            cudaError_t e = cudaFuncSetAttribute(weights_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 80 * 1024);
-            if (e != cudaSuccess) return e;
-            attr_set[dev % NMRFIT_MAX_DEVICES] = true;
-        }
+        cudaError_t e = opt_in_smem<weights_kernel>(80 * 1024);
+        if (e != cudaSuccess) return e;
     }
     // numpy evaluates (1. - omega) * x[1:-1] + omega * 0.5 * (x[2:] + x[:-2]) with the scalars folded first
     weights_kernel<<<B, kWThreads, smem, st>>>(spec, scratch, bounds_dev, values_dev, N, n_windows, sweeps, 1.0 - omega,

@@ -537,6 +537,17 @@ def _check_noise_args(noise, max_lag, noise_acf, B, N, P):
     return rho.shape[1] - 1, rho
 
 
+def stack_fits(fits, fields):
+    """The device inputs of a batch of fits of equal length and peak count: ``W, U, V, weights`` [B, N] from each
+    fit's data and weights, then one [B, D] array per attribute named in ``fields``, all float64."""
+    N, D = len(fits[0].data.w), len(fits[0].params)
+    for f in fits:
+        if len(f.data.w) != N or len(f.params) != D:
+            raise ValueError('every fit of a batch must have the same number of points and peaks')
+    rows = [(f.data.w, f.data.u, f.data.v, f.weights) + tuple(getattr(f, k) for k in fields) for f in fits]
+    return tuple(np.stack([_cabi.as_f64(a) for a in arrs]) for arrs in zip(*rows))
+
+
 def compute_uncertainties_batch(fits, noise='white', max_lag=32, noise_acf=None):
     """``compute_uncertainties()`` for many fits of equal length and peak count (what ``fit_batch`` returns) in one
     device pass: the normal equations of every spectrum at its fitted ``params`` with its fit's ``weights``, then
@@ -568,10 +579,8 @@ def compute_uncertainties_batch(fits, noise='white', max_lag=32, noise_acf=None)
         if f.fit_im:
             raise NotImplementedError('uncertainties are not available with fit_im: that objective is a sum of two '
                                       'RMSEs, not a least-squares problem')
-    N, D = len(fits[0].data.w), len(fits[0].params)
-    for f in fits:
-        if len(f.data.w) != N or len(f.params) != D:
-            raise ValueError('every fit of a batch must have the same number of points and peaks')
+    W, U, V, weights, X = stack_fits(fits, ('params',))
+    N, D = W.shape[1], X.shape[1]
     ties = [getattr(f, 'ties', None) for f in fits]
     losses = [getattr(f, 'loss', None) for f in fits]
     if noise == 'correlated' and any(lo is not None for lo in losses):
@@ -582,9 +591,6 @@ def compute_uncertainties_batch(fits, noise='white', max_lag=32, noise_acf=None)
         raise ValueError('the spectrum has %d points for %d parameters: no residual degrees of freedom' % (N, d))
     B, P = len(fits), (D - 4) // 3
     L, rho = _check_noise_args(noise, max_lag, noise_acf, B, N, P)
-    W, U, V, weights = (np.stack([_cabi.as_f64(a) for a in arrs])
-                        for arrs in zip(*[(f.data.w, f.data.u, f.data.v, f.weights) for f in fits]))
-    X = np.stack([_cabi.as_f64(f.params) for f in fits])
     with _cabi.pooled_context(B, N, P, device=fits[0].options.get('device')) as ctx:
         ctx.set_spectra(W, U, V, weights)
         H, M, g, ssr = ctx.normal_equations(X)
@@ -714,16 +720,11 @@ def refine_batch(fits, max_iter=None, xtol=1e-6, ties=None, loss='linear', f_sca
         return []
     for f in fits:
         _check_refinable(f, fitted=True)
-    N, D = len(fits[0].data.w), len(fits[0].params)
-    for f in fits:
-        if len(f.data.w) != N or len(f.params) != D:
-            raise ValueError('every fit of a batch must have the same number of points and peaks')
+    W, U, V, weights, X, LB, UB = stack_fits(fits, ('params', 'lower', 'upper'))
+    N, D = W.shape[1], X.shape[1]
     per, arrays = batch_ties(ties, len(fits), (D - 4) // 3)
     _cabi.check_loss(loss, f_scale, len(fits))
     max_iter = default_max_iter(max_iter, loss)
-    W, U, V, weights = (np.stack([_cabi.as_f64(a) for a in arrs])
-                        for arrs in zip(*[(f.data.w, f.data.u, f.data.v, f.weights) for f in fits]))
-    X, LB, UB = (np.stack([_cabi.as_f64(getattr(f, k)) for f in fits]) for k in ('params', 'lower', 'upper'))
     if arrays is None:
         _cabi.check_refine_args(X, LB, UB, max_iter, xtol, len(fits), N, (D - 4) // 3)
     else:
