@@ -1,6 +1,6 @@
-// Host build of nmrfit_b200/csrc/nmrfit_math.cuh for accuracy tests without a GPU.
-// Compiled by tests/test_host_math.py with g++ into a shared object; the product
-// never links or loads it.
+// Host build of nmrfit_b200/csrc/nmrfit_math.cuh and robust_loss.cuh for accuracy tests without a GPU.
+// Compiled by tests/test_host_math.py and tests/test_robust_loss_host.py with g++ into a shared object;
+// the product never links or loads it.
 #define NMRFIT_HOST_MATH 1
 #define __device__
 #define __host__
@@ -8,6 +8,13 @@
 #define __forceinline__ inline
 #include <vector>
 #include "../nmrfit_b200/csrc/nmrfit_math.cuh"
+#include "../nmrfit_b200/csrc/robust_loss.cuh"
+
+// Loss::eval of one loss (NMRFIT_LOSS_*) at z[0..n): rho, rho' and psi' = rho' + 2 z rho''
+template <typename Loss>
+static void loss_eval(const double* z, int n, double* rho, double* d1, double* dpsi) {
+    for (int i = 0; i < n; ++i) Loss::eval(z[i], rho + i, d1 + i, dpsi + i);
+}
 
 // Sum of peaks over a uniform grid w_i = w[0] + i*h, evaluated span by span exactly as
 // objective_uniform_kernel does it: anchors at the true w of every R-th point.
@@ -136,6 +143,15 @@ void h_span_fit(const double* w, int n, double h, const double* x, int P, int R,
         if (R == 4) spans<4, 10>(w, n, h, x, P, NMRFIT_EXP2_TAB10, vfit);
         else if (R == 8) spans<8, 10>(w, n, h, x, P, NMRFIT_EXP2_TAB10, vfit);
         else spans<16, 10>(w, n, h, x, P, NMRFIT_EXP2_TAB10, vfit);
+    }
+}
+
+void h_loss(int loss, const double* z, int n, double* rho, double* d1, double* dpsi) {
+    switch (loss) {
+        case NMRFIT_LOSS_HUBER: loss_eval<nmrfit::LossHuber>(z, n, rho, d1, dpsi); break;
+        case NMRFIT_LOSS_SOFT_L1: loss_eval<nmrfit::LossSoftL1>(z, n, rho, d1, dpsi); break;
+        case NMRFIT_LOSS_CAUCHY: loss_eval<nmrfit::LossCauchy>(z, n, rho, d1, dpsi); break;
+        default: loss_eval<nmrfit::LossLinear>(z, n, rho, d1, dpsi); break;
     }
 }
 

@@ -11,7 +11,8 @@ LOSSES = ('linear', 'huber', 'soft_l1', 'cauchy')
 
 
 def loss_terms(z, loss):
-    """``(rho, rho', rho'')`` of ``loss`` at z >= 0 (scipy.optimize.least_squares' convention), in z's dtype."""
+    """``(rho, rho', rho'')`` of ``loss`` at z >= 0 (scipy.optimize.least_squares' convention), in z's dtype, in forms
+    without cancellation (soft-L1's rho = 2 z / (sqrt(1 + z) + 1), not scipy's 2 (sqrt(1 + z) - 1))."""
     z = np.asarray(z)
     one = np.ones_like(z)
     if loss == 'linear':
@@ -22,7 +23,8 @@ def loss_terms(z, loss):
         return np.where(inner, z, 2 * s - 1), np.where(inner, one, 1 / s), np.where(inner, 0 * z, -0.5 / (s * s * s))
     if loss == 'soft_l1':
         t = 1 + z
-        return 2 * (np.sqrt(t) - 1), 1 / np.sqrt(t), -0.5 / (t * np.sqrt(t))
+        s = np.sqrt(t)
+        return 2 * z / (s + 1), 1 / s, -0.5 / (t * s)
     if loss == 'cauchy':
         t = 1 + z
         return np.log1p(z), 1 / t, -1 / (t * t)
@@ -30,9 +32,21 @@ def loss_terms(z, loss):
 
 
 def psi_prime(z, loss):
-    """psi'(r) = rho'(z) + 2 z rho''(z) at z = (r/c)^2."""
-    _, d1, d2 = loss_terms(z, loss)
-    return d1 + 2 * z * d2
+    """psi'(r) = rho'(z) + 2 z rho''(z) at z = (r/c)^2, in z's dtype, in closed form: 1 inside c and exactly 0 beyond
+    for Huber (rho' + 2 z rho'' leaves a rounding residue of either sign there, which decides the sign of sum psi' when
+    no point lies inside c), (1 + z)^-1.5 for soft-L1 and (1 - z) / (1 + z)^2 for Cauchy."""
+    z = np.asarray(z)
+    one = np.ones_like(z)
+    if loss == 'linear':
+        return one
+    if loss == 'huber':
+        return np.where(z <= 1, one, 0 * z)
+    t = 1 + z
+    if loss == 'soft_l1':
+        return 1 / (t * np.sqrt(t))
+    if loss == 'cauchy':
+        return (1 - z) / t / t
+    raise ValueError(loss)
 
 
 def _terms(x, w, u, v, weights, loss, c):
@@ -57,8 +71,8 @@ def robust_pass(x, w, u, v, weights, loss, c):
 
 def moments(x, w, u, v, weights, loss, c):
     """(cost, sum w^2 res^2, sum psi^2, sum psi', sum psi'^2) in long double, psi = rho' res."""
-    r, _, w2, c, z, rho, d1, d2 = _terms(x, w, u, v, weights, loss, 1.0 if loss == 'linear' else c)
-    psi, dpsi = d1 * r, d1 + 2 * z * d2
+    r, _, w2, c, z, rho, d1, _ = _terms(x, w, u, v, weights, loss, 1.0 if loss == 'linear' else c)
+    psi, dpsi = d1 * r, psi_prime(z, loss)
     cost = np.sum(w2 * r * r) if loss == 'linear' else np.sum(w2 * c * c * rho)
     return np.array([cost, np.sum(w2 * r * r), np.sum(psi * psi), np.sum(dpsi), np.sum(dpsi * dpsi)],
                     dtype=np.float64)

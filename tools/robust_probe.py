@@ -1,10 +1,11 @@
 #!/usr/bin/env python
-"""Huber against least-squares refinement (DESIGN K16) on one GPU, from the same swarm answers.
+"""A robust loss (Huber by default) against least-squares refinement (DESIGN K16) on one GPU, from the same swarm
+answers.
 
-    python tools/robust_probe.py [--reps 10] [--out profiles/robust_probe.json]
+    python tools/robust_probe.py [--reps 10] [--loss huber|soft_l1|cauchy] [--out profiles/robust_probe.json]
 
 For each workload the swarm runs once (fit_batch, device RNG), then Context.refine is timed from its answers with the
-linear loss (max_iter 50) and with Huber at c = 1.345 sigma (sigma = 1e-4, synth.multiplet's noise; max_iter
+linear loss (max_iter 50) and with the robust loss at c = 1.345 sigma (sigma = 1e-4, synth.multiplet's noise; max_iter
 utils.ROBUST_MAX_ITER, the library's default for a robust loss), which also gives how many spectra would end MAX_ITER
 at 50 passes (those that need more: the trajectory does not depend on max_iter): CUDA events on the call's
 stream, median of --reps calls, L2 overwritten (256 MiB fill) before each, outside the event pair; the two are timed
@@ -30,10 +31,9 @@ WORKLOADS = [
     dict(name='65536x24', B=1, N=65536, P=24, swarmsize=204, maxiter=200),
 ]
 C = 1.345e-4
-MAX_ITER = dict(linear=50, huber=utils.ROBUST_MAX_ITER)
 
 
-def probe(wl, reps, flush):
+def probe(wl, reps, flush, loss):
     import torch
     B, N, P = wl['B'], wl['N'], wl['P']
     datas, lows, ups = [], [], []
@@ -50,9 +50,9 @@ def probe(wl, reps, flush):
     with _cabi.Context(B, N, P) as ctx:
         ctx.set_spectra(*(np.stack([getattr(d, k) for d in datas]) for k in ('w', 'u', 'v')),
                         np.stack([f.weights for f in fits]))
-        runs = dict(linear=lambda: ctx.refine(X, LB, UB, max_iter=MAX_ITER['linear'], stream=stream),
-                    huber=lambda: ctx.refine(X, LB, UB, max_iter=MAX_ITER['huber'], stream=stream, loss='huber',
-                                             f_scale=C))
+        max_iter = {'linear': 50, loss: utils.ROBUST_MAX_ITER}
+        runs = {'linear': lambda: ctx.refine(X, LB, UB, max_iter=max_iter['linear'], stream=stream),
+                loss: lambda: ctx.refine(X, LB, UB, max_iter=max_iter[loss], stream=stream, loss=loss, f_scale=C)}
         results = {k: fn() for k, fn in runs.items()}
         times = {k: [] for k in runs}
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -68,10 +68,10 @@ def probe(wl, reps, flush):
             split = kernel_split(runs[k])
             x, f, passes, accepted, status = results[k]
             n_pass = int(passes.max())
-            iters = min(-(-n_pass // 8) * 8, MAX_ITER[k])   # passes launched: the running count is read every 8
+            iters = min(-(-n_pass // 8) * 8, max_iter[k])   # passes launched: the running count is read every 8
             ms = float(np.median(times[k]))
             rows[k] = dict(refine_ms=ms, refine_ms_min=float(np.min(times[k])), passes_max=n_pass,
-                           passes_median=float(np.median(passes)), iterations_run=iters, max_iter=MAX_ITER[k],
+                           passes_median=float(np.median(passes)), iterations_run=iters, max_iter=max_iter[k],
                            max_iter_at_50=int(np.sum(passes > 50)),
                            ms_per_iteration=ms / iters, normal_eq_ms_per_pass=split['normal_eq_ms'] / iters,
                            status_counts={str(a): int(c) for a, c in zip(*np.unique(status, return_counts=True))},
@@ -82,7 +82,8 @@ def probe(wl, reps, flush):
                       rows[k]['normal_eq_ms_per_pass'], rows[k]['status_counts'], rows[k]['max_iter_at_50']), flush=True)
     return dict(workload=wl['name'], spectra=B, n_points=N, n_peaks=P, D=4 + 3 * P, f_scale=C,
                 swarm=dict(swarmsize=wl['swarmsize'], maxiter=wl['maxiter']),
-                robust_pass_over_k12=rows['huber']['normal_eq_ms_per_pass'] / rows['linear']['normal_eq_ms_per_pass'],
+                loss=loss, robust_pass_over_k12=rows[loss]['normal_eq_ms_per_pass'] /
+                rows['linear']['normal_eq_ms_per_pass'],
                 **rows)
 
 
@@ -90,6 +91,7 @@ def main():
     import torch
     ap = argparse.ArgumentParser()
     ap.add_argument('--reps', type=int, default=10)
+    ap.add_argument('--loss', default='huber', choices=('huber', 'soft_l1', 'cauchy'))
     ap.add_argument('--out', default=os.path.join(ROOT, 'profiles', 'robust_probe.json'))
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -97,9 +99,10 @@ def main():
     gpu = gpu_identity()
     print('%s, power limit %s' % (gpu['name'], gpu.get('power_limit')), flush=True)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device='cuda')
-    rows = [probe(wl, args.reps, flush) for wl in WORKLOADS]
+    rows = [probe(wl, args.reps, flush, args.loss) for wl in WORKLOADS]
     out = dict(gpu=gpu, timing=dict(method='CUDA events around Context.refine on its stream, median of %d calls, '
-                                           'huber and linear alternated, L2 overwritten before each' % args.reps),
+                                           '%s and linear alternated, L2 overwritten before each'
+                                           % (args.reps, args.loss)),
                workloads=rows)
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, 'w') as fh:
