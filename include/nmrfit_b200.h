@@ -217,6 +217,19 @@ int nmrfit_ctx_refine_loss(nmrfit_ctx* ctx, double* x_inout, const double* lb, c
                            int max_iter, double xtol, double* f_out, int* passes_out, int* accepted_out,
                            int* status_out, void* stream);
 
+/* The residual scale (DESIGN K17), from the spectra the context holds, at one x [n_spectra][D] per spectrum, with
+ * res_i the unweighted residual of nmrfit_ctx_normal_equations over all n_points points:
+ *   nmrfit_ctx_residuals:      res_out [n_spectra][n_points] = res;
+ *   nmrfit_ctx_residual_scale: out [n_spectra][2] = (med, MAD), med = median(res) and MAD = median(|res - med|), each
+ *                              the value numpy's median gives (the middle order statistic, or (a + b) / 2 of the two
+ *                              middle ones for an even count; NaN for a row holding a NaN; -0 and +0 compare equal).
+ * The normal-consistent noise level is sigma = MAD / 0.6744897501960817 (the standard normal quantile at 3/4), as
+ * scipy.stats.median_abs_deviation(res, scale='normal').  Both run in FP64 on FP32 contexts too, and the selection is
+ * exact: the result is the same alone or in a batch and from call to call.  Host or device pointers; they return
+ * when the outputs are written.  NMRFIT_ERR_ARG for NULL pointers and more than 64 peaks. */
+int nmrfit_ctx_residuals(nmrfit_ctx* ctx, const double* x, double* res_out, void* stream);
+int nmrfit_ctx_residual_scale(nmrfit_ctx* ctx, const double* x, double* out, void* stream);
+
 /* Which objective kernel runs (default NMRFIT_ALGO_AUTO), and which one a launch with this fit_im would use.
  * Both kernels evaluate equations.objective (equations.py:152-212); the uniform-axis one exploits
  * w_i = w_0 + i*h (what core.load builds, core.py:58-60) to replace most exponentials by a recurrence. */

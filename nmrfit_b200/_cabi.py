@@ -62,6 +62,8 @@ SIGNATURES = {
     'nmrfit_ctx_loss_moments': (_i, [_vp, _vp, _i, _vp, _vp, _vp]),
     'nmrfit_ctx_refine_loss': (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
     'nmrfit_ctx_residual_acf': (_i, [_vp, _vp, _i, _vp, _vp]),
+    'nmrfit_ctx_residuals': (_i, [_vp, _vp, _vp, _vp]),
+    'nmrfit_ctx_residual_scale': (_i, [_vp, _vp, _vp, _vp]),
     'nmrfit_ctx_normal_m_lagged': (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     'nmrfit_lagged_plan': (_i, [_i, _i, _i, c_int_p]),
     'nmrfit_ctx_set_algorithm': (_i, [_vp, _i]),
@@ -522,6 +524,24 @@ class Context(_Handle):
         r = np.empty((self.B, L + 1))
         check(lib().nmrfit_ctx_residual_acf(self._h, ptr(x), L, ptr(r), ptr(stream)))
         return r
+
+    def residuals(self, x, stream=None):
+        """The unweighted residuals res = Vdata - Vfit at ``x`` [B, D] over the spectra the context holds, the residual
+        of ``normal_equations``: returns [B, N] on the host (DESIGN K17)."""
+        x = self._params(x)
+        res = np.empty((self.B, self.N))
+        check(lib().nmrfit_ctx_residuals(self._h, ptr(x), ptr(res), ptr(stream)))
+        return res
+
+    def residual_scale(self, x, stream=None):
+        """The median of the residuals at ``x`` [B, D] and their median absolute deviation, each as ``np.median`` gives
+        it (exact selection on the device, DESIGN K17): returns ``(median [B], MAD [B])``.  MAD / 0.6744897501960817
+        (``utils.NORMAL_MAD``) is the normal-consistent noise level, ``scipy.stats.median_abs_deviation(res,
+        scale='normal')``."""
+        x = self._params(x)
+        out = np.empty((self.B, 2))
+        check(lib().nmrfit_ctx_residual_scale(self._h, ptr(x), ptr(out), ptr(stream)))
+        return out[:, 0].copy(), out[:, 1].copy()
 
     def normal_m_lagged(self, x, rho, stream=None):
         """Lag-weighted M at ``x`` [B, D]: returns [B, D, D] = sum_i sum_{|k| <= L} rho_|k| a_i^T a_{i+k}, a_i = w_i^2 A_i

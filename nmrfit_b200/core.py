@@ -35,8 +35,8 @@ def fit_batch(datas, lowers, uppers, expon=0.5, dynamic_weighting=True, fit_im=F
     options['seeds'] = [k_0, k_1, ...], spectrum b reproduces the reference fit run
     after ``np.random.seed(k_b)``.  With options['refine'] every fit is then refined (``utils.refine_batch``) in the
     same context, where the spectra and weights already are, with options['ties'] (one ``utils.Ties`` for every
-    spectrum or a list of them) and options['loss'] / options['f_scale'] (one scale for every spectrum or one per
-    spectrum) if given.  Returns a list of ``FitUtility``.
+    spectrum or a list of them) and options['loss'] / options['f_scale'] (one scale for every spectrum, one per
+    spectrum, or 'auto' for each spectrum's own from its least-squares residuals) if given.  Returns a list of ``FitUtility``.
     """
     fits = [utils.FitUtility(d, lo, up, expon, dynamic_weighting, fit_im, 1, summary, options)
             for d, lo, up in zip(datas, lowers, uppers)]
@@ -45,7 +45,7 @@ def fit_batch(datas, lowers, uppers, expon=0.5, dynamic_weighting=True, fit_im=F
     B = len(fits)
     if refine and fits:
         utils._check_refinable(fits[0])
-        _cabi.check_loss(opt.get('loss', 'linear'), opt.get('f_scale'), B)
+        utils.check_loss_scale(opt.get('loss', 'linear'), opt.get('f_scale'), B)
     if not refine:
         utils.check_unrefined_options(opt)
     lb = np.array(lowers, dtype=np.float64)

@@ -147,6 +147,7 @@ struct nmrfit_ctx {
     DevBuf<int> rf_tie_i;              // tied refinement: the tie map of each spectrum (RefineTies)
     DevBuf<double> rf_tie_d;
     DevBuf<double> rb_scale, rb_part, rb_out;   // robust losses: f_scale [B], moments chunk partials, moments [B][5]
+    DevBuf<double> sc_res, sc_out;     // residual scale: residuals [B][N], (median, MAD) [B][2]
     Stream pipe[2];                    // nmrfit_objective_batch_host: slices of a large particle set
     PinnedBuf<double> h_f;             // ... and staging of their values
     int far_cells = 0;                 // far-field cells per region: 0 = far_cells_per_region(N, R), else 1 | 2 | 4
@@ -785,6 +786,38 @@ int nmrfit_ctx_loss_moments(nmrfit_ctx* c, const double* x, int loss, const doub
     CK(cudaMemcpyAsync(out, c->rb_out.ptr, sizeof(double) * B * 5, cudaMemcpyDefault, st));
     CK(cudaStreamSynchronize(st));                         // x and out may be pageable host memory
     return NMRFIT_OK;
+}
+
+// Both residual-scale entry points (DESIGN K17): the residuals at x into sc_res, then with `scale` their median and
+// MAD into sc_out; `out` receives whichever was asked for.
+static int residual_scale_pass(nmrfit_ctx* c, const double* x, bool scale, double* out, cudaStream_t st) {
+    const double* xd = nullptr;
+    if (int r = post_fit_begin(
+            c, [&] { return x && out ? NMRFIT_OK : fail(NMRFIT_ERR_ARG, "x and out must be non-NULL"); },
+            "the residual passes support", no_checks, "its residuals are computed", x, st, &xd))
+        return r;
+    const size_t B = (size_t)c->B, N = (size_t)c->N;
+    CK(c->sc_res.reserve(B * N));
+    cudaError_t e = launch_residuals(c->spec.ptr, xd, c->B, c->N, c->P, c->sc_res.ptr, st);
+    if (e != cudaSuccess) return fail_cuda(e, "residuals launch");
+    if (scale) {
+        CK(c->sc_out.reserve(B * 2));
+        e = launch_median_mad(c->sc_res.ptr, c->B, c->N, c->sc_out.ptr, st);
+        if (e != cudaSuccess) return fail_cuda(e, "median and MAD launch");
+        CK(cudaMemcpyAsync(out, c->sc_out.ptr, sizeof(double) * B * 2, cudaMemcpyDefault, st));
+    } else {
+        CK(cudaMemcpyAsync(out, c->sc_res.ptr, sizeof(double) * B * N, cudaMemcpyDefault, st));
+    }
+    CK(cudaStreamSynchronize(st));                         // x and out may be pageable host memory
+    return NMRFIT_OK;
+}
+
+int nmrfit_ctx_residuals(nmrfit_ctx* c, const double* x, double* res_out, void* stream) {
+    return residual_scale_pass(c, x, false, res_out, (cudaStream_t)stream);
+}
+
+int nmrfit_ctx_residual_scale(nmrfit_ctx* c, const double* x, double* out, void* stream) {
+    return residual_scale_pass(c, x, true, out, (cudaStream_t)stream);
 }
 
 // the lag checks of both lagged passes; fills the plan

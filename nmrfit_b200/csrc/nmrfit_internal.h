@@ -247,6 +247,9 @@ cudaError_t launch_normal_eq_loss(const double* spec, const double* x, int loss,
 size_t loss_moments_scratch_doubles(int B, int N);
 cudaError_t launch_loss_moments(const double* spec, const double* x, int loss, const double* fscale, int B, int N,
                                 int P, double* part, double* out, cudaStream_t st);
+// K17 (scale.cu): x [B][D] -> res [B][N], the residual of K12; res [B][N] -> out [B][2] = (median, MAD), numpy's median
+cudaError_t launch_residuals(const double* spec, const double* x, int B, int N, int P, double* res, cudaStream_t st);
+cudaError_t launch_median_mad(const double* res, int B, int N, double* out, cudaStream_t st);
 
 // ---- K14 residual autocorrelation and lag-weighted M (lagged.cu) --------------------
 // Tiling of both passes: a function of N, P and the largest lag L only.

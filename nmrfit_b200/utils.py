@@ -103,7 +103,8 @@ class FitUtility:
                     honour ties).  ``fit_batch`` takes one ``Ties`` for every spectrum or a list of them.
       ``loss``, ``f_scale``   a robust loss the refinement minimises (``refine(loss=..., f_scale=...)``; needs
                     ``refine``: the swarm keeps the reference's objective).  ``fit_batch`` takes one f_scale for every
-                    spectrum or one per spectrum.
+                    spectrum or one per spectrum; f_scale 'auto' estimates each spectrum's scale from its
+                    least-squares residuals (``refine(f_scale='auto')``).
     ``processes`` is accepted and ignored (the GPU evaluates every particle at once).
     """
 
@@ -124,7 +125,7 @@ class FitUtility:
         ``options['refine']``)."""
         if self.options.get('refine', False):
             _check_refinable(self)
-            _cabi.check_loss(self.options.get('loss', 'linear'), self.options.get('f_scale'), 1)
+            check_loss_scale(self.options.get('loss', 'linear'), self.options.get('f_scale'), 1)
         else:
             check_unrefined_options(self.options)
         self.weights = self._compute_weights()
@@ -221,9 +222,24 @@ class FitUtility:
         passes than least squares (DESIGN K16): ``max_iter`` None is 50 for linear and ``ROBUST_MAX_ITER`` = 200 for a
         robust loss.  The loop stops as soon as every spectrum has finished, so the larger cap costs nothing then.
 
+        ``f_scale='auto'`` sets c from the data (DESIGN K17): a least-squares refinement first (``max_iter`` None is 50
+        there), then sigma = MAD / 0.6744897501960817 of its unweighted residuals over all points (``noise_level()``,
+        as ``scipy.stats.median_abs_deviation(scale='normal')``; the median ignores the few points an impurity line
+        spoils, where the least-squares sigma does not), c = ``AUTO_SCALE_K[loss]`` * sigma, and the robust
+        refinement from the least-squares point with that c.  The result is that of ``refine()`` followed by
+        ``refine(loss=loss, f_scale=c)`` bit for bit, except that ``refine_info`` keeps the start of the first stage
+        and gains ``scale`` = dict(sigma, median, k, lsq_passes, lsq_accepted, lsq_status).  ValueError naming the
+        spectrum, with no fit changed, if a sigma is 0 or not finite (more than half of the residuals equal, or the
+        least-squares stage ended ``REFINE_NONFINITE``).
+
         Raises RuntimeError before ``fit()`` and NotImplementedError with ``fit_im``."""
         refine_batch([self], max_iter, xtol, ties=None if ties is None else [ties], loss=loss, f_scale=f_scale)
         return self.params
+
+    def noise_level(self):
+        """The noise level sigma = MAD / 0.6744897501960817 of the unweighted residuals at ``params`` over all points
+        (``noise_level_batch``): one device pass, no refinement."""
+        return float(noise_level_batch([self])[0])
 
     def compute_uncertainties(self, noise='white', max_lag=32, noise_acf=None):
         """Standard errors of ``params`` from the linearised least-squares problem at the fitted point (one pass
@@ -656,6 +672,48 @@ def apply_refinement(fits, x, fval, passes, accepted, status, ties=None, loss='l
 
 
 ROBUST_MAX_ITER = 200
+NORMAL_MAD = 0.6744897501960817          # scipy.special.ndtri(0.75): E MAD = NORMAL_MAD sigma for Gaussian noise
+# c / sigma of each robust loss at 95 % asymptotic efficiency on Gaussian noise, (E psi')^2 / E psi^2 = 0.95
+AUTO_SCALE_K = {'huber': 1.345, 'soft_l1': 1.287, 'cauchy': 2.385}
+AUTO_SCALE_LIST = ("f_scale 'auto' estimates the scale of every spectrum of the call: give it once, not in a list "
+                   "of scales")
+
+
+def check_loss_scale(loss, f_scale, B):
+    """``_cabi.check_loss`` that also takes ``f_scale='auto'`` for a robust loss: returns ``(code, 'auto')`` then, else
+    what ``check_loss`` returns.  ValueError for any other string and for 'auto' inside a list of scales.  With the
+    linear loss ``f_scale`` is not read."""
+    code, _ = _cabi.check_loss(loss, 1.0, B)
+    if code == _cabi.LOSS_LINEAR:
+        return code, None
+    if isinstance(f_scale, str):
+        if f_scale != 'auto':
+            raise ValueError("f_scale must be a number, one number per spectrum, or 'auto', got %r" % f_scale)
+        return code, 'auto'
+    if isinstance(f_scale, (list, tuple, np.ndarray)) and \
+            any(isinstance(v, str) for v in np.ravel(np.asarray(f_scale, dtype=object))):
+        raise ValueError(AUTO_SCALE_LIST)
+    return _cabi.check_loss(code, f_scale, B)
+
+
+def noise_level_batch(fits):
+    """``noise_level()`` for many fits of equal length and peak count in one device pass: sigma = MAD / NORMAL_MAD of
+    each spectrum's unweighted residuals at its ``params`` (``Context.residual_scale``, DESIGN K17), as
+    ``scipy.stats.median_abs_deviation(res, scale='normal')``.  Returns sigma [B]."""
+    fits = list(fits)
+    if not fits:
+        return np.empty(0)
+    for f in fits:
+        if getattr(f, 'params', None) is None:
+            raise RuntimeError('noise_level needs a fitted model: call fit() first')
+        if f.fit_im:
+            raise NotImplementedError('noise_level is not available with fit_im: that objective is a sum of two '
+                                      'RMSEs, not one residual')
+    W, U, V, weights, X = stack_fits(fits, ('params',))
+    with _cabi.pooled_context(len(fits), W.shape[1], (X.shape[1] - 4) // 3,
+                              device=fits[0].options.get('device')) as ctx:
+        ctx.set_spectra(W, U, V, weights)
+        return ctx.residual_scale(X)[1] / NORMAL_MAD
 
 
 def default_max_iter(max_iter, loss):
@@ -669,13 +727,34 @@ def default_max_iter(max_iter, loss):
 def refine_with_loss(ctx, fits, x, lb, ub, ties=None, ties_per=None, loss='linear', f_scale=None, max_iter=None,
                      xtol=1e-6):
     """``ctx.refine`` (its spectra and weights set) and ``apply_refinement``, with the moments pass at the result for a
-    robust loss.  ``loss`` and ``f_scale`` must have passed ``_cabi.check_loss``; ``max_iter`` None is
-    ``default_max_iter``."""
-    out = ctx.refine(x, lb, ub, ties=ties, loss=loss, f_scale=f_scale, max_iter=default_max_iter(max_iter, loss),
-                     xtol=xtol)
-    code, fs = _cabi.check_loss(loss, f_scale, len(fits))
-    moments = None if code == _cabi.LOSS_LINEAR else ctx.loss_moments(out[0], code, fs)
+    robust loss.  ``loss`` and ``f_scale`` must have passed ``check_loss_scale``; ``max_iter`` None is
+    ``default_max_iter``.  ``f_scale='auto'`` runs the two stages of ``FitUtility.refine``: the least-squares
+    refinement, the scale from the MAD of its residuals, then the robust refinement from its result."""
+    code, fs = check_loss_scale(loss, f_scale, len(fits))
     name = [k for k, v in _cabi.LOSSES.items() if v == code][0]
+    if isinstance(fs, str):
+        starts = [(np.array(f.params, dtype=np.float64), f.error) for f in fits]
+        lsq = ctx.refine(x, lb, ub, ties=ties, max_iter=default_max_iter(max_iter, 'linear'), xtol=xtol)
+        med, mad = ctx.residual_scale(lsq[0])
+        sigma = mad / NORMAL_MAD
+        for b in range(len(fits)):                       # every scale is checked before any fit changes
+            if lsq[4][b] == _cabi.REFINE_NONFINITE or not (np.isfinite(sigma[b]) and sigma[b] > 0):
+                raise ValueError("spectrum %d: f_scale='auto' needs a noise level > 0 from the least-squares residuals,"
+                                 " got sigma = MAD / %r = %r (least-squares status %d)"
+                                 % (b, NORMAL_MAD, sigma[b], lsq[4][b]))
+        apply_refinement(fits, *lsq, ties=ties_per)
+        fs = AUTO_SCALE_K[name] * sigma
+        refine_with_loss(ctx, fits, lsq[0], lb, ub, ties=ties, ties_per=ties_per, loss=code, f_scale=fs,
+                         max_iter=max_iter, xtol=xtol)
+        for b, f in enumerate(fits):
+            f.refine_info.update(start_params=starts[b][0], start_error=starts[b][1],
+                                 scale=dict(sigma=float(sigma[b]), median=float(med[b]), k=AUTO_SCALE_K[name],
+                                            lsq_passes=int(lsq[2][b]), lsq_accepted=int(lsq[3][b]),
+                                            lsq_status=int(lsq[4][b])))
+        return
+    out = ctx.refine(x, lb, ub, ties=ties, loss=code, f_scale=fs, max_iter=default_max_iter(max_iter, code),
+                     xtol=xtol)
+    moments = None if code == _cabi.LOSS_LINEAR else ctx.loss_moments(out[0], code, fs)
     apply_refinement(fits, *out, ties=ties_per, loss=name, f_scale=fs, moments=moments)
 
 
@@ -713,8 +792,8 @@ def refine_batch(fits, max_iter=None, xtol=1e-6, ties=None, loss='linear', f_sca
     the spectra and each fit's ``weights`` go to a pooled context, and every spectrum runs bounded Levenberg-Marquardt
     (``Context.refine``, DESIGN K13) from its ``params`` within its box.  ``ties``: one ``Ties`` for every fit, or a
     list with one ``Ties`` (or None) per fit (DESIGN K15); each fit keeps its own as ``ties``.  ``loss`` and
-    ``f_scale`` (a scalar or one per fit) and ``max_iter`` (None: ``default_max_iter``) as ``FitUtility.refine``
-    (DESIGN K16).  Returns the list of refined ``params``."""
+    ``f_scale`` (a scalar, one per fit, or 'auto' for each fit's own, DESIGN K17) and ``max_iter`` (None:
+    ``default_max_iter``) as ``FitUtility.refine`` (DESIGN K16).  Returns the list of refined ``params``."""
     fits = list(fits)
     if not fits:
         return []
@@ -723,12 +802,12 @@ def refine_batch(fits, max_iter=None, xtol=1e-6, ties=None, loss='linear', f_sca
     W, U, V, weights, X, LB, UB = stack_fits(fits, ('params', 'lower', 'upper'))
     N, D = W.shape[1], X.shape[1]
     per, arrays = batch_ties(ties, len(fits), (D - 4) // 3)
-    _cabi.check_loss(loss, f_scale, len(fits))
-    max_iter = default_max_iter(max_iter, loss)
+    check_loss_scale(loss, f_scale, len(fits))
+    cap = default_max_iter(max_iter, loss)
     if arrays is None:
-        _cabi.check_refine_args(X, LB, UB, max_iter, xtol, len(fits), N, (D - 4) // 3)
+        _cabi.check_refine_args(X, LB, UB, cap, xtol, len(fits), N, (D - 4) // 3)
     else:
-        _cabi.check_refine_args(X, LB, UB, max_iter, xtol, len(fits), N, (D - 4) // 3, box=False)
+        _cabi.check_refine_args(X, LB, UB, cap, xtol, len(fits), N, (D - 4) // 3, box=False)
         _cabi.check_ties(*arrays, LB, UB, len(fits), N, (D - 4) // 3)
     with _cabi.pooled_context(len(fits), N, (D - 4) // 3, device=fits[0].options.get('device')) as ctx:
         ctx.set_spectra(W, U, V, weights)
