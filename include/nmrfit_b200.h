@@ -238,7 +238,9 @@ int nmrfit_ctx_get_algorithm(nmrfit_ctx* ctx, int fit_im, int* algorithm);
 
 /* Launch geometry of the objective kernel; 0 keeps the automatic choice for that field.
  * threads in {128, 256}; points_per_thread in {2, 4, 8} (general kernel) or {4, 8, 16} (uniform-axis
- * kernel); exp_table_bits in {-1 (no table), 6, 8, 10}. */
+ * kernel); exp_table_bits in {-1 (no table), 6, 8, 10}.  nmrfit_ctx_get_tuning reports the geometry that runs for a
+ * real-only call of n_particles: FP32 contexts run 4 or 8 points per thread on a uniform axis (16 runs as 8) and
+ * 256 threads x 4 points on any other axis. */
 int nmrfit_ctx_set_tuning(nmrfit_ctx* ctx, int threads, int points_per_thread, int exp_table_bits,
                           int particles_per_cta);
 int nmrfit_ctx_get_tuning(nmrfit_ctx* ctx, int n_particles, int* threads, int* points_per_thread, int* exp_table_bits,

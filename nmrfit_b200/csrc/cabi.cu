@@ -199,109 +199,15 @@ bool axis_is_uniform(const double* hw, int N, double* grid) {
     return uni;
 }
 
-// Which objective kernel a launch uses: the uniform-axis kernels (FP64 or FP32) need every spectrum of the
-// batch on a uniform axis and the real-only fit; anything else runs the general kernel of that precision.
-bool use_uniform(const nmrfit_ctx* c, int fit_im) {
-    if (c->algorithm == NMRFIT_ALGO_GENERAL) return false;
-    // real-only fit in both precisions; fit_im with the reference's semantics (last peak's counterpart) in FP64
-    if (fit_im == NMRFIT_IM_SUM || (fit_im == NMRFIT_IM_REFERENCE && c->precision != NMRFIT_FP64)) return false;
-    for (char u : c->uniform)
-        if (!u) return false;
-    return true;
+// The launch plan of an objective call on this context (objective_plan.h)
+ObjPlan ctx_plan(const nmrfit_ctx* c, int S, int fit_im, size_t slots_total = 0) {
+    bool uniform_axis = true;
+    for (char u : c->uniform) uniform_axis = uniform_axis && u;
+    return objective_plan(c->N, c->P, S, c->B, c->precision, fit_im, uniform_axis, c->algorithm, c->user_tune,
+                          c->far_cells, slots_total);
 }
 
-// far-field cells per region of the FP64 uniform-axis kernels (every kernel of a context uses the same split)
-int ctx_cells(const nmrfit_ctx* c, int r) { return c->far_cells ? c->far_cells : far_cells_per_region(c->N, r); }
-
-ObjTune pick_tune(const nmrfit_ctx* c, int S, bool uni) {
-    ObjTune t;
-    // The point tiling fixes the summation order of the residual, so it may depend on
-    // N alone (never on how many particles or spectra a rank happens to hold).
-    if (uni) {
-        // 2,048-point tiles from 2,048 points up (measured 9 % faster than 1,024-point tiles at 2,048 and 4,096
-        // points, 6 peaks: tools/tune_probe.py)
-        if (c->N >= 2048) { t.threads = 256; t.r = 8; }
-        else { t.threads = 128; t.r = 4; }
-    } else {
-        if (c->N >= 8192) { t.threads = 256; t.r = 4; }
-        else if (c->N >= 1024) { t.threads = 128; t.r = 4; }
-        else { t.threads = 128; t.r = 2; }
-    }
-    t.tb = 6;
-    if (c->user_tune.threads) t.threads = c->user_tune.threads;
-    if (c->user_tune.r) t.r = c->user_tune.r;
-    if (c->user_tune.tb == -1) t.tb = 0;            // -1: polynomial-only exp
-    else if (c->user_tune.tb > 0) t.tb = c->user_tune.tb;
-    // particles per CTA: amortise the spectrum/coefficients over as many particles as
-    // still leaves >= ~4 CTAs per SM
-    int n_tiles = (c->N + t.threads * t.r - 1) / (t.threads * t.r);
-    long long ctas1 = (long long)n_tiles * S * c->B;
-    int sp = (int)std::max<long long>(1, std::min<long long>(16, ctas1 / (148 * 4)));
-    sp = std::min(sp, std::max(1, S));
-    if (c->user_tune.sp > 0) sp = std::min(c->user_tune.sp, std::max(1, S));
-    t.sp = sp;
-    // FP64 uniform-axis path: the streamed evaluation kernel (objective_stream.cu) unless the caller asked for the
-    // one-group-per-CTA kernel.  Its `sp` is the particles per pipeline stage: as many as leave three CTAs per SM.
-    t.variant = 0;
-    t.stages = 0;
-    t.occ = 3;
-    // ... when there is enough work to stream: a small swarm (a single fit's 100-204 particles on a short axis) is a few
-    // dozen CTAs either way, and then one group per CTA finishes sooner than a handful of CTAs walking several groups each
-    const long long particle_tiles = (long long)((c->N + t.threads * t.r - 1) / (t.threads * t.r)) * S * c->B;
-    const bool enough = particle_tiles >= 8192 || c->user_tune.variant == 1;
-    if (uni && c->precision == NMRFIT_FP64 && c->user_tune.variant != 0 && t.tb == 6 && enough) {   // (built for the default table)
-        t.variant = 1;
-        t.occ = c->user_tune.occ == 3 ? 3 : 2;
-        // two CTAs: the B200's 228 KB of shared memory per SM less 1 KB reserved per CTA, halved
-        const size_t budget = t.occ == 2 ? 115712 : 74 * 1024;
-        // at two CTAs per SM a warp evaluates one particle per far-field cell of a region at once (objective_stream.cu):
-        // a group that is not a multiple of that would leave lanes idle in its last step
-        const int cells = ctx_cells(c, t.r), per_warp = t.occ == 2 ? cells : 1;
-        auto fit_sp = [&](int stg) {
-            t.stages = stg;
-            int spg = 0;
-            for (int cand = 1; cand <= 16; ++cand) {
-                t.sp = cand;
-                if (objective_stream_smem_bytes(c->P, t, cells) <= budget && (cand < per_warp || cand % per_warp == 0))
-                    spg = cand;
-            }
-            return spg;
-        };
-        int stg = c->user_tune.stages > 0 ? c->user_tune.stages : 3;
-        int spg = fit_sp(stg);
-        // heavy per-particle constants (many peaks, or four far-field cells per region): two deeper stages rather than
-        // three shallow ones - a group of 7 instead of 5 particles amortises the per-group handshakes (r02ae: -5 % at
-        // 6 peaks x 4,096 points; groups of 7+ gain nothing from the switch)
-        if (c->user_tune.stages == 0 && spg < 6) {
-            const int spg2 = fit_sp(2);
-            if (spg2 > spg) { stg = 2; spg = spg2; }
-        }
-        t.stages = stg;
-        t.sp = std::max(1, spg);
-        bool fits = true;
-        if (c->user_tune.sp > 0) {                         // an explicit group size: fewer stages if need be, else the
-            t.sp = c->user_tune.sp;                        // one-group-per-CTA kernel below (which takes any size)
-            if (objective_stream_smem_bytes(c->P, t, ctx_cells(c, t.r)) > 200 * 1024 && c->user_tune.stages == 0) t.stages = 2;
-            fits = objective_stream_smem_bytes(c->P, t, ctx_cells(c, t.r)) <= 200 * 1024;
-        }
-        if (fits) {
-            t.sp = std::min(t.sp, std::max(1, S));
-            return t;
-        }
-        t.variant = 0;
-        t.stages = 0;
-        t.occ = 3;
-    }
-    // per-particle coefficients live in shared memory: keep the CTA under the 200 KB opt-in limit
-    const bool f32 = c->precision == NMRFIT_FP32;
-    auto uni_bytes = [&]() { return f32 ? objective_f32_smem_bytes(c->P, t) : objective_uniform_smem_bytes(c->P, t, ctx_cells(c, t.r)); };
-    while (t.sp > 1 && (uni ? uni_bytes() : objective_smem_bytes(c->P, t, 2)) > 200 * 1024)
-        t.sp /= 2;
-    // uniform-axis kernels: three CTAs per SM if a smaller particle tile achieves it (227 KB / 3)
-    if (uni && c->user_tune.sp <= 0)
-        while (t.sp > 4 && uni_bytes() > 74 * 1024) t.sp -= 1;
-    return t;
-}
+bool two_pass(const ObjPlan& p) { return p.kernel == OBJ_UNIFORM || p.kernel == OBJ_STREAM; }
 
 int check_ctx(const nmrfit_ctx* c) {
     if (!c) return fail(NMRFIT_ERR_ARG, "ctx is NULL");
@@ -335,76 +241,42 @@ int run_objective(nmrfit_ctx* c, const double* x_dev, int S, int fit_im, double*
     for (int b = 0; b < c->B; ++b)
         if (!c->spec_set[b]) return fail(NMRFIT_ERR_STATE, "spectrum " + std::to_string(b) + " was never set");
     if (fit_im < 0 || fit_im > 2) return fail(NMRFIT_ERR_ARG, "fit_im must be 0, 1 or 2");
-    const bool uni = use_uniform(c, fit_im);
-    if (c->algorithm == NMRFIT_ALGO_UNIFORM && !uni)
-        return fail(NMRFIT_ERR_STATE, "the uniform-axis kernel needs uniformly spaced w in every spectrum and fit_im off");
-    if (c->precision == NMRFIT_FP32 && fit_im != NMRFIT_REAL_ONLY)
-        return fail(NMRFIT_ERR_ARG, "fit_im is not available in FP32 mode (the Kramers-Kronig term runs in FP64 only)");
-    ObjTune t = pick_tune(c, S, uni);
-    if (uni && c->precision == NMRFIT_FP32 && t.r == 16) t.r = 8;      // the FP32 kernel is built for 4 and 8
-    if (uni ? (t.r != 4 && t.r != 8 && t.r != 16) : (t.r != 2 && t.r != 4 && t.r != 8))
-        return fail(NMRFIT_ERR_ARG, uni ? "points_per_thread must be 4, 8 or 16 for the uniform-axis kernel"
-                                        : "points_per_thread must be 2, 4 or 8 for the general kernel");
-    int n_tiles = objective_tiles(c->N, t);
-    const size_t part_per = (size_t)n_tiles * 2 * (t.variant == 1 ? t.threads / 32 : 1);
-    CK(c->partials.reserve(std::max((size_t)c->B * S, in.slots_total) * part_per));
+    const ObjPlan p = ctx_plan(c, S, fit_im, in.slots_total);
+    if (p.refuse) return fail(p.refuse, p.why);
+    CK(c->partials.reserve(p.slots * p.part_per));
     ObjArgs a{};
-    const int sub = (uni && c->precision == NMRFIT_FP64) ? ctx_cells(c, t.r) : 1;
-    if (uni) {
-        size_t nc, np, nf, na, nm;
-        int pad = 0;
-        objective_uniform_prep_sizes(c->N, c->P, t, sub, &nc, &np, &nf, &na, &nm, &pad);
-        const size_t slots = std::max((size_t)c->B * S, in.slots_total) + pad;
-        CK(c->prep_coef.reserve(slots * nc));
-        CK(c->prep_part.reserve(slots * np));
-        CK(c->prep_far.reserve(slots * nf));
-        CK(c->prep_anchor.reserve(slots * na));
-        CK(c->prep_mask.reserve(slots * nm));
-        a.prep_coef = c->prep_coef.ptr + in.slot0 * nc; a.prep_part = c->prep_part.ptr + in.slot0 * np;
-        a.prep_far = c->prep_far.ptr + in.slot0 * nf; a.prep_anchor = c->prep_anchor.ptr + in.slot0 * na;
-        a.prep_mask = c->prep_mask.ptr + in.slot0 * nm;
+    if (p.prep_threads) {
+        const size_t slots = p.slots + p.pad;
+        CK(c->prep_coef.reserve(slots * p.coef));
+        CK(c->prep_part.reserve(slots * p.part));
+        CK(c->prep_far.reserve(slots * p.far));
+        CK(c->prep_anchor.reserve(slots * p.anchor));
+        CK(c->prep_mask.reserve(slots * p.mask));
+        a.prep_coef = c->prep_coef.ptr + in.slot0 * p.coef; a.prep_part = c->prep_part.ptr + in.slot0 * p.part;
+        a.prep_far = c->prep_far.ptr + in.slot0 * p.far; a.prep_anchor = c->prep_anchor.ptr + in.slot0 * p.anchor;
+        a.prep_mask = c->prep_mask.ptr + in.slot0 * p.mask;
     }
     a.spec = c->spec.ptr;
     a.x = x_dev;
     a.x_in = in.x_in;                                      // (two-pass FP64 path only: the caller checks)
-    a.partials = c->partials.ptr + in.slot0 * part_per;
+    a.partials = c->partials.ptr + in.slot0 * p.part_per;
     a.frozen = in.frozen;
     a.grid_h = c->grid_h.ptr;
-    a.N = c->N; a.P = c->P; a.S = S; a.kk = fit_im; a.sp = t.sp; a.sub = sub;
+    a.N = c->N; a.P = c->P; a.S = S; a.kk = fit_im;
     // profiling: three events per launch - before the prepare pass, between it and the evaluation kernel, after
-    cudaEvent_t ev0 = nullptr, evm = nullptr, ev1 = nullptr;
+    cudaEvent_t ev[3] = {};
     if (c->profiling) {
-        if (c->prof_used + 3 > c->prof_events.size()) {
-            for (int k = 0; k < 3; ++k) {
-                cudaEvent_t ev;
-                CK(cudaEventCreate(&ev));
-                c->prof_events.emplace_back(ev);
-            }
+        while (c->prof_events.size() < c->prof_used + 3) {
+            cudaEvent_t e;
+            CK(cudaEventCreate(&e));
+            c->prof_events.emplace_back(e);
         }
-        ev0 = c->prof_events[c->prof_used].h;
-        evm = c->prof_events[c->prof_used + 1].h;
-        ev1 = c->prof_events[c->prof_used + 2].h;
+        for (int k = 0; k < 3; ++k) ev[k] = c->prof_events[c->prof_used + k].h;
         c->prof_used += 3;
     }
-    const bool two_pass = uni && c->precision == NMRFIT_FP64;
-    if (evm && !two_pass) {                                // no separate prepare pass on this path: zero-length first leg
-        CK(cudaEventRecord(ev0, st));
-        CK(cudaEventRecord(evm, st));
-        ev0 = nullptr;
-    }
-    const MoveArgs* mv = in.move;
-    const bool move_in_prepare = mv && uni && c->precision == NMRFIT_FP64;
-    if (mv && !move_in_prepare) {                          // paths without a prepare pass move the swarm on their own
-        cudaError_t em = launch_swarm_move(mv->s, mv->rp, mv->rg, mv->generation, st);
-        if (em != cudaSuccess) return fail_cuda(em, "swarm move");
-    }
-    ObjOut o;
-    o.nsum = c->precision == NMRFIT_FP32 ? 1 : (fit_im ? 2 : 1);
-    cudaError_t e = c->precision == NMRFIT_FP32 ? launch_objective_f32(a, t, c->B, f_dev, uni, st, ev0, ev1, &o.n_tiles)
-                    : uni ? launch_objective_uniform(a, t, c->B, f_dev, st, ev0, ev1, move_in_prepare ? mv : nullptr, &o.n_tiles, evm, &o.nw)
-                          : launch_objective(a, t, c->B, f_dev, st, ev0, ev1, &o.n_tiles);
+    cudaError_t e = run_objective_plan(p, a, c->B, in.move, f_dev, st, ev[0], ev[1], ev[2]);
     if (e != cudaSuccess) return fail_cuda(e, "objective launch");
-    if (out) *out = o;
+    if (out) *out = ObjOut{p.n_tiles, p.nsum, p.nw};
     return NMRFIT_OK;
 }
 
@@ -443,9 +315,9 @@ int no_checks() { return NMRFIT_OK; }
 int fused_setup(nmrfit_ctx* c, int n_gen, const double* rp_d, const double* rg_d, FusedArgs* a, FusedPlan* plan) {
     plan->ok = false;
     if (c->fused_mode == NMRFIT_FUSED_OFF) return NMRFIT_OK;
-    if (c->precision != NMRFIT_FP64 || c->kk != NMRFIT_REAL_ONLY || !use_uniform(c, NMRFIT_REAL_ONLY)) return NMRFIT_OK;
     const SwarmState& s = c->sw;
-    ObjTune t = pick_tune(c, s.S, true);
+    const ObjPlan p = ctx_plan(c, s.S, NMRFIT_REAL_ONLY);
+    if (c->precision != NMRFIT_FP64 || c->kk != NMRFIT_REAL_ONLY || !two_pass(p)) return NMRFIT_OK;
     *a = FusedArgs{};
     a->s = s;
     a->spec = c->spec.ptr;
@@ -453,13 +325,13 @@ int fused_setup(nmrfit_ctx* c, int n_gen, const double* rp_d, const double* rg_d
     a->rp = rp_d;
     a->rg = rg_d;
     a->N = c->N; a->P = c->P;
-    a->n_vtiles = objective_tiles(c->N, t);
-    a->vw = t.threads / 32;
-    a->sub = ctx_cells(c, t.r);
+    a->n_vtiles = p.n_tiles;
+    a->vw = p.t.threads / 32;
+    a->sub = p.sub;
     a->n_gen = n_gen;
     a->gen0 = c->generation + 1;
     a->maxiter = c->maxiter;
-    cudaError_t e = swarm_fused_plan(*a, c->D, s.B, s.S, t, c->device, c->fused_mode == NMRFIT_FUSED_REQUIRE, plan);
+    cudaError_t e = swarm_fused_plan(*a, c->D, s.B, s.S, p.t, c->device, c->fused_mode == NMRFIT_FUSED_REQUIRE, plan);
     if (e != cudaSuccess) return fail_cuda(e, "fused swarm plan");
     if (!plan->ok) return NMRFIT_OK;
     CK(c->frec_f.reserve(2 * (size_t)s.B * s.S));
@@ -1145,7 +1017,8 @@ int nmrfit_ctx_set_algorithm(nmrfit_ctx* c, int algorithm) {
 int nmrfit_ctx_get_algorithm(nmrfit_ctx* c, int fit_im, int* algorithm) {
     if (int r = check_ctx(c)) return r;
     if (!algorithm) return fail(NMRFIT_ERR_ARG, "algorithm is NULL");
-    *algorithm = use_uniform(c, fit_im) ? NMRFIT_ALGO_UNIFORM : NMRFIT_ALGO_GENERAL;
+    const int k = ctx_plan(c, 1, fit_im).kernel;
+    *algorithm = k == OBJ_GENERAL || k == OBJ_F32_GENERAL ? NMRFIT_ALGO_GENERAL : NMRFIT_ALGO_UNIFORM;
     return NMRFIT_OK;
 }
 
@@ -1181,7 +1054,7 @@ int nmrfit_ctx_set_far_cells(nmrfit_ctx* c, int cells) {
 
 int nmrfit_ctx_get_variant(nmrfit_ctx* c, int S, int* variant, int* stages) {
     if (int rc = check_ctx(c)) return rc;
-    ObjTune t = pick_tune(c, S < 1 ? 1 : S, use_uniform(c, NMRFIT_REAL_ONLY));
+    const ObjTune t = ctx_plan(c, S < 1 ? 1 : S, NMRFIT_REAL_ONLY).t;
     if (variant) *variant = t.variant;
     if (stages) *stages = t.stages;
     return NMRFIT_OK;
@@ -1189,12 +1062,13 @@ int nmrfit_ctx_get_variant(nmrfit_ctx* c, int S, int* variant, int* stages) {
 
 int nmrfit_ctx_get_tuning(nmrfit_ctx* c, int S, int* threads, int* r, int* tb, int* sp, int* n_tiles) {
     if (int rc = check_ctx(c)) return rc;
-    ObjTune t = pick_tune(c, S < 1 ? 1 : S, use_uniform(c, NMRFIT_REAL_ONLY));
+    const ObjPlan p = ctx_plan(c, S < 1 ? 1 : S, NMRFIT_REAL_ONLY);
+    const ObjTune& t = p.t;
     if (threads) *threads = t.threads;
     if (r) *r = t.r;
     if (tb) *tb = t.tb;
     if (sp) *sp = t.sp;
-    if (n_tiles) *n_tiles = objective_tiles(c->N, t);
+    if (n_tiles) *n_tiles = p.n_tiles;
     return NMRFIT_OK;
 }
 
@@ -1272,8 +1146,8 @@ int nmrfit_objective_batch(nmrfit_ctx* c, const double* x_dev, int S, int fit_im
 
 namespace {
 // Page-locked host positions as the device sees them (null: pageable memory, or a path without the prepare pass)
-const double* mapped_positions(const nmrfit_ctx* c, const double* x_host, int fit_im) {
-    if (!use_uniform(c, fit_im) || c->precision != NMRFIT_FP64) return nullptr;
+const double* mapped_positions(const nmrfit_ctx* c, const double* x_host, int S, int fit_im) {
+    if (!two_pass(ctx_plan(c, S, fit_im))) return nullptr;
     cudaPointerAttributes at{};
     const cudaError_t pe = cudaPointerGetAttributes(&at, x_host);
     if (pe != cudaSuccess) (void)cudaGetLastError();
@@ -1294,7 +1168,7 @@ int nmrfit_objective_batch_host(nmrfit_ctx* c, const double* x_host, int S, int 
     // Page-locked host positions (cudaHostAlloc / cudaHostRegister: mapped into the device under unified addressing) are
     // read by the prepare pass ITSELF, each element crossing PCIe once while other CTAs compute - no staging copy in
     // front of the kernels.  Pageable arrays take the copies below.
-    const double* x_map = mapped_positions(c, x_host, fit_im);     // the caller's array as the device sees it, or null
+    const double* x_map = mapped_positions(c, x_host, S, fit_im);     // the caller's array as the device sees it, or null
     constexpr int kPad = 64;
     // (slices of ~12k particles, two to six of them: 1.24 / 1.15 / 1.13 / 1.12 ms per call with 1 / 2 / 4 / 6 slices
     // at 65,536 particles of 6 peaks x 4,096 points, tools/e2e_probe.py)
@@ -1345,7 +1219,7 @@ int nmrfit_objective_spectrum_host(nmrfit_ctx* c, const double* w, const double*
     const size_t N = (size_t)c->N;
     const bool have = c->spec_set[0] && !c->shadow.empty() && c->shadow[0].size() == 4 * N && !is_device_pointer(w) &&
                       !is_device_pointer(u) && !is_device_pointer(v) && !is_device_pointer(weights);
-    const double* x_map = have && !c->profiling ? mapped_positions(c, x_host, fit_im) : nullptr;
+    const double* x_map = have && !c->profiling ? mapped_positions(c, x_host, S, fit_im) : nullptr;
     if (!x_map) {
         if (int rc = nmrfit_ctx_set_spectrum(c, 0, w, u, v, weights)) return rc;
         return nmrfit_objective_batch_host(c, x_host, S, fit_im, f_host);

@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <cstddef>
 #include <cstdint>
+#include <type_traits>
+#include "objective_plan.h"
 
 #define NMRFIT_MAX_DEVICES 16
 
@@ -51,60 +53,44 @@ struct ObjArgs {
                             // `sub` entries per region
 };
 
-// Far-field cells per warp region (uniform_eval.cuh): the shorter the axis, the shorter the cells, down to 64 points.
-// A function of the axis length and the points per thread ONLY, so that every kernel that evaluates a given spectrum
-// (one group per CTA, streamed, fused swarm) splits it the same way and stays bit-identical to the others.
-__host__ __device__ inline int far_cells_per_region(int N, int R) {
-    const int target = N < 8192 ? 64 : (N < 32768 ? 128 : 256);    // cell length aimed at, in points
-    int sub = 32 * R / target;
-    return sub < 1 ? 1 : (sub > 4 ? 4 : sub);
+// Calls f(std::integral_constant<int, V>{}) for the V among Vs that equals v, cudaErrorInvalidValue for any other v:
+// each launcher lists the values it is built for, and only those are instantiated.
+template <int... Vs, typename F>
+cudaError_t dispatch(int v, F&& f) {
+    cudaError_t e = cudaErrorInvalidValue;
+    (void)((v == Vs ? (e = f(std::integral_constant<int, Vs>{}), true) : false) || ...);
+    return e;
 }
+// a plan's threads per CTA (128 | 256) and points per thread (among Rs): f(THREADS, R)
+template <int... Rs, typename F>
+cudaError_t dispatch_geometry(const ObjTune& t, F&& f) {
+    return dispatch<128, 256>(t.threads, [&](auto T) { return dispatch<Rs...>(t.r, [&](auto R) { return f(T, R); }); });
+}
+// exp table bits of the kernels built for every table
+template <typename F>
+cudaError_t dispatch_tb(int tb, F&& f) { return dispatch<0, 6, 8, 10>(tb, f); }
 
-struct ObjTune {
-    int threads;            // 128 | 256
-    int r;                  // grid points per thread: 2 | 4 | 8 (general kernel), 4 | 8 | 16 (uniform-grid kernel)
-    int tb;                 // exp table bits: 0 | 6 | 8 | 10
-    int sp;                 // particles per CTA (streamed kernel: per pipeline stage)
-    int variant;            // uniform-axis FP64 evaluation kernel: 0 one particle group per CTA, 1 streamed (objective_stream.cu)
-    int stages;             // streamed kernel: pipeline depth
-    int occ;                // streamed kernel: CTAs of 256 threads per SM (2 or 3)
-};
+struct MoveArgs;
+// One objective evaluation as `p` plans it (objective.cu): the stand-alone move of the swarm `mv` or the prepare pass
+// (which folds the move in), the evaluation kernel, and the finalize pass when f is set (f == nullptr: the swarm's
+// finish kernel sums the tiles itself).  ev0 / evm / ev1 (nullable) are recorded before the first leg, between it and
+// the evaluation kernel (at its start on paths without a prepare pass), and after the evaluation kernel.
+cudaError_t run_objective_plan(const ObjPlan& p, ObjArgs a, int B, const MoveArgs* mv, double* f, cudaStream_t st,
+                               cudaEvent_t ev0, cudaEvent_t evm, cudaEvent_t ev1);
 
-int objective_tiles(int N, const ObjTune& t);
-size_t objective_smem_bytes(int P, const ObjTune& t, int kk);
-// ev0/ev1 (nullable) are recorded immediately before/after the main kernel on `st`
-// f == nullptr skips the finalize pass; tiles_out receives the number of partial sums per particle
-cudaError_t launch_objective(ObjArgs a, const ObjTune& t, int B, double* f, cudaStream_t st, cudaEvent_t ev0 = nullptr,
-                             cudaEvent_t ev1 = nullptr, int* tiles_out = nullptr);
+// The evaluation kernel of each file at the plan's geometry (`a` as run_objective_plan fills it)
+cudaError_t launch_objective_general(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st);   // objective.cu
+cudaError_t launch_objective_uniform(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st);   // objective_uniform.cu
+cudaError_t launch_objective_stream(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st);    // objective_stream.cu
+cudaError_t launch_objective_f32(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st);       // objective_f32.cu
+// the prepare pass of the uniform-axis kernels (objective_uniform.cu); mv != nullptr moves the swarm (pso.cu's update)
+// in it, one launch fewer per generation
+cudaError_t launch_objective_prepare(const ObjPlan& p, const ObjArgs& a, int B, const MoveArgs* mv, cudaStream_t st);
 
 // fixed-order sum over point tiles + sqrt(mean) (shared by the objective kernels)
 // `nw` > 1: the partial sums are per REGION, [n_tiles][nw]: the nw regions of a tile are summed first, then the tiles
 cudaError_t launch_objective_finalize(const double* partials, int n_tiles, int nsum, int N, int S, int B,
                                       const int* frozen, double* f, cudaStream_t st, int nw = 1);
-
-// uniform-axis objective (objective_uniform.cu): real-only fit, FP64
-size_t objective_uniform_smem_bytes(int P, const ObjTune& t, int sub = 1);
-// per-particle sizes (in doubles / 32-bit words) of the prepare pass's outputs; `sub` far-field cells per region
-void objective_uniform_prep_sizes(int N, int P, const ObjTune& t, int sub, size_t* coef, size_t* part, size_t* far,
-                                  size_t* anchor, size_t* mask_words, int* pad_particles);
-struct SwarmState;
-struct MoveArgs;
-// f == nullptr skips the finalize pass (the swarm's finish kernel sums the tiles itself); mv != nullptr moves the
-// swarm (pso.cu's update) inside the prepare pass, one launch fewer per generation
-cudaError_t launch_objective_uniform(ObjArgs a, const ObjTune& t, int B, double* f, cudaStream_t st,
-                                     cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr, const MoveArgs* mv = nullptr,
-                                     int* tiles_out = nullptr, cudaEvent_t evm = nullptr, int* nw_out = nullptr);
-
-cudaError_t launch_objective_prepare(ObjArgs& a, const ObjTune& t, int B, cudaStream_t st, const MoveArgs* mv = nullptr);
-
-// streamed evaluation kernel (objective_stream.cu): shared-memory need and launch; partial sums per region
-size_t objective_stream_smem_bytes(int P, const ObjTune& t, int sub);
-cudaError_t launch_objective_stream(const ObjArgs& a, const ObjTune& t, int B, cudaStream_t st);
-
-// opt-in FP32 objective: uniform-axis kernel when `uniform`, else a plain FP32 kernel for any axis (real-only fit)
-size_t objective_f32_smem_bytes(int P, const ObjTune& t);
-cudaError_t launch_objective_f32(ObjArgs a, const ObjTune& t, int B, double* f, bool uniform, cudaStream_t st,
-                                 cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr, int* tiles_out = nullptr);
 
 // ---- K2/K3 swarm --------------------------------------------------------------
 struct SwarmState {

@@ -13,6 +13,7 @@
 //   exp_neg<10>   7 slots   (1024-entry table, degree 3)
 #pragma once
 #include "nmrfit_coeffs.cuh"
+#include "objective_smem.h"     // kFarPoly
 
 #ifdef NMRFIT_HOST_MATH
 #include <cmath>
@@ -55,6 +56,12 @@ constexpr double kSqrtLn2OverPi = 0.46971863934982566689;    // sqrt(ln 2 / pi)
 constexpr double kTwoOverSqrtPi = 1.12837916709551257390;    // 2 / sqrt(pi)
 constexpr double kMagic = 6755399441055744.0;                // 1.5 * 2^52: round-to-nearest-int shifter
 constexpr int kExpClampHi = (int)0xC085E000;                 // high word of -700.0
+
+// The table of exp_neg<TB> in global memory (copied into shared memory by the kernels that use one); none for TB = 0
+template <int TB> struct ExpTab { static NMRFIT_HD const double* src() { return nullptr; } };
+template <> struct ExpTab<6> { static NMRFIT_HD const double* src() { return NMRFIT_EXP2_TAB6; } };
+template <> struct ExpTab<8> { static NMRFIT_HD const double* src() { return NMRFIT_EXP2_TAB8; } };
+template <> struct ExpTab<10> { static NMRFIT_HD const double* src() { return NMRFIT_EXP2_TAB10; } };
 
 // 1/q for q >= 1 (the Lorentzian denominator 1 + t^2).  One MUFU seed with
 // ~2^-20 relative error, then a cubic correction y0*(1 + e + e^2), e = 1 - q*y0:
@@ -430,7 +437,6 @@ NMRFIT_HD bool far_accumulate(double Dc, const SpanCoef& c, double H, double (&C
 // 16^-10/512) = 1.8e-15 of a far peak's height - the size of the series' own truncation error - and leaves a
 // polynomial of degree 9: two FMAs fewer per point in the evaluation kernels, ten more per cell here.  The factors
 // are exact binary fractions.
-constexpr int kFarPoly = 10;                               // coefficients stored per far-field cell
 NMRFIT_HD void far_economise(double (&C)[kFarTerms]) {
     static_assert(kFarTerms == 12 && kFarPoly == 10, "economisation is written for 12 -> 10 coefficients");
     const double a = C[11], b = C[10];

@@ -24,28 +24,6 @@
 
 namespace nmrfit {
 
-constexpr int kCoefStride = 8;   // loc kL2 aL nkG2 | aG kL kG pad
-
-template <int TB> struct ExpTab { static __device__ __forceinline__ const double* src() { return nullptr; } };
-template <> struct ExpTab<6> { static __device__ __forceinline__ const double* src() { return NMRFIT_EXP2_TAB6; } };
-template <> struct ExpTab<8> { static __device__ __forceinline__ const double* src() { return NMRFIT_EXP2_TAB8; } };
-template <> struct ExpTab<10> { static __device__ __forceinline__ const double* src() { return NMRFIT_EXP2_TAB10; } };
-
-// shared-memory carve-up (in doubles), shared by kernel and launcher
-struct ObjSmem {
-    int coef, pyoff, elo, emid, wpart, tab, total;
-    __host__ __device__ ObjSmem(int sp, int P, int nwarps, int R, int TB, int nsum) {
-        int o = 0;
-        coef = o;  o += sp * P * kCoefStride;
-        elo = o;   o += sp * 32 * 2;
-        emid = o;  o += sp * nwarps * R * 2;
-        tab = o;   o += TB ? (1 << TB) : 0;
-        pyoff = o; o += sp;
-        wpart = o; o += sp * nwarps * nsum;
-        total = o;
-    }
-};
-
 // KK: 0 = real only; 1 = reference semantics (equations.py:199 overwrites I_fit, so
 // only the LAST peak's Kramers-Kronig curve is compared); 2 = sum over peaks.
 template <int THREADS, int R, int TB, int KK>
@@ -232,61 +210,56 @@ __global__ void objective_finalize_kernel(const double* __restrict__ partials, i
     f[idx] = rm;
 }
 
-// ---- launcher -----------------------------------------------------------------
+// ---- launchers ----------------------------------------------------------------
 template <int THREADS, int R, int TB, int KK>
-static cudaError_t launch_one(const ObjArgs& a, dim3 grid, cudaStream_t st) {
-    ObjSmem L(a.sp, a.P, THREADS / 32, R, TB, KK ? 2 : 1);
-    size_t bytes = (size_t)L.total * sizeof(double);
+static cudaError_t launch_one(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st) {
     cudaError_t e = opt_in_smem<objective_kernel<THREADS, R, TB, KK>>(200 * 1024);
     if (e != cudaSuccess) return e;
-    objective_kernel<THREADS, R, TB, KK><<<grid, THREADS, bytes, st>>>(a);
+    dim3 grid((a.S + p.t.sp - 1) / p.t.sp, p.n_tiles, B);
+    objective_kernel<THREADS, R, TB, KK><<<grid, THREADS, p.smem, st>>>(a);
     return cudaGetLastError();
 }
 
-template <int THREADS, int R, int TB>
-static cudaError_t launch_kk(const ObjArgs& a, dim3 grid, cudaStream_t st) {
-    switch (a.kk) {
-        case 0: return launch_one<THREADS, R, TB, 0>(a, grid, st);
-        case 1: return launch_one<THREADS, R, TB, 1>(a, grid, st);
-        default: return launch_one<THREADS, R, TB, 2>(a, grid, st);
-    }
+cudaError_t launch_objective_general(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st) {
+    return dispatch_geometry<2, 4, 8>(p.t, [&](auto T, auto R) {
+        return dispatch_tb(p.t.tb, [&](auto TB) {
+            return dispatch<0, 1, 2>(a.kk, [&](auto KK) { return launch_one<T, R, TB, KK>(p, a, B, st); });
+        });
+    });
 }
 
-template <int THREADS, int R>
-static cudaError_t launch_tb(const ObjArgs& a, int tb, dim3 grid, cudaStream_t st) {
-    switch (tb) {
-        case 0: return launch_kk<THREADS, R, 0>(a, grid, st);
-        case 6: return launch_kk<THREADS, R, 6>(a, grid, st);
-        case 8: return launch_kk<THREADS, R, 8>(a, grid, st);
-        case 10: return launch_kk<THREADS, R, 10>(a, grid, st);
-        default: return cudaErrorInvalidValue;
-    }
-}
-
-int objective_tiles(int N, const ObjTune& t) { return (N + t.threads * t.r - 1) / (t.threads * t.r); }
-
-size_t objective_smem_bytes(int P, const ObjTune& t, int kk) {
-    return (size_t)ObjSmem(t.sp, P, t.threads / 32, t.r, t.tb, kk ? 2 : 1).total * sizeof(double);
-}
-
-cudaError_t launch_objective(ObjArgs a, const ObjTune& t, int B, double* f, cudaStream_t st, cudaEvent_t ev0,
-                             cudaEvent_t ev1, int* tiles_out) {
-    a.sp = t.sp;
-    const int n_tiles = objective_tiles(a.N, t);
-    if (tiles_out) *tiles_out = n_tiles;
-    dim3 grid((a.S + t.sp - 1) / t.sp, n_tiles, B);
-    cudaError_t e = cudaErrorInvalidValue;
+cudaError_t run_objective_plan(const ObjPlan& p, ObjArgs a, int B, const MoveArgs* mv, double* f, cudaStream_t st,
+                               cudaEvent_t ev0, cudaEvent_t evm, cudaEvent_t ev1) {
+    a.sp = p.t.sp;
+    a.n_tiles = p.n_tiles;
+    a.nw = p.t.threads / 32;
+    a.sub = p.sub;
+    a.tile_major = p.tile_major;
+    a.stages = p.t.stages;
+    a.gpc = p.gpc;
+    a.occ = p.t.occ;
+    // the FP64 uniform-axis path times its prepare pass (with the swarm's move folded in) as the first leg; the others
+    // move the swarm on their own and leave the first leg empty
+    const bool two_pass = p.kernel == OBJ_UNIFORM || p.kernel == OBJ_STREAM;
+    cudaError_t e;
     if (ev0) cudaEventRecord(ev0, st);
-    if (t.threads == 128 && t.r == 2) e = launch_tb<128, 2>(a, t.tb, grid, st);
-    else if (t.threads == 128 && t.r == 4) e = launch_tb<128, 4>(a, t.tb, grid, st);
-    else if (t.threads == 128 && t.r == 8) e = launch_tb<128, 8>(a, t.tb, grid, st);
-    else if (t.threads == 256 && t.r == 2) e = launch_tb<256, 2>(a, t.tb, grid, st);
-    else if (t.threads == 256 && t.r == 4) e = launch_tb<256, 4>(a, t.tb, grid, st);
-    else if (t.threads == 256 && t.r == 8) e = launch_tb<256, 8>(a, t.tb, grid, st);
+    if (!two_pass) {
+        if (evm) cudaEventRecord(evm, st);
+        if (mv && (e = launch_swarm_move(mv->s, mv->rp, mv->rg, mv->generation, st)) != cudaSuccess) return e;
+    }
+    const bool prepare = p.prep_threads > 0;
+    if (prepare && (e = launch_objective_prepare(p, a, B, two_pass ? mv : nullptr, st)) != cudaSuccess) return e;
+    if (two_pass && evm) cudaEventRecord(evm, st);
+    switch (p.kernel) {
+        case OBJ_GENERAL: e = launch_objective_general(p, a, B, st); break;
+        case OBJ_UNIFORM: e = launch_objective_uniform(p, a, B, st); break;
+        case OBJ_STREAM: e = launch_objective_stream(p, a, B, st); break;
+        default: e = launch_objective_f32(p, a, B, st); break;
+    }
     if (ev1) cudaEventRecord(ev1, st);
     if (e != cudaSuccess) return e;
-    if (f) e = launch_objective_finalize(a.partials, n_tiles, a.kk ? 2 : 1, a.N, a.S, B, a.frozen, f, st);
-    count_launches(f ? 2 : 1);
+    if (f) e = launch_objective_finalize(a.partials, p.n_tiles, p.nsum, a.N, a.S, B, a.frozen, f, st, p.nw);
+    count_launches(prepare + 1 + (f ? 1 : 0));
     return e;
 }
 

@@ -70,31 +70,6 @@ __device__ __forceinline__ void peak_span_f32(float t0, float s0, float dT, floa
     }
 }
 
-// shared-memory carve-up (in doubles): as UniSmem without the exp table
-struct F32Smem {
-    int uv, wt, bar, wpart, coef, part, far, anchor, mask, coef32, far32, mw, total;
-    __host__ __device__ F32Smem(int sp, int P, int threads, int R) {
-        const int nw = threads / 32;
-        mw = (P + 31) / 32;
-        int o = 0;
-        uv = o;     o += threads * R * 2;
-        wt = o;     o += threads * R;
-        bar = o;    o += 2;
-        wpart = o;  o += sp * nw;
-        coef = o;   o += sp * P * 8;
-        part = o;   o += sp * kPartDoubles;
-        far = o;    o += sp * nw * kFarPoly;
-        anchor = o; o += sp * nw * 2;
-        mask = o;   o += ((sp * nw * (mw + 1) + 3) / 4) * 2;
-        // single-precision copies made once per CTA (a double -> float conversion costs four FP64 issue slots: doing
-        // it per thread and particle was 30 conversions per 8 points, now 1.5 + the 8 of the residual)
-        coef32 = o; o += sp * P * 4;                       // 8 floats per peak: kL, kG, dT, aL, aG, c2, thr, -
-        far32 = o;  o += (sp * nw * kFarPoly + 1) / 2;
-        o = (o + 1) & ~1;
-        total = o;
-    }
-};
-
 template <int THREADS, int R>
 __global__ void __launch_bounds__(THREADS, 768 / THREADS)
 objective_uniform_f32_kernel(ObjArgs a) {
@@ -240,8 +215,6 @@ objective_uniform_f32_kernel(ObjArgs a) {
 }
 
 // ---- any axis: every peak at every point ------------------------------------------------------------
-constexpr int kGenThreads32 = 256;
-constexpr int kGenR32 = 4;
 __global__ void __launch_bounds__(kGenThreads32)
 objective_general_f32_kernel(ObjArgs a, int n_tiles) {
     extern __shared__ __align__(16) double smem[];         // [sp][P][4] floats packed: kL, kG, aL, aG ; then loc doubles
@@ -319,55 +292,25 @@ objective_general_f32_kernel(ObjArgs a, int n_tiles) {
     }
 }
 
-// ---- launchers ------------------------------------------------------------------------------------
-size_t objective_f32_smem_bytes(int P, const ObjTune& t) {
-    return (size_t)F32Smem(t.sp, P, t.threads, t.r).total * sizeof(double);
-}
-
+// ---- launcher ------------------------------------------------------------------------------------
 template <int THREADS, int R>
-static cudaError_t launch_uniform_f32(const ObjArgs& a, int B, cudaStream_t st) {
-    const size_t bytes = (size_t)F32Smem(a.sp, a.P, THREADS, R).total * sizeof(double);
+static cudaError_t launch_uniform_f32(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st) {
     cudaError_t e = opt_in_smem<objective_uniform_f32_kernel<THREADS, R>>(200 * 1024);
     if (e != cudaSuccess) return e;
-    dim3 grid((a.S + a.sp - 1) / a.sp, a.n_tiles, B);
-    objective_uniform_f32_kernel<THREADS, R><<<grid, THREADS, bytes, st>>>(a);
+    dim3 grid((a.S + p.t.sp - 1) / p.t.sp, p.n_tiles, B);
+    objective_uniform_f32_kernel<THREADS, R><<<grid, THREADS, p.smem, st>>>(a);
     return cudaGetLastError();
 }
 
-cudaError_t launch_objective_f32(ObjArgs a, const ObjTune& t, int B, double* f, bool uniform, cudaStream_t st,
-                                 cudaEvent_t ev0, cudaEvent_t ev1, int* tiles_out) {
+cudaError_t launch_objective_f32(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st) {
     if (a.kk != 0) return cudaErrorNotSupported;           // fit_im needs the FP64 general kernel
-    cudaError_t e;
-    int n_tiles;
-    if (ev0) cudaEventRecord(ev0, st);
-    if (uniform) {
-        a.sub = 1;                                         // the FP32 kernel keeps one far-field cell per region
-        a.tile_major = 0;
-        e = launch_objective_prepare(a, t, B, st);
-        if (e != cudaSuccess) return e;
-        e = cudaErrorInvalidValue;
-        if (t.threads == 128 && t.r == 4) e = launch_uniform_f32<128, 4>(a, B, st);
-        else if (t.threads == 128 && t.r == 8) e = launch_uniform_f32<128, 8>(a, B, st);
-        else if (t.threads == 256 && t.r == 4) e = launch_uniform_f32<256, 4>(a, B, st);
-        else if (t.threads == 256 && t.r == 8) e = launch_uniform_f32<256, 8>(a, B, st);
-        n_tiles = a.n_tiles;
-        count_launches(1);
-    } else {
-        e = opt_in_smem<objective_general_f32_kernel>(200 * 1024);
-        if (e != cudaSuccess) return e;
-        a.sp = t.sp;
-        n_tiles = (a.N + kGenThreads32 * kGenR32 - 1) / (kGenThreads32 * kGenR32);
-        const size_t bytes = ((size_t)a.sp * a.P * 3 + (size_t)a.sp * (kGenThreads32 / 32)) * sizeof(double);
-        dim3 grid((a.S + a.sp - 1) / a.sp, n_tiles, B);
-        objective_general_f32_kernel<<<grid, kGenThreads32, bytes, st>>>(a, n_tiles);
-        e = cudaGetLastError();
-    }
-    if (ev1) cudaEventRecord(ev1, st);
+    if (p.kernel == OBJ_F32_UNIFORM)
+        return dispatch_geometry<4, 8>(p.t, [&](auto T, auto R) { return launch_uniform_f32<T, R>(p, a, B, st); });
+    cudaError_t e = opt_in_smem<objective_general_f32_kernel>(200 * 1024);
     if (e != cudaSuccess) return e;
-    if (tiles_out) *tiles_out = n_tiles;
-    if (f) e = launch_objective_finalize(a.partials, n_tiles, 1, a.N, a.S, B, a.frozen, f, st);
-    count_launches(f ? 2 : 1);
-    return e;
+    dim3 grid((a.S + p.t.sp - 1) / p.t.sp, p.n_tiles, B);
+    objective_general_f32_kernel<<<grid, kGenThreads32, p.smem, st>>>(a, p.n_tiles);
+    return cudaGetLastError();
 }
 
 }  // namespace nmrfit

@@ -39,36 +39,6 @@ namespace nmrfit {
 
 namespace {
 
-template <int TB> struct ExpTabS { static __device__ __forceinline__ const double* src() { return nullptr; } };
-template <> struct ExpTabS<6> { static __device__ __forceinline__ const double* src() { return NMRFIT_EXP2_TAB6; } };
-
-// shared-memory carve-up (in doubles); every offset is even (16-byte alignment)
-struct StreamSmem {
-    int tab, uv, wt, wfirst, bars, tickets, slot0, slot, coef, part, far, anchor, mask, mw, total;
-    __host__ __device__ StreamSmem(int spg, int stages, int P, int threads, int R, int TB, int sub) {
-        const int nw = threads / 32;
-        mw = (P + 31) / 32;
-        int o = 0;
-        tab = o;     o += TB ? (1 << TB) : 0;
-        uv = o;      o += threads * R * 2;
-        wt = o;      o += threads * R;
-        wfirst = o;  o += threads;                          // stored abscissa of every thread span's first point
-        bars = o;    o += stages;                           // one mbarrier per slot
-        tickets = o; o += (stages + 1) / 2 * 2;             // one 32-bit release counter per slot (two per double)
-        if (o & 1) ++o;
-        slot0 = o;
-        // one slot (offsets relative to its start)
-        int q = 0;
-        coef = q;    q += spg * P * 8;
-        part = q;    q += spg * kPartDoubles;
-        far = q;     q += spg * nw * sub * kFarPoly;       // per far-field cell (uniform_eval.cuh)
-        anchor = q;  q += spg * nw * 2;
-        mask = q;    q += ((spg * nw * mask_words_per_region(P, sub) + 3) / 4) * 2;
-        slot = q;
-        total = slot0 + stages * slot;
-    }
-};
-
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // OCC: CTAs of 256 threads per SM the kernel is compiled for (3: 80 registers, 75 KB of shared memory each; 2: up to
@@ -150,7 +120,7 @@ objective_stream_kernel(ObjArgs a) {
         swf[tid] = i_first < N ? sw[i_first] : fma((double)i_first, h, sw[0]);
     }
     if (TB) {
-        const double* src = ExpTabS<TB>::src();
+        const double* src = ExpTab<TB>::src();
         for (int i = tid; i < (1 << TB); i += THREADS) tab[i] = src[i];
     }
     constexpr double H = 16.0 * R;                         // half a region, in points
@@ -224,58 +194,30 @@ objective_stream_kernel(ObjArgs a) {
 }
 
 template <int THREADS, int R, int TB, int KK, int OCC, int SUB>
-cudaError_t launch_sub(const ObjArgs& a, int B, cudaStream_t st) {
-    StreamSmem L(a.sp, a.stages, a.P, THREADS, R, TB, a.sub);
-    const size_t bytes = (size_t)L.total * sizeof(double);
+cudaError_t launch_one(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st) {
     cudaError_t e = opt_in_smem<objective_stream_kernel<THREADS, R, TB, KK, OCC, SUB>>(200 * 1024);
     if (e != cudaSuccess) return e;
-    const int n_groups = (a.S + a.sp - 1) / a.sp;
-    dim3 grid((n_groups + a.gpc - 1) / a.gpc, a.n_tiles, B);
-    objective_stream_kernel<THREADS, R, TB, KK, OCC, SUB><<<grid, THREADS, bytes, st>>>(a);
+    const int n_groups = (a.S + p.t.sp - 1) / p.t.sp;
+    dim3 grid((n_groups + p.gpc - 1) / p.gpc, p.n_tiles, B);
+    objective_stream_kernel<THREADS, R, TB, KK, OCC, SUB><<<grid, THREADS, p.smem, st>>>(a);
     return cudaGetLastError();
-}
-
-// far-field cells per region as a compile-time constant: the lane's cell, the mirror lane and the cell coordinate's
-// step fold into immediates instead of being recomputed per particle (the kernel runs at its register limit)
-template <int THREADS, int R, int TB, int KK, int OCC>
-cudaError_t launch_occ(const ObjArgs& a, int B, cudaStream_t st) {
-    switch (a.sub) {
-        case 1: return launch_sub<THREADS, R, TB, KK, OCC, 1>(a, B, st);
-        case 2: return launch_sub<THREADS, R, TB, KK, OCC, 2>(a, B, st);
-        case 4: return launch_sub<THREADS, R, TB, KK, OCC, 4>(a, B, st);
-        default: return cudaErrorInvalidValue;
-    }
-}
-
-template <int THREADS, int R, int TB, int KK>
-cudaError_t launch_one(const ObjArgs& a, int B, cudaStream_t st) {
-    return a.occ == 2 ? launch_occ<THREADS, R, TB, KK, 2>(a, B, st) : launch_occ<THREADS, R, TB, KK, 3>(a, B, st);
-}
-
-template <int THREADS, int R>
-cudaError_t launch_tb(const ObjArgs& a, int tb, int B, cudaStream_t st) {
-    switch (tb) {
-        // (built for the default exp table only: the launcher routes every other table to the one-group kernel)
-        case 6: return a.kk ? launch_one<THREADS, R, 6, 1>(a, B, st) : launch_one<THREADS, R, 6, 0>(a, B, st);
-        default: return cudaErrorInvalidValue;
-    }
 }
 
 }  // namespace
 
-size_t objective_stream_smem_bytes(int P, const ObjTune& t, int sub) {
-    return (size_t)StreamSmem(t.sp, t.stages, P, t.threads, t.r, t.tb, sub).total * sizeof(double);
-}
-
-// a.sp / a.stages / a.gpc / a.n_tiles / a.nw are set by the caller (launch_objective_uniform)
-cudaError_t launch_objective_stream(const ObjArgs& a, const ObjTune& t, int B, cudaStream_t st) {
-    if (t.threads == 128 && t.r == 4) return launch_tb<128, 4>(a, t.tb, B, st);
-    if (t.threads == 128 && t.r == 8) return launch_tb<128, 8>(a, t.tb, B, st);
-    if (t.threads == 128 && t.r == 16) return launch_tb<128, 16>(a, t.tb, B, st);
-    if (t.threads == 256 && t.r == 4) return launch_tb<256, 4>(a, t.tb, B, st);
-    if (t.threads == 256 && t.r == 8) return launch_tb<256, 8>(a, t.tb, B, st);
-    if (t.threads == 256 && t.r == 16) return launch_tb<256, 16>(a, t.tb, B, st);
-    return cudaErrorInvalidValue;
+// Built for the default exp table only (the plan sends every other table to the one-group kernel).  The far-field
+// cells per region are a compile-time constant: the lane's cell, the mirror lane and the cell coordinate's step fold
+// into immediates instead of being recomputed per particle (the kernel runs at its register limit).
+cudaError_t launch_objective_stream(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st) {
+    return dispatch_geometry<4, 8, 16>(p.t, [&](auto T, auto R) {
+        return dispatch<6>(p.t.tb, [&](auto TB) {
+            return dispatch<0, 1>(a.kk ? 1 : 0, [&](auto KK) {
+                return dispatch<2, 3>(p.t.occ == 2 ? 2 : 3, [&](auto OCC) {
+                    return dispatch<1, 2, 4>(p.sub, [&](auto SUB) { return launch_one<T, R, TB, KK, OCC, SUB>(p, a, B, st); });
+                });
+            });
+        });
+    });
 }
 
 }  // namespace nmrfit

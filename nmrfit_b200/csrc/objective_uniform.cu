@@ -52,12 +52,6 @@
 
 namespace nmrfit {
 
-template <int TB> struct ExpTabU { static __device__ __forceinline__ const double* src() { return nullptr; } };
-template <> struct ExpTabU<6> { static __device__ __forceinline__ const double* src() { return NMRFIT_EXP2_TAB6; } };
-template <> struct ExpTabU<8> { static __device__ __forceinline__ const double* src() { return NMRFIT_EXP2_TAB8; } };
-template <> struct ExpTabU<10> { static __device__ __forceinline__ const double* src() { return NMRFIT_EXP2_TAB10; } };
-
-
 // Where particle s of spectrum b keeps its per-region constants (in regions; times sub*12, 2 or mask words each):
 // particle-major [B][S][n_tiles*nw] for objective_uniform_kernel, tile-major [B][n_tiles][S][nw] for the streamed
 // kernel, whose CTA reads one tile's regions of a whole particle group as ONE contiguous block.
@@ -86,7 +80,6 @@ struct RegionDst {
 // MOVE: the swarm's move (pso.cu's swarm_move_kernel for these particles) in front: one launch fewer per generation.
 // Regions are stored in axis order, padded to a whole number of tiles; the slots of regions past the end of the axis
 // are neutral.
-constexpr int kPrepThreads = 256;                          // at most; 128 when a particle alone fills the CTA
 template <int R, bool MOVE>
 __global__ void __launch_bounds__(kPrepThreads, 4)
 objective_prepare_kernel(ObjArgs a, MoveArgs mv, int G) {
@@ -184,27 +177,6 @@ objective_prepare_kernel(ObjArgs a, MoveArgs mv, int G) {
 }
 
 // ---- pass 2: evaluation ------------------------------------------------------------------------------
-// shared-memory carve-up (in doubles), shared by kernel and launcher; every offset is even (16-byte alignment)
-struct UniSmem {
-    int tab, uv, wt, bar, wpart, coef, part, far, anchor, mask, mw, total;
-    __host__ __device__ UniSmem(int sp, int P, int threads, int R, int TB, int nsum = 1, int sub = 1) {
-        const int nw = threads / 32;
-        mw = (P + 31) / 32;                               // near-peak mask words per region, + 1 has-far word
-        int o = 0;
-        tab = o;    o += TB ? (1 << TB) : 0;
-        uv = o;     o += threads * R * 2;
-        wt = o;     o += threads * R;
-        bar = o;    o += 2;                               // one mbarrier
-        wpart = o;  o += sp * nw * nsum;                   // nsum = 2: real and imaginary sums of fit_im
-        coef = o;   o += sp * P * 8;
-        part = o;   o += sp * kPartDoubles;
-        far = o;    o += sp * nw * sub * kFarPoly;       // far-field polynomial per (particle, cell of a warp region)
-        anchor = o; o += sp * nw * 2;                     // phase at the first point of each warp region
-        mask = o;   o += ((sp * nw * mask_words_per_region(P, sub) + 3) / 4) * 2;
-        total = o;
-    }
-};
-
 template <int THREADS, int R, int TB, int KK>
 __global__ void __launch_bounds__(THREADS, (R <= 8 ? 768 : 512) / THREADS)    // 24 (16 for R = 16) resident warps per SM
 objective_uniform_kernel(ObjArgs a) {
@@ -269,7 +241,7 @@ objective_uniform_kernel(ObjArgs a) {
     const int i_first = tile0 + tid * R;                   // this thread's first point
     const double w_first = i_first < N ? sw[i_first] : fma((double)i_first, h, sw[0]);
     if (TB) {
-        const double* src = ExpTabU<TB>::src();
+        const double* src = ExpTab<TB>::src();
         for (int i = tid; i < (1 << TB); i += THREADS) tab[i] = src[i];
     }
     const double xi0 = cell_xi0<R>(lane, SUB);             // first point's position inside its far-field cell
@@ -301,128 +273,33 @@ objective_uniform_kernel(ObjArgs a) {
     }
 }
 
-// ---- launcher -----------------------------------------------------------------
+// ---- launchers ----------------------------------------------------------------
 template <int THREADS, int R, int TB, int KK>
-static cudaError_t launch_one(const ObjArgs& a, int B, cudaStream_t st) {
-    UniSmem L(a.sp, a.P, THREADS, R, TB, KK ? 2 : 1, a.sub);
-    const size_t bytes = (size_t)L.total * sizeof(double);
+static cudaError_t launch_one(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st) {
     cudaError_t e = opt_in_smem<objective_uniform_kernel<THREADS, R, TB, KK>>(200 * 1024);
     if (e != cudaSuccess) return e;
-    dim3 grid((a.S + a.sp - 1) / a.sp, a.n_tiles, B);
-    objective_uniform_kernel<THREADS, R, TB, KK><<<grid, THREADS, bytes, st>>>(a);
+    dim3 grid((a.S + p.t.sp - 1) / p.t.sp, p.n_tiles, B);
+    objective_uniform_kernel<THREADS, R, TB, KK><<<grid, THREADS, p.smem, st>>>(a);
     return cudaGetLastError();
 }
 
-template <int THREADS, int R>
-static cudaError_t launch_tb(const ObjArgs& a, int tb, int B, cudaStream_t st) {
-    switch (tb) {
-        case 0: return a.kk ? launch_one<THREADS, R, 0, 1>(a, B, st) : launch_one<THREADS, R, 0, 0>(a, B, st);
-        case 6: return a.kk ? launch_one<THREADS, R, 6, 1>(a, B, st) : launch_one<THREADS, R, 6, 0>(a, B, st);
-        case 8: return a.kk ? launch_one<THREADS, R, 8, 1>(a, B, st) : launch_one<THREADS, R, 8, 0>(a, B, st);
-        case 10: return a.kk ? launch_one<THREADS, R, 10, 1>(a, B, st) : launch_one<THREADS, R, 10, 0>(a, B, st);
-        default: return cudaErrorInvalidValue;
-    }
+cudaError_t launch_objective_uniform(const ObjPlan& p, const ObjArgs& a, int B, cudaStream_t st) {
+    return dispatch_geometry<4, 8, 16>(p.t, [&](auto T, auto R) {
+        return dispatch_tb(p.t.tb, [&](auto TB) {
+            return dispatch<0, 1>(a.kk ? 1 : 0, [&](auto KK) { return launch_one<T, R, TB, KK>(p, a, B, st); });
+        });
+    });
 }
 
-void objective_uniform_prep_sizes(int N, int P, const ObjTune& t, int sub, size_t* coef, size_t* part, size_t* far,
-                                  size_t* anchor, size_t* mask_words, int* pad_particles) {
-    const size_t nrp = (size_t)objective_tiles(N, t) * (t.threads / 32);
-    *coef = (size_t)P * 8;                      // doubles per particle
-    *part = kPartDoubles;
-    *far = nrp * sub * kFarPoly;
-    *anchor = nrp * 2;
-    *mask_words = nrp * mask_words_per_region(P, sub);    // 32-bit words per particle
-    *pad_particles = kPadParticles;
-}
-
-size_t objective_uniform_smem_bytes(int P, const ObjTune& t, int sub) {
-    return (size_t)UniSmem(t.sp, P, t.threads, t.r, t.tb, 2, sub).total * sizeof(double);
-}
-
-// pass 1 (shared with the FP32 evaluation kernel); fills a.sp / a.n_tiles / a.nw
-cudaError_t launch_objective_prepare(ObjArgs& a, const ObjTune& t, int B, cudaStream_t st, const MoveArgs* mv) {
-    if (t.sp > kPadParticles) return cudaErrorInvalidValue;
-    a.sp = t.sp;
-    a.n_tiles = objective_tiles(a.N, t);
-    a.nw = t.threads / 32;
-    if (a.sub < 1) a.sub = 1;
-    // particles per CTA: about four rounds of far-field cells for its 256 threads (0.184 / 0.182 / 0.179 ms with 8 / 12 /
-    // 16 particles at 6 peaks x 4,096 points; 0.202 with 4)
-    const int nc = a.n_tiles * a.nw * a.sub;
-    const size_t per_particle = (size_t)(a.P * 12 + 4 + 3 * a.P) * sizeof(double);
-    int G = std::max(1, std::min(16, std::min(a.S, 4 * kPrepThreads / nc)));
-    while (G > 1 && G * per_particle > 40 * 1024) --G;     // stay inside the default dynamic shared-memory limit
-    // a particle with >= 128 cells fills a CTA of 128 threads on its own (and many small CTAs schedule better)
-    int pthreads = nc >= 128 ? 128 : kPrepThreads;
-    if (nc >= 128) G = 1;
-    // a small swarm (a single fit): as many CTAs as there are particles - the critical path of one CTA, not the
-    // machine's throughput, is what the generation waits for
-    const long long want_ctas = 2 * 148;
-    if ((long long)a.S * B / G < want_ctas) {
-        G = (int)std::max<long long>(1, std::min<long long>(G, (long long)a.S * B / want_ctas));
-        if (G == 1) pthreads = 128;
-    }
-    dim3 pgrid((a.S + G - 1) / G, B);
-    const size_t bytes = G * per_particle;
-    const MoveArgs none{};
-    if (mv) {
-        if (t.r == 4) objective_prepare_kernel<4, true><<<pgrid, pthreads, bytes, st>>>(a, *mv, G);
-        else if (t.r == 8) objective_prepare_kernel<8, true><<<pgrid, pthreads, bytes, st>>>(a, *mv, G);
-        else if (t.r == 16) objective_prepare_kernel<16, true><<<pgrid, pthreads, bytes, st>>>(a, *mv, G);
-        else return cudaErrorInvalidValue;
+// pass 1 (shared with the FP32 evaluation kernel)
+cudaError_t launch_objective_prepare(const ObjPlan& p, const ObjArgs& a, int B, const MoveArgs* mv, cudaStream_t st) {
+    if (p.t.sp > kPadParticles) return cudaErrorInvalidValue;
+    const dim3 grid((a.S + p.prep_g - 1) / p.prep_g, B);
+    return dispatch<4, 8, 16>(p.t.r, [&](auto R) {
+        if (mv) objective_prepare_kernel<R, true><<<grid, p.prep_threads, p.prep_smem, st>>>(a, *mv, p.prep_g);
+        else objective_prepare_kernel<R, false><<<grid, p.prep_threads, p.prep_smem, st>>>(a, MoveArgs{}, p.prep_g);
         return cudaGetLastError();
-    }
-    if (t.r == 4) objective_prepare_kernel<4, false><<<pgrid, pthreads, bytes, st>>>(a, none, G);
-    else if (t.r == 8) objective_prepare_kernel<8, false><<<pgrid, pthreads, bytes, st>>>(a, none, G);
-    else if (t.r == 16) objective_prepare_kernel<16, false><<<pgrid, pthreads, bytes, st>>>(a, none, G);
-    else return cudaErrorInvalidValue;
-    return cudaGetLastError();
-}
-
-// Groups per CTA of the streamed kernel: enough CTAs for ~5 waves of the 3-per-SM residency (the hardware's CTA
-// scheduler evens out the tiles' different costs), few enough that the tile staging is amortised over >= 4 groups.
-static int stream_groups_per_cta(int S, int sp, int n_tiles, int B) {
-    const long long n_groups = (S + sp - 1) / sp;
-    long long gpc = n_groups * n_tiles * B / (148 * 3 * 5);
-    gpc = std::max<long long>(4, std::min<long long>(32, gpc));
-    const long long chunks = (n_groups + gpc - 1) / gpc;
-    return (int)((n_groups + chunks - 1) / chunks);        // equal chunks
-}
-
-cudaError_t launch_objective_uniform(ObjArgs a, const ObjTune& t, int B, double* f, cudaStream_t st, cudaEvent_t ev0,
-                                     cudaEvent_t ev1, const MoveArgs* mv, int* tiles_out, cudaEvent_t evm, int* nw_out) {
-    if (ev0) cudaEventRecord(ev0, st);
-    a.tile_major = t.variant == 1;
-    cudaError_t e = launch_objective_prepare(a, t, B, st, mv);
-    if (e != cudaSuccess) return e;
-    if (evm) cudaEventRecord(evm, st);
-    if (nw_out) *nw_out = 1;
-    if (t.variant == 1) {
-        a.stages = t.stages;
-        a.occ = t.occ;
-        a.gpc = stream_groups_per_cta(a.S, a.sp, a.n_tiles, B);
-        e = launch_objective_stream(a, t, B, st);
-        if (ev1) cudaEventRecord(ev1, st);
-        if (e != cudaSuccess) return e;
-        if (tiles_out) *tiles_out = a.n_tiles;
-        if (nw_out) *nw_out = a.nw;
-        if (f) e = launch_objective_finalize(a.partials, a.n_tiles, a.kk ? 2 : 1, a.N, a.S, B, a.frozen, f, st, a.nw);
-        count_launches(f ? 3 : 2);
-        return e;
-    }
-    e = cudaErrorInvalidValue;
-    if (t.threads == 128 && t.r == 4) e = launch_tb<128, 4>(a, t.tb, B, st);
-    else if (t.threads == 128 && t.r == 8) e = launch_tb<128, 8>(a, t.tb, B, st);
-    else if (t.threads == 128 && t.r == 16) e = launch_tb<128, 16>(a, t.tb, B, st);
-    else if (t.threads == 256 && t.r == 4) e = launch_tb<256, 4>(a, t.tb, B, st);
-    else if (t.threads == 256 && t.r == 8) e = launch_tb<256, 8>(a, t.tb, B, st);
-    else if (t.threads == 256 && t.r == 16) e = launch_tb<256, 16>(a, t.tb, B, st);
-    if (ev1) cudaEventRecord(ev1, st);
-    if (e != cudaSuccess) return e;
-    if (tiles_out) *tiles_out = a.n_tiles;
-    if (f) e = launch_objective_finalize(a.partials, a.n_tiles, a.kk ? 2 : 1, a.N, a.S, B, a.frozen, f, st);
-    count_launches(f ? 3 : 2);
-    return e;
+    });
 }
 
 }  // namespace nmrfit

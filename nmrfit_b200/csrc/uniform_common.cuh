@@ -2,11 +2,9 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cstdint>
+#include "objective_smem.h"
 
 namespace nmrfit {
-
-constexpr int kPartDoubles = 68;   // per particle: e^{i p1 lane R/N} for 32 lanes (64), cos/sin(p1/N), P*yoff, #exact peaks
-constexpr int kPadParticles = 64;  // slack at the end of the prepare buffers: the last group is copied whole
 
 // TMA bulk copy (global -> shared, 1-D) completing on an mbarrier, and the barrier's own operations.
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }

@@ -17,7 +17,7 @@
 // its Gaussian cannot reach the cell), so shorter cells leave fewer peaks to evaluate one by one: on a 4,096-point
 // axis with 6 peaks, 4.75 of them are near the average 256-point region but only 1.6 near the average 64-point cell.
 // The price is `sub` times the polynomials in the prepare pass, so long axes (where the Gaussian's reach, not the
-// series, decides what is near) keep sub = 1: far_cells_per_region() in nmrfit_internal.h, a function of the axis
+// series, decides what is near) keep sub = 1: far_cells_per_region() in objective_smem.h, a function of the axis
 // length and R alone - never of how particles or spectra are sharded.
 #pragma once
 #include <cuda_runtime.h>
@@ -25,10 +25,6 @@
 #include "uniform_common.cuh"
 
 namespace nmrfit {
-
-// 32-bit mask words per region: one cell - [MW near words][has-far]; several cells - the same block for the UNION of
-// the region's cells first (what the warp as a whole has to visit), then one block per cell.
-__host__ __device__ inline int mask_words_per_region(int P, int sub) { return (sub == 1 ? 1 : sub + 1) * ((P + 31) / 32 + 1); }
 
 // ---- the items of the prepare pass.  One particle's constants are a few dozen independent work items; the prepare
 // kernel (objective_uniform.cu) spreads the items of SEVERAL particles over the threads of a CTA so that no warp idles,

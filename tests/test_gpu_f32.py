@@ -28,13 +28,17 @@ def test_fp32_matches_reference_golden(case):
     assert relerr(f, g['f']) < TOL32
 
 
-@pytest.mark.parametrize('threads,r', [(128, 4), (128, 8), (256, 4), (256, 8)])
+@pytest.mark.parametrize('threads,r', [(128, 4), (128, 8), (128, 16), (256, 4), (256, 8), (256, 16)])
 def test_fp32_uniform_variants(threads, r):
     g = load_golden('objective_ragged_1000x6')
+    runs = min(r, 8)                                     # the FP32 kernel is built for 4 and 8 points per thread
     with _cabi.Context(1, g['w'].size, 6, precision=_cabi.FP32) as ctx:
         ctx.set_spectrum(0, g['w'], g['u'], g['v'], g['weights'])
         for sp in (1, 5, 16):
             ctx.set_tuning(threads, r, 0, sp)
+            t = ctx.get_tuning(len(g['xs']))
+            assert (t['threads'], t['points_per_thread']) == (threads, runs)
+            assert t['n_point_tiles'] == -(-g['w'].size // (threads * runs))
             assert relerr(ctx.objective_host(g['xs']), g['f']) < TOL32
 
 
@@ -48,6 +52,8 @@ def test_fp32_non_uniform_axis_and_extreme_widths():
     with _cabi.Context(1, 1500, 6, precision=_cabi.FP32) as ctx:
         ctx.set_spectrum(0, w, data.u, data.v, wts)
         assert ctx.get_algorithm() == _cabi.ALGO_GENERAL
+        t = ctx.get_tuning(len(xs))                      # the any-axis FP32 kernel's fixed geometry
+        assert (t['threads'], t['points_per_thread'], t['n_point_tiles']) == (256, 4, 2)
         assert relerr(ctx.objective_host(xs), want) < TOL32
     # uniform axis, widths that leave the recurrence (exact FP64 path inside the FP32 kernel) and far-away peaks
     xs = []

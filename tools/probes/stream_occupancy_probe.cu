@@ -1,6 +1,6 @@
 // Resident CTAs per SM of the streamed evaluation kernel at the headline shape (6 peaks, 4,096 points: 256 threads,
-// R = 8, four far-field cells per region), around the two-CTA shared-memory budget of pick_tune (cabi.cu): two stages of
-// 7 and of 8 particles, the budget itself and one byte over it.
+// R = 8, four far-field cells per region), around the two-CTA shared-memory budget of objective_plan
+// (objective_plan.h): two stages of 7 and of 8 particles, the budget itself and one byte over it.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -o stream_occupancy_probe stream_occupancy_probe.cu
 #include "../../nmrfit_b200/csrc/objective_stream.cu"
 #include <cstdio>
